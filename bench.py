@@ -1,7 +1,7 @@
 #!/usr/bin/env python
 """Benchmark of the Factorizer hot path on B200 (see BASELINE.json: metric / configs).
 
-    python bench.py [--gpus N] [--steps K] [--warmup W] [--impl ours|reference]
+    python bench.py [--gpus N] [--steps K] [--warmup W] [--impl ours|reference] [--dump-outputs DIR]
 
 Workload (config.workload): BASELINE config 3 -- ft.FactorizerBlock(32, 128^3, LayerNorm, SWMatricize(head_dim 8, patch 8),
 HALS rank 1 x 5 sweeps, mlp_ratio 2, dropout 0), forward + backward including every parameter gradient, one (1,32,128^3)
@@ -29,6 +29,16 @@ cpu_baseline / --impl reference
            pure Python and absent on the GPU box) -- on the SAME workload (the whole block at (1,32,128^3), all host
            threads); the C/OpenMP port of the core (oracle/nmf_oracle.c) is reported beside it
 Multi-GPU: one process per GPU (torchrun), batch-sharded (one volume per rank, no data-path collective), weak scaling.
+
+--dump-outputs DIR
+           after the timed steps, rank 0 writes what the last timed block step returned to its caller: DIR/out.npy,
+           DIR/dx.npy and DIR/grad.<parameter name>.npy, float32.  Inputs and parameters are seeded, so two builds run with
+           the same arguments can be compared file by file.  out and dx (2^26 entries each at 128^3) are written as their
+           entries at a fixed sample of flat indices (see dump_outputs), about 32 MB in all.  The parameter gradients are
+           fp32 sums over 2^21 voxels reduced in no fixed order, so expect them to differ in the last bits from run to
+           run; compare them with a tolerance.
+--steps K  the number of timed steps of the headline block step (and of --impl reference); the side measurements
+           (kernels_us, e2e, model, cpu_baseline) use their own fixed or capped counts.
 """
 from __future__ import annotations
 
@@ -71,9 +81,10 @@ def _host_threads() -> int:
         return os.cpu_count() or 1
 
 
-def torch_port_block(steps: int, warmup: int, budget_s: float):
+def torch_port_block(steps: int, warmup: int, budget_s: float | None):
     """The reference's PyTorch CPU path (restated: oracle/torch_port.py) on the whole workload; returns
-    (voxels/s, per-step seconds, threads, steps timed)."""
+    (voxels/s, per-step seconds, threads, steps timed).  With a budget, timing stops early once at least two steps
+    are timed and the budget is spent."""
     import torch
 
     from oracle import torch_port as TP
@@ -100,8 +111,7 @@ def torch_port_block(steps: int, warmup: int, budget_s: float):
         dt = time.perf_counter() - t0
         if k >= warmup:
             times.append(dt)
-        # a bounded run: always at least two timed steps, then stop when the budget is spent
-        if len(times) >= 2 and time.perf_counter() - t_start > budget_s:
+        if budget_s is not None and len(times) >= 2 and time.perf_counter() - t_start > budget_s:
             break
     return N ** 3 / statistics.mean(times), times, torch.get_num_threads(), len(times)
 
@@ -132,9 +142,9 @@ def run_reference(args):
     rank = int(os.environ.get("RANK", "0"))
     if rank != 0:
         return
-    rate, times, threads, timed = torch_port_block(max(args.steps, 2), min(args.warmup, 1), budget_s=150.0)
-    sample = (f"the whole workload: FactorizerBlock fwd+bwd on (1,{C},{N}^3), {timed} timed steps of the {args.steps} requested "
-              f"(bounded to ~150 s of CPU work; {statistics.mean(times):.2f} s per step), after {min(args.warmup, 1)} warm-up")
+    rate, times, threads, timed = torch_port_block(args.steps, min(args.warmup, 1), budget_s=None)
+    sample = (f"the whole workload: FactorizerBlock fwd+bwd on (1,{C},{N}^3), {timed} timed steps "
+              f"({statistics.mean(times):.2f} s per step), after {min(args.warmup, 1)} warm-up")
     line = {
         "impl": "reference", "metric": METRIC, "value": rate, "unit": UNIT, "n_gpus": args.gpus,
         "steps": args.steps, "warmup": args.warmup, "ms_per_step": 1e3 * statistics.mean(times), "higher_is_better": True,
@@ -221,6 +231,24 @@ def tol_ratio(got, ref, rtol=1e-4, atol=1e-5):
     import torch
     ref = ref.to(torch.float64)
     return float(((got.to(torch.float64) - ref).abs() / (atol + rtol * ref.abs())).max())
+
+
+DUMP_SAMPLE = 1 << 22
+
+
+def dump_outputs(directory, arrays):
+    """Write every tensor of `arrays` as <directory>/<name>.npy in float32.  A tensor of more than DUMP_SAMPLE entries is
+    reduced to its flattened entries at DUMP_SAMPLE indices drawn by numpy's default_rng(0) (sorted, repeats dropped):
+    the same positions in every run."""
+    import numpy as np
+    import torch
+    os.makedirs(directory, exist_ok=True)
+    for name, t in arrays.items():
+        t = t.detach()
+        if t.numel() > DUMP_SAMPLE:
+            idx = np.unique(np.random.default_rng(0).integers(0, t.numel(), DUMP_SAMPLE))
+            t = t.reshape(-1)[torch.from_numpy(idx).to(t.device)]
+        np.save(os.path.join(directory, f"{name}.npy"), t.float().cpu().numpy())
 
 
 def model_leg(dev, world, rank, n=128, steps=3):
@@ -463,6 +491,7 @@ def run_ours(args):
     # AccumulateGrad nodes keep running on this stream and invalidate the capture)
     y_block = out_timed.detach().clone()
     gx_block = xb.grad.detach().clone()
+    gp_block = {k: p_.grad.detach().clone() for k, p_ in blk.named_parameters()}
     del out_timed
     bgraph = None
     try:        # the same step replayed from one CUDA graph (forward, autograd backward, gradient accumulation)
@@ -494,6 +523,7 @@ def run_ours(args):
             timed_launches = per_step_launches * args.steps
             y_block = out_graph.detach().clone()
             gx_block = xb.grad.detach().clone()
+            gp_block = {k: p_.grad.detach().clone() for k, p_ in blk.named_parameters()}
     except Exception as e:
         launch_mode = f"stream launches from autograd (graph capture failed: {type(e).__name__}: {str(e)[:160]})"
         torch.cuda.synchronize(dev)
@@ -775,6 +805,8 @@ def run_ours(args):
             line["cpu_baseline_c_port"] = {"value": crate, "unit": UNIT, "cores": cthreads, "kind": "port",
                                            "sample": f"the fused core alone (config 2) on the whole (1,{C},{N}^3) volume through "
                                                      f"oracle/nmf_oracle.c (C/OpenMP), median of 3 ({1e3 * statistics.median(ctimes):.0f} ms)"}
+        if args.dump_outputs:
+            dump_outputs(args.dump_outputs, {"out": y_block, "dx": gx_block, **{f"grad.{k}": g for k, g in gp_block.items()}})
         print(json.dumps(line))
     if world > 1:
         dist.destroy_process_group()
@@ -783,13 +815,18 @@ def run_ours(args):
 def main():
     ap = argparse.ArgumentParser()
     ap.add_argument("--gpus", type=int, default=1)
-    ap.add_argument("--steps", type=int, default=20)
+    ap.add_argument("--steps", type=int, default=20, help="timed steps of the headline block step (and of --impl reference)")
     ap.add_argument("--warmup", type=int, default=3)
     ap.add_argument("--impl", default="ours", choices=["ours", "reference"])
     ap.add_argument("--no-model", action="store_true", help="skip the whole-model (configs 4-5) side measurement")
     ap.add_argument("--no-cpu", action="store_true", help="skip the CPU baseline leg")
     ap.add_argument("--no-parity", action="store_true", help="skip the parity check of the timed buffers")
+    ap.add_argument("--dump-outputs", metavar="DIR", help="write the last timed step's output and gradients under DIR (.npy)")
     args = ap.parse_args()
+    if args.steps < 1:
+        ap.error("--steps must be at least 1")
+    if args.dump_outputs and args.impl != "ours":
+        ap.error("--dump-outputs applies to --impl ours")
     if args.impl == "reference":
         run_reference(args)
     else:

@@ -6,6 +6,7 @@ only the reference's *outputs* (and its torch-RNG-initialised u0/v0 buffers) liv
 from __future__ import annotations
 
 import hashlib
+import os
 
 import numpy as np
 
@@ -140,3 +141,62 @@ def make_array(name: str, shape, dist: str, tag: str = "x") -> np.ndarray:
 def digest(a: np.ndarray) -> str:
     a = np.ascontiguousarray(a)
     return hashlib.sha256(a.tobytes()).hexdigest()
+
+
+# --- storage of the golden outputs --------------------------------------------------------------------------------
+# Each family (nmf, sw, fused, block, model) is one file, <family>.npz, below 1 MB.  Inputs (u0, v0, state dicts), factors
+# and parameter gradients are stored whole.  The outputs y, gx, y64, gx64 of a case with more than SAMPLE[family] entries
+# are stored at SAMPLE[family] flat indices drawn once per case from a seeded generator: "<case>/sample_index" and
+# "<case>/sample_shape" hold the indices and the full shape, "<key>@sample" the values there.  load_golden returns such
+# an output as a Sample, and conftest.tol_ratio compares a computed array with it at those indices.
+OUTPUTS = ("y", "gx", "y64", "gx64")
+SAMPLE = {"nmf": 1536, "fused": 4096, "block": 8192}
+
+
+class Sample(np.ndarray):
+    """Reference values at the flat indices ``index`` of an array of shape ``full_shape``."""
+
+    def __new__(cls, values, index, full_shape):
+        obj = np.asarray(values).view(cls)
+        obj.index, obj.full_shape = index, tuple(int(n) for n in full_shape)
+        return obj
+
+    def __array_finalize__(self, obj):
+        self.index = getattr(obj, "index", None)
+        self.full_shape = getattr(obj, "full_shape", None)
+
+
+def save_golden(directory: str, family: str, arrays: dict) -> None:
+    """Write ``arrays`` (insertion order kept) as <directory>/<family>.npz, the larger outputs sampled as above."""
+    keep = SAMPLE.get(family)
+    out = {}
+    for key, a in arrays.items():
+        a = np.asarray(a)
+        case, name = key.split("/", 1)
+        if keep is None or name not in OUTPUTS or a.size <= keep:
+            out[key] = a
+            continue
+        if f"{case}/sample_index" not in out:
+            rng = np.random.Generator(np.random.PCG64(_seed(case + ":sample")))
+            out[f"{case}/sample_index"] = np.sort(rng.choice(a.size, keep, replace=False)).astype(np.int32)
+            out[f"{case}/sample_shape"] = np.array(a.shape, dtype=np.int64)
+        assert tuple(out[f"{case}/sample_shape"]) == a.shape, key      # one index set per case
+        out[f"{key}@sample"] = a.reshape(-1)[out[f"{case}/sample_index"]]
+    path = os.path.join(directory, f"{family}.npz")
+    np.savez(path, **out)
+    assert os.path.getsize(path) < 1_000_000, (path, os.path.getsize(path))
+
+
+def load_golden(directory: str, family: str) -> dict:
+    """All arrays of ``family`` by key, in the order they were saved; sampled outputs as Sample."""
+    with np.load(os.path.join(directory, f"{family}.npz")) as f:
+        raw = {k: f[k] for k in f.files}
+    out = {}
+    for key, a in raw.items():
+        if key.endswith("@sample"):
+            key = key[:-len("@sample")]
+            case = key.split("/", 1)[0]
+            out[key] = Sample(a, raw[f"{case}/sample_index"], raw[f"{case}/sample_shape"])
+        elif not key.endswith(("/sample_index", "/sample_shape")):
+            out[key] = a
+    return out

@@ -6,7 +6,8 @@ Build-container only (the reference does not exist on the GPU box):
     python tests/golden/make_golden.py
 
 The reference imports ``opt_einsum`` (factorizer/factorization/matrix_factorization.py:8) but never
-uses it; an empty stub module stands in for it.  Outputs: nmf.npz, sw.npz, fused.npz, block.npz, model.npz.
+uses it; an empty stub module stands in for it.  Outputs: nmf.npz, sw.npz, fused.npz, block.npz, model.npz
+(cases.save_golden: the outputs of the larger cases at a seeded sample of indices, each file below 1 MB).
 """
 from __future__ import annotations
 
@@ -62,7 +63,7 @@ def gen_nmf():
         (gx64,) = torch.autograd.grad((y64 * gy.double()).sum(), x64)
         out[f"{name}/y64"] = y64.detach().numpy()
         out[f"{name}/gx64"] = gx64.numpy()
-    np.savez(os.path.join(HERE, "nmf.npz"), **out)
+    cases.save_golden(HERE, "nmf", out)
     print("nmf.npz", len(out), "arrays")
 
 
@@ -90,7 +91,7 @@ def gen_sw():
         rt = mod.inverse_forward(y)
         out[f"{name}/roundtrip_equal"] = np.array(bool(torch.equal(rt, x)))
         out[f"{name}/rt_digest"] = np.array(cases.digest(rt.numpy()))
-    np.savez(os.path.join(HERE, "sw.npz"), **out)
+    cases.save_golden(HERE, "sw", out)
     print("sw.npz", len(out), "arrays")
 
 
@@ -114,7 +115,7 @@ def gen_fused():
         out[f"{name}/v0"] = nmf.init.v0.numpy().copy()
         out[f"{name}/y"] = y.detach().numpy()
         out[f"{name}/gx"] = gx.numpy()
-    np.savez(os.path.join(HERE, "fused.npz"), **out)
+    cases.save_golden(HERE, "fused", out)
     print("fused.npz", len(out), "arrays")
 
 
@@ -143,7 +144,7 @@ def gen_block():
         out[f"{name}/gx"] = grads[0].numpy()
         for (k, _), g in zip(blk.named_parameters(), grads[1:]):
             out[f"{name}/gp/{k}"] = g.numpy()
-    np.savez(os.path.join(HERE, "block.npz"), **out)
+    cases.save_golden(HERE, "block", out)
     print("block.npz", len(out), "arrays")
 
 
@@ -170,7 +171,7 @@ def gen_model():
         out[f"{name}/gx"] = grads[0].numpy()
         for (k, _), g in zip(net.named_parameters(), grads[1:]):
             out[f"{name}/gp/{k}"] = g.numpy()
-    np.savez(os.path.join(HERE, "model.npz"), **out)
+    cases.save_golden(HERE, "model", out)
     print("model.npz", len(out), "arrays")
 
 

@@ -197,7 +197,7 @@ def test_factorizer_block_matches_reference(ft, dev, golden, name):
     blk = ft.FactorizerBlock(channels=c["channels"], spatial_size=c["spatial"], norm=ft.LayerNorm,
                              reshape=(ft.SWMatricize, c["kw"]), act=nn.ReLU, factorize=ft.NMF,
                              mlp_ratio=c["mlp_ratio"], dropout=0.0, **c["nmf"])
-    sd = {k.split("/sd/")[1]: torch.from_numpy(g[k]) for k in g.files if k.startswith(name + "/sd/")}
+    sd = {k.split("/sd/")[1]: torch.from_numpy(g[k]) for k in g if k.startswith(name + "/sd/")}
     blk.load_state_dict(sd)
     blk = blk.to(dev)
     xs = (c["batch"], c["channels"], *c["spatial"])
@@ -230,7 +230,7 @@ def test_factorizer_model_matches_reference(ft, dev, golden, name):
     net = ft.Factorizer(in_channels=c["in_channels"], out_channels=c["out_channels"], spatial_size=c["spatial"],
                         norm=ft.LayerNorm, reshape=(ft.SWMatricize, c["reshape_kw"]), act=nn.ReLU, factorize=ft.NMF,
                         **c["kw"])
-    net.load_state_dict({k.split("/sd/")[1]: torch.from_numpy(g[k]) for k in g.files if k.startswith(name + "/sd/")})
+    net.load_state_dict({k.split("/sd/")[1]: torch.from_numpy(g[k]) for k in g if k.startswith(name + "/sd/")})
     net = net.to(dev).eval()
     xs = (c["batch"], c["in_channels"], *c["spatial"])
     x = torch.from_numpy(cases.make_array(name, xs, "randn")).to(dev).requires_grad_(True)
@@ -398,14 +398,13 @@ def test_reference_test_nmf_port(ft, dev):
     assert loss.shape == size[:1] and (loss >= 0).all()
 
 
-def test_standalone_nmf_on_large_matrices(ft, dev):
+def test_standalone_nmf_on_large_matrices(ft, dev, golden):
     """ft.NMF on matrices beyond a CTA's shared memory (rank 1): forward and input gradient against the reference
     golden of the identical computation through Matricize(num_heads=1, grid_size=1), which is a pure view."""
     from factorizer_b200 import _lib
     name = "fused_global_mu_big"
     c = cases.FUSED_CASES[name]
-    import os
-    gold = np.load(os.path.join(os.path.dirname(__file__), "golden", "fused.npz"))
+    gold = golden["fused"]
     xs = c["x_shape"]
     M, N = xs[1], int(np.prod(xs[2:]))
     nmf = ft.NMF(size=(M, N), rank=1, num_iters=5, init="uniform", solver="mu")

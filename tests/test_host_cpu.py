@@ -66,7 +66,7 @@ def test_readme_shapes_and_state_dict_keys(ft, golden):
     blk = ft.FactorizerBlock(channels=c["channels"], spatial_size=c["spatial"], norm=ft.LayerNorm,
                              reshape=(ft.SWMatricize, c["kw"]), act=nn.ReLU, factorize=ft.NMF,
                              mlp_ratio=c["mlp_ratio"], dropout=0.0, **c["nmf"])
-    ref_keys = [k.split("/sd/")[1] for k in golden["block"].files if k.startswith("block_c16_16/sd/")]
+    ref_keys = [k.split("/sd/")[1] for k in golden["block"] if k.startswith("block_c16_16/sd/")]
     assert list(blk.state_dict().keys()) == ref_keys
     for k, v in blk.state_dict().items():
         assert tuple(v.shape) == golden["block"][f"block_c16_16/sd/{k}"].shape
@@ -86,7 +86,7 @@ def test_factorizer_model_state_dict_matches_reference(ft, golden, name):
     c, g = cases.MODEL_CASES[name], golden["model"]
     torch.manual_seed(cases._seed(name) % (2**31))
     net = _build_model(ft, c)
-    ref_keys = [k.split("/sd/")[1] for k in g.files if k.startswith(name + "/sd/")]
+    ref_keys = [k.split("/sd/")[1] for k in g if k.startswith(name + "/sd/")]
     sd = net.state_dict()
     assert list(sd.keys()) == ref_keys
     for k, v in sd.items():

@@ -135,11 +135,11 @@ def test_gram_form_is_well_conditioned(golden, name):
     gy = cases.make_array(name, c["shape"], "randn", tag="gy").reshape(-1, M, N)
     v0 = g[f"{name}/v0"][:, 0]
     kw = dict(num_iters=c["num_iters"], num_grad_steps=c["num_grad_steps"])
-    y64, gx64 = g[f"{name}/y64"].reshape(x.shape), g[f"{name}/gx64"].reshape(x.shape)
-    yr, gr = g[f"{name}/y"].reshape(x.shape), g[f"{name}/gx"].reshape(x.shape)
-    y, dx = O.hals_r1_gram(x.astype(np.float64), v0.astype(np.float64), gy.astype(np.float64), **kw)
+    y64, gx64 = g[f"{name}/y64"], g[f"{name}/gx64"]
+    yr, gr = g[f"{name}/y"], g[f"{name}/gx"]
+    y, dx = (a.reshape(c["shape"]) for a in O.hals_r1_gram(x.astype(np.float64), v0.astype(np.float64), gy.astype(np.float64), **kw))
     assert tol_ratio(y, y64) < 1e-6 and tol_ratio(dx, gx64) < 1e-6
-    y, dx = O.hals_r1_gram(x, v0, gy, **kw)
+    y, dx = (a.reshape(c["shape"]) for a in O.hals_r1_gram(x, v0, gy, **kw))
     assert_close(y, yr, what="y")
     assert_close(dx, gr, what="gx")
     assert tol_ratio(y, y64) <= tol_ratio(yr, y64) + 0.02
@@ -152,7 +152,7 @@ def test_oracle_block_matches_reference(golden, name):
     and hand-derived backward, against the reference's own forward + autograd (block.npz); fp64 arithmetic
     on the fp32 inputs, so the bound is the reference's fp32 rounding."""
     c, g = cases.BLOCK_CASES[name], golden["block"]
-    sd = {k.split("/sd/")[1]: g[k].astype(np.float64) for k in g.files if k.startswith(name + "/sd/")}
+    sd = {k.split("/sd/")[1]: g[k].astype(np.float64) for k in g if k.startswith(name + "/sd/")}
     xs = (c["batch"], c["channels"], *c["spatial"])
     x = cases.make_array(name, xs, "randn").astype(np.float64)
     gy = cases.make_array(name, xs, "randn", tag="gy").astype(np.float64)
@@ -175,7 +175,7 @@ def test_torch_port_matches_golden(golden, name):
     import torch
     from oracle import torch_port as TP
     c, g = cases.BLOCK_CASES[name], golden["block"]
-    sd = {k.split("/sd/")[1]: torch.from_numpy(g[k]).requires_grad_(True) for k in g.files if k.startswith(name + "/sd/")}
+    sd = {k.split("/sd/")[1]: torch.from_numpy(g[k]).requires_grad_(True) for k in g if k.startswith(name + "/sd/")}
     xs = (c["batch"], c["channels"], *c["spatial"])
     x = torch.from_numpy(cases.make_array(name, xs, "randn")).requires_grad_(True)
     gy = torch.from_numpy(cases.make_array(name, xs, "randn", tag="gy"))
