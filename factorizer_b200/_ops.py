@@ -440,11 +440,13 @@ def _channel_map(x, w, bias, epi=EPI_NONE, aux=None, transposed=False):
 
 
 def _channel_map_wgrad(gy, x, want_bias: bool):
-    """dW = sum over (batch, voxels) of gy x^T, db = sum of gy."""
+    """dW = sum over (batch, voxels) of gy x^T, db = sum of gy.  Views the kernels do not take (non-contiguous, or not
+    16-byte aligned) run the same arithmetic in torch."""
     lib = L.lib()
     B, cout, vox = gy.shape
     cin = x.shape[1]
-    if gy.is_contiguous() and x.is_contiguous() and lib.fz_linear_wgrad_supported(cout, cin, vox):
+    if (gy.is_contiguous() and x.is_contiguous() and (gy.data_ptr() | x.data_ptr()) % 16 == 0
+            and lib.fz_linear_wgrad_supported(cout, cin, vox)):
         gw = torch.empty(cout, cin, device=x.device, dtype=torch.float32)
         gb = torch.empty(cout, device=x.device, dtype=torch.float32) if want_bias else None
         _call(lib.fz_linear_wgrad, L.ptr(gy), L.ptr(x), L.ptr(gw), L.ptr(gb), B, cout, cin, vox, L.stream_ptr(x.device))
@@ -594,7 +596,7 @@ class LayerNormCF(torch.autograd.Function):
 # ---- pointwise channel map (k = 1 Conv1d) with a hand-written weight gradient -------------------
 def space_depth2_supported(x: torch.Tensor) -> bool:
     return (isinstance(x, torch.Tensor) and x.is_cuda and x.dtype == torch.float32 and x.dim() == 5 and x.is_contiguous()
-            and bool(L.lib().fz_space_depth2_supported(*x.shape[2:])))
+            and x.data_ptr() % 16 == 0 and bool(L.lib().fz_space_depth2_supported(*x.shape[2:])))
 
 
 class SpaceDepth2(torch.autograd.Function):
@@ -610,6 +612,10 @@ class SpaceDepth2(torch.autograd.Function):
     @staticmethod
     def _run(x, B, D, H, W, to_depth):
         x = L.require_cuda_f32(x, "x")
+        if x.data_ptr() % 16:               # the kernel moves float4 words: the same permutation in torch
+            if to_depth:
+                return x.view(B, -1, D // 2, 2, H // 2, 2, W // 2, 2).permute(0, 1, 3, 5, 7, 2, 4, 6).reshape(B, -1, (D // 2) * (H // 2) * (W // 2))
+            return x.view(B, -1, 2, 2, 2, D // 2, H // 2, W // 2).permute(0, 1, 5, 2, 6, 3, 7, 4).reshape(B, -1, D, H, W)
         if to_depth:
             C = x.shape[1]
             out = torch.empty(B, C * 8, (D // 2) * (H // 2) * (W // 2), device=x.device, dtype=torch.float32)
@@ -631,7 +637,7 @@ def linear_wgrad_supported(x: torch.Tensor, out_channels: int, min_voxels: int =
                            voxels: Optional[int] = None) -> bool:
     """The contraction over voxels is worth a kernel of its own when it is long (library SGEMMs take their slow
     large-K route there); short ones stay with cuBLAS."""
-    if not (isinstance(x, torch.Tensor) and x.is_cuda and x.dtype == torch.float32 and x.dim() >= 3):
+    if not (isinstance(x, torch.Tensor) and x.is_cuda and x.dtype == torch.float32 and x.dim() >= 3 and x.data_ptr() % 16 == 0):
         return False
     if torch.is_autocast_enabled():          # the fp32 kernels are not autocast-aware: leave mixed precision to the library
         return False
@@ -681,18 +687,13 @@ class LinearCF(torch.autograd.Function):
     @once_differentiable
     def backward(ctx, gy):
         x, weight = ctx.saved_tensors
-        lib = L.lib()
         gy = L.require_cuda_f32(gy, "grad")
-        B, cin, vox = x.shape
-        cout = weight.shape[0]
         gx = gw = gb = None
         if ctx.needs_input_grad[0]:
             gx = linear_forward(gy.contiguous(), weight, None, transposed=True)
         if ctx.needs_input_grad[1] or (ctx.has_bias and ctx.needs_input_grad[2]):
-            gw = torch.empty(weight.shape, device=x.device, dtype=torch.float32)     # row-major whatever the weight's strides
-            gb = torch.empty(cout, device=x.device, dtype=torch.float32) if ctx.has_bias else None
-            with torch.cuda.device(x.device):
-                _call(lib.fz_linear_wgrad, L.ptr(gy), L.ptr(x), L.ptr(gw), L.ptr(gb), B, cout, cin, vox, L.stream_ptr(x.device))
+            with torch.cuda.device(x.device):                                       # gw row-major whatever the weight's strides
+                gw, gb = _channel_map_wgrad(gy, x, ctx.has_bias)
         return gx, gw, gb
 
 
@@ -700,6 +701,7 @@ def stem_conv_supported(x: torch.Tensor, weight: torch.Tensor, padding) -> bool:
     """3x3x3, stride 1, padding 1, 1..4 -> 32 channels on a contiguous CUDA fp32 volume: csrc/fz_linear.cu has a direct
     kernel for the forward (the caller checks stride / dilation / groups)."""
     return (isinstance(x, torch.Tensor) and x.is_cuda and x.dtype == torch.float32 and x.dim() == 5 and x.is_contiguous()
+            and x.data_ptr() % 16 == 0
             and not torch.is_autocast_enabled() and weight.dim() == 5 and tuple(weight.shape[2:]) == (3, 3, 3) and tuple(padding) == (1, 1, 1)
             and weight.is_contiguous() and weight.dtype == torch.float32
             and bool(L.lib().fz_conv3d_stem_supported(x.shape[1], weight.shape[0], *x.shape[2:])))
@@ -736,7 +738,6 @@ class ConvWgradCF(torch.autograd.Function):
     def backward(ctx, gy):
         import itertools
         x, weight = ctx.saved_tensors
-        lib = L.lib()
         nd = weight.dim() - 2
         gy = L.require_cuda_f32(gy, "grad")
         gx = gw = gb = None
@@ -747,10 +748,7 @@ class ConvWgradCF(torch.autograd.Function):
             xp = torch.nn.functional.pad(x, [q for p in reversed(ctx.padding) for q in (p, p)])
             cols = torch.stack([xp[(slice(None), slice(None)) + tuple(slice(o, o + n) for o, n in zip(off, out_sp))]
                                 for off in itertools.product(*[range(q) for q in k])], dim=2)   # (B, C_in, K, *out)
-            rows = cols.shape[1] * cols.shape[2]
-            gw = torch.empty(weight.shape, device=x.device, dtype=torch.float32)
-            gb = torch.empty(cout, device=x.device, dtype=torch.float32) if ctx.has_bias else None
             with torch.cuda.device(x.device):
-                _call(lib.fz_linear_wgrad, L.ptr(gy), L.ptr(cols), L.ptr(gw), L.ptr(gb), B, cout, rows, gy[0, 0].numel(),
-                      L.stream_ptr(x.device))
+                gw, gb = _channel_map_wgrad(gy.view(B, cout, -1), cols.view(B, cols.shape[1] * cols.shape[2], -1), ctx.has_bias)
+            gw = gw.view(weight.shape)
         return gx, gw, gb, None

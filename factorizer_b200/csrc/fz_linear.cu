@@ -338,6 +338,9 @@ __global__ void __launch_bounds__(128, 2) conv3_stem_fwd(const float* __restrict
     }
 }
 
+// the kernels above move float4 (and cp.async 16-byte) words of the caller's buffers
+bool unaligned16(const void* p) { return (reinterpret_cast<uintptr_t>(p) & 15) != 0; }
+
 }  // namespace
 }  // namespace fz
 
@@ -356,6 +359,7 @@ int fz_linear_wgrad(const float* dy, const float* x, float* dW, float* db, int64
         return fail(FZ_ERR_UNSUPPORTED, "linear wgrad kernel needs a voxel count divisible by 4 (got %d x %d x %lld)", cout, cin,
                     (long long)voxels);
     if (!dW) return fail(FZ_ERR_INVALID, "linear wgrad: null dW");
+    if (unaligned16(dy) || unaligned16(x)) return fail(FZ_ERR_UNSUPPORTED, "linear wgrad kernels need 16-byte aligned dy and x");
     cudaStream_t st = (cudaStream_t)stream;
     FZ_CUDA_CHECK(cudaMemsetAsync(dW, 0, sizeof(float) * (size_t)cout * cin, st));
     if (db) FZ_CUDA_CHECK(cudaMemsetAsync(db, 0, sizeof(float) * (size_t)cout, st));
@@ -442,6 +446,7 @@ int fz_space_depth2(const float* in, float* out, int64_t batch, int32_t channels
         return fail(FZ_ERR_UNSUPPORTED, "space/depth kernel needs even D, H and W divisible by 4 (got %d x %d x %d)", D, H, W);
     if (batch == 0) return FZ_OK;
     if (!in || !out) return fail(FZ_ERR_INVALID, "space/depth: null buffer");
+    if (unaligned16(in) || unaligned16(out)) return fail(FZ_ERR_UNSUPPORTED, "space/depth kernel needs 16-byte aligned buffers");
     const long long total4 = (long long)batch * channels * D * H * (W / 4);
     int dev = 0, sms = 148;
     FZ_CUDA_CHECK(cudaGetDevice(&dev));
@@ -466,6 +471,7 @@ int fz_conv3d_stem_forward(const float* x, const float* weight, const float* bia
         return fail(FZ_ERR_UNSUPPORTED, "stem convolution kernel handles 1..4 -> 32 channels, W divisible by 4 (got %d -> %d, W = %d)", cin, cout, W);
     if (batch == 0) return FZ_OK;
     if (!x || !weight || !y) return fail(FZ_ERR_INVALID, "stem convolution: null buffer");
+    if (unaligned16(x) || unaligned16(y)) return fail(FZ_ERR_UNSUPPORTED, "stem convolution kernel needs 16-byte aligned x and y");
     const long long total4 = (long long)batch * D * H * (W / 4);
     int dev = 0, sms = 148;
     FZ_CUDA_CHECK(cudaGetDevice(&dev));

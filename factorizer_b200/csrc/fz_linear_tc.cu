@@ -572,9 +572,11 @@ int linear_wgrad_tc_launch(const float* dy, const float* x, float* dW, float* db
     const int bo = (cout + kBlk - 1) / kBlk, bi = (cin + kBlk - 1) / kBlk;
     long long gx = (2LL * num_sms() + bo * bi - 1) / (bo * bi);
     // The tensor core adds into its fp32 accumulator with truncation, so the error of a TMEM accumulation chain grows linearly
-    // with its length (measured 2.6e-5 of max |dW| after 1 770 MMAs, 6e-7 for the FP32-pipe kernel): at most kMaxChain stages
-    // (4 MMAs each) per CTA, more CTAs along the voxel axis instead
-    constexpr long long kMaxChain = 64;
+    // with its length: on same-sign operands about 2^-24 S per MMA of the chain, S = sum |dy| |x| (B200: 1.7e-5 S after 64
+    // stages, 9.8e-5 S after 443; the FP32-pipe kernels stay below 1.1e-6 S).  At most kMaxChain stages (4 MMAs each) per
+    // CTA, more CTAs along the voxel axis instead: 32 stages keep the error at 0.8-1.04e-5 S
+    // (tests/test_gpu_channel_map_scale.py holds it to 2e-5 S).
+    constexpr long long kMaxChain = 32;
     if (gx * kMaxChain < tiles) gx = (tiles + kMaxChain - 1) / kMaxChain;
     if (gx > tiles) gx = tiles;
     if (gx < 1) gx = 1;

@@ -160,8 +160,9 @@ int fz_layernorm_cf_backward_add(const float* x, const float* gamma, const float
  * dW[o][i] = sum over batch and voxels of dy[b][o][v] x[b][i][v]   (cout x cin floats, OVERWRITTEN)
  * db[o]    = sum over batch and voxels of dy[b][o][v]              (cout floats, OVERWRITTEN; may be NULL)
  * dy is (batch, cout, voxels), x is (batch, cin, voxels), fp32 contiguous.  voxels must be a multiple of 4 (channel
- * counts are free: blocks of 32 x 32 are zero-padded); fz_linear_wgrad_supported() tells.  Replaces the large-K library SGEMM autograd picks
- * for the 64..512-channel stages of the Swin Factorizer. */
+ * counts are free: blocks of 32 x 32 are zero-padded); fz_linear_wgrad_supported() tells.  dy and x must be 16-byte aligned
+ * (FZ_ERR_UNSUPPORTED otherwise, before anything is written).  Replaces the large-K library SGEMM autograd picks for the
+ * 64..512-channel stages of the Swin Factorizer. */
 int fz_linear_wgrad_supported(int32_t cout, int32_t cin, int64_t voxels);
 int fz_linear_wgrad(const float* dy, const float* x, float* dW, float* db, int64_t batch, int32_t cout, int32_t cin,
                     int64_t voxels, void* stream);
@@ -189,14 +190,14 @@ int fz_linear_forward_ex(const float* x, const float* W, const float* bias, floa
 /* (batch, channels, D, H, W) <-> (batch, channels*8, D/2*H/2*W/2) with rows ordered (c, kd, kh, kw): the view on which
  * the reference U-Net's kernel-2 stride-2 down-sampling convolution (factorizer/unet.py:53) and transposed up-sampling
  * convolution (unet.py:97-99) are channel maps.  to_depth != 0: full resolution -> patch rows; 0: the inverse.
- * D, H even and W divisible by 4. */
+ * D, H even and W divisible by 4; in and out 16-byte aligned (FZ_ERR_UNSUPPORTED otherwise). */
 int fz_space_depth2_supported(int32_t D, int32_t H, int32_t W);
 int fz_space_depth2(const float* in, float* out, int64_t batch, int32_t channels, int32_t D, int32_t H, int32_t W,
                     int32_t to_depth, void* stream);
 
 /* 3x3x3 convolution, stride 1, zero padding 1, 1..4 input channels -> 32 output channels: the Swin Factorizer's stem
  * (reference factorizer/factorizer.py:139-140).  x (batch, cin, D, H, W), weight (32, cin, 3, 3, 3), bias 32 floats or
- * NULL, y (batch, 32, D, H, W); fp32 contiguous, W divisible by 4. */
+ * NULL, y (batch, 32, D, H, W); fp32 contiguous, W divisible by 4, x and y 16-byte aligned (FZ_ERR_UNSUPPORTED otherwise). */
 int fz_conv3d_stem_supported(int32_t cin, int32_t cout, int32_t D, int32_t H, int32_t W);
 int fz_conv3d_stem_forward(const float* x, const float* weight, const float* bias, float* y, int64_t batch, int32_t cin,
                            int32_t cout, int32_t D, int32_t H, int32_t W, void* stream);

@@ -288,8 +288,8 @@ def _glue_call(fn, *args):
 
 @pytest.fixture(params=[0, 5, 7], ids=["fp32-pipe", "tc-mlp", "tc-mlp+linear-wgrad"])
 def glue_mode(request):
-    """0 = every glue kernel on the FP32 pipe; bit 0 = forward MLP kernel on tcgen05, bit 2 = MLP backward on tcgen05 (5 is
-    the default), bit 1 = also linear_bwd's weight gradient."""
+    """0 = every glue kernel on the FP32 pipe; bit 0 = forward MLP kernel on tcgen05, bit 2 = MLP backward on tcgen05, bit 1 =
+    also linear_bwd's weight gradient and fz_linear_wgrad (7, all three, is the default)."""
     from factorizer_b200 import _lib as L
     lib = L.lib()
     before = lib.fz_get_glue_mode()
