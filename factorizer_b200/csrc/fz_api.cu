@@ -19,6 +19,26 @@ int fail(int code, const char* fmt, ...) {
     return code;
 }
 
+int encode_tiled_map(CUtensorMap* m, const char* what, CUtensorMapDataType type, cuuint32_t rank, const void* ptr,
+                     const cuuint64_t* dims, const cuuint64_t* strides, const cuuint32_t* box, CUtensorMapSwizzle swizzle) {
+    typedef CUresult (*EncodeTiledFn)(CUtensorMap*, CUtensorMapDataType, cuuint32_t, void*, const cuuint64_t*, const cuuint64_t*,
+                                      const cuuint32_t*, const cuuint32_t*, CUtensorMapInterleave, CUtensorMapSwizzle,
+                                      CUtensorMapL2promotion, CUtensorMapFloatOOBfill);
+    static EncodeTiledFn enc = nullptr;
+    if (!enc) {
+        void* p = nullptr;
+        cudaDriverEntryPointQueryResult q;
+        if (cudaGetDriverEntryPoint("cuTensorMapEncodeTiled", &p, cudaEnableDefault, &q) == cudaSuccess && q == cudaDriverEntryPointSuccess)
+            enc = reinterpret_cast<EncodeTiledFn>(p);
+    }
+    if (!enc) return fail(FZ_ERR_CUDA, "cuTensorMapEncodeTiled entry point not available");
+    const cuuint32_t es[5] = {1, 1, 1, 1, 1};
+    const CUresult r = enc(m, type, rank, const_cast<void*>(ptr), dims, strides, box, es, CU_TENSOR_MAP_INTERLEAVE_NONE, swizzle,
+                           CU_TENSOR_MAP_L2_PROMOTION_L2_128B, CU_TENSOR_MAP_FLOAT_OOB_FILL_NONE);
+    if (r != CUDA_SUCCESS) return fail(FZ_ERR_CUDA, "cuTensorMapEncodeTiled (%s) failed with CUresult %d", what, (int)r);
+    return FZ_OK;
+}
+
 // One window per (sample, head), no roll, and more elements than a CTA can hold: Matricize(grid_size=1), the
 // reference's default FactMixer reshape (factorizer/factorizer.py:17).  The matrix is the contiguous block
 // x[b, h*d:(h+1)*d, :].

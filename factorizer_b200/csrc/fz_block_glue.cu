@@ -23,15 +23,11 @@
 // Every kernel here has a tensor-core twin (tcgen05 / TMEM, 3xTF32: fz_block_glue_fwd_tc.cu, fz_block_glue_lin_tc.cu,
 // fz_block_glue_bwd_tc.cu), which is the default where its shape restrictions hold (hidden width 64 for the MLP backward,
 // 32 or 64 for the forward); these FP32-pipe kernels take every other hidden width and fz_set_glue_mode(0).
-#include "fz_common.cuh"
+#include "fz_device.cuh"
 #include "fz_internal.cuh"
 
 namespace fz {
 namespace {
-
-typedef float2 f2;
-__device__ __forceinline__ f2 fma2(f2 a, f2 b, f2 c) { return __ffma2_rn(a, b, c); }
-__device__ __forceinline__ f2 dup(float a) { return make_float2(a, a); }
 
 constexpr int kC = 32;            // channels the kernels are written for
 constexpr int kMaxHidden = 64;    // hidden units per launch of the backward kernel (shared memory); wider MLPs go slice by slice
@@ -103,61 +99,6 @@ __device__ __forceinline__ f2 normalize(f2 (&v)[C], float eps) {
 #pragma unroll
     for (int c = 0; c < C; ++c) { v[c].x *= rstd.x; v[c].y *= rstd.y; }
     return rstd;
-}
-
-// Transposing warp reduction: every lane passes N values; returns, in every lane, the warp-wide total of
-// element (lane / (32 / N)).  N = 32: 31 shuffles.
-template <int N>
-__device__ __forceinline__ float warp_vec_sum(float (&v)[N], int lane) {
-    static_assert(N == 32 || N == 16 || N == 8 || N == 4, "N");
-    int off = 16;
-#pragma unroll
-    for (int n = N; n > 1; n >>= 1) {
-        const bool up = (lane & off) != 0;
-#pragma unroll
-        for (int i = 0; i < n / 2; ++i) {
-            const float keep = up ? v[i + n / 2] : v[i];
-            const float send = up ? v[i] : v[i + n / 2];
-            v[i] = keep + __shfl_xor_sync(0xffffffffu, send, off);
-        }
-        off >>= 1;
-    }
-    float r = v[0];
-    for (; off > 0; off >>= 1) r += __shfl_xor_sync(0xffffffffu, r, off);
-    return r;
-}
-
-// Exact (erf) GELU through Abramowitz-Stegun 7.1.26: erf(z) = 1 - (a1 t + ... + a5 t^5) exp(-z^2), t = 1/(1 + p z),
-// |error| <= 1.5e-7 for z >= 0, odd extension below.  With z = |h|/sqrt(2) the exponential is exp(-h^2/2), which is
-// also the density the derivative needs; two MUFU ops (RCP, EX2) and ~12 FP32 ops instead of erff + expf (~45).
-// gauss_cdf2 returns Phi(h) = (1 + erf(h/sqrt 2))/2 and e = exp(-h^2/2).
-__device__ __forceinline__ float ex2_approx(float x) { float y; asm("ex2.approx.ftz.f32 %0, %1;" : "=f"(y) : "f"(x)); return y; }
-__device__ __forceinline__ float rcp_approx(float x) { float y; asm("rcp.approx.ftz.f32 %0, %1;" : "=f"(y) : "f"(x)); return y; }
-// two values at a time: the polynomial in packed FFMA2, one MUFU.RCP + one MUFU.EX2 per value
-__device__ __forceinline__ f2 gauss_cdf2(f2 h, f2& e) {
-    const f2 z = make_float2(fabsf(h.x) * 0.70710678118654752f, fabsf(h.y) * 0.70710678118654752f);
-    const f2 d = fma2(dup(0.3275911f), z, dup(1.f));
-    const f2 t = make_float2(rcp_approx(d.x), rcp_approx(d.y));
-    const f2 hh = __fmul2_rn(h, h);
-    e = make_float2(ex2_approx(hh.x * -0.72134752044448170f), ex2_approx(hh.y * -0.72134752044448170f));   // exp(-h^2/2)
-    f2 p = fma2(t, dup(1.061405429f), dup(-1.453152027f));
-    p = fma2(t, p, dup(1.421413741f));
-    p = fma2(t, p, dup(-0.284496736f));
-    p = fma2(t, p, dup(0.254829592f));
-    const f2 pt = __fmul2_rn(p, t);
-    const f2 erf_abs = fma2(make_float2(-pt.x, -pt.y), e, dup(1.f));
-    return fma2(make_float2(copysignf(0.5f, h.x), copysignf(0.5f, h.y)), erf_abs, dup(0.5f));
-}
-__device__ __forceinline__ f2 gelu2(f2 h) {
-    f2 e;
-    return __fmul2_rn(h, gauss_cdf2(h, e));
-}
-// gelu(h) and its derivative Phi(h) + h phi(h)  (torch: GeluBackward, approximate='none')
-__device__ __forceinline__ void gelu_grad2(f2 h, f2& g, f2& gp) {
-    f2 e;
-    const f2 cdf = gauss_cdf2(h, e);
-    g = __fmul2_rn(h, cdf);
-    gp = fma2(__fmul2_rn(h, dup(0.39894228040143268f)), e, cdf);
 }
 
 template <int C>
@@ -645,8 +586,6 @@ __global__ void __launch_bounds__(kTT, 1) mlp_bwd(const float* __restrict__ x1, 
 // backward; all on by default.  fz_set_glue_mode() exists for the parity tests and the benchmark's FP32-pipe comparison.
 int glue_mode() { return tls().glue_mode; }
 
-int sm_count() { return num_sms(); }
-
 int check_common(long long batch, int channels, long long voxels) {
     if (batch < 0 || voxels < 0) return fail(FZ_ERR_INVALID, "negative size");
     if (channels != kC) return fail(FZ_ERR_UNSUPPORTED, "block glue kernels are built for %d channels, got %d", kC, channels);
@@ -685,7 +624,7 @@ int fz_ln_linear_forward(const float* x, const float* gamma, const float* beta, 
     if (glue_mode() & 1) return ln_linear_tc_launch(x, gamma, beta, W, y, batch, voxels, eps, (cudaStream_t)stream);
     const long long pps = voxels / 2, total = batch * pps;
     long long blocks = (total + 127) / 128;
-    const long long cap = 3LL * sm_count();
+    const long long cap = 3LL * num_sms();
     if (blocks > cap) blocks = cap;
     ln_linear_fwd<kC><<<(unsigned)blocks, 128, 0, (cudaStream_t)stream>>>(x, gamma, beta, W, y, pps, total, eps);
     FZ_LAUNCH_CHECK();
@@ -712,7 +651,7 @@ int fz_mixer_mlp_forward(const float* x, const float* m, const float* Wout, cons
     FZ_CUDA_CHECK(cfg.ensure(mixer_mlp_fwd<kC>, smem));
     const long long pps = voxels / 2, total = batch * pps;
     long long blocks = (total + 127) / 128;
-    const long long cap = 2LL * sm_count();
+    const long long cap = 2LL * num_sms();
     if (blocks > cap) blocks = cap;
     mixer_mlp_fwd<kC><<<(unsigned)blocks, 128, smem, (cudaStream_t)stream>>>(x, m, Wout, bout, gamma, beta, W1, b1, W2, b2, x1, out,
                                                                              hidden, pps, total, eps);
@@ -746,7 +685,7 @@ int fz_linear_backward(const float* dy, const float* a, const float* gamma, cons
     FZ_CUDA_CHECK(cfg_plain.ensure(linear_bwd<kC, false>, smem));
     const int tps = (int)((voxels + kLV - 1) / kLV);
     const long long tiles = batch * tps;
-    const unsigned blocks = (unsigned)(tiles < 2LL * sm_count() ? tiles : 2LL * sm_count());
+    const unsigned blocks = (unsigned)(tiles < 2LL * num_sms() ? tiles : 2LL * num_sms());
     if (layernorm)
         linear_bwd<kC, true><<<blocks, kLT, smem, st>>>(dy, a, gamma, beta, W, resid, da, dW, db, dgamma, dbeta, voxels, tps, tiles, eps);
     else
@@ -779,7 +718,7 @@ int fz_mlp_backward(const float* x1, const float* dout, const float* gamma, cons
         return mlp_bwd_tc_launch(x1, dout, gamma, beta, W1, b1, W2, dx1, dgamma, dbeta, dW1, db1, dW2, db2, batch, hidden, voxels, eps, st);
     const int tps = (int)((voxels + kTV - 1) / kTV);
     const long long tiles = batch * tps;
-    const unsigned blocks = (unsigned)(tiles < sm_count() ? tiles : sm_count());
+    const unsigned blocks = (unsigned)(tiles < num_sms() ? tiles : num_sms());
     // the kernel holds the weights and weight-gradient accumulators of at most kMaxHidden hidden units in shared
     // memory; wider MLPs (mlp_ratio 4: model_zoo/factorizer_brats23/configs/train.yaml) run slice by slice
     for (int h0 = 0; h0 < hidden; h0 += kMaxHidden) {

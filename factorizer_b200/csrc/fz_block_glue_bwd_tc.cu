@@ -62,26 +62,6 @@ __device__ long long* g_mlp_bwd_trace = nullptr;
 #define FZ_TR(slot) do { } while (0)
 #endif
 
-// transposing warp reduction of N values: lane l ends with the warp total of element l / (32 / N)
-template <int N>
-__device__ __forceinline__ float warp_vec_sum(float (&v)[N], int lane) {
-    int off = 16;
-#pragma unroll
-    for (int n = N; n > 1; n >>= 1) {
-        const bool up = (lane & off) != 0;
-#pragma unroll
-        for (int i = 0; i < n / 2; ++i) {
-            const float keep = up ? v[i + n / 2] : v[i];
-            const float send = up ? v[i] : v[i + n / 2];
-            v[i] = keep + __shfl_xor_sync(0xffffffffu, send, off);
-        }
-        off >>= 1;
-    }
-    float r = v[0];
-    for (; off > 0; off >>= 1) r += __shfl_xor_sync(0xffffffffu, r, off);
-    return r;
-}
-
 __global__ void __launch_bounds__(kThreads, 1)
 mlp_bwd_tc(const float* __restrict__ x1, const float* __restrict__ dout, const float* __restrict__ gamma,
            const float* __restrict__ beta, const float* __restrict__ W1, const float* __restrict__ b1,
@@ -127,15 +107,15 @@ mlp_bwd_tc(const float* __restrict__ x1, const float* __restrict__ dout, const f
         par[j] = s;
     }
     if (tid == 0) {
-        bar_init(bar_p1a, kWorkers); bar_init(bar_p1b, kWorkers); bar_init(bar_g1, 1); bar_init(bar_g2, 1); bar_init(bar_p2, kWorkers);
-        bar_init(bar_g3, 1); bar_init(bar_wg, 1);
-        asm volatile("fence.mbarrier_init.release.cluster;" ::: "memory");
+        mbar_init(bar_p1a, kWorkers); mbar_init(bar_p1b, kWorkers); mbar_init(bar_g1, 1); mbar_init(bar_g2, 1); mbar_init(bar_p2, kWorkers);
+        mbar_init(bar_g3, 1); mbar_init(bar_wg, 1);
+        fence_mbarrier_init();
     }
     if (warp == kMmaWarp) {
-        asm volatile("tcgen05.alloc.cta_group::1.sync.aligned.shared::cta.b32 [%0], %1;" :: "r"(sbase + oTmem), "n"(kTmemCols) : "memory");
-        asm volatile("tcgen05.relinquish_alloc_permit.cta_group::1.sync.aligned;" ::: "memory");
+        tmem_alloc<kTmemCols>(sbase + oTmem);
+        tmem_relinquish_alloc_permit();
     }
-    fence_async_smem();
+    fence_proxy_async_smem();
     tc_fence_before();
     __syncthreads();
     tc_fence_after();
@@ -162,7 +142,7 @@ mlp_bwd_tc(const float* __restrict__ x1, const float* __restrict__ dout, const f
             const uint64_t k_xh = make_desc(sbase + oXH, kAtom, 512, 1);
             for (long long it = 0; it < my_tiles; ++it) {
                 const uint32_t ph = (uint32_t)(it & 1);
-                bar_wait(bar_p1a, ph);
+                mbar_wait(bar_p1a, ph);
                 tc_fence_after();
                 FZ_TR(8);
                 if (elect_one()) {
@@ -176,7 +156,7 @@ mlp_bwd_tc(const float* __restrict__ x1, const float* __restrict__ dout, const f
                 }
                 __syncwarp();
                 FZ_TR(9);
-                bar_wait(bar_p1b, ph);
+                mbar_wait(bar_p1b, ph);
                 tc_fence_after();
                 FZ_TR(14);
                 if (elect_one()) {
@@ -190,7 +170,7 @@ mlp_bwd_tc(const float* __restrict__ x1, const float* __restrict__ dout, const f
                 }
                 __syncwarp();
                 FZ_TR(15);
-                bar_wait(bar_p2, ph);
+                mbar_wait(bar_p2, ph);
                 tc_fence_after();
                 FZ_TR(10);
                 if (elect_one()) {
@@ -291,7 +271,7 @@ mlp_bwd_tc(const float* __restrict__ x1, const float* __restrict__ dout, const f
                     xh[i] = xr[i]; go[i] = dr[i];
                     l8[i] = tf32_lo(xh[i]); th[i] = __float_as_uint(xh[i]); tl[i] = __float_as_uint(l8[i]);
                 }
-                if (it > 0) bar_wait(bar_wg, pph);                       // the previous tile's contractions have read their operands
+                if (it > 0) mbar_wait(bar_wg, pph);                       // the previous tile's contractions have read their operands
                 tc_fence_after();
                 if (warp == 0) FZ_TR(1);
                 st_row_chunk(sbase + oXH + cx, swap, xh);
@@ -300,8 +280,8 @@ mlp_bwd_tc(const float* __restrict__ x1, const float* __restrict__ dout, const f
                 tmem_st8(lane_addr + cA + 32 + qq * 8, tl);
                 tmem_st_wait();
                 tc_fence_before();
-                fence_async_smem();
-                bar_arrive(bar_p1a);
+                fence_proxy_async_smem();
+                mbar_arrive(bar_p1a);
 #pragma unroll
                 for (int i = 0; i < 8; ++i) {
                     l8[i] = tf32_lo(go[i]); th[i] = __float_as_uint(go[i]); tl[i] = __float_as_uint(l8[i]);
@@ -314,8 +294,8 @@ mlp_bwd_tc(const float* __restrict__ x1, const float* __restrict__ dout, const f
                 tmem_st8(lane_addr + cA + 96 + qq * 8, tl);
                 tmem_st_wait();
                 tc_fence_before();
-                fence_async_smem();
-                bar_arrive(bar_p1b);
+                fence_proxy_async_smem();
+                mbar_arrive(bar_p1b);
             }
             if (warp == 0) FZ_TR(3);
             // next tile's loads: in flight during this tile's GELU phase
@@ -325,7 +305,7 @@ mlp_bwd_tc(const float* __restrict__ x1, const float* __restrict__ dout, const f
             {
                 uint32_t hr[16], dh_hi[16], dh_lo[16];
                 float gp[16];
-                bar_wait(bar_g1, ph);
+                mbar_wait(bar_g1, ph);
                 tc_fence_after();
                 if (warp == 0) FZ_TR(4);
                 tmem_ld16_nowait(lane_addr + cH + qq * 16, hr);
@@ -346,7 +326,7 @@ mlp_bwd_tc(const float* __restrict__ x1, const float* __restrict__ dout, const f
                     st_row_chunk(sbase + oG + cg, swap, g8);
                     st_row_chunk(sbase + oG + 2 * kAtom + cg, swap, gl8);
                 }
-                bar_wait(bar_g2, ph);
+                mbar_wait(bar_g2, ph);
                 tc_fence_after();
                 tmem_ld16_nowait(lane_addr + cDG + qq * 16, hr);
                 tmem_ld_wait();
@@ -370,12 +350,12 @@ mlp_bwd_tc(const float* __restrict__ x1, const float* __restrict__ dout, const f
                 tmem_st_wait();
             }
             tc_fence_before();
-            fence_async_smem();
-            bar_arrive(bar_p2);
+            fence_proxy_async_smem();
+            mbar_arrive(bar_p2);
             if (warp == 0) FZ_TR(5);
             // the next tile's LayerNorm while GEMM3 runs
             if (it + 1 < my_tiles) normalise();
-            bar_wait(bar_g3, ph);
+            mbar_wait(bar_g3, ph);
             tc_fence_after();
             if (warp == 0) FZ_TR(6);
             // ---- P3: through LayerNorm, plus the residual branch ----
@@ -407,7 +387,7 @@ mlp_bwd_tc(const float* __restrict__ x1, const float* __restrict__ dout, const f
             tc_fence_before();
             if (warp == 0) FZ_TR(7);
         }
-        if (my_tiles > 0) bar_wait(bar_wg, (uint32_t)((my_tiles - 1) & 1));
+        if (my_tiles > 0) mbar_wait(bar_wg, (uint32_t)((my_tiles - 1) & 1));
         tc_fence_after();
         // ---- per-CTA totals of the register accumulators ----
         {
@@ -477,7 +457,7 @@ mlp_bwd_tc(const float* __restrict__ x1, const float* __restrict__ dout, const f
     __syncthreads();
     if (warp == kMmaWarp) {
         __syncwarp();
-        asm volatile("tcgen05.dealloc.cta_group::1.sync.aligned.b32 %0, %1;" :: "r"(tmem), "n"(kTmemCols) : "memory");
+        tmem_dealloc<kTmemCols>(tmem);
     }
 }
 

@@ -82,14 +82,14 @@ mixer_mlp_fwd_tc2(const float* __restrict__ x, const float* __restrict__ m, cons
     }
     for (int j = tid; j < HID; j += kThreads) par[4 * kC + j] = b1 ? b1[j] : 0.f;
     if (tid == 0) {
-        bar_init(bar, 1);
-        asm volatile("fence.mbarrier_init.release.cluster;" ::: "memory");
+        mbar_init(bar, 1);
+        fence_mbarrier_init();
     }
     if (warp == 0) {
-        asm volatile("tcgen05.alloc.cta_group::1.sync.aligned.shared::cta.b32 [%0], %1;" :: "r"(sbase + L::oTmem), "n"(kTmemCols) : "memory");
-        asm volatile("tcgen05.relinquish_alloc_permit.cta_group::1.sync.aligned;" ::: "memory");
+        tmem_alloc<kTmemCols>(sbase + L::oTmem);
+        tmem_relinquish_alloc_permit();
     }
-    fence_async_smem();
+    fence_proxy_async_smem();
     tc_fence_before();
     __syncthreads();
     tc_fence_after();
@@ -146,7 +146,7 @@ mixer_mlp_fwd_tc2(const float* __restrict__ x, const float* __restrict__ m, cons
         }
     };
     auto wait_gemm = [&]() {
-        bar_wait(bar, parity);
+        mbar_wait(bar, parity);
         parity ^= 1;
         tc_fence_after();
     };
@@ -242,7 +242,7 @@ mixer_mlp_fwd_tc2(const float* __restrict__ x, const float* __restrict__ m, cons
     }
     tc_fence_before();
     __syncthreads();
-    if (warp == 0) asm volatile("tcgen05.dealloc.cta_group::1.sync.aligned.b32 %0, %1;" :: "r"(tmem), "n"(kTmemCols) : "memory");
+    if (warp == 0) tmem_dealloc<kTmemCols>(tmem);
 }
 
 // --------------------------------------------------------------------------------------------------------------------
@@ -277,14 +277,14 @@ ln_linear_fwd_tc(const float* __restrict__ x, const float* __restrict__ gamma, c
         wb[o] = s;
     }
     if (tid == 0) {
-        bar_init(bar, 1);
-        asm volatile("fence.mbarrier_init.release.cluster;" ::: "memory");
+        mbar_init(bar, 1);
+        fence_mbarrier_init();
     }
     if (warp == 0) {
-        asm volatile("tcgen05.alloc.cta_group::1.sync.aligned.shared::cta.b32 [%0], 128;" :: "r"(sbase + lTmem) : "memory");
-        asm volatile("tcgen05.relinquish_alloc_permit.cta_group::1.sync.aligned;" ::: "memory");
+        tmem_alloc<128>(sbase + lTmem);
+        tmem_relinquish_alloc_permit();
     }
-    fence_async_smem();
+    fence_proxy_async_smem();
     tc_fence_before();
     __syncthreads();
     tc_fence_after();
@@ -353,7 +353,7 @@ ln_linear_fwd_tc(const float* __restrict__ x, const float* __restrict__ gamma, c
             __syncwarp();
         }
         if (it + 1 < my_tiles) fetch();
-        bar_wait(bar, parity);
+        mbar_wait(bar, parity);
         parity ^= 1;
         tc_fence_after();
         {
@@ -370,7 +370,7 @@ ln_linear_fwd_tc(const float* __restrict__ x, const float* __restrict__ gamma, c
     }
     tc_fence_before();
     __syncthreads();
-    if (warp == 0) asm volatile("tcgen05.dealloc.cta_group::1.sync.aligned.b32 %0, 128;" :: "r"(tmem) : "memory");
+    if (warp == 0) tmem_dealloc<128>(tmem);
 }
 
 }  // namespace

@@ -33,25 +33,6 @@ constexpr uint32_t kSmem = oTmem + 8;
 // TMEM columns: A = dy hi | lo, D = d(xh), contraction accumulator (64 rows x 64 columns)
 constexpr uint32_t cA = 0, cD = 64, cWG = 96, kTmemCols = 256;
 
-template <int N>
-__device__ __forceinline__ float warp_vec_sum(float (&v)[N], int lane) {
-    int off = 16;
-#pragma unroll
-    for (int n = N; n > 1; n >>= 1) {
-        const bool up = (lane & off) != 0;
-#pragma unroll
-        for (int i = 0; i < n / 2; ++i) {
-            const float keep = up ? v[i + n / 2] : v[i];
-            const float send = up ? v[i] : v[i + n / 2];
-            v[i] = keep + __shfl_xor_sync(0xffffffffu, send, off);
-        }
-        off >>= 1;
-    }
-    float r = v[0];
-    for (; off > 0; off >>= 1) r += __shfl_xor_sync(0xffffffffu, r, off);
-    return r;
-}
-
 template <bool LN>
 __global__ void __launch_bounds__(kThreads, 2)
 linear_bwd_tc2(const float* __restrict__ dy, const float* __restrict__ a, const float* __restrict__ gamma,
@@ -77,14 +58,14 @@ linear_bwd_tc2(const float* __restrict__ dy, const float* __restrict__ a, const 
         par[kC + c] = LN && beta ? beta[c] : 0.f;
     }
     if (tid == 0) {
-        bar_init(bar_g, 1); bar_init(bar_wg, 1);
-        asm volatile("fence.mbarrier_init.release.cluster;" ::: "memory");
+        mbar_init(bar_g, 1); mbar_init(bar_wg, 1);
+        fence_mbarrier_init();
     }
     if (warp == 0) {
-        asm volatile("tcgen05.alloc.cta_group::1.sync.aligned.shared::cta.b32 [%0], %1;" :: "r"(sbase + oTmem), "n"(kTmemCols) : "memory");
-        asm volatile("tcgen05.relinquish_alloc_permit.cta_group::1.sync.aligned;" ::: "memory");
+        tmem_alloc<kTmemCols>(sbase + oTmem);
+        tmem_relinquish_alloc_permit();
     }
-    fence_async_smem();
+    fence_proxy_async_smem();
     tc_fence_before();
     __syncthreads();
     tc_fence_after();
@@ -149,7 +130,7 @@ linear_bwd_tc2(const float* __restrict__ dy, const float* __restrict__ a, const 
             for (int c = 0; c < 16; ++c) xh[c] = ar[c];
         }
         // ---- dy -> TMEM (A of the GEMM) and voxel rows; xh -> voxel rows ----
-        if (it > 0) bar_wait(bar_wg, ph ^ 1);                // the previous tile's contraction has read the rows
+        if (it > 0) mbar_wait(bar_wg, ph ^ 1);                // the previous tile's contraction has read the rows
         tc_fence_after();
         {
             uint32_t th[16], tl[16];
@@ -175,7 +156,7 @@ linear_bwd_tc2(const float* __restrict__ dy, const float* __restrict__ a, const 
             tmem_st_wait();
         }
         tc_fence_before();
-        fence_async_smem();
+        fence_proxy_async_smem();
         __syncthreads();
         if (issuer) {
             tc_fence_after();
@@ -202,7 +183,7 @@ linear_bwd_tc2(const float* __restrict__ dy, const float* __restrict__ a, const 
             for (int c = 0; c < 16; ++c) { rs[c] = (resid && cur_valid) ? __ldg(pr) : 0.f; pr += vox; }
         }
         if (it + 1 < my_tiles) fetch();
-        bar_wait(bar_g, ph);
+        mbar_wait(bar_g, ph);
         tc_fence_after();
         // ---- da ----
         if (LN) {
@@ -234,7 +215,7 @@ linear_bwd_tc2(const float* __restrict__ dy, const float* __restrict__ a, const 
         }
         tc_fence_before();
     }
-    if (my_tiles > 0) bar_wait(bar_wg, ph ^ 1);
+    if (my_tiles > 0) mbar_wait(bar_wg, ph ^ 1);
     tc_fence_after();
     // ---- per-CTA totals ----
     {
@@ -290,7 +271,7 @@ linear_bwd_tc2(const float* __restrict__ dy, const float* __restrict__ a, const 
     }
     tc_fence_before();
     __syncthreads();
-    if (warp == 0) asm volatile("tcgen05.dealloc.cta_group::1.sync.aligned.b32 %0, %1;" :: "r"(tmem), "n"(kTmemCols) : "memory");
+    if (warp == 0) tmem_dealloc<kTmemCols>(tmem);
 }
 
 }  // namespace

@@ -1,5 +1,6 @@
 // Shared host/device helpers for the factorizer_b200 CUDA library (sm_100a only).
 #pragma once
+#include <cuda.h>
 #include <cuda_runtime.h>
 #include <stdint.h>
 #include <stdio.h>
@@ -18,6 +19,12 @@ struct TlsState {
 };
 TlsState& tls();
 int fail(int code, const char* fmt, ...);
+
+// cuTensorMapEncodeTiled (driver entry point, looked up once) with element strides of 1, no interleave, L2 promotion in
+// 128-byte lines and out-of-bounds elements read as zeros; every tensor map of the library is encoded here.  On failure:
+// fail(FZ_ERR_CUDA, ...) naming the map (`what`).
+int encode_tiled_map(CUtensorMap* m, const char* what, CUtensorMapDataType type, cuuint32_t rank, const void* ptr,
+                     const cuuint64_t* dims, const cuuint64_t* strides, const cuuint32_t* box, CUtensorMapSwizzle swizzle);
 
 #define FZ_CUDA_CHECK(expr)                                                                     \
     do {                                                                                        \

@@ -262,9 +262,6 @@ __global__ void __launch_bounds__(kLnThreads) layernorm_cf_bwd_any(const float* 
     }
 }
 
-int sm_count();
-int sm_count_cached() { return sm_count(); }
-
 // ---- few voxels, many channels (the deep stages: 128 ch at 32^3 ... 512 ch at 8^3) -------------------------------------
 // A thread walking all C channels of its voxel pair is one long latency chain there and the grid is a handful of CTAs.
 // Sliced form: blockDim = (32 voxel pairs, SL channel slices); every warp owns C / SL channels of the CTA's 32 pairs,
@@ -418,17 +415,15 @@ __global__ void __launch_bounds__(32 * kLnMaxSlices, 2) layernorm_cf_bwd_sliced(
 
 // slices for the sliced kernels: 0 = use the one-thread-per-voxel-pair kernels
 int ln_slices(int channels, long long total_pairs) {
-    if (channels < 64 || total_pairs >= 256LL * sm_count_cached()) return 0;
+    if (channels < 64 || total_pairs >= 256LL * num_sms()) return 0;
     return channels >= 256 ? 8 : (channels >= 128 ? 4 : 2);
 }
-
-int sm_count() { return num_sms(); }
 
 template <int C>
 int launch_fwd(const float* x, const float* gamma, const float* beta, float* y, long long batch, long long voxels, float eps, cudaStream_t st) {
     const long long pps = voxels / 2, total = batch * pps;
     long long blocks = (total + kLnThreads - 1) / kLnThreads;
-    const long long cap = 8LL * sm_count();
+    const long long cap = 8LL * num_sms();
     if (blocks > cap) blocks = cap;
     layernorm_cf_fwd<C><<<(unsigned)blocks, kLnThreads, 0, st>>>(x, gamma, beta, y, pps, total, eps);
     FZ_LAUNCH_CHECK();
@@ -439,7 +434,7 @@ int launch_bwd(const float* x, const float* gamma, const float* dy, const float*
                long long voxels, float eps, cudaStream_t st) {
     const long long pps = voxels / 2, total = batch * pps;
     long long blocks = (total + kLnThreads - 1) / kLnThreads;
-    const long long cap = 2LL * sm_count();
+    const long long cap = 2LL * num_sms();
     if (blocks > cap) blocks = cap;
     if (dgamma) FZ_CUDA_CHECK(cudaMemsetAsync(dgamma, 0, C * sizeof(float), st));
     if (dbeta) FZ_CUDA_CHECK(cudaMemsetAsync(dbeta, 0, C * sizeof(float), st));
@@ -485,14 +480,14 @@ int fz_layernorm_cf_forward(const float* x, const float* gamma, const float* bet
         const long long pps = voxels / 2, total = batch * pps;
         if (const int sl = ln_slices(channels, total)) {
             long long groups = (total + 31) / 32;
-            if (groups > 8LL * sm_count()) groups = 8LL * sm_count();
+            if (groups > 8LL * num_sms()) groups = 8LL * num_sms();
             layernorm_cf_fwd_sliced<<<(unsigned)groups, dim3(32, sl), 0, st>>>(x, gamma, beta, y, channels, pps, total, eps);
             FZ_LAUNCH_CHECK();
             return FZ_OK;
         }
-        const int threads = total >= 256LL * sm_count() ? kLnThreads : 64;   // few voxels: spread them over more SMs
+        const int threads = total >= 256LL * num_sms() ? kLnThreads : 64;   // few voxels: spread them over more SMs
         long long blocks = (total + threads - 1) / threads;
-        const long long cap = 8LL * sm_count();
+        const long long cap = 8LL * num_sms();
         if (blocks > cap) blocks = cap;
         layernorm_cf_fwd_any<<<(unsigned)blocks, threads, 0, st>>>(x, gamma, beta, y, channels, pps, total, eps);
         FZ_LAUNCH_CHECK();
@@ -524,15 +519,15 @@ int fz_layernorm_cf_backward_add(const float* x, const float* gamma, const float
     }
     {
         const long long pps = voxels / 2, total = batch * pps;
-        const int threads = total >= 256LL * sm_count() ? kLnThreads : 64;
+        const int threads = total >= 256LL * num_sms() ? kLnThreads : 64;
         long long blocks = (total + threads - 1) / threads;
-        const long long cap = 4LL * sm_count();
+        const long long cap = 4LL * num_sms();
         if (blocks > cap) blocks = cap;
         if (dgamma) FZ_CUDA_CHECK(cudaMemsetAsync(dgamma, 0, channels * sizeof(float), st));
         if (dbeta) FZ_CUDA_CHECK(cudaMemsetAsync(dbeta, 0, channels * sizeof(float), st));
         if (const int sl = ln_slices(channels, total)) {
             long long groups = (total + 31) / 32;
-            if (groups > 4LL * sm_count()) groups = 4LL * sm_count();
+            if (groups > 4LL * num_sms()) groups = 4LL * num_sms();
             layernorm_cf_bwd_sliced<<<(unsigned)groups, dim3(32, sl), sizeof(float) * 3 * channels, st>>>(x, gamma, dy, add, dx, dgamma, dbeta,
                                                                                                          channels, pps, total, eps);
             FZ_LAUNCH_CHECK();

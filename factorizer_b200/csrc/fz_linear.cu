@@ -12,7 +12,7 @@
 // 256 voxels of its 32 + 32 rows in shared memory, keeps the partial sums in registers (a warp takes every 4th float4 column,
 // a lane an 8 x 4 sub-block read with broadcast LDS.128) and adds them to dW once at the end.  linear_wgrad64 (further down):
 // 64 x 64 or 32 x 128 blocks, cp.async double buffering, 8 x 8 register tiles.  FP32 pipe, exact fp32 products.
-#include "fz_common.cuh"
+#include "fz_device.cuh"
 #include "fz_internal.cuh"
 
 namespace fz {
@@ -22,10 +22,6 @@ constexpr int kWT = 128;            // threads
 constexpr int kWV = 256;            // voxels per tile
 constexpr int kWRS = kWV + 4;       // staged row stride (floats), = 4 mod 32: conflict-free row-broadcast reads
 constexpr int kWWarps = kWT / 32;
-
-__device__ __forceinline__ float2 ffma2(float2 a, float2 b, float2 c) {
-    return __ffma2_rn(a, b, c);
-}
 
 // rows [r0, r0+32) x voxels [v0, v0+256) of a (rows_total, vox) matrix -> S[32][kWRS]; past-the-end voxels and rows
 // (rows_left = rows_total - r0 may be below 32) read as 0
@@ -85,8 +81,8 @@ __global__ void __launch_bounds__(kWT, 3) linear_wgrad(const float* __restrict__
                 const float4 A = *reinterpret_cast<const float4*>(SA + (ro + 4 * i) * kWRS + v);
 #pragma unroll
                 for (int k = 0; k < 4; ++k) {
-                    acc[i][k] = ffma2(make_float2(A.x, A.y), make_float2(B[k].x, B[k].y), acc[i][k]);
-                    acc[i][k] = ffma2(make_float2(A.z, A.w), make_float2(B[k].z, B[k].w), acc[i][k]);
+                    acc[i][k] = fma2(make_float2(A.x, A.y), make_float2(B[k].x, B[k].y), acc[i][k]);
+                    acc[i][k] = fma2(make_float2(A.z, A.w), make_float2(B[k].z, B[k].w), acc[i][k]);
                 }
             }
         }
@@ -126,12 +122,6 @@ __global__ void __launch_bounds__(kWT, 3) linear_wgrad(const float* __restrict__
 // owns 32 dy rows (w & 1) x all 64 x rows of every fourth float4 column (w >> 1).
 constexpr int kW2T = 256, kW2V = 128, kW2RS = kW2V + 4;
 
-__device__ __forceinline__ void cp_async16(float* dst, const float* src, bool real) {
-    const unsigned d = (unsigned)__cvta_generic_to_shared(dst);
-    const int n = real ? 16 : 0;
-    asm volatile("cp.async.cg.shared.global [%0], [%1], 16, %2;" ::"r"(d), "l"(src), "r"(n) : "memory");
-}
-
 // RB x CB = 2 x 1: a 64 x 64 block (warp halves split the dy rows); 1 x 2: a 32 x 128 block for layers with at most 32
 // outputs (the stem's unfolded 32 x 108 gradient, the decoder adapters), where the warp halves split the x rows.
 template <int RB, int CB>
@@ -170,9 +160,9 @@ __global__ void __launch_bounds__(kW2T, 1) linear_wgrad64(const float* __restric
             const int ch = isx ? i0 + r - NA : o0 + r;
             const bool real = in_v && ch < (isx ? cin : cout);
             const float* src = real ? (isx ? gx : gdy) + (long long)ch * vox + v : dy;
-            cp_async16(S + r * kW2RS, src, real);
+            cp_async16_zfill(S + r * kW2RS, src, real);
         }
-        asm volatile("cp.async.commit_group;" ::: "memory");
+        cp_async_commit();
     };
 
     long long tile = blockIdx.x;
@@ -181,9 +171,9 @@ __global__ void __launch_bounds__(kW2T, 1) linear_wgrad64(const float* __restric
     for (; tile < total_tiles; tile += gridDim.x, stage ^= 1) {
         if (tile + gridDim.x < total_tiles) {
             issue(tile + gridDim.x, stage ^ 1);
-            asm volatile("cp.async.wait_group 1;" ::: "memory");
+            cp_async_wait<1>();
         } else {
-            asm volatile("cp.async.wait_group 0;" ::: "memory");
+            cp_async_wait<0>();
         }
         __syncthreads();
         const float* SA = sm + stage * kW2Stage + (32 * sr) * kW2RS;
@@ -200,8 +190,8 @@ __global__ void __launch_bounds__(kW2T, 1) linear_wgrad64(const float* __restric
                 if (sums) rs[i] += (A.x + A.y) + (A.z + A.w);
 #pragma unroll
                 for (int k = 0; k < 8; ++k) {
-                    acc[i][k] = ffma2(make_float2(A.x, A.y), make_float2(B[k].x, B[k].y), acc[i][k]);
-                    acc[i][k] = ffma2(make_float2(A.z, A.w), make_float2(B[k].z, B[k].w), acc[i][k]);
+                    acc[i][k] = fma2(make_float2(A.x, A.y), make_float2(B[k].x, B[k].y), acc[i][k]);
+                    acc[i][k] = fma2(make_float2(A.z, A.w), make_float2(B[k].z, B[k].w), acc[i][k]);
                 }
             }
         }
@@ -325,8 +315,8 @@ __global__ void __launch_bounds__(128, 2) conv3_stem_fwd(const float* __restrict
                     const float wa[4] = {wv.x, wv.y, wv.z, wv.w};
 #pragma unroll
                     for (int e = 0; e < 4; ++e) {
-                        acc[4 * o4 + e][0] = ffma2(make_float2(wa[e], wa[e]), p[kw][0], acc[4 * o4 + e][0]);
-                        acc[4 * o4 + e][1] = ffma2(make_float2(wa[e], wa[e]), p[kw][1], acc[4 * o4 + e][1]);
+                        acc[4 * o4 + e][0] = fma2(make_float2(wa[e], wa[e]), p[kw][0], acc[4 * o4 + e][0]);
+                        acc[4 * o4 + e][1] = fma2(make_float2(wa[e], wa[e]), p[kw][1], acc[4 * o4 + e][1]);
                     }
                 }
             c = cn; lft = lftn; rgt = rgtn;
@@ -368,9 +358,7 @@ int fz_linear_wgrad(const float* dy, const float* x, float* dW, float* db, int64
     // tensor-core path (csrc/fz_linear_tc.cu: TMA-fed K-major operands, 3xTF32) unless the calling thread asked for the FP32 pipe
     if ((tls().glue_mode & 2) && batch * voxels >= 4096 && linear_wgrad_tc_supported(dy, x, batch, cout, cin, voxels))
         return linear_wgrad_tc_launch(dy, x, dW, db, batch, cout, cin, voxels, st);
-    int dev = 0, sms = 148;
-    FZ_CUDA_CHECK(cudaGetDevice(&dev));
-    FZ_CUDA_CHECK(cudaDeviceGetAttribute(&sms, cudaDevAttrMultiProcessorCount, dev));
+    const int sms = num_sms();
     // fewer voxels: the smaller CTAs of the 32 x 32 kernel spread better; a 32 x 128 block pays from 65 input rows on
     if ((cout >= 64 ? cin >= 64 : cin > 64) && batch * voxels >= 32768) {
         const int tps = (int)((voxels + kW2V - 1) / kW2V);
@@ -448,9 +436,7 @@ int fz_space_depth2(const float* in, float* out, int64_t batch, int32_t channels
     if (!in || !out) return fail(FZ_ERR_INVALID, "space/depth: null buffer");
     if (unaligned16(in) || unaligned16(out)) return fail(FZ_ERR_UNSUPPORTED, "space/depth kernel needs 16-byte aligned buffers");
     const long long total4 = (long long)batch * channels * D * H * (W / 4);
-    int dev = 0, sms = 148;
-    FZ_CUDA_CHECK(cudaGetDevice(&dev));
-    FZ_CUDA_CHECK(cudaDeviceGetAttribute(&sms, cudaDevAttrMultiProcessorCount, dev));
+    const int sms = num_sms();
     long long blocks = (total4 + 255) / 256;
     if (blocks > 16LL * sms) blocks = 16LL * sms;
     cudaStream_t st = (cudaStream_t)stream;
@@ -473,9 +459,7 @@ int fz_conv3d_stem_forward(const float* x, const float* weight, const float* bia
     if (!x || !weight || !y) return fail(FZ_ERR_INVALID, "stem convolution: null buffer");
     if (unaligned16(x) || unaligned16(y)) return fail(FZ_ERR_UNSUPPORTED, "stem convolution kernel needs 16-byte aligned x and y");
     const long long total4 = (long long)batch * D * H * (W / 4);
-    int dev = 0, sms = 148;
-    FZ_CUDA_CHECK(cudaGetDevice(&dev));
-    FZ_CUDA_CHECK(cudaDeviceGetAttribute(&sms, cudaDevAttrMultiProcessorCount, dev));
+    const int sms = num_sms();
     long long blocks = (total4 + 127) / 128;
     if (blocks > 16LL * sms) blocks = 16LL * sms;
     cudaStream_t st = (cudaStream_t)stream;

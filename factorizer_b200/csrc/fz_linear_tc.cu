@@ -12,8 +12,6 @@
 // voxels and are added up, then added to the global gradient with one atomic per element and CTA.
 // Warp roles: warp 0 = TMA producer, warp 1 = MMA issue (warp-uniform code under elect.sync), warps 2-5 = remainder tiles and
 // epilogue.  Three stages of 32 KB, two CTAs per SM.
-#include <cuda.h>
-
 #include "fz_tc.cuh"
 
 namespace fz {
@@ -32,40 +30,13 @@ constexpr uint32_t oBarFull = kStages * kStage, oBarLo = oBarFull + 8 * kStages,
                    oBarDone = oBarEmpty + 8 * kStages, oTmemSlot = oBarDone + 8, kSmemW = oTmemSlot + 8;
 constexpr int kN = 2 * kBlk + 16;              // 144 accumulator columns
 
-typedef CUresult (*EncodeTiledFn)(CUtensorMap*, CUtensorMapDataType, cuuint32_t, void*, const cuuint64_t*, const cuuint64_t*,
-                                  const cuuint32_t*, const cuuint32_t*, CUtensorMapInterleave, CUtensorMapSwizzle,
-                                  CUtensorMapL2promotion, CUtensorMapFloatOOBfill);
-EncodeTiledFn encode_fn() {
-    static EncodeTiledFn fn = nullptr;
-    if (!fn) {
-        void* p = nullptr;
-        cudaDriverEntryPointQueryResult q;
-        if (cudaGetDriverEntryPoint("cuTensorMapEncodeTiled", &p, cudaEnableDefault, &q) == cudaSuccess && q == cudaDriverEntryPointSuccess)
-            fn = reinterpret_cast<EncodeTiledFn>(p);
-    }
-    return fn;
-}
 // (batch, channels, voxels) fp32, box (1, 64, 32): rows beyond `channels` read as zeros, so do voxels beyond the end
 int make_map(CUtensorMap* m, const float* ptr, long long batch, int channels, long long voxels) {
-    EncodeTiledFn enc = encode_fn();
-    if (!enc) return fail(FZ_ERR_CUDA, "cuTensorMapEncodeTiled entry point not available");
     cuuint64_t dims[3] = {(cuuint64_t)voxels, (cuuint64_t)channels, (cuuint64_t)batch};
     cuuint64_t strides[2] = {(cuuint64_t)voxels * 4, (cuuint64_t)voxels * channels * 4};
     cuuint32_t box[3] = {kVT, kBlk, 1};
-    cuuint32_t es[3] = {1, 1, 1};
-    const CUresult r = enc(m, CU_TENSOR_MAP_DATA_TYPE_FLOAT32, 3, const_cast<float*>(ptr), dims, strides, box, es,
-                           CU_TENSOR_MAP_INTERLEAVE_NONE, CU_TENSOR_MAP_SWIZZLE_128B, CU_TENSOR_MAP_L2_PROMOTION_L2_128B,
-                           CU_TENSOR_MAP_FLOAT_OOB_FILL_NONE);
-    if (r != CUDA_SUCCESS) return fail(FZ_ERR_CUDA, "cuTensorMapEncodeTiled failed with CUresult %d", (int)r);
-    return FZ_OK;
-}
-
-__device__ __forceinline__ void tma_load_3d(uint32_t dst, const CUtensorMap* m, uint32_t bar, int c0, int c1, int c2) {
-    asm volatile("cp.async.bulk.tensor.3d.shared::cluster.global.tile.mbarrier::complete_tx::bytes [%0], [%1, {%3, %4, %5}], [%2];"
-                 :: "r"(dst), "l"(m), "r"(bar), "r"(c0), "r"(c1), "r"(c2) : "memory");
-}
-__device__ __forceinline__ void bar_expect_tx(uint32_t bar, uint32_t bytes) {
-    asm volatile("{\n.reg .b64 st;\nmbarrier.arrive.expect_tx.shared::cta.b64 st, [%0], %1;\n}" :: "r"(bar), "r"(bytes) : "memory");
+    return encode_tiled_map(m, "dy / x", CU_TENSOR_MAP_DATA_TYPE_FLOAT32, 3, ptr, dims, strides, box,
+                            CU_TENSOR_MAP_SWIZZLE_128B);
 }
 
 __global__ void __launch_bounds__(kThreads, 2)
@@ -80,12 +51,12 @@ linear_wgrad_tc(const __grid_constant__ CUtensorMap map_dy, const __grid_constan
 
     if (tid == 0) {
         for (int s = 0; s < kStages; ++s) {
-            bar_init(sbase + oBarFull + 8 * s, 1);
-            bar_init(sbase + oBarLo + 8 * s, 4);
-            bar_init(sbase + oBarEmpty + 8 * s, 1);
+            mbar_init(sbase + oBarFull + 8 * s, 1);
+            mbar_init(sbase + oBarLo + 8 * s, 4);
+            mbar_init(sbase + oBarEmpty + 8 * s, 1);
         }
-        bar_init(sbase + oBarDone, 1);
-        asm volatile("fence.mbarrier_init.release.cluster;" ::: "memory");
+        mbar_init(sbase + oBarDone, 1);
+        fence_mbarrier_init();
     }
     // the ones block of every stage (constant): row 0 = ones, rows 1 .. 15 = zeros (a 128-byte row of equal words: no swizzle to mind)
     for (int i = tid; i < kStages * 16 * 32; i += kThreads) {
@@ -93,10 +64,10 @@ linear_wgrad_tc(const __grid_constant__ CUtensorMap map_dy, const __grid_constan
         reinterpret_cast<float*>(smem + s * kStage + oOnes)[i % (16 * 32)] = r == 0 ? 1.f : 0.f;
     }
     if (warp == 1) {
-        asm volatile("tcgen05.alloc.cta_group::1.sync.aligned.shared::cta.b32 [%0], 256;" :: "r"(sbase + oTmemSlot) : "memory");
-        asm volatile("tcgen05.relinquish_alloc_permit.cta_group::1.sync.aligned;" ::: "memory");
+        tmem_alloc<256>(sbase + oTmemSlot);
+        tmem_relinquish_alloc_permit();
     }
-    fence_async_smem();
+    fence_proxy_async_smem();
     tc_fence_before();
     __syncthreads();
     tc_fence_after();
@@ -110,9 +81,9 @@ linear_wgrad_tc(const __grid_constant__ CUtensorMap map_dy, const __grid_constan
             for (long long it = 0; it < my_tiles; ++it) {
                 const int s = (int)(it % kStages);
                 const uint32_t round = (uint32_t)(it / kStages);
-                if (round > 0) bar_wait(sbase + oBarEmpty + 8 * s, (round - 1) & 1);
+                if (round > 0) mbar_wait(sbase + oBarEmpty + 8 * s, (round - 1) & 1);
                 const uint32_t full = sbase + oBarFull + 8 * s;
-                bar_expect_tx(full, 2 * kTile);
+                mbar_arrive_expect_tx(full, 2 * kTile);
                 tma_load_3d(sbase + s * kStage + oA, &map_dy, full, nt * kVT, ob * kBlk, (int)nb);
                 tma_load_3d(sbase + s * kStage + oB, &map_x, full, nt * kVT, ib * kBlk, (int)nb);
                 nt += (int)gridDim.x;
@@ -126,7 +97,7 @@ linear_wgrad_tc(const __grid_constant__ CUtensorMap map_dy, const __grid_constan
         for (long long it = 0; it < my_tiles; ++it) {
             const int s = (int)(it % kStages);
             const uint32_t round = (uint32_t)(it / kStages);
-            bar_wait(sbase + oBarLo + 8 * s, round & 1);
+            mbar_wait(sbase + oBarLo + 8 * s, round & 1);
             tc_fence_after();
             if (elect_one()) {
                 const uint64_t ad = make_desc(sbase + s * kStage + oA, 16, 1024, 2);
@@ -144,7 +115,7 @@ linear_wgrad_tc(const __grid_constant__ CUtensorMap map_dy, const __grid_constan
         for (long long it = 0; it < my_tiles; ++it) {
             const int s = (int)(it % kStages);
             const uint32_t round = (uint32_t)(it / kStages);
-            bar_wait(sbase + oBarFull + 8 * s, round & 1);
+            mbar_wait(sbase + oBarFull + 8 * s, round & 1);
             unsigned char* st = smem + s * kStage;
 #pragma unroll
             for (int half = 0; half < 2; ++half) {             // dy tile, then x tile
@@ -156,15 +127,15 @@ linear_wgrad_tc(const __grid_constant__ CUtensorMap map_dy, const __grid_constan
                     lo[i * 128 + t] = make_float4(tf32_lo(v.x), tf32_lo(v.y), tf32_lo(v.z), tf32_lo(v.w));
                 }
             }
-            fence_async_smem();
+            fence_proxy_async_smem();
             __syncwarp();
-            if (lane == 0) bar_arrive(sbase + oBarLo + 8 * s);
+            if (lane == 0) mbar_arrive(sbase + oBarLo + 8 * s);
         }
     }
     // ---- epilogue: accumulator row r (TMEM lane r) = output channel r % 64 (hi block for r < 64, lo block above); column n =
     //      input channel n % 64 (hi for n < 64, lo for 64 <= n < 128), column 128 = the bias sums ----
     if (my_tiles > 0) {
-        bar_wait(sbase + oBarDone, 0);
+        mbar_wait(sbase + oBarDone, 0);
         tc_fence_after();
     }
     __syncthreads();                                           // the stages are free: they take the scratch copy of the accumulator
@@ -199,7 +170,7 @@ linear_wgrad_tc(const __grid_constant__ CUtensorMap map_dy, const __grid_constan
         if (db && ib == 0 && tid < kBlk && ob * kBlk + tid < cout) atomicAdd(db + ob * kBlk + tid, S[tid * 145 + 128] + S[(64 + tid) * 145 + 128]);
     }
     __syncthreads();
-    if (warp == 1) asm volatile("tcgen05.dealloc.cta_group::1.sync.aligned.b32 %0, 256;" :: "r"(tmem) : "memory");
+    if (warp == 1) tmem_dealloc<256>(tmem);
 }
 
 // =====================================================================================================================
@@ -228,51 +199,29 @@ __host__ __device__ constexpr uint32_t g_smem_bytes(int stages) { return stages 
 
 // x as (batch, channels, voxels): box (1, 32, 32), the 128-byte rows swizzled in 32-byte atoms
 int make_map_x(CUtensorMap* m, const float* ptr, long long batch, int channels, long long voxels) {
-    EncodeTiledFn enc = encode_fn();
-    if (!enc) return fail(FZ_ERR_CUDA, "cuTensorMapEncodeTiled entry point not available");
     cuuint64_t dims[3] = {(cuuint64_t)voxels, (cuuint64_t)channels, (cuuint64_t)batch};
     cuuint64_t strides[2] = {(cuuint64_t)voxels * 4, (cuuint64_t)voxels * channels * 4};
     cuuint32_t box[3] = {32, kGK, 1};
-    cuuint32_t es[3] = {1, 1, 1};
-    const CUresult r = enc(m, CU_TENSOR_MAP_DATA_TYPE_FLOAT32, 3, const_cast<float*>(ptr), dims, strides, box, es,
-                           CU_TENSOR_MAP_INTERLEAVE_NONE, CU_TENSOR_MAP_SWIZZLE_128B_ATOM_32B, CU_TENSOR_MAP_L2_PROMOTION_L2_128B,
-                           CU_TENSOR_MAP_FLOAT_OOB_FILL_NONE);
-    if (r != CUDA_SUCCESS) return fail(FZ_ERR_CUDA, "cuTensorMapEncodeTiled (x) failed with CUresult %d", (int)r);
-    return FZ_OK;
+    return encode_tiled_map(m, "x", CU_TENSOR_MAP_DATA_TYPE_FLOAT32, 3, ptr, dims, strides, box,
+                            CU_TENSOR_MAP_SWIZZLE_128B_ATOM_32B);
 }
 // W as (outputs, inputs) row-major: box (64 outputs, 32 inputs)
 int make_map_w(CUtensorMap* m, const float* ptr, int cout, int cin) {
-    EncodeTiledFn enc = encode_fn();
-    if (!enc) return fail(FZ_ERR_CUDA, "cuTensorMapEncodeTiled entry point not available");
     cuuint64_t dims[2] = {(cuuint64_t)cin, (cuuint64_t)cout};
     cuuint64_t strides[1] = {(cuuint64_t)cin * 4};
     cuuint32_t box[2] = {kGK, kGN};
-    cuuint32_t es[2] = {1, 1};
-    const CUresult r = enc(m, CU_TENSOR_MAP_DATA_TYPE_FLOAT32, 2, const_cast<float*>(ptr), dims, strides, box, es,
-                           CU_TENSOR_MAP_INTERLEAVE_NONE, CU_TENSOR_MAP_SWIZZLE_128B, CU_TENSOR_MAP_L2_PROMOTION_L2_128B,
-                           CU_TENSOR_MAP_FLOAT_OOB_FILL_NONE);
-    if (r != CUDA_SUCCESS) return fail(FZ_ERR_CUDA, "cuTensorMapEncodeTiled (W) failed with CUresult %d", (int)r);
-    return FZ_OK;
+    return encode_tiled_map(m, "W", CU_TENSOR_MAP_DATA_TYPE_FLOAT32, 2, ptr, dims, strides, box,
+                            CU_TENSOR_MAP_SWIZZLE_128B);
 }
 // W stored as (inputs, outputs) row-major, used transposed (the input gradient reads the layer's weight as it lies): the
 // outputs are contiguous, i.e. the B operand is MN-major like x: boxes of (32 outputs x 32 inputs), 128-byte rows swizzled in
 // 32-byte atoms
 int make_map_wt(CUtensorMap* m, const float* ptr, int cout, int cin) {
-    EncodeTiledFn enc = encode_fn();
-    if (!enc) return fail(FZ_ERR_CUDA, "cuTensorMapEncodeTiled entry point not available");
     cuuint64_t dims[2] = {(cuuint64_t)cout, (cuuint64_t)cin};
     cuuint64_t strides[1] = {(cuuint64_t)cout * 4};
     cuuint32_t box[2] = {32, kGK};
-    cuuint32_t es[2] = {1, 1};
-    const CUresult r = enc(m, CU_TENSOR_MAP_DATA_TYPE_FLOAT32, 2, const_cast<float*>(ptr), dims, strides, box, es,
-                           CU_TENSOR_MAP_INTERLEAVE_NONE, CU_TENSOR_MAP_SWIZZLE_128B_ATOM_32B, CU_TENSOR_MAP_L2_PROMOTION_L2_128B,
-                           CU_TENSOR_MAP_FLOAT_OOB_FILL_NONE);
-    if (r != CUDA_SUCCESS) return fail(FZ_ERR_CUDA, "cuTensorMapEncodeTiled (W^T) failed with CUresult %d", (int)r);
-    return FZ_OK;
-}
-__device__ __forceinline__ void tma_load_2d(uint32_t dst, const CUtensorMap* m, uint32_t bar, int c0, int c1) {
-    asm volatile("cp.async.bulk.tensor.2d.shared::cluster.global.tile.mbarrier::complete_tx::bytes [%0], [%1, {%3, %4}], [%2];"
-                 :: "r"(dst), "l"(m), "r"(bar), "r"(c0), "r"(c1) : "memory");
+    return encode_tiled_map(m, "W^T", CU_TENSOR_MAP_DATA_TYPE_FLOAT32, 2, ptr, dims, strides, box,
+                            CU_TENSOR_MAP_SWIZZLE_128B_ATOM_32B);
 }
 
 // STAGES = 2: two CTAs per SM (the streaming shapes); STAGES = 4: one CTA per SM with four K chunks in flight, for launches with
@@ -295,19 +244,19 @@ linear_fwd_tc(const __grid_constant__ CUtensorMap map_x, const __grid_constant__
 
     if (tid == 0) {
         for (int s = 0; s < kGStages; ++s) {
-            bar_init(sbase + gBarFull + 8 * s, 1);
-            bar_init(sbase + gBarLo + 8 * s, 8);
-            bar_init(sbase + gBarEmpty + 8 * s, 1);
+            mbar_init(sbase + gBarFull + 8 * s, 1);
+            mbar_init(sbase + gBarLo + 8 * s, 8);
+            mbar_init(sbase + gBarEmpty + 8 * s, 1);
         }
         for (int a = 0; a < 2; ++a) {
-            bar_init(sbase + gBarAccFull + 8 * a, 1);
-            bar_init(sbase + gBarAccFree + 8 * a, 8);
+            mbar_init(sbase + gBarAccFull + 8 * a, 1);
+            mbar_init(sbase + gBarAccFree + 8 * a, 8);
         }
-        asm volatile("fence.mbarrier_init.release.cluster;" ::: "memory");
+        fence_mbarrier_init();
     }
     if (warp == 1) {
-        asm volatile("tcgen05.alloc.cta_group::1.sync.aligned.shared::cta.b32 [%0], 256;" :: "r"(sbase + gTmemSlot) : "memory");
-        asm volatile("tcgen05.relinquish_alloc_permit.cta_group::1.sync.aligned;" ::: "memory");
+        tmem_alloc<256>(sbase + gTmemSlot);
+        tmem_relinquish_alloc_permit();
     }
     tc_fence_before();
     __syncthreads();
@@ -327,9 +276,9 @@ linear_fwd_tc(const __grid_constant__ CUtensorMap map_x, const __grid_constant__
                 for (int kc = 0; kc < kchunks; ++kc, ++g) {
                     const int s = (int)(g % kGStages);
                     const uint32_t round = (uint32_t)(g / kGStages);
-                    if (round > 0) bar_wait(sbase + gBarEmpty + 8 * s, (round - 1) & 1);
+                    if (round > 0) mbar_wait(sbase + gBarEmpty + 8 * s, (round - 1) & 1);
                     const uint32_t full = sbase + gBarFull + 8 * s, st = sbase + s * kGStage;
-                    bar_expect_tx(full, kGA + kGB);
+                    mbar_arrive_expect_tx(full, kGA + kGB);
 #pragma unroll
                     for (int a = 0; a < 4; ++a) tma_load_3d(st + gA + a * (kGA / 4), &map_x, full, v0 + 32 * a, kc * kGK, b);
                     if (wt) {
@@ -352,12 +301,12 @@ linear_fwd_tc(const __grid_constant__ CUtensorMap map_x, const __grid_constant__
                 const int ks = kc % kGSeg;                                 // position inside the segment
                 const uint32_t acc = (uint32_t)(seg & 1), use = (uint32_t)(seg >> 1);
                 if (ks == 0) {
-                    if (use > 0) bar_wait(sbase + gBarAccFree + 8 * acc, (use - 1) & 1);      // the workers have drained this pair
+                    if (use > 0) mbar_wait(sbase + gBarAccFree + 8 * acc, (use - 1) & 1);      // the workers have drained this pair
                     tc_fence_after();
                 }
                 const int s = (int)(g % kGStages);
                 const uint32_t round = (uint32_t)(g / kGStages);
-                bar_wait(sbase + gBarLo + 8 * s, round & 1);
+                mbar_wait(sbase + gBarLo + 8 * s, round & 1);
                 tc_fence_after();
                 const bool seg_end = ks + 1 == kGSeg || kc + 1 == kchunks;
                 if (elect_one()) {
@@ -431,7 +380,7 @@ linear_fwd_tc(const __grid_constant__ CUtensorMap map_x, const __grid_constant__
         start_item(0);
         auto drain = [&](long long seg) {
             const uint32_t acc = (uint32_t)(seg & 1), use = (uint32_t)(seg >> 1);
-            bar_wait(sbase + gBarAccFull + 8 * acc, use & 1);
+            mbar_wait(sbase + gBarAccFull + 8 * acc, use & 1);
             tc_fence_after();
             const uint32_t ta = tmem + ((uint32_t)(wq * 32) << 16) + acc * (2 * kGN) + wh * 32;
 #pragma unroll
@@ -445,7 +394,7 @@ linear_fwd_tc(const __grid_constant__ CUtensorMap map_x, const __grid_constant__
             }
             tc_fence_before();
             __syncwarp();
-            if (lane == 0) bar_arrive(sbase + gBarAccFree + 8 * acc);
+            if (lane == 0) mbar_arrive(sbase + gBarAccFree + 8 * acc);
             if (seg % spi == spi - 1) {                                    // the item's last segment: epilogue, store, start over
                 const long long it = seg / spi;
                 long long off;
@@ -518,7 +467,7 @@ linear_fwd_tc(const __grid_constant__ CUtensorMap map_x, const __grid_constant__
             for (int kc = 0; kc < kchunks; ++kc, ++g) {
                 const int s = (int)(g % kGStages);
                 const uint32_t round = (uint32_t)(g / kGStages);
-                bar_wait(sbase + gBarFull + 8 * s, round & 1);
+                mbar_wait(sbase + gBarFull + 8 * s, round & 1);
                 unsigned char* st = smem + s * kGStage;
                 {
                     const float4* hi = reinterpret_cast<const float4*>(st + gA);
@@ -538,9 +487,9 @@ linear_fwd_tc(const __grid_constant__ CUtensorMap map_x, const __grid_constant__
                         lo[i * 256 + t] = make_float4(tf32_lo(v4.x), tf32_lo(v4.y), tf32_lo(v4.z), tf32_lo(v4.w));
                     }
                 }
-                fence_async_smem();
+                fence_proxy_async_smem();
                 __syncwarp();
-                if (lane == 0) bar_arrive(sbase + gBarLo + 8 * s);
+                if (lane == 0) mbar_arrive(sbase + gBarLo + 8 * s);
                 if (kc % kGSeg == 0 && seg > 0) drain(seg - 1);            // the previous segment, now that this one is under way
                 if (kc % kGSeg == kGSeg - 1 || kc + 1 == kchunks) ++seg;
             }
@@ -549,7 +498,7 @@ linear_fwd_tc(const __grid_constant__ CUtensorMap map_x, const __grid_constant__
     }
     tc_fence_before();
     __syncthreads();
-    if (warp == 1) asm volatile("tcgen05.dealloc.cta_group::1.sync.aligned.b32 %0, 256;" :: "r"(tmem) : "memory");
+    if (warp == 1) tmem_dealloc<256>(tmem);
 }
 
 }  // namespace

@@ -14,7 +14,7 @@
 // (c_bar, v_bar, the rank-1 updates of dX), per matrix the M-vector parts (u_bar, a_bar, b_bar) rebuilt in the
 // prologue of the next pass from the sums the previous pass accumulated.  K + 1 launches for K differentiated sweeps.
 // Same math as csrc/fz_swnmf_small.cu (and oracle/factorizer_oracle.py::_half_bwd), spread over the grid.
-#include "fz_common.cuh"
+#include "fz_device.cuh"
 #include "fz_internal.cuh"
 
 namespace fz {
@@ -42,12 +42,6 @@ struct BigParams {
     int M, n, T, K, kind, relu, t, pass;
     float eps;
 };
-
-__device__ __forceinline__ float rcp_nr(float d) {
-    float r;
-    asm("rcp.approx.ftz.f32 %0, %1;" : "=f"(r) : "f"(d));
-    return fmaf(r, fmaf(-d, r, 1.f), r);
-}
 
 // red[warp][i] <- warp sums; then rows 0..count-1 are added to dst[] with one atomic per row
 __device__ __forceinline__ void flush_rows(float* red, int count, float* dst) {

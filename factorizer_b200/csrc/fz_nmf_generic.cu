@@ -493,10 +493,7 @@ static int launch_generic(const NmfArgs& a_in, bool bwd, cudaStream_t st) {
     int per_sm = 1;
     FZ_CUDA_CHECK(cudaOccupancyMaxActiveBlocksPerMultiprocessor(&per_sm, kern, kThreads, smem));
     if (per_sm < 1) per_sm = 1;
-    int dev = 0, sms = 148;
-    FZ_CUDA_CHECK(cudaGetDevice(&dev));
-    FZ_CUDA_CHECK(cudaDeviceGetAttribute(&sms, cudaDevAttrMultiProcessorCount, dev));
-    long long grid = (long long)sms * per_sm;
+    long long grid = (long long)num_sms() * per_sm;
     if (grid > a.n) grid = a.n;
     kern<<<(unsigned)grid, kThreads, smem, st>>>(a);
     FZ_LAUNCH_CHECK();

@@ -35,12 +35,12 @@
 //  * arithmetic: packed FFMA2 (fma.rn.f32x2) for every GEMV / rank-1 update -- same FP32 pipe rate,
 //    half the issue slots, which is what the scalar overhead (shuffles, selects, addressing) needs;
 //    reciprocals are MUFU.RCP + one Newton step, (a+eps)/(b+eps) is evaluated as fma(a, r, eps*r).
-#include <cuda.h>
 #include <stdlib.h>
 #include <string.h>
 
 #include <algorithm>
 
+#include "fz_device.cuh"
 #include "fz_internal.cuh"
 
 namespace fz {
@@ -80,66 +80,7 @@ struct alignas(64) FastParams {
     unsigned order[kMaxOrder];  // (set << 29) | (head << 20) | (g0 << 10) | g1, in processing order
 };
 
-typedef float2 f2;
-__device__ __forceinline__ f2 fma2(f2 a, f2 b, f2 c) { return __ffma2_rn(a, b, c); }
-__device__ __forceinline__ f2 mul2(f2 a, f2 b) { return __fmul2_rn(a, b); }
-__device__ __forceinline__ f2 add2(f2 a, f2 b) { return __fadd2_rn(a, b); }
-__device__ __forceinline__ f2 dup(float a) { return make_float2(a, a); }
-
-// 1 / d for d >= eps > 0: MUFU.RCP (1 ulp) + one Newton step
-__device__ __forceinline__ float rcp_nr(float d) {
-    float r;
-    asm("rcp.approx.ftz.f32 %0, %1;" : "=f"(r) : "f"(d));
-    return fmaf(r, fmaf(-d, r, 1.f), r);
-}
-
 // ---- PTX helpers ------------------------------------------------------------------------------------
-__device__ __forceinline__ uint32_t smem_u32(const void* p) { return (uint32_t)__cvta_generic_to_shared(p); }
-__device__ __forceinline__ void mbar_init(uint64_t* b, int n) {
-    asm volatile("mbarrier.init.shared::cta.b64 [%0], %1;" ::"r"(smem_u32(b)), "r"(n));
-}
-__device__ __forceinline__ void mbar_expect_tx(uint64_t* b, uint32_t bytes) {   // no arrival
-    asm volatile("mbarrier.expect_tx.relaxed.cta.shared::cta.b64 [%0], %1;" ::"r"(smem_u32(b)), "r"(bytes) : "memory");
-}
-__device__ __forceinline__ void mbar_arrive(uint64_t* b) {
-    asm volatile("mbarrier.arrive.shared::cta.b64 _, [%0];" ::"r"(smem_u32(b)) : "memory");
-}
-// arrival that fires once every cp.async this thread has issued so far has landed
-__device__ __forceinline__ void mbar_arrive_after_cp_async(uint64_t* b) {
-    asm volatile("cp.async.mbarrier.arrive.noinc.shared::cta.b64 [%0];" ::"r"(smem_u32(b)) : "memory");
-}
-__device__ __forceinline__ bool mbar_try_wait(uint64_t* b, uint32_t parity) {
-    uint32_t ok;
-    asm volatile("{\n.reg .pred p;\nmbarrier.try_wait.parity.shared::cta.b64 p, [%1], %2;\nselp.u32 %0, 1, 0, p;\n}"
-                 : "=r"(ok) : "r"(smem_u32(b)), "r"(parity) : "memory");
-    return ok != 0;
-}
-__device__ __forceinline__ void mbar_wait(uint64_t* b, uint32_t parity) { while (!mbar_try_wait(b, parity)) {} }
-__device__ __forceinline__ void tma_load_tile(void* dst, const CUtensorMap* m, uint64_t* bar, int cw, int ch, int cd, int cc, int cb) {
-    asm volatile("cp.async.bulk.tensor.5d.shared::cluster.global.tile.mbarrier::complete_tx::bytes [%0], [%1, {%3, %4, %5, %6, %7}], [%2];"
-                 ::"r"(smem_u32(dst)), "l"(m), "r"(smem_u32(bar)), "r"(cw), "r"(ch), "r"(cd), "r"(cc), "r"(cb) : "memory");
-}
-__device__ __forceinline__ void tma_store_tile(const CUtensorMap* m, const void* src, int cw, int ch, int cd, int cc, int cb) {
-    asm volatile("cp.async.bulk.tensor.5d.global.shared::cta.tile.bulk_group [%0, {%2, %3, %4, %5, %6}], [%1];"
-                 ::"l"(m), "r"(smem_u32(src)), "r"(cw), "r"(ch), "r"(cd), "r"(cc), "r"(cb) : "memory");
-}
-// contiguous shared -> global bulk copy (bytes: multiple of 16), completion through the bulk async-group
-__device__ __forceinline__ void bulk_store_1d(void* dst, const void* src, uint32_t bytes) {
-    asm volatile("cp.async.bulk.global.shared::cta.bulk_group [%0], [%1], %2;" ::"l"(dst), "r"(smem_u32(src)), "r"(bytes) : "memory");
-}
-__device__ __forceinline__ void bulk_commit() { asm volatile("cp.async.bulk.commit_group;" ::: "memory"); }
-__device__ __forceinline__ void bulk_wait_all() { asm volatile("cp.async.bulk.wait_group 0;" ::: "memory"); }
-__device__ __forceinline__ void bulk_wait_read_all() { asm volatile("cp.async.bulk.wait_group.read 0;" ::: "memory"); }
-__device__ __forceinline__ void fence_proxy_async_smem() { asm volatile("fence.proxy.async.shared::cta;" ::: "memory"); }
-__device__ __forceinline__ void fence_proxy_async_all() { asm volatile("fence.proxy.async;" ::: "memory"); }
-__device__ __forceinline__ void cp_async16(void* dst, const void* src) {
-    asm volatile("cp.async.cg.shared.global [%0], [%1], 16;" ::"r"(smem_u32(dst)), "l"(src) : "memory");
-}
-__device__ __forceinline__ void cp_async_commit() { asm volatile("cp.async.commit_group;" ::: "memory"); }
-__device__ __forceinline__ void cp_async_wait_all() { asm volatile("cp.async.wait_group 0;" ::: "memory"); }
-__device__ __forceinline__ void cp_async4(void* dst, const void* src) {
-    asm volatile("cp.async.ca.shared.global [%0], [%1], 4;" ::"r"(smem_u32(dst)), "l"(src) : "memory");
-}
 __device__ __forceinline__ void pair_bar(int id) { asm volatile("bar.sync %0, 64;" ::"r"(id) : "memory"); }
 // Completion counters are polled with relaxed gpu-scope loads (an acquire on every poll costs an L1 invalidation,
 // ~1 us, per iteration); once a poll shows "done" the observer issues ONE acquire fence, plus a proxy fence because
@@ -152,7 +93,7 @@ __device__ __forceinline__ int ld_poll(const int* p) {
 }
 __device__ __forceinline__ void acquire_after_poll() {
     asm volatile("fence.acq_rel.gpu;" ::: "memory");
-    asm volatile("fence.proxy.async;" ::: "memory");
+    fence_proxy_async_all();
 }
 __device__ __forceinline__ void red_release_add(int* p, int v) {
     asm volatile("red.release.gpu.global.add.s32 [%0], %1;" ::"l"(p), "r"(v) : "memory");
@@ -472,7 +413,7 @@ __global__ void __launch_bounds__(kFwdPairs * 64, 1) swnmf_fwd_fast(const __grid
     int claimed = 0;     // leader: item claimed ahead, not yet decoded
     if (c.leader) {
         mbar_init(&ps.xfull, 64);
-        asm volatile("fence.mbarrier_init.release.cluster;" ::: "memory");
+        fence_mbarrier_init();
         decode(P, claim(P), &ps.info[0]);
         decode(P, claim(P), &ps.info[1]);
         claimed = claim(P);
@@ -645,7 +586,7 @@ __global__ void __launch_bounds__(kBwdPairs * 64, 1) swnmf_bwd_fast(const __grid
         mbar_init(&ps.gfull, 64);
         mbar_init(&ps.ofull, 64);
         ps.oready = 0;
-        asm volatile("fence.mbarrier_init.release.cluster;" ::: "memory");
+        fence_mbarrier_init();
         decode(P, claim(P), &ps.info[0]);
         decode(P, claim(P), &ps.info[1]);
         claimed = claim(P);
@@ -864,36 +805,13 @@ __global__ void __launch_bounds__(kBwdPairs * 64, 1) swnmf_bwd_fast(const __grid
 // =====================================================================================================
 // host side
 // =====================================================================================================
-typedef CUresult (*EncodeTiledFn)(CUtensorMap*, CUtensorMapDataType, cuuint32_t, void*, const cuuint64_t*,
-                                  const cuuint64_t*, const cuuint32_t*, const cuuint32_t*, CUtensorMapInterleave,
-                                  CUtensorMapSwizzle, CUtensorMapL2promotion, CUtensorMapFloatOOBfill);
-
-static EncodeTiledFn encode_fn() {
-    static EncodeTiledFn fn = nullptr;
-    if (!fn) {
-        void* p = nullptr;
-        cudaDriverEntryPointQueryResult q;
-        if (cudaGetDriverEntryPoint("cuTensorMapEncodeTiled", &p, cudaEnableDefault, &q) == cudaSuccess &&
-            q == cudaDriverEntryPointSuccess)
-            fn = reinterpret_cast<EncodeTiledFn>(p);
-    }
-    return fn;
-}
-
 static int make_map(CUtensorMap* m, const void* ptr, const DevGeom& G, int box_d = 8) {
-    EncodeTiledFn enc = encode_fn();
-    if (!enc) return fail(FZ_ERR_CUDA, "cuTensorMapEncodeTiled entry point not available");
     if (reinterpret_cast<uintptr_t>(ptr) & 15) return fail(FZ_ERR_INVALID, "volume pointer %p is not 16-byte aligned", ptr);
     cuuint64_t dims[5] = {(cuuint64_t)G.n[2], (cuuint64_t)G.n[1], (cuuint64_t)G.n[0], (cuuint64_t)G.C, (cuuint64_t)G.B};
     cuuint64_t strides[4] = {(cuuint64_t)G.n[2] * 4, (cuuint64_t)G.n[2] * G.n[1] * 4, (cuuint64_t)G.vox * 4,
                              (cuuint64_t)G.vox * G.C * 4};
     cuuint32_t box[5] = {8, 8, (cuuint32_t)box_d, 8, 1};
-    cuuint32_t es[5] = {1, 1, 1, 1, 1};
-    CUresult r = enc(m, CU_TENSOR_MAP_DATA_TYPE_FLOAT32, 5, const_cast<void*>(ptr), dims, strides, box, es,
-                     CU_TENSOR_MAP_INTERLEAVE_NONE, CU_TENSOR_MAP_SWIZZLE_NONE, CU_TENSOR_MAP_L2_PROMOTION_L2_128B,
-                     CU_TENSOR_MAP_FLOAT_OOB_FILL_NONE);
-    if (r != CUDA_SUCCESS) return fail(FZ_ERR_CUDA, "cuTensorMapEncodeTiled failed with CUresult %d", (int)r);
-    return FZ_OK;
+    return encode_tiled_map(m, "volume", CU_TENSOR_MAP_DATA_TYPE_FLOAT32, 5, ptr, dims, strides, box, CU_TENSOR_MAP_SWIZZLE_NONE);
 }
 
 static int rec_head_for(int T) { return ((9 * T + 3) / 4) * 4; }

@@ -142,7 +142,7 @@ __global__ void __launch_bounds__(kGFwdWarps * 32, 1) swnmf_fwd_gram(const __gri
     }
     if (lane == 0) {
         mbar_init(full, 32);
-        asm volatile("fence.mbarrier_init.release.cluster;" ::: "memory");
+        fence_mbarrier_init();
     }
     __syncthreads();
 
@@ -399,7 +399,7 @@ __global__ void __launch_bounds__(kGFwdWarps * 32, 1) swnmf_fwd_gram(const __gri
             const LaneAddr4 la = lane_addr4(P, it, lane);
             int i1 = it.c1 + ((lane >> 1) & 7); if (i1 >= P.n1) i1 -= P.n1;
             if (fac_staged) {
-                cp_async_wait_all();
+                cp_async_wait<0>();
                 const float4* st4 = reinterpret_cast<const float4*>(stage);
 #pragma unroll
                 for (int j = 0; j < 4; ++j) {
@@ -545,7 +545,7 @@ __global__ void __launch_bounds__(kGBwdPairs * 64, 1) swnmf_bwd_gram(const __gri
         mbar_init(&ps.gfull, 64);
         mbar_init(&ps.ofull, 64);
         ps.oready = 0;
-        asm volatile("fence.mbarrier_init.release.cluster;" ::: "memory");
+        fence_mbarrier_init();
         decode(P, claim(P), &ps.info[0]);
         decode(P, claim(P), &ps.info[1]);
         claimed = claim(P);

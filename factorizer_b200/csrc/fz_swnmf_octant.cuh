@@ -20,12 +20,12 @@
 //           where s runs over the unshifted window of the tile and the shifted window of the voxel's octant.
 // There are no wrapped or misaligned boxes and no partial-sum round trip through the volume.
 #pragma once
-#include <cuda.h>
 #include <cuda_bf16.h>
 #include <type_traits>
 #include <stdlib.h>
 #include <string.h>
 
+#include "fz_device.cuh"
 #include "fz_internal.cuh"
 
 namespace fz {
@@ -38,41 +38,6 @@ constexpr int kFacF = 12;             // per window: u_T (8), rd_T, pad
 constexpr int kBwdOct = 12;           // per (octant, set): w (8), e, pad
 constexpr int kBwdTileRec = 8 * 2 * kBwdOct;   // 192 floats per tile
 constexpr int kMbF = 100;             // per window: M (64) | m (8) | abar_1 (8) | rd_T u_T (8) | u_T (8) | pad (4); 400 B keeps 8 records in distinct banks
-
-typedef float2 f2;
-__device__ __forceinline__ f2 fma2(f2 a, f2 b, f2 c) { return __ffma2_rn(a, b, c); }
-__device__ __forceinline__ f2 mul2(f2 a, f2 b) { return __fmul2_rn(a, b); }
-__device__ __forceinline__ f2 add2(f2 a, f2 b) { return __fadd2_rn(a, b); }
-__device__ __forceinline__ f2 dup(float a) { return make_float2(a, a); }
-__device__ __forceinline__ float rcp_nr(float d) {
-    float r;
-    asm("rcp.approx.ftz.f32 %0, %1;" : "=f"(r) : "f"(d));
-    return fmaf(r, fmaf(-d, r, 1.f), r);
-}
-__device__ __forceinline__ uint32_t smem_u32(const void* p) { return (uint32_t)__cvta_generic_to_shared(p); }
-__device__ __forceinline__ void mbar_init(uint64_t* b, int n) {
-    asm volatile("mbarrier.init.shared::cta.b64 [%0], %1;" ::"r"(smem_u32(b)), "r"(n));
-}
-__device__ __forceinline__ void mbar_arrive_expect_tx(uint64_t* b, uint32_t bytes) {
-    asm volatile("mbarrier.arrive.expect_tx.shared::cta.b64 _, [%0], %1;" ::"r"(smem_u32(b)), "r"(bytes) : "memory");
-}
-__device__ __forceinline__ bool mbar_try_wait(uint64_t* b, uint32_t parity) {
-    uint32_t ok;
-    asm volatile("{\n.reg .pred p;\nmbarrier.try_wait.parity.shared::cta.b64 p, [%1], %2;\nselp.u32 %0, 1, 0, p;\n}"
-                 : "=r"(ok) : "r"(smem_u32(b)), "r"(parity) : "memory");
-    return ok != 0;
-}
-__device__ __forceinline__ void mbar_wait(uint64_t* b, uint32_t parity) { while (!mbar_try_wait(b, parity)) {} }
-__device__ __forceinline__ void tma_load_tile(void* dst, const CUtensorMap* m, uint64_t* bar, int cw, int ch, int cd, int cc, int cb) {
-    asm volatile("cp.async.bulk.tensor.5d.shared::cluster.global.tile.mbarrier::complete_tx::bytes [%0], [%1, {%3, %4, %5, %6, %7}], [%2];"
-                 ::"r"(smem_u32(dst)), "l"(m), "r"(smem_u32(bar)), "r"(cw), "r"(ch), "r"(cd), "r"(cc), "r"(cb) : "memory");
-}
-// the same load with an L2 eviction-priority hint (createpolicy value)
-__device__ __forceinline__ void tma_load_tile_hint(void* dst, const CUtensorMap* m, uint64_t* bar, int cw, int ch, int cd, int cc,
-                                                   int cb, uint64_t policy) {
-    asm volatile("cp.async.bulk.tensor.5d.shared::cluster.global.tile.mbarrier::complete_tx::bytes.L2::cache_hint [%0], [%1, {%3, %4, %5, %6, %7}], [%2], %8;"
-                 ::"r"(smem_u32(dst)), "l"(m), "r"(smem_u32(bar)), "r"(cw), "r"(ch), "r"(cd), "r"(cc), "r"(cb), "l"(policy) : "memory");
-}
 
 // How the pipelined launch (fz_swnmf_pipe.cu) walks the volume: sub-volumes (sample, head) are taken `gs` at a time
 // (a gang); a PLANE-GROUP is one plane t0 of tiles of every sub-volume of a gang (nA = gs * G1 * G2 tiles), and
@@ -326,7 +291,7 @@ __device__ __forceinline__ void fwd_tile_gram(const Tile tile, float* scratch, c
         float4* o4 = reinterpret_cast<float4*>(rec_out);
         for (int q = lane; q < kTileRec / 4; q += 32) o4[q] = s4[q * SPITCH];
     }
-    asm volatile("fence.proxy.async.shared::cta;" ::: "memory");   // the buffer goes back to TMA
+    fence_proxy_async_smem();   // the buffer goes back to TMA
 }
 // fp32 tile: the tile buffer itself is the scratch area
 __device__ __forceinline__ void fwd_tile_gram(float* tile, const float* v0s, const int (&dst)[15], int lane, float* rec_out) {
@@ -826,8 +791,7 @@ __device__ __forceinline__ void bwd_fetch_records(const PhaseParams& P, float* m
     for (int q = lane; q < 9 * (kMbF / 4); q += 32) {
         const int wdx = q / (kMbF / 4), part = q - wdx * (kMbF / 4);
         const long long wid = wdx == 0 ? (long long)tid : (long long)P.tiles + shifted_window_of(P, c, wdx - 1);
-        asm volatile("cp.async.cg.shared.global [%0], [%1], 16;" ::"r"(smem_u32(mbs + wdx * kMbF + 4 * part)),
-                     "l"(P.mb + wid * kMbF + 4 * part) : "memory");
+        cp_async16(mbs + wdx * kMbF + 4 * part, P.mb + wid * kMbF + 4 * part);
     }
 }
 
@@ -901,37 +865,16 @@ __device__ __forceinline__ void bwd_tile_apply(const PhaseParams& P, const float
 }
 
 // ---- host helpers shared by both launch schemes ---------------------------------------------------------
-typedef CUresult (*EncodeTiledFn)(CUtensorMap*, CUtensorMapDataType, cuuint32_t, void*, const cuuint64_t*,
-                                  const cuuint64_t*, const cuuint32_t*, const cuuint32_t*, CUtensorMapInterleave,
-                                  CUtensorMapSwizzle, CUtensorMapL2promotion, CUtensorMapFloatOOBfill);
-inline EncodeTiledFn encode_fn() {
-    static EncodeTiledFn fn = nullptr;
-    if (!fn) {
-        void* p = nullptr;
-        cudaDriverEntryPointQueryResult q;
-        if (cudaGetDriverEntryPoint("cuTensorMapEncodeTiled", &p, cudaEnableDefault, &q) == cudaSuccess &&
-            q == cudaDriverEntryPointSuccess)
-            fn = reinterpret_cast<EncodeTiledFn>(p);
-    }
-    return fn;
-}
 // box (8,8,8,8,1) of fp32, or -- bf16 activations -- (16,8,8,8,1) of bf16: two tiles side by side along W
 inline int make_tile_map(CUtensorMap* m, const void* ptr, const DevGeom& G) {
-    EncodeTiledFn enc = encode_fn();
-    if (!enc) return fail(FZ_ERR_CUDA, "cuTensorMapEncodeTiled entry point not available");
     if (reinterpret_cast<uintptr_t>(ptr) & 15) return fail(FZ_ERR_INVALID, "volume pointer %p is not 16-byte aligned", ptr);
     cuuint64_t dims[5] = {(cuuint64_t)G.n[2], (cuuint64_t)G.n[1], (cuuint64_t)G.n[0], (cuuint64_t)G.C, (cuuint64_t)G.B};
     const cuuint64_t e = G.dtype == FZ_DTYPE_BF16 ? 2 : 4;
     cuuint64_t strides[4] = {(cuuint64_t)G.n[2] * e, (cuuint64_t)G.n[2] * G.n[1] * e, (cuuint64_t)G.vox * e,
                              (cuuint64_t)G.vox * G.C * e};
     cuuint32_t box[5] = {G.dtype == FZ_DTYPE_BF16 ? 16u : 8u, 8, 8, 8, 1};
-    cuuint32_t es[5] = {1, 1, 1, 1, 1};
-    CUresult r = enc(m, G.dtype == FZ_DTYPE_BF16 ? CU_TENSOR_MAP_DATA_TYPE_BFLOAT16 : CU_TENSOR_MAP_DATA_TYPE_FLOAT32, 5,
-                     const_cast<void*>(ptr), dims, strides, box, es,
-                     CU_TENSOR_MAP_INTERLEAVE_NONE, CU_TENSOR_MAP_SWIZZLE_NONE, CU_TENSOR_MAP_L2_PROMOTION_L2_128B,
-                     CU_TENSOR_MAP_FLOAT_OOB_FILL_NONE);
-    if (r != CUDA_SUCCESS) return fail(FZ_ERR_CUDA, "cuTensorMapEncodeTiled failed with CUresult %d", (int)r);
-    return FZ_OK;
+    return encode_tiled_map(m, "volume tile", G.dtype == FZ_DTYPE_BF16 ? CU_TENSOR_MAP_DATA_TYPE_BFLOAT16 : CU_TENSOR_MAP_DATA_TYPE_FLOAT32,
+                            5, ptr, dims, strides, box, CU_TENSOR_MAP_SWIZZLE_NONE);
 }
 inline size_t align_up(size_t v, size_t a) { return (v + a - 1) / a * a; }
 inline int rec_head_for(int T) { return ((9 * T + 3) / 4) * 4; }

@@ -52,7 +52,7 @@ __global__ void __launch_bounds__(kW1 * 32, 1) phase_fwd_gram(const __grid_const
     if (lane == 0) {
         mbar_init(&bars[warp][0], 1);
         mbar_init(&bars[warp][1], 1);
-        asm volatile("fence.mbarrier_init.release.cluster;" ::: "memory");
+        fence_mbarrier_init();
     }
     __syncthreads();
     if (blockIdx.x == 0 && warp == 0) {
@@ -126,7 +126,7 @@ __global__ void __launch_bounds__(kW3 * 32, 1) phase_fwd_apply(const __grid_cons
     if (lane == 0) {
         mbar_init(&bars[warp][0], 1);
         mbar_init(&bars[warp][1], 1);
-        asm volatile("fence.mbarrier_init.release.cluster;" ::: "memory");
+        fence_mbarrier_init();
     }
     __syncthreads();
     constexpr int kPer = BF16 ? 2 : 1;
@@ -189,7 +189,7 @@ __global__ void __launch_bounds__(kWB * 32, 1) phase_bwd_reduce(const __grid_con
     if (lane == 0) {
         mbar_init(&bars[warp][0], 1);
         mbar_init(&bars[warp][1], 1);
-        asm volatile("fence.mbarrier_init.release.cluster;" ::: "memory");
+        fence_mbarrier_init();
     }
     __syncthreads();
     constexpr int kPer = BF16 ? 2 : 1;
@@ -270,7 +270,7 @@ __global__ void __launch_bounds__(kWB * 32, 1) phase_bwd_apply(const __grid_cons
     if (lane == 0) {
         mbar_init(&bars[warp][0], 1);
         mbar_init(&bars[warp][1], 1);
-        asm volatile("fence.mbarrier_init.release.cluster;" ::: "memory");
+        fence_mbarrier_init();
     }
     __syncthreads();
     Stream S; S.gw = blockIdx.x * kWB + warp; S.nw = gridDim.x * kWB; S.lane = lane; S.begin = P.t_begin / kPer; S.count = P.t_count / kPer; S.reverse = P.reverse;
@@ -296,7 +296,7 @@ __global__ void __launch_bounds__(kWB * 32, 1) phase_bwd_apply(const __grid_cons
     auto fetch = [&](int q) {
         const int tid = tile_of(q);
         if (tid < P.tiles) bwd_fetch_records(P, mbs_all[warp][q & 1], tid, tile_coord(P, tid), lane);
-        asm volatile("cp.async.commit_group;" ::: "memory");
+        cp_async_commit();
     };
     issue(0);
     fetch(0);
@@ -309,7 +309,7 @@ __global__ void __launch_bounds__(kWB * 32, 1) phase_bwd_apply(const __grid_cons
         for (int half = 0; half < kPer; ++half) {
             const int q = k * kPer + half;
             fetch(q + 1);
-            asm volatile("cp.async.wait_group 1;" ::: "memory");     // this lane's copies of tile q have landed ...
+            cp_async_wait<1>();     // this lane's copies of tile q have landed ...
             __syncwarp();                                             // ... and so have everyone else's
             if (half == 0) {
                 mbar_wait(&bars[warp][st], parity[st]);
@@ -324,8 +324,6 @@ __global__ void __launch_bounds__(kWB * 32, 1) phase_bwd_apply(const __grid_cons
 }
 
 // ---- host ------------------------------------------------------------------------------------------------
-int make_map(CUtensorMap* m, const void* ptr, const DevGeom& G) { return make_tile_map(m, ptr, G); }
-
 struct Layout { size_t oct, b1, fac, mb, total; };
 Layout layout(const DevGeom& G) {
     const size_t tiles = (size_t)G.mats_per_shift;
@@ -382,7 +380,7 @@ int phase_forward(const float* x, const float* v0, float* y, void* saved, void* 
     if (reinterpret_cast<uintptr_t>(y) & 15) return fail(FZ_ERR_INVALID, "output pointer %p is not 16-byte aligned", (void*)y);
     static thread_local PhaseParams P;
     fill(P, G, s, 0, workspace);
-    if (int e = make_map(&P.tm_x, x, G)) return e;
+    if (int e = make_tile_map(&P.tm_x, x, G)) return e;
     P.x = x; P.out = y; P.v0 = v0; P.saved = static_cast<float*>(saved);
     const bool bf16 = G.dtype == FZ_DTYPE_BF16;
     static SmemConfig cfg_gram, cfg_apply, cfg_gram_h, cfg_apply_h;
@@ -416,8 +414,8 @@ int phase_backward(const float* x, const float* gy, const float* v0, const void*
     if (reinterpret_cast<uintptr_t>(gx) & 15) return fail(FZ_ERR_INVALID, "output pointer %p is not 16-byte aligned", (void*)gx);
     static thread_local PhaseParams P;
     fill(P, G, s, K, workspace);
-    if (int e = make_map(&P.tm_x, x, G)) return e;
-    if (int e = make_map(&P.tm_g, gy, G)) return e;
+    if (int e = make_tile_map(&P.tm_x, x, G)) return e;
+    if (int e = make_tile_map(&P.tm_g, gy, G)) return e;
     P.x = x; P.gy = gy; P.out = gx; P.v0 = v0;
     P.saved = const_cast<float*>(static_cast<const float*>(saved));
     const bool bf16 = G.dtype == FZ_DTYPE_BF16;

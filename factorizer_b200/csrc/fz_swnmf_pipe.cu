@@ -69,13 +69,6 @@ __device__ __forceinline__ void wait_known(const int* p, int need, int lane) {
     }
     __syncwarp();
 }
-__device__ __forceinline__ void mbar_arrive(uint64_t* b) {
-    asm volatile("mbarrier.arrive.shared::cta.b64 _, [%0];" ::"r"(smem_u32(b)) : "memory");
-}
-__device__ __forceinline__ void bulk_copy(void* dst, const void* src, uint32_t bytes, uint64_t* bar) {
-    asm volatile("cp.async.bulk.shared::cluster.global.mbarrier::complete_tx::bytes [%0], [%1], %2, [%3];"
-                 ::"r"(smem_u32(dst)), "l"(src), "r"(bytes), "r"(smem_u32(bar)) : "memory");
-}
 // L2 eviction priorities (createpolicy): pass 1 reads a tile that pass 3 will want again, pass 3 reads it for the last time
 __device__ __forceinline__ uint64_t policy_evict_last() {
     uint64_t p;
@@ -389,7 +382,7 @@ __device__ __forceinline__ void ring_init(RingShared& R, int slots) {
     R.known[0] = R.known[1] = R.known[2] = 0;
     R.next_seq = 0;
     for (int s = 0; s < slots; ++s) { mbar_init(&R.full[s], 1); mbar_init(&R.empty[s], 1); }
-    asm volatile("fence.mbarrier_init.release.cluster;" ::: "memory");
+    fence_mbarrier_init();
 }
 // next slot of the ring for a consumer warp: its sequence number's slot, once the producer's data has landed; false at
 // the end of the stream

@@ -17,7 +17,7 @@
 // (operations.py:426-433); consecutive sub-warps take windows that are neighbours along W, so a warp-wide
 // load still covers whole 32-byte sectors.  Division is reciprocal (MUFU + one Newton step) times numerator,
 // <= 1 ulp from the reference's true division (same deviation as the 8x512 kernels, DESIGN.md section 2).
-#include "fz_common.cuh"
+#include "fz_device.cuh"
 #include "fz_internal.cuh"
 
 namespace fz {
@@ -37,12 +37,6 @@ struct SmallParams {
     float eps;
     DevGeom G;
 };
-
-__device__ __forceinline__ float rcp_nr(float d) {
-    float r;
-    asm("rcp.approx.ftz.f32 %0, %1;" : "=f"(r) : "f"(d));
-    return fmaf(r, fmaf(-d, r, 1.f), r);
-}
 
 template <int L>
 __device__ __forceinline__ float group_sum(float v) {
@@ -105,10 +99,6 @@ struct Locator {
         return ((long long)b * G.C + (long long)h * G.d) * G.vox;
     }
 };
-
-typedef float2 f2;
-__device__ __forceinline__ f2 fma2(f2 a, f2 b, f2 c) { return __ffma2_rn(a, b, c); }
-__device__ __forceinline__ f2 dup(float a) { return make_float2(a, a); }
 
 // Columns come in pairs (float2, packed FFMA2): pair kp of a lane = columns 2 (kp L + lane), +1.
 // one half-step for the M side: a = X v (all-reduced), b = v.v;  u <- update
@@ -514,13 +504,11 @@ __global__ void __launch_bounds__(kSmallThreads) small_bwd(const SmallParams P) 
     }
 }
 
-int small_sm_count() { return num_sms(); }
-
 template <int M, int CPL, int L>
 int launch_small(const SmallParams& P, bool bwd, cudaStream_t st) {
     const long long per_cta = kSmallThreads / L;
     long long ctas = (P.n + per_cta - 1) / per_cta;
-    const long long cap = 8LL * small_sm_count();
+    const long long cap = 8LL * num_sms();
     if (ctas > cap) ctas = cap;
     if (bwd) {
         const size_t smem = sizeof(float) * Hist<M, CPL, L>::floats * (kSmallThreads / L);

@@ -1,5 +1,6 @@
-// tcgen05 / TMEM building blocks shared by the tensor-core glue kernels (sm_100a): shared-memory matrix descriptors,
-// kind::tf32 MMA issue, commit / mbarrier waits, TMEM loads, the 3xTF32 split, and the exact-erf GELU.
+// tcgen05 / TMEM building blocks shared by the tensor-core kernels (sm_100a): shared-memory matrix descriptors,
+// kind::tf32 MMA issue and commit, TMEM allocation, loads and stores, and the 3xTF32 split.  The primitives that are not
+// specific to tcgen05 (mbarriers, TMA, fences, the exact-erf GELU) are in fz_device.cuh.
 //
 // Operand forms used by these kernels (all pinned on B200 by bench_probes/tcgen05_*probe.cu; kind::tf32):
 //   * A in TENSOR MEMORY (per-voxel GEMMs, M = 128 voxels = TMEM lanes): column c of lane v = A(v, k = c); every thread
@@ -11,12 +12,10 @@
 //     128-byte row whose 32-byte chunks are XOR-ed with (voxel % 4) -- a thread stores its voxel's row with STS.128.
 //   * K-major without swizzle (layout type 0; the weights): 8 x 16-byte core matrices, LBO along K, SBO along M / N.
 #pragma once
-#include "fz_common.cuh"
+#include "fz_device.cuh"
 
 namespace fz {
 namespace tc {
-
-__device__ __forceinline__ uint32_t smem_u32(const void* p) { return (uint32_t)__cvta_generic_to_shared(p); }
 
 __device__ __forceinline__ uint64_t make_desc(uint32_t saddr, uint32_t lbo_bytes, uint32_t sbo_bytes, uint32_t layout_type) {
     uint64_t d = 0;
@@ -55,20 +54,19 @@ __device__ __forceinline__ uint32_t uniform_u32(uint32_t v) { return __shfl_sync
 __device__ __forceinline__ void commit(uint32_t bar) {
     asm volatile("tcgen05.commit.cta_group::1.mbarrier::arrive::one.shared::cluster.b64 [%0];" :: "r"(bar) : "memory");
 }
-__device__ __forceinline__ void bar_init(uint32_t bar, uint32_t count) {
-    asm volatile("mbarrier.init.shared::cta.b64 [%0], %1;" :: "r"(bar), "r"(count));
+// TMEM allocation by one warp: COLS columns (a power of two, 32 .. 512), their address written to the shared-memory word at
+// `slot`; the allocating warp then gives up the permit to allocate more, and frees the same COLS columns at the end
+template <uint32_t COLS>
+__device__ __forceinline__ void tmem_alloc(uint32_t slot) {
+    asm volatile("tcgen05.alloc.cta_group::1.sync.aligned.shared::cta.b32 [%0], %1;" :: "r"(slot), "n"(COLS) : "memory");
 }
-__device__ __forceinline__ void bar_arrive(uint32_t bar) {
-    asm volatile("{\n.reg .b64 st;\nmbarrier.arrive.shared::cta.b64 st, [%0];\n}" :: "r"(bar) : "memory");
+__device__ __forceinline__ void tmem_relinquish_alloc_permit() {
+    asm volatile("tcgen05.relinquish_alloc_permit.cta_group::1.sync.aligned;" ::: "memory");
 }
-__device__ __forceinline__ void bar_wait(uint32_t bar, uint32_t parity) {
-    uint32_t ok = 0;
-    while (!ok) {
-        asm volatile("{\n.reg .pred p;\nmbarrier.try_wait.parity.shared::cta.b64 p, [%1], %2;\nselp.u32 %0, 1, 0, p;\n}"
-                     : "=r"(ok) : "r"(bar), "r"(parity) : "memory");
-    }
+template <uint32_t COLS>
+__device__ __forceinline__ void tmem_dealloc(uint32_t taddr) {
+    asm volatile("tcgen05.dealloc.cta_group::1.sync.aligned.b32 %0, %1;" :: "r"(taddr), "n"(COLS) : "memory");
 }
-__device__ __forceinline__ void fence_async_smem() { asm volatile("fence.proxy.async.shared::cta;" ::: "memory"); }
 __device__ __forceinline__ void tc_fence_before() { asm volatile("tcgen05.fence::before_thread_sync;" ::: "memory"); }
 __device__ __forceinline__ void tc_fence_after() { asm volatile("tcgen05.fence::after_thread_sync;" ::: "memory"); }
 
@@ -155,34 +153,6 @@ __device__ __forceinline__ float2 pair_sum2(float2 mine, float2* slots, uint32_t
     const float2 other = s[(hh ^ 1) * 128 + v];
     ++turn;
     return make_float2(mine.x + other.x, mine.y + other.y);
-}
-
-__device__ __forceinline__ float ex2_approx(float x) { float y; asm("ex2.approx.ftz.f32 %0, %1;" : "=f"(y) : "f"(x)); return y; }
-__device__ __forceinline__ float rcp_approx(float x) { float y; asm("rcp.approx.ftz.f32 %0, %1;" : "=f"(y) : "f"(x)); return y; }
-
-// Exact (erf) GELU through Abramowitz-Stegun 7.1.26 (|error| <= 1.5e-7; the formula of csrc/fz_block_glue.cu), two values
-// at a time: Phi(h) and e = exp(-h^2 / 2)
-__device__ __forceinline__ float2 gauss_cdf2(float2 h, float2& e) {
-    const float2 one = make_float2(1.f, 1.f);
-    const float2 z = make_float2(fabsf(h.x) * 0.70710678118654752f, fabsf(h.y) * 0.70710678118654752f);
-    const float2 d = __ffma2_rn(make_float2(0.3275911f, 0.3275911f), z, one);
-    const float2 t = make_float2(rcp_approx(d.x), rcp_approx(d.y));
-    const float2 hh = __fmul2_rn(h, h);
-    e = make_float2(ex2_approx(hh.x * -0.72134752044448170f), ex2_approx(hh.y * -0.72134752044448170f));
-    float2 p = __ffma2_rn(t, make_float2(1.061405429f, 1.061405429f), make_float2(-1.453152027f, -1.453152027f));
-    p = __ffma2_rn(t, p, make_float2(1.421413741f, 1.421413741f));
-    p = __ffma2_rn(t, p, make_float2(-0.284496736f, -0.284496736f));
-    p = __ffma2_rn(t, p, make_float2(0.254829592f, 0.254829592f));
-    const float2 pt = __fmul2_rn(p, t);
-    const float2 erf_abs = __ffma2_rn(make_float2(-pt.x, -pt.y), e, one);
-    return __ffma2_rn(make_float2(copysignf(0.5f, h.x), copysignf(0.5f, h.y)), erf_abs, make_float2(0.5f, 0.5f));
-}
-// gelu(h) and its derivative Phi(h) + h phi(h)  (torch GeluBackward, approximate='none')
-__device__ __forceinline__ void gelu_grad2(float2 h, float2& g, float2& gp) {
-    float2 e;
-    const float2 cdf = gauss_cdf2(h, e);
-    g = __fmul2_rn(h, cdf);
-    gp = __ffma2_rn(__fmul2_rn(h, make_float2(0.39894228040143268f, 0.39894228040143268f)), e, cdf);
 }
 
 }  // namespace tc
