@@ -1,0 +1,166 @@
+"""FactorizerBlock forward + backward on bf16 activations against the fp32 block and today's layer-by-layer bf16 autocast route.
+
+Per shape and route, the block step (forward, backward of <out, gout>) is captured in one CUDA graph and replayed; CUDA
+events time --reps replays after --warmup.  Routes:
+    fp32        x fp32, no autocast: the fused fp32 block (FactorizerBlockFn at 32 channels, FactorizerBlockWideFn otherwise)
+    bf16-old    x bf16 under bf16 autocast with the bf16 block path switched off: the layers one by one
+    bf16-new    x bf16: FactorizerBlockBf16Fn
+The whole Swin Factorizer's training step (forward, sigmoid-BCE + soft-Dice, backward; no optimizer) at 128^3 is timed
+eagerly for fp32, bf16-old and bf16-new.  Achieved bandwidth is against the block's algorithmic bytes: every activation
+each step reads or writes once, 32 C + 8 H elements per voxel for forward + backward (C channels, H hidden), 4 bytes each
+in fp32, 2 in bf16.  Writes JSON (the card's name and power limit included) to --out.
+
+    python bench_probes/bf16_block_time.py --out /tmp/bf16_block_time.json
+"""
+import argparse
+import json
+import os
+import subprocess
+import sys
+
+import torch
+from torch import nn
+
+sys.path.insert(0, os.path.dirname(os.path.dirname(os.path.abspath(__file__))))
+import factorizer_b200 as ft  # noqa: E402
+from factorizer_b200 import _ops  # noqa: E402
+
+SHAPES = [(1, 32, 128), (1, 64, 64), (1, 128, 32), (1, 256, 16)]
+
+
+def card():
+    try:
+        q = subprocess.run(["nvidia-smi", "--query-gpu=name,power.limit", "--format=csv,noheader"], capture_output=True, text=True)
+        return q.stdout.strip().splitlines()[torch.cuda.current_device()]
+    except Exception as e:  # noqa: BLE001
+        return f"{torch.cuda.get_device_name()} (power limit not read: {e})"
+
+
+class _Route:
+    def __init__(self, name):
+        self.name = name
+        self.saved = _ops.bf16_block_supported
+
+    def __enter__(self):
+        if self.name == "bf16-old":
+            _ops.bf16_block_supported = lambda x, hidden: False
+        self.ac = torch.autocast("cuda", dtype=torch.bfloat16, enabled=self.name == "bf16-old")
+        self.ac.__enter__()
+
+    def __exit__(self, *exc):
+        self.ac.__exit__(*exc)
+        _ops.bf16_block_supported = self.saved
+
+
+def block(C, n, ratio=2):
+    torch.manual_seed(0)
+    return ft.FactorizerBlock(channels=C, spatial_size=(n, n, n), norm=ft.LayerNorm,
+                              reshape=(ft.SWMatricize, {"head_dim": 8, "patch_size": 8}), act=nn.ReLU, factorize=ft.NMF, rank=1,
+                              num_iters=5, init="uniform", solver="hals", mlp_ratio=ratio, dropout=0.0).cuda()
+
+
+def time_graph(fn, warmup, reps):
+    side = torch.cuda.Stream()
+    side.wait_stream(torch.cuda.current_stream())
+    with torch.cuda.stream(side):
+        for _ in range(3):
+            fn()
+        g = torch.cuda.CUDAGraph()
+        with torch.cuda.graph(g, stream=side):
+            fn()
+    torch.cuda.current_stream().wait_stream(side)
+    for _ in range(warmup):
+        g.replay()
+    a, b = torch.cuda.Event(enable_timing=True), torch.cuda.Event(enable_timing=True)
+    a.record()
+    for _ in range(reps):
+        g.replay()
+    b.record()
+    torch.cuda.synchronize()
+    return a.elapsed_time(b) / reps
+
+
+def block_leg(B, C, n, route, warmup, reps):
+    blk = block(C, n)
+    H = blk.mlp.block[0].linear.out_channels
+    dtype = torch.float32 if route == "fp32" else torch.bfloat16
+    x = torch.randn(B, C, n, n, n, device="cuda").to(dtype).requires_grad_(True)
+    gout = torch.randn(B, C, n, n, n, device="cuda").to(dtype)
+    params = list(blk.parameters())
+
+    def step():
+        for p in params:
+            p.grad = None
+        x.grad = None
+        with _Route(route):
+            out = blk(x)
+        out.backward(gout.to(out.dtype))
+        return out
+
+    with _Route(route):
+        node = type(blk(x).grad_fn).__name__
+    ms = time_graph(step, warmup, reps)
+    nbytes = (32 * C + 8 * H) * B * n ** 3 * (4 if route == "fp32" else 2)
+    del blk
+    return {"shape": [B, C, n, n, n], "route": route, "node": node, "ms": ms, "algorithmic_bytes": nbytes,
+            "achieved_GBps": nbytes / ms / 1e6}
+
+
+def model_leg(route, warmup, reps, n=128):
+    torch.manual_seed(1234)
+    net = ft.Factorizer(in_channels=4, out_channels=3, spatial_size=(n, n, n), encoder_depth=(1, 1, 1, 1, 1),
+                        encoder_width=(32, 64, 128, 256, 512), strides=(1, 2, 2, 2, 2), decoder_depth=(1, 1, 1, 1),
+                        norm=ft.LayerNorm, reshape=(ft.SWMatricize, {"head_dim": 8, "patch_size": 8}), act=nn.ReLU,
+                        factorize=ft.NMF, rank=1, num_iters=5, init="uniform", solver="hals", mlp_ratio=2, dropout=0.1).cuda()
+    net.train()
+    x = torch.rand(1, 4, n, n, n, device="cuda")
+    target = torch.randint(0, 2, (1, 3, n, n, n), device="cuda").float()
+
+    def step():
+        net.zero_grad(set_to_none=True)
+        with _Route(route), torch.autocast("cuda", dtype=torch.bfloat16, enabled=route != "fp32"):
+            logits = net(x).float()
+        p = torch.sigmoid(logits)
+        dice = 1 - (2 * (p * target).sum((2, 3, 4)) + 1e-5) / (p.sum((2, 3, 4)) + target.sum((2, 3, 4)) + 1e-5)
+        loss = nn.functional.binary_cross_entropy_with_logits(logits, target) + dice.mean()
+        loss.backward()
+
+    for _ in range(warmup):
+        step()
+    torch.cuda.synchronize()
+    a, b = torch.cuda.Event(enable_timing=True), torch.cuda.Event(enable_timing=True)
+    a.record()
+    for _ in range(reps):
+        step()
+    b.record()
+    torch.cuda.synchronize()
+    return {"route": route, "train_step_ms_eager": a.elapsed_time(b) / reps}
+
+
+def main():
+    ap = argparse.ArgumentParser()
+    ap.add_argument("--out", required=True, help="JSON file to write")
+    ap.add_argument("--warmup", type=int, default=5)
+    ap.add_argument("--reps", type=int, default=30)
+    ap.add_argument("--no-model", action="store_true")
+    args = ap.parse_args()
+    torch.backends.cuda.matmul.allow_tf32 = False
+    torch.backends.cudnn.allow_tf32 = False
+    res = {"card": card(), "blocks": [], "model": []}
+    for B, C, n in SHAPES:
+        row = {r: block_leg(B, C, n, r, args.warmup, args.reps) for r in ("fp32", "bf16-old", "bf16-new")}
+        row["new_vs_old"] = row["bf16-old"]["ms"] / row["bf16-new"]["ms"]
+        row["new_vs_fp32"] = row["fp32"]["ms"] / row["bf16-new"]["ms"]
+        res["blocks"].append(row)
+        print(json.dumps(row), flush=True)
+    if not args.no_model:
+        for r in ("fp32", "bf16-old", "bf16-new"):
+            res["model"].append(model_leg(r, 3, 5))
+            print(json.dumps(res["model"][-1]), flush=True)
+    os.makedirs(os.path.dirname(os.path.abspath(args.out)), exist_ok=True)
+    with open(args.out, "w") as f:
+        json.dump(res, f, indent=1)
+
+
+if __name__ == "__main__":
+    main()

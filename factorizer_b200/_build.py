@@ -10,7 +10,7 @@ CSRC = os.path.join(HERE, "csrc")
 OUT_DIR = os.path.join(HERE, "_C")
 LIB_PATH = os.path.join(OUT_DIR, "libfactorizer_b200.so")
 SOURCES = ["fz_api.cu", "fz_swmat.cu", "fz_nmf_generic.cu", "fz_swnmf_fast.cu", "fz_swnmf_phase.cu", "fz_swnmf_pipe.cu", "fz_layernorm.cu",
-           "fz_block_glue.cu", "fz_swnmf_small.cu", "fz_nmf_big.cu", "fz_block_glue_bwd_tc.cu", "fz_block_glue_fwd_tc.cu", "fz_block_glue_lin_tc.cu", "fz_linear.cu", "fz_linear_tc.cu"]
+           "fz_block_glue.cu", "fz_swnmf_small.cu", "fz_nmf_big.cu", "fz_block_glue_bwd_tc.cu", "fz_block_glue_fwd_tc.cu", "fz_block_glue_lin_tc.cu", "fz_linear.cu", "fz_linear_tc.cu", "fz_bf16_block.cu"]
 
 OBJ_DIR = os.path.join(OUT_DIR, "obj")
 NVCC_FLAGS = [

@@ -73,6 +73,19 @@ _SIGNATURES = {
                                          c_int64, c_float, c_void_p]),
     "fz_layernorm_cf_backward_add": (c_int, [c_void_p, c_void_p, c_void_p, c_void_p, c_void_p, c_void_p, c_void_p, c_int64, c_int32,
                                              c_int64, c_float, c_void_p]),
+    "fz_linear_forward_bf16_supported": (c_int, [c_int32, c_int32, c_int64]),
+    "fz_linear_forward_bf16": (c_int, [c_void_p, c_void_p, c_int32, c_void_p, c_void_p, c_int64, c_int32, c_int32, c_int64, c_int32,
+                                       c_void_p, c_void_p, c_void_p]),
+    "fz_linear_wgrad_bf16_supported": (c_int, [c_int32, c_int32, c_int64]),
+    "fz_linear_wgrad_bf16": (c_int, [c_void_p, c_void_p, c_void_p, c_void_p, c_int64, c_int32, c_int32, c_int64, c_void_p]),
+    "fz_bf16_stage_weights_supported": (c_int, [c_int32, c_int32]),
+    "fz_bf16_staged_elems": (c_int64, [c_int32, c_int32]),
+    "fz_bf16_stage_weights": (c_int, [c_void_p, c_int32, c_int32] * 4 + [c_void_p, c_void_p]),
+    "fz_layernorm_cf_bf16_supported": (c_int, [c_int32, c_int64]),
+    "fz_layernorm_cf_forward_bf16": (c_int, [c_void_p, c_void_p, c_void_p, c_void_p, c_int64, c_int32, c_int64, c_float, c_void_p]),
+    "fz_layernorm_cf_backward_add_bf16": (c_int, [c_void_p, c_void_p, c_void_p, c_void_p, c_void_p, c_void_p, c_void_p, c_int64,
+                                                  c_int32, c_int64, c_float, c_void_p]),
+    "fz_swnmf_bf16_supported": (c_int, [POINTER(FzGeom), POINTER(FzSolver), c_int32]),
     "fz_set_glue_mode": (None, [c_int32]),
     "fz_get_glue_mode": (c_int, []),
     "fz_glue_supported": (c_int, [c_int32, c_int32, c_int64]),

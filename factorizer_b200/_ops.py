@@ -546,6 +546,162 @@ class FactorizerBlockWideFn(_GradModeFunction):
                 None, None, None, None, None, None)
 
 
+# ---- FactorizerBlock on bf16 activations: bf16 tensor-core channel maps around the bf16 fused core ------------------
+def _ld8(n: int) -> int:
+    return (int(n) + 7) & ~7
+
+
+def bf16_core_supported(geom: Geometry, spec: SolverSpec, relu: bool = True) -> bool:
+    """The fused core takes bf16 volumes of this geometry (the octant kernels: head_dim 8, patch 8^3, shifts [0, 4], rank-1
+    HALS, an even number of patches along W)."""
+    g, s = geom.c_geom(1, torch.bfloat16), spec.c_solver()
+    return bool(L.lib().fz_swnmf_bf16_supported(ctypes.byref(g), ctypes.byref(s), int(relu)))
+
+
+def bf16_block_supported(x: torch.Tensor, hidden: int) -> bool:
+    """FactorizerBlockBf16Fn: a contiguous, 16-byte aligned bf16 CUDA volume whose voxel count is a multiple of 8 (the bf16
+    TMA boxes need 16-byte row strides), channel counts the LayerNorm kernels take (up to 512); with or without autocast.
+    The caller checks the core's geometry (bf16_core_supported)."""
+    if not (isinstance(x, torch.Tensor) and x.is_cuda and x.dtype == torch.bfloat16 and x.dim() >= 3 and x.is_contiguous()
+            and x.data_ptr() % 16 == 0):
+        return False
+    B, C = x.shape[0], x.shape[1]
+    vox = x.numel() // max(B * C, 1)
+    lib, H = L.lib(), int(hidden)
+    return bool(B > 0 and vox > 0 and lib.fz_layernorm_cf_bf16_supported(C, vox)
+                and lib.fz_linear_forward_bf16_supported(C, C, vox) and lib.fz_linear_forward_bf16_supported(H, C, vox)
+                and lib.fz_linear_forward_bf16_supported(C, H, vox) and lib.fz_linear_wgrad_bf16_supported(H, C, vox)
+                and lib.fz_linear_wgrad_bf16_supported(C, H, vox))
+
+
+def _staged_views(buf, shapes):
+    """Per weight of shape (R, C) in `buf`, the (W, W^T) bf16 copies fz_bf16_stage_weights wrote there, each as (view, row
+    stride)."""
+    views, off = [], 0
+    for R, C in shapes:
+        n = R * _ld8(C) + C * _ld8(R)
+        views.append(((buf[off:off + R * _ld8(C)], _ld8(C)), (buf[off + R * _ld8(C):off + n], _ld8(R))))
+        off += n
+    return views
+
+
+def _stage_weights_bf16(ws):
+    """One launch: the four fp32 weights as bf16, each as stored and transposed; returns the buffer."""
+    lib = L.lib()
+    n = sum(int(lib.fz_bf16_staged_elems(w.shape[0], w.shape[1])) for w in ws)
+    buf = torch.empty(n, device=ws[0].device, dtype=torch.bfloat16)
+    args = []
+    for w in ws:
+        args += [L.ptr(w), w.shape[0], w.shape[1]]
+    _call(lib.fz_bf16_stage_weights, *args, L.ptr(buf), L.stream_ptr(buf.device))
+    return buf
+
+
+def _channel_map_bf16(x, w, cout, bias, epi=EPI_NONE, aux=None):
+    """r = W x + bias on bf16 (B, C_in, voxels), w = (staged bf16 weight, row stride); returns y, or (y, gelu(y)) for
+    EPI_GELU (fz_linear_forward_bf16)."""
+    B, cin, vox = x.shape
+    y = torch.empty(B, cout, vox, device=x.device, dtype=torch.bfloat16)
+    y2 = torch.empty_like(y) if epi == EPI_GELU else None
+    wb, ldw = w
+    _call(L.lib().fz_linear_forward_bf16, L.ptr(x), L.ptr(wb), ldw, L.ptr(bias), L.ptr(y), B, cin, cout, vox, epi, L.ptr(aux),
+          L.ptr(y2), L.stream_ptr(x.device))
+    return (y, y2) if epi == EPI_GELU else y
+
+
+def _channel_map_wgrad_bf16(gy, x, want_bias: bool):
+    B, cout, vox = gy.shape
+    cin = x.shape[1]
+    gw = torch.empty(cout, cin, device=x.device, dtype=torch.float32)
+    gb = torch.empty(cout, device=x.device, dtype=torch.float32) if want_bias else None
+    _call(L.lib().fz_linear_wgrad_bf16, L.ptr(gy), L.ptr(x), L.ptr(gw), L.ptr(gb), B, cout, cin, vox, L.stream_ptr(x.device))
+    return gw, gb
+
+
+def _ln_forward_bf16(x3, gamma, beta, eps):
+    B, C, vox = x3.shape
+    y = torch.empty_like(x3)
+    _call(L.lib().fz_layernorm_cf_forward_bf16, L.ptr(x3), L.ptr(gamma), L.ptr(beta), L.ptr(y), B, C, vox, float(eps),
+          L.stream_ptr(x3.device))
+    return y
+
+
+def _ln_backward_add_bf16(x3, gamma, gy, add, eps):
+    """dx = add + LN'(gy) in bf16, d(gamma), d(beta) in fp32."""
+    B, C, vox = x3.shape
+    dx, dg, db = torch.empty_like(x3), torch.empty_like(gamma), torch.empty_like(gamma)
+    _call(L.lib().fz_layernorm_cf_backward_add_bf16, L.ptr(x3), L.ptr(gamma), L.ptr(gy), L.ptr(add), L.ptr(dx), L.ptr(dg),
+          L.ptr(db), B, C, vox, float(eps), L.stream_ptr(x3.device))
+    return dx, dg, db
+
+
+class FactorizerBlockBf16Fn(_GradModeFunction):
+    """FactorizerBlockWideFn's steps on bf16 activations: every activation (n1, z, m, x1, n2, h, g, the output, dx) is bf16 in
+    memory and in the saved tensors; the parameters and their gradients stay fp32 (master weights), every sum accumulates
+    in fp32, the LayerNorm statistics are fp32, and bias, residual, GELU and GELU' are applied before the one rounding to
+    bf16.  One launch stages the four weights in bf16 (as stored and transposed), then norm1 | in_proj | core x3 |
+    out_proj + residual | norm2 | fc1 + GELU | fc2 + residual; the backward runs the same steps in reverse with the
+    weight gradients from fz_linear_wgrad_bf16."""
+
+    @staticmethod
+    def forward(ctx, x, g1, b1n, w_in, w_out, b_out, g2, b2n, w1, bb1, w2, bb2, u0, v0, geom, spec, eps1, eps2):
+        if x.dtype != torch.bfloat16:
+            raise NotImplementedError(f"factorizer_b200: FactorizerBlockBf16Fn takes bf16 activations, got {x.dtype}")
+        x = _check_vol(x, geom, "x", allow_bf16=True)
+        params = [L.require_cuda_f32(t, "parameter") for t in (g1, b1n, w_in, w_out, b_out, g2, b2n, w1, bb1, w2, bb2)]
+        g1, b1n, w_in, w_out, b_out, g2, b2n, w1, bb1, w2, bb2 = params
+        u0 = L.require_cuda_f32(u0, "u0")
+        v0 = L.require_cuda_f32(v0, "v0")
+        B, C = x.shape[0], x.shape[1]
+        H = w1.shape[0]
+        need_grad = _GradModeFunction.wants_grad(ctx, 12)
+        x3 = x.view(B, C, -1)
+        with torch.cuda.device(x.device):
+            staged = _stage_weights_bf16((w_in, w_out, w1, w2))
+            (wi, _), (wo, _), (f1, _), (f2, _) = _staged_views(staged, [tuple(w.shape) for w in (w_in, w_out, w1, w2)])
+            n1 = _ln_forward_bf16(x3, g1, b1n, eps1)
+            z = _channel_map_bf16(n1, wi, C, None)
+            m, saved = _swnmf_forward(z.view(x.shape), u0, v0, geom, spec, True, need_grad)
+            m3 = m.view(B, C, -1)
+            x1 = _channel_map_bf16(m3, wo, C, b_out, EPI_RESIDUAL, x3)
+            n2 = _ln_forward_bf16(x1, g2, b2n, eps2)
+            if need_grad:
+                h, g = _channel_map_bf16(n2, f1, H, bb1, EPI_GELU)
+            else:                                                       # inference: the pre-activation is not kept
+                h, g = None, _channel_map_bf16(n2, f1, H, bb1, EPI_GELU_ONLY)
+            out = _channel_map_bf16(g, f2, C, bb2, EPI_RESIDUAL, x1)
+        if need_grad:
+            ctx.save_for_backward(x3, n1, z, m3, x1, n2, h, g, saved, g1, g2, u0, v0, staged)
+            ctx.geom, ctx.spec, ctx.eps, ctx.C, ctx.H = geom, spec, (float(eps1), float(eps2)), C, H
+        return out.view(x.shape)
+
+    @staticmethod
+    @once_differentiable
+    def backward(ctx, gout):
+        x3, n1, z, m3, x1, n2, h, g, saved, g1, g2, u0, v0, staged = ctx.saved_tensors
+        geom, H = ctx.geom, ctx.H
+        gout = _check_vol(gout.to(torch.bfloat16), geom, "grad", allow_bf16=True)
+        B, C = x3.shape[0], x3.shape[1]
+        eps1, eps2 = ctx.eps
+        (_, wit), (_, wot), (_, f1t), (_, f2t) = _staged_views(staged, [(C, C), (C, C), (H, C), (C, H)])
+        go3 = gout.view(B, C, -1)
+        with torch.cuda.device(x3.device):
+            dh = _channel_map_bf16(go3, f2t, H, None, EPI_GELU_GRAD, h)     # (W2^T dOut) * gelu'(h)
+            dw2, dbb2 = _channel_map_wgrad_bf16(go3, g, True)
+            dw1, dbb1 = _channel_map_wgrad_bf16(dh, n2, True)
+            dn2 = _channel_map_bf16(dh, f1t, C, None)
+            dx1, dg2, db2n = _ln_backward_add_bf16(x1, g2, dn2, go3, eps2)   # dOut + norm2'(..)
+            dm = _channel_map_bf16(dx1, wot, C, None)
+            dw_out, db_out = _channel_map_wgrad_bf16(dx1, m3, True)
+            vol = (B, C, *geom.size)
+            dz = _swnmf_backward(z.view(vol), dm.view(vol), u0, v0, saved, geom, ctx.spec, True).view(B, C, -1)
+            dw_in, _ = _channel_map_wgrad_bf16(dz, n1, False)
+            dn1 = _channel_map_bf16(dz, wit, C, None)
+            dx, dg1, db1n = _ln_backward_add_bf16(x3, g1, dn1, dx1, eps1)   # dx1 + norm1'(..)
+        return (dx.view(vol), dg1, db1n, dw_in, dw_out, db_out, dg2, db2n, dw1, dbb1, dw2, dbb2,
+                None, None, None, None, None, None)
+
+
 # ---- channels-first LayerNorm (glue around the mixer) --------------------------------------------
 def layernorm_cf_supported(x: torch.Tensor) -> bool:
     if not (isinstance(x, torch.Tensor) and x.is_cuda and x.dtype == torch.float32 and x.dim() >= 3):

@@ -180,6 +180,16 @@ size_t fz_swnmf_workspace_bytes(const fz_geom* g, const fz_solver* s) {
     return a;
 }
 
+int fz_swnmf_bf16_supported(const fz_geom* g, const fz_solver* s, int32_t relu_input) {
+    if (!g || !s) return 0;
+    fz_geom gb = *g;
+    gb.dtype = FZ_DTYPE_BF16;
+    DevGeom G;
+    int K;
+    if (make_dev_geom(&gb, &G) || check_solver(s, G.d, G.P, &K)) return 0;
+    return phase_supported(G, *s, relu_input) ? 1 : 0;
+}
+
 int fz_swnmf_forward(const float* x, const float* u0, const float* v0, float* y, void* saved,
                      void* workspace, const fz_geom* g, const fz_solver* s, int32_t relu_input,
                      void* stream) {

@@ -8,16 +8,33 @@
 // accumulates d(gamma), d(beta) per thread across its voxels, reduces them per CTA in shared memory and
 // issues one atomicAdd per channel and CTA.  HBM-bound: forward reads x and writes y once, backward reads
 // x and dy once and writes dx once.
+//
+// The kernels are templated on the element type T of x, y, dy, add and dx: float, or bf16 (the bf16 FactorizerBlock), which is
+// read and written as bf16 pairs and computed in fp32; gamma, beta, their gradients and the statistics stay fp32.
+#include <cuda_bf16.h>
+
 #include "fz_common.cuh"
 
 namespace fz {
 namespace {
 
+template <typename T> struct Pair2;
+template <> struct Pair2<float> { typedef float2 type; };
+template <> struct Pair2<__nv_bfloat16> { typedef __nv_bfloat162 type; };
+template <typename T> using pair_t = typename Pair2<T>::type;   // two neighbouring voxels of one channel
+
+__device__ __forceinline__ float2 ld2(const float2* p) { return __ldg(p); }
+__device__ __forceinline__ float2 ld2(const __nv_bfloat162* p) { return __bfloat1622float2(__ldg(p)); }
+__device__ __forceinline__ float2 ld2cs(const float2* p) { return __ldcs(p); }
+__device__ __forceinline__ float2 ld2cs(const __nv_bfloat162* p) { return __bfloat1622float2(__ldcs(p)); }
+__device__ __forceinline__ void st2(float2* p, float2 v) { *p = v; }
+__device__ __forceinline__ void st2(__nv_bfloat162* p, float2 v) { *p = __float22bfloat162_rn(v); }
+
 constexpr int kLnThreads = 256;
 
-template <int C>
-__global__ void __launch_bounds__(kLnThreads) layernorm_cf_fwd(const float* __restrict__ x, const float* __restrict__ gamma,
-                                                               const float* __restrict__ beta, float* __restrict__ y,
+template <int C, typename T>
+__global__ void __launch_bounds__(kLnThreads) layernorm_cf_fwd(const T* __restrict__ x, const float* __restrict__ gamma,
+                                                               const float* __restrict__ beta, T* __restrict__ y,
                                                                long long pairs_per_sample, long long total_pairs, float eps) {
     __shared__ float gs[C], bs[C];
     for (int c = threadIdx.x; c < C; c += blockDim.x) { gs[c] = gamma ? gamma[c] : 1.f; bs[c] = beta ? beta[c] : 0.f; }
@@ -25,11 +42,11 @@ __global__ void __launch_bounds__(kLnThreads) layernorm_cf_fwd(const float* __re
     const long long vox = 2 * pairs_per_sample;
     for (long long p = (long long)blockIdx.x * blockDim.x + threadIdx.x; p < total_pairs; p += (long long)gridDim.x * blockDim.x) {
         const long long b = p / pairs_per_sample, v = p - b * pairs_per_sample;
-        const float2* xp = reinterpret_cast<const float2*>(x + b * C * vox) + v;
+        const pair_t<T>* xp = reinterpret_cast<const pair_t<T>*>(x + b * C * vox) + v;
         float2 val[C];
         float2 sum = make_float2(0.f, 0.f);
 #pragma unroll
-        for (int c = 0; c < C; ++c) { val[c] = __ldcs(xp + (long long)c * pairs_per_sample); sum.x += val[c].x; sum.y += val[c].y; }
+        for (int c = 0; c < C; ++c) { val[c] = ld2cs(xp + (long long)c * pairs_per_sample); sum.x += val[c].x; sum.y += val[c].y; }
         const float2 mean = make_float2(sum.x * (1.f / C), sum.y * (1.f / C));
         float2 var = make_float2(0.f, 0.f);
 #pragma unroll
@@ -38,21 +55,21 @@ __global__ void __launch_bounds__(kLnThreads) layernorm_cf_fwd(const float* __re
             var.x = fmaf(dx, dx, var.x); var.y = fmaf(dy, dy, var.y);
         }
         const float2 rstd = make_float2(rsqrtf(var.x * (1.f / C) + eps), rsqrtf(var.y * (1.f / C) + eps));
-        float2* yp = reinterpret_cast<float2*>(y + b * C * vox) + v;
+        pair_t<T>* yp = reinterpret_cast<pair_t<T>*>(y + b * C * vox) + v;
 #pragma unroll
         for (int c = 0; c < C; ++c) {
             float2 o;
             o.x = fmaf((val[c].x - mean.x) * rstd.x, gs[c], bs[c]);
             o.y = fmaf((val[c].y - mean.y) * rstd.y, gs[c], bs[c]);
-            yp[(long long)c * pairs_per_sample] = o;
+            st2(yp + (long long)c * pairs_per_sample, o);
         }
     }
 }
 
-template <int C>
-__global__ void __launch_bounds__(kLnThreads) layernorm_cf_bwd(const float* __restrict__ x, const float* __restrict__ gamma,
-                                                               const float* __restrict__ dy, const float* __restrict__ add,
-                                                               float* __restrict__ dx, float* __restrict__ dgamma, float* __restrict__ dbeta,
+template <int C, typename T>
+__global__ void __launch_bounds__(kLnThreads) layernorm_cf_bwd(const T* __restrict__ x, const float* __restrict__ gamma,
+                                                               const T* __restrict__ dy, const T* __restrict__ add,
+                                                               T* __restrict__ dx, float* __restrict__ dgamma, float* __restrict__ dbeta,
                                                                long long pairs_per_sample, long long total_pairs, float eps) {
     __shared__ float gs[C];
     __shared__ float red[2][C][kLnThreads / 32];
@@ -64,14 +81,14 @@ __global__ void __launch_bounds__(kLnThreads) layernorm_cf_bwd(const float* __re
     for (int c = 0; c < C; ++c) { dg[c] = 0.f; db[c] = 0.f; }
     for (long long p = (long long)blockIdx.x * blockDim.x + threadIdx.x; p < total_pairs; p += (long long)gridDim.x * blockDim.x) {
         const long long b = p / pairs_per_sample, v = p - b * pairs_per_sample;
-        const float2* xp = reinterpret_cast<const float2*>(x + b * C * vox) + v;
-        const float2* gp = reinterpret_cast<const float2*>(dy + b * C * vox) + v;
+        const pair_t<T>* xp = reinterpret_cast<const pair_t<T>*>(x + b * C * vox) + v;
+        const pair_t<T>* gp = reinterpret_cast<const pair_t<T>*>(dy + b * C * vox) + v;
         float2 xh[C], g[C];
         float2 sum = make_float2(0.f, 0.f);
 #pragma unroll
         for (int c = 0; c < C; ++c) {
-            xh[c] = __ldcs(xp + (long long)c * pairs_per_sample);
-            g[c] = __ldcs(gp + (long long)c * pairs_per_sample);
+            xh[c] = ld2cs(xp + (long long)c * pairs_per_sample);
+            g[c] = ld2cs(gp + (long long)c * pairs_per_sample);
             sum.x += xh[c].x; sum.y += xh[c].y;
         }
         const float2 mean = make_float2(sum.x * (1.f / C), sum.y * (1.f / C));
@@ -94,15 +111,15 @@ __global__ void __launch_bounds__(kLnThreads) layernorm_cf_bwd(const float* __re
             m2.x = fmaf(g[c].x, xh[c].x, m2.x); m2.y = fmaf(g[c].y, xh[c].y, m2.y);
         }
         m1.x *= (1.f / C); m1.y *= (1.f / C); m2.x *= (1.f / C); m2.y *= (1.f / C);
-        float2* op = reinterpret_cast<float2*>(dx + b * C * vox) + v;
-        const float2* ap = add ? reinterpret_cast<const float2*>(add + b * C * vox) + v : nullptr;
+        pair_t<T>* op = reinterpret_cast<pair_t<T>*>(dx + b * C * vox) + v;
+        const pair_t<T>* ap = add ? reinterpret_cast<const pair_t<T>*>(add + b * C * vox) + v : nullptr;
 #pragma unroll
         for (int c = 0; c < C; ++c) {
             float2 o;
             o.x = rstd.x * (g[c].x - m1.x - xh[c].x * m2.x);
             o.y = rstd.y * (g[c].y - m1.y - xh[c].y * m2.y);
-            if (ap) { const float2 r = __ldcs(ap + (long long)c * pairs_per_sample); o.x += r.x; o.y += r.y; }
-            op[(long long)c * pairs_per_sample] = o;
+            if (ap) { const float2 r = ld2cs(ap + (long long)c * pairs_per_sample); o.x += r.x; o.y += r.y; }
+            st2(op + (long long)c * pairs_per_sample, o);
         }
     }
     if (dgamma || dbeta) {
@@ -129,12 +146,13 @@ __global__ void __launch_bounds__(kLnThreads) layernorm_cf_bwd(const float* __re
 // L1 / L2) instead of three times; the backward keeps per-warp rows of d(gamma), d(beta) partials in shared memory.
 constexpr int kLnMaxC = 512;
 
-__device__ __forceinline__ void ln_stats(const float2* __restrict__ xp, long long pps, int C, float eps, float2& mean, float2& rstd) {
-    const float2 k = __ldg(xp);
+template <typename P>
+__device__ __forceinline__ void ln_stats(const P* __restrict__ xp, long long pps, int C, float eps, float2& mean, float2& rstd) {
+    const float2 k = ld2(xp);
     float2 s1 = make_float2(0.f, 0.f), s2 = make_float2(0.f, 0.f);
 #pragma unroll 8
     for (int c = 0; c < C; ++c) {
-        const float2 v = __ldg(xp + (long long)c * pps);
+        const float2 v = ld2(xp + (long long)c * pps);
         const float dx = v.x - k.x, dy = v.y - k.y;
         s1.x += dx; s1.y += dy;
         s2.x = fmaf(dx, dx, s2.x); s2.y = fmaf(dy, dy, s2.y);
@@ -145,8 +163,9 @@ __device__ __forceinline__ void ln_stats(const float2* __restrict__ xp, long lon
     rstd = make_float2(rsqrtf(fmaxf(s2.x * inv - mx * mx, 0.f) + eps), rsqrtf(fmaxf(s2.y * inv - my * my, 0.f) + eps));
 }
 
-__global__ void __launch_bounds__(kLnThreads) layernorm_cf_fwd_any(const float* __restrict__ x, const float* __restrict__ gamma,
-                                                                   const float* __restrict__ beta, float* __restrict__ y, int C,
+template <typename T>
+__global__ void __launch_bounds__(kLnThreads) layernorm_cf_fwd_any(const T* __restrict__ x, const float* __restrict__ gamma,
+                                                                   const float* __restrict__ beta, T* __restrict__ y, int C,
                                                                    long long pairs_per_sample, long long total_pairs, float eps) {
     __shared__ float gs[kLnMaxC], bs[kLnMaxC];
     for (int c = threadIdx.x; c < C; c += blockDim.x) { gs[c] = gamma ? gamma[c] : 1.f; bs[c] = beta ? beta[c] : 0.f; }
@@ -154,15 +173,15 @@ __global__ void __launch_bounds__(kLnThreads) layernorm_cf_fwd_any(const float* 
     const long long vox = 2 * pairs_per_sample;
     for (long long p = (long long)blockIdx.x * blockDim.x + threadIdx.x; p < total_pairs; p += (long long)gridDim.x * blockDim.x) {
         const long long b = p / pairs_per_sample, v = p - b * pairs_per_sample;
-        const float2* xp = reinterpret_cast<const float2*>(x + b * C * vox) + v;
-        float2* yp = reinterpret_cast<float2*>(y + b * C * vox) + v;
+        const pair_t<T>* xp = reinterpret_cast<const pair_t<T>*>(x + b * C * vox) + v;
+        pair_t<T>* yp = reinterpret_cast<pair_t<T>*>(y + b * C * vox) + v;
         float2 mean, rstd;
         ln_stats(xp, pairs_per_sample, C, eps, mean, rstd);
 #pragma unroll 8
         for (int c = 0; c < C; ++c) {
-            const float2 val = __ldg(xp + (long long)c * pairs_per_sample);
-            yp[(long long)c * pairs_per_sample] = make_float2(fmaf((val.x - mean.x) * rstd.x, gs[c], bs[c]),
-                                                              fmaf((val.y - mean.y) * rstd.y, gs[c], bs[c]));
+            const float2 val = ld2(xp + (long long)c * pairs_per_sample);
+            st2(yp + (long long)c * pairs_per_sample, make_float2(fmaf((val.x - mean.x) * rstd.x, gs[c], bs[c]),
+                                                              fmaf((val.y - mean.y) * rstd.y, gs[c], bs[c])));
         }
     }
 }
@@ -185,9 +204,10 @@ __device__ __forceinline__ float warp_transpose_sum32(float (&v)[32], int lane) 
     return v[0];
 }
 
-__global__ void __launch_bounds__(kLnThreads) layernorm_cf_bwd_any(const float* __restrict__ x, const float* __restrict__ gamma,
-                                                                   const float* __restrict__ dy, const float* __restrict__ add,
-                                                                   float* __restrict__ dx, float* __restrict__ dgamma, float* __restrict__ dbeta, int C,
+template <typename T>
+__global__ void __launch_bounds__(kLnThreads) layernorm_cf_bwd_any(const T* __restrict__ x, const float* __restrict__ gamma,
+                                                                   const T* __restrict__ dy, const T* __restrict__ add,
+                                                                   T* __restrict__ dx, float* __restrict__ dgamma, float* __restrict__ dbeta, int C,
                                                                    long long pairs_per_sample, long long total_pairs, float eps) {
     extern __shared__ float lsm[];
     const int CP = (C + 31) & ~31;                     // channels rounded up to whole chunks of 32
@@ -207,9 +227,9 @@ __global__ void __launch_bounds__(kLnThreads) layernorm_cf_bwd_any(const float* 
         const bool valid = p < total_pairs;
         const long long pc = valid ? p : 0;
         const long long b = pc / pairs_per_sample, v = pc - b * pairs_per_sample;
-        const float2* xp = reinterpret_cast<const float2*>(x + b * C * vox) + v;
-        const float2* gp = reinterpret_cast<const float2*>(dy + b * C * vox) + v;
-        float2* op = reinterpret_cast<float2*>(dx + b * C * vox) + v;
+        const pair_t<T>* xp = reinterpret_cast<const pair_t<T>*>(x + b * C * vox) + v;
+        const pair_t<T>* gp = reinterpret_cast<const pair_t<T>*>(dy + b * C * vox) + v;
+        pair_t<T>* op = reinterpret_cast<pair_t<T>*>(dx + b * C * vox) + v;
         float2 mean, rstd;
         ln_stats(xp, pairs_per_sample, C, eps, mean, rstd);
         float2 m1 = make_float2(0.f, 0.f), m2 = make_float2(0.f, 0.f);
@@ -218,8 +238,8 @@ __global__ void __launch_bounds__(kLnThreads) layernorm_cf_bwd_any(const float* 
 #pragma unroll
             for (int j = 0; j < 32; ++j) {
                 const int c = min(c0 + j, C - 1);                  // the tail chunk re-reads the last channel, weighted 0
-                const float2 xv = __ldg(xp + (long long)c * pairs_per_sample);
-                float2 g = __ldg(gp + (long long)c * pairs_per_sample);
+                const float2 xv = ld2(xp + (long long)c * pairs_per_sample);
+                float2 g = ld2(gp + (long long)c * pairs_per_sample);
                 if (!valid || c0 + j >= C) g = make_float2(0.f, 0.f);
                 const float hx = (xv.x - mean.x) * rstd.x, hy = (xv.y - mean.y) * rstd.y;
                 sg[j] = fmaf(g.x, hx, g.y * hy);
@@ -239,15 +259,15 @@ __global__ void __launch_bounds__(kLnThreads) layernorm_cf_bwd_any(const float* 
         if (valid) {
 #pragma unroll 8
             for (int c = 0; c < C; ++c) {
-                const float2 xv = __ldg(xp + (long long)c * pairs_per_sample);
-                const float2 g = __ldg(gp + (long long)c * pairs_per_sample);
+                const float2 xv = ld2(xp + (long long)c * pairs_per_sample);
+                const float2 g = ld2(gp + (long long)c * pairs_per_sample);
                 const float hx = (xv.x - mean.x) * rstd.x, hy = (xv.y - mean.y) * rstd.y;
                 float2 o = make_float2(rstd.x * (g.x * gs[c] - m1.x - hx * m2.x), rstd.y * (g.y * gs[c] - m1.y - hy * m2.y));
                 if (add) {
-                    const float2 r = __ldg(reinterpret_cast<const float2*>(add + b * C * vox) + v + (long long)c * pairs_per_sample);
+                    const float2 r = ld2(reinterpret_cast<const pair_t<T>*>(add + b * C * vox) + v + (long long)c * pairs_per_sample);
                     o.x += r.x; o.y += r.y;
                 }
-                op[(long long)c * pairs_per_sample] = o;
+                st2(op + (long long)c * pairs_per_sample, o);
             }
         }
     }
@@ -275,14 +295,15 @@ __device__ __forceinline__ void slice_range(int C, int& cbeg, int& cend) {
 }
 
 // partial shifted sums of this slice -> totals over all slices (every thread of a pair column gets the same values)
-__device__ __forceinline__ void sliced_stats(const float2* __restrict__ xp, long long pps, int C, int cbeg, int cend, float eps,
+template <typename P>
+__device__ __forceinline__ void sliced_stats(const P* __restrict__ xp, long long pps, int C, int cbeg, int cend, float eps,
                                              float2 (*sa)[32], float2 (*sb)[32], float2& mean, float2& rstd) {
     const int lane = threadIdx.x;
-    const float2 k = __ldg(xp);
+    const float2 k = ld2(xp);
     float2 s1 = make_float2(0.f, 0.f), s2 = make_float2(0.f, 0.f);
 #pragma unroll 8
     for (int c = cbeg; c < cend; ++c) {
-        const float2 v = __ldg(xp + (long long)c * pps);
+        const float2 v = ld2(xp + (long long)c * pps);
         const float dx = v.x - k.x, dy = v.y - k.y;
         s1.x += dx; s1.y += dy;
         s2.x = fmaf(dx, dx, s2.x); s2.y = fmaf(dy, dy, s2.y);
@@ -301,8 +322,9 @@ __device__ __forceinline__ void sliced_stats(const float2* __restrict__ xp, long
     rstd = make_float2(rsqrtf(fmaxf(s2.x * inv - mx * mx, 0.f) + eps), rsqrtf(fmaxf(s2.y * inv - my * my, 0.f) + eps));
 }
 
-__global__ void __launch_bounds__(32 * kLnMaxSlices) layernorm_cf_fwd_sliced(const float* __restrict__ x, const float* __restrict__ gamma,
-                                                                             const float* __restrict__ beta, float* __restrict__ y, int C,
+template <typename T>
+__global__ void __launch_bounds__(32 * kLnMaxSlices) layernorm_cf_fwd_sliced(const T* __restrict__ x, const float* __restrict__ gamma,
+                                                                             const float* __restrict__ beta, T* __restrict__ y, int C,
                                                                              long long pairs_per_sample, long long total_pairs, float eps) {
     __shared__ float2 sa[kLnMaxSlices][32], sb[kLnMaxSlices][32];
     const int lane = threadIdx.x;
@@ -314,25 +336,26 @@ __global__ void __launch_bounds__(32 * kLnMaxSlices) layernorm_cf_fwd_sliced(con
         const bool valid = p < total_pairs;
         const long long pc = valid ? p : 0;
         const long long b = pc / pairs_per_sample, v = pc - b * pairs_per_sample;
-        const float2* xp = reinterpret_cast<const float2*>(x + b * C * vox) + v;
-        float2* yp = reinterpret_cast<float2*>(y + b * C * vox) + v;
+        const pair_t<T>* xp = reinterpret_cast<const pair_t<T>*>(x + b * C * vox) + v;
+        pair_t<T>* yp = reinterpret_cast<pair_t<T>*>(y + b * C * vox) + v;
         float2 mean, rstd;
         sliced_stats(xp, pairs_per_sample, C, cbeg, cend, eps, sa, sb, mean, rstd);
         if (valid) {
 #pragma unroll 8
             for (int c = cbeg; c < cend; ++c) {
-                const float2 val = __ldg(xp + (long long)c * pairs_per_sample);
+                const float2 val = ld2(xp + (long long)c * pairs_per_sample);
                 const float g = gamma ? __ldg(gamma + c) : 1.f, bb = beta ? __ldg(beta + c) : 0.f;
-                yp[(long long)c * pairs_per_sample] = make_float2(fmaf((val.x - mean.x) * rstd.x, g, bb), fmaf((val.y - mean.y) * rstd.y, g, bb));
+                st2(yp + (long long)c * pairs_per_sample, make_float2(fmaf((val.x - mean.x) * rstd.x, g, bb), fmaf((val.y - mean.y) * rstd.y, g, bb)));
             }
         }
         __syncthreads();          // sa / sb are rewritten by the next group
     }
 }
 
-__global__ void __launch_bounds__(32 * kLnMaxSlices, 2) layernorm_cf_bwd_sliced(const float* __restrict__ x, const float* __restrict__ gamma,
-                                                                             const float* __restrict__ dy, const float* __restrict__ add,
-                                                                             float* __restrict__ dx, float* __restrict__ dgamma, float* __restrict__ dbeta, int C,
+template <typename T>
+__global__ void __launch_bounds__(32 * kLnMaxSlices, 2) layernorm_cf_bwd_sliced(const T* __restrict__ x, const float* __restrict__ gamma,
+                                                                             const T* __restrict__ dy, const T* __restrict__ add,
+                                                                             T* __restrict__ dx, float* __restrict__ dgamma, float* __restrict__ dbeta, int C,
                                                                              long long pairs_per_sample, long long total_pairs, float eps) {
     extern __shared__ float lsm[];
     __shared__ float2 sa[kLnMaxSlices][32], sb[kLnMaxSlices][32];
@@ -350,9 +373,9 @@ __global__ void __launch_bounds__(32 * kLnMaxSlices, 2) layernorm_cf_bwd_sliced(
         const bool valid = p < total_pairs;
         const long long pc = valid ? p : 0;
         const long long b = pc / pairs_per_sample, v = pc - b * pairs_per_sample;
-        const float2* xp = reinterpret_cast<const float2*>(x + b * C * vox) + v;
-        const float2* gp = reinterpret_cast<const float2*>(dy + b * C * vox) + v;
-        float2* op = reinterpret_cast<float2*>(dx + b * C * vox) + v;
+        const pair_t<T>* xp = reinterpret_cast<const pair_t<T>*>(x + b * C * vox) + v;
+        const pair_t<T>* gp = reinterpret_cast<const pair_t<T>*>(dy + b * C * vox) + v;
+        pair_t<T>* op = reinterpret_cast<pair_t<T>*>(dx + b * C * vox) + v;
         float2 mean, rstd;
         sliced_stats(xp, pairs_per_sample, C, cbeg, cend, eps, sa, sb, mean, rstd);
         float2 m1 = make_float2(0.f, 0.f), m2 = make_float2(0.f, 0.f);
@@ -362,8 +385,8 @@ __global__ void __launch_bounds__(32 * kLnMaxSlices, 2) layernorm_cf_bwd_sliced(
             for (int j = 0; j < 32; ++j) {
                 const bool live = c0 + j < cend;
                 const int c = live ? c0 + j : cend - 1;            // the tail chunk re-reads the last channel, weighted 0
-                const float2 xv = __ldg(xp + (long long)c * pairs_per_sample);
-                float2 g = __ldg(gp + (long long)c * pairs_per_sample);
+                const float2 xv = ld2(xp + (long long)c * pairs_per_sample);
+                float2 g = ld2(gp + (long long)c * pairs_per_sample);
                 if (!valid || !live) g = make_float2(0.f, 0.f);
                 const float hx = (xv.x - mean.x) * rstd.x, hy = (xv.y - mean.y) * rstd.y;
                 sg[j] = fmaf(g.x, hx, g.y * hy);
@@ -392,16 +415,16 @@ __global__ void __launch_bounds__(32 * kLnMaxSlices, 2) layernorm_cf_bwd_sliced(
         if (valid) {
 #pragma unroll 8
             for (int c = cbeg; c < cend; ++c) {
-                const float2 xv = __ldg(xp + (long long)c * pairs_per_sample);
-                const float2 g = __ldg(gp + (long long)c * pairs_per_sample);
+                const float2 xv = ld2(xp + (long long)c * pairs_per_sample);
+                const float2 g = ld2(gp + (long long)c * pairs_per_sample);
                 const float w = gs[c];
                 const float hx = (xv.x - mean.x) * rstd.x, hy = (xv.y - mean.y) * rstd.y;
                 float2 o = make_float2(rstd.x * (g.x * w - m1.x - hx * m2.x), rstd.y * (g.y * w - m1.y - hy * m2.y));
                 if (add) {
-                    const float2 r = __ldg(reinterpret_cast<const float2*>(add + b * C * vox) + v + (long long)c * pairs_per_sample);
+                    const float2 r = ld2(reinterpret_cast<const pair_t<T>*>(add + b * C * vox) + v + (long long)c * pairs_per_sample);
                     o.x += r.x; o.y += r.y;
                 }
-                op[(long long)c * pairs_per_sample] = o;
+                st2(op + (long long)c * pairs_per_sample, o);
             }
         }
         __syncthreads();          // sa / sb are rewritten by the next group
@@ -419,8 +442,8 @@ int ln_slices(int channels, long long total_pairs) {
     return channels >= 256 ? 8 : (channels >= 128 ? 4 : 2);
 }
 
-template <int C>
-int launch_fwd(const float* x, const float* gamma, const float* beta, float* y, long long batch, long long voxels, float eps, cudaStream_t st) {
+template <int C, typename T>
+int launch_fwd(const T* x, const float* gamma, const float* beta, T* y, long long batch, long long voxels, float eps, cudaStream_t st) {
     const long long pps = voxels / 2, total = batch * pps;
     long long blocks = (total + kLnThreads - 1) / kLnThreads;
     const long long cap = 8LL * num_sms();
@@ -429,8 +452,8 @@ int launch_fwd(const float* x, const float* gamma, const float* beta, float* y, 
     FZ_LAUNCH_CHECK();
     return FZ_OK;
 }
-template <int C>
-int launch_bwd(const float* x, const float* gamma, const float* dy, const float* add, float* dx, float* dgamma, float* dbeta, long long batch,
+template <int C, typename T>
+int launch_bwd(const T* x, const float* gamma, const T* dy, const T* add, T* dx, float* dgamma, float* dbeta, long long batch,
                long long voxels, float eps, cudaStream_t st) {
     const long long pps = voxels / 2, total = batch * pps;
     long long blocks = (total + kLnThreads - 1) / kLnThreads;
@@ -443,32 +466,24 @@ int launch_bwd(const float* x, const float* gamma, const float* dy, const float*
     return FZ_OK;
 }
 
-int check_args(const void* a, const void* b, long long batch, int channels, long long voxels) {
+// `align`: the byte alignment of a voxel pair of the element type
+int check_args(const void* a, const void* b, long long batch, int channels, long long voxels, uintptr_t align) {
     if (!a || !b) return fail(FZ_ERR_INVALID, "null buffer");
     if (batch < 0 || voxels < 0) return fail(FZ_ERR_INVALID, "negative size");
     if (channels < 1 || channels > kLnMaxC)
         return fail(FZ_ERR_UNSUPPORTED, "channels-first LayerNorm kernel handles 1..%d channels, got %d", kLnMaxC, channels);
     if (voxels % 2) return fail(FZ_ERR_UNSUPPORTED, "channels-first LayerNorm kernel needs an even number of voxels, got %lld", voxels);
-    if ((reinterpret_cast<uintptr_t>(a) | reinterpret_cast<uintptr_t>(b)) & 7) return fail(FZ_ERR_INVALID, "buffers must be 8-byte aligned");
+    if ((reinterpret_cast<uintptr_t>(a) | reinterpret_cast<uintptr_t>(b)) & (align - 1))
+        return fail(FZ_ERR_INVALID, "buffers must be %d-byte aligned", (int)align);
     return FZ_OK;
 }
 
-}  // namespace
-}  // namespace fz
-
-using namespace fz;
-
-extern "C" {
-
-int fz_layernorm_cf_supported(int32_t channels, int64_t voxels) {
-    return channels >= 1 && channels <= kLnMaxC && voxels % 2 == 0;
-}
-
-int fz_layernorm_cf_forward(const float* x, const float* gamma, const float* beta, float* y, int64_t batch,
-                            int32_t channels, int64_t voxels, float eps, void* stream) {
+template <typename T>
+int ln_forward(const T* x, const float* gamma, const float* beta, T* y, int64_t batch, int32_t channels, int64_t voxels, float eps,
+               void* stream) {
     tls().launches = 0;
     if (batch == 0 || voxels == 0) return FZ_OK;          // empty tensors carry null data pointers
-    if (int e = check_args(x, y, batch, channels, voxels)) return e;
+    if (int e = check_args(x, y, batch, channels, voxels, sizeof(pair_t<T>))) return e;
     cudaStream_t st = (cudaStream_t)stream;
     switch (channels) {
         case 8: return launch_fwd<8>(x, gamma, beta, y, batch, voxels, eps, st);
@@ -495,13 +510,9 @@ int fz_layernorm_cf_forward(const float* x, const float* gamma, const float* bet
     }
 }
 
-int fz_layernorm_cf_backward(const float* x, const float* gamma, const float* dy, float* dx, float* dgamma,
-                             float* dbeta, int64_t batch, int32_t channels, int64_t voxels, float eps, void* stream) {
-    return fz_layernorm_cf_backward_add(x, gamma, dy, nullptr, dx, dgamma, dbeta, batch, channels, voxels, eps, stream);
-}
-
-int fz_layernorm_cf_backward_add(const float* x, const float* gamma, const float* dy, const float* add, float* dx, float* dgamma,
-                                 float* dbeta, int64_t batch, int32_t channels, int64_t voxels, float eps, void* stream) {
+template <typename T>
+int ln_backward_add(const T* x, const float* gamma, const T* dy, const T* add, T* dx, float* dgamma, float* dbeta, int64_t batch,
+                    int32_t channels, int64_t voxels, float eps, void* stream) {
     tls().launches = 0;
     cudaStream_t st = (cudaStream_t)stream;
     if (batch == 0 || voxels == 0) {
@@ -509,7 +520,7 @@ int fz_layernorm_cf_backward_add(const float* x, const float* gamma, const float
         if (dbeta) FZ_CUDA_CHECK(cudaMemsetAsync(dbeta, 0, channels * sizeof(float), st));
         return FZ_OK;
     }
-    if (int e = check_args(x, dx, batch, channels, voxels)) return e;
+    if (int e = check_args(x, dx, batch, channels, voxels, sizeof(pair_t<T>))) return e;
     if (!dy) return fail(FZ_ERR_INVALID, "null buffer");
     switch (channels) {
         case 8: return launch_bwd<8>(x, gamma, dy, add, dx, dgamma, dbeta, batch, voxels, eps, st);
@@ -536,11 +547,52 @@ int fz_layernorm_cf_backward_add(const float* x, const float* gamma, const float
         const size_t cp = ((size_t)channels + 31) & ~(size_t)31;
         const size_t smem = sizeof(float) * (cp + (threads / 32) * 2 * cp);
         static SmemConfig cfg;
-        FZ_CUDA_CHECK(cfg.ensure(layernorm_cf_bwd_any, sizeof(float) * (kLnMaxC + (kLnThreads / 32) * 2 * kLnMaxC)));
+        FZ_CUDA_CHECK(cfg.ensure(layernorm_cf_bwd_any<T>, sizeof(float) * (kLnMaxC + (kLnThreads / 32) * 2 * kLnMaxC)));
         layernorm_cf_bwd_any<<<(unsigned)blocks, threads, smem, st>>>(x, gamma, dy, add, dx, dgamma, dbeta, channels, pps, total, eps);
         FZ_LAUNCH_CHECK();
         return FZ_OK;
     }
+}
+
+}  // namespace
+}  // namespace fz
+
+using namespace fz;
+
+extern "C" {
+
+int fz_layernorm_cf_supported(int32_t channels, int64_t voxels) {
+    return channels >= 1 && channels <= kLnMaxC && voxels % 2 == 0;
+}
+
+int fz_layernorm_cf_forward(const float* x, const float* gamma, const float* beta, float* y, int64_t batch,
+                            int32_t channels, int64_t voxels, float eps, void* stream) {
+    return ln_forward(x, gamma, beta, y, batch, channels, voxels, eps, stream);
+}
+
+int fz_layernorm_cf_backward(const float* x, const float* gamma, const float* dy, float* dx, float* dgamma,
+                             float* dbeta, int64_t batch, int32_t channels, int64_t voxels, float eps, void* stream) {
+    return fz_layernorm_cf_backward_add(x, gamma, dy, nullptr, dx, dgamma, dbeta, batch, channels, voxels, eps, stream);
+}
+
+int fz_layernorm_cf_backward_add(const float* x, const float* gamma, const float* dy, const float* add, float* dx, float* dgamma,
+                                 float* dbeta, int64_t batch, int32_t channels, int64_t voxels, float eps, void* stream) {
+    return ln_backward_add(x, gamma, dy, add, dx, dgamma, dbeta, batch, channels, voxels, eps, stream);
+}
+
+int fz_layernorm_cf_bf16_supported(int32_t channels, int64_t voxels) { return fz_layernorm_cf_supported(channels, voxels); }
+
+int fz_layernorm_cf_forward_bf16(const void* x, const float* gamma, const float* beta, void* y, int64_t batch, int32_t channels,
+                                 int64_t voxels, float eps, void* stream) {
+    return ln_forward(static_cast<const __nv_bfloat16*>(x), gamma, beta, static_cast<__nv_bfloat16*>(y), batch, channels, voxels, eps,
+                      stream);
+}
+
+int fz_layernorm_cf_backward_add_bf16(const void* x, const float* gamma, const void* dy, const void* add, void* dx, float* dgamma,
+                                      float* dbeta, int64_t batch, int32_t channels, int64_t voxels, float eps, void* stream) {
+    typedef __nv_bfloat16 bf16;
+    return ln_backward_add(static_cast<const bf16*>(x), gamma, static_cast<const bf16*>(dy), static_cast<const bf16*>(add),
+                           static_cast<bf16*>(dx), dgamma, dbeta, batch, channels, voxels, eps, stream);
 }
 
 }  // extern "C"

@@ -40,6 +40,20 @@ __device__ __forceinline__ void mma_tf32(uint32_t tmem_d, uint64_t adesc, uint64
         "tcgen05.mma.cta_group::1.kind::tf32 [%0], %1, %2, %3, p;\n\t}\n"
         :: "r"(tmem_d), "l"(adesc), "l"(bdesc), "r"(idesc), "r"(accumulate) : "memory");
 }
+// kind::f16 with A = B = BF16 and D = F32 (bench_probes/tcgen05_bf16_layout_probe.cu): one MMA per 16 values of K.  16-bit
+// operands use the plain SWIZZLE_128B layout (type 2) in both majors -- K-major: 128-byte rows of 64 K values, SBO = 1024
+// between groups of 8 rows, a K step of 16 is +32 bytes; MN-major: 128-byte rows of 64 MN values, one row per K, SBO = 1024
+// between groups of 8 K, LBO between groups of 64 MN, a K step of 16 is +2048 bytes
+__device__ __forceinline__ uint32_t make_idesc_bf16(int m, int n, bool a_mn_major, bool b_mn_major) {
+    return (1u << 4) | (1u << 7) | (1u << 10) | ((a_mn_major ? 1u : 0u) << 15) | ((b_mn_major ? 1u : 0u) << 16) |
+           ((uint32_t)(n >> 3) << 17) | ((uint32_t)(m >> 4) << 24);
+}
+__device__ __forceinline__ void mma_bf16(uint32_t tmem_d, uint64_t adesc, uint64_t bdesc, uint32_t idesc, uint32_t accumulate) {
+    asm volatile(
+        "{\n\t.reg .pred p;\n\tsetp.ne.b32 p, %4, 0;\n\t"
+        "tcgen05.mma.cta_group::1.kind::f16 [%0], %1, %2, %3, p;\n\t}\n"
+        :: "r"(tmem_d), "l"(adesc), "l"(bdesc), "r"(idesc), "r"(accumulate) : "memory");
+}
 // UTCHMMA takes its operands from UNIFORM registers.  Issued under `if (threadIdx.x == 0)` the compiler wraps every MMA in
 // an ELECT / R2UR.BROADCAST / BRA.U.ANY loop (~70 cycles per MMA, measured); issued from warp-uniform control flow on
 // warp-uniform values (uniform_u32) under elect_one() it is a single predicated instruction.

@@ -7,10 +7,12 @@ reference's constructor signatures and parameter names (factorizer/factorizer.py
 any other combination runs the same steps through the standalone kernels.  A FactorizerBlock with LayerNorm / ReLU / GELU
 and no active dropout runs entirely in hand-written kernels: 32 channels in the fused glue kernels (csrc/fz_block_glue*.cu)
 around the fused core, any other width in the tcgen05 channel-map kernel with fused epilogues (csrc/fz_linear_tc.cu) and the
-channels-first LayerNorm kernels; other blocks run the glue layer by layer.
+channels-first LayerNorm kernels, bf16 inputs (bf16 autocast) in the bf16 channel maps (csrc/fz_bf16_block.cu) around the
+bf16 core; other blocks run the glue layer by layer.
 """
 from __future__ import annotations
 
+import torch
 from torch import nn
 
 from . import _ops
@@ -48,8 +50,10 @@ class FactMixer(nn.Module):
         out = self.in_proj(x)
         if self._fusable():
             f = self.factorize
-            out = _ops.SWNMF.apply(out, f.init.u0, f.init.v0, self.reshape._geom, f.solver_spec(),
-                                   isinstance(self.act, nn.ReLU))
+            relu = isinstance(self.act, nn.ReLU)
+            if out.dtype == torch.bfloat16 and not _ops.bf16_core_supported(self.reshape._geom, f.solver_spec(), relu):
+                out = out.float()           # the core takes bf16 volumes at the default Swin geometry only (not the 8^3 bottleneck)
+            out = _ops.SWNMF.apply(out, f.init.u0, f.init.v0, self.reshape._geom, f.solver_spec(), relu)
         else:
             out = self.reshape(out)
             out = self.act(out)
@@ -89,7 +93,13 @@ class FactorizerBlock(nn.Module):
         C = x.shape[1] if x.dim() >= 3 else -1
         if tuple(n1.normalized_shape) != (C,) or tuple(n2.normalized_shape) != (C,) or fc2.linear.out_channels != C:
             return None
-        if _ops.block_glue_supported(x, fc1.linear.out_channels):
+        if isinstance(x, torch.Tensor) and x.dtype == torch.bfloat16:
+            # bf16 activations (bf16 autocast, or bf16 inputs): the bf16 channel maps around the bf16 core, where both apply
+            if not (_ops.bf16_block_supported(x, fc1.linear.out_channels)
+                    and _ops.bf16_core_supported(f.reshape._geom, f.factorize.solver_spec())):
+                return None
+            fn = _ops.FactorizerBlockBf16Fn
+        elif _ops.block_glue_supported(x, fc1.linear.out_channels):
             fn = _ops.FactorizerBlockFn            # 32 channels: fused glue kernels (csrc/fz_block_glue*.cu)
         elif _ops.wide_block_supported(x, fc1.linear.out_channels):
             fn = _ops.FactorizerBlockWideFn        # any other width: channel-map kernels with fused epilogues

@@ -187,6 +187,42 @@ enum { FZ_EPILOGUE_NONE = 0, FZ_EPILOGUE_RESIDUAL = 1, FZ_EPILOGUE_GELU = 2, FZ_
 int fz_linear_forward_ex(const float* x, const float* W, const float* bias, float* y, int64_t batch, int32_t cin, int32_t cout,
                          int64_t voxels, int32_t epilogue, int32_t w_transposed, const float* aux, float* y2, void* stream);
 
+/* ---- bf16 activations (the FactorizerBlock under bf16 autocast, or fed bf16 tensors) -------------------------------------
+ * Buffers typed `void*` below hold bf16 (torch.bfloat16) values; parameters, their gradients and the LayerNorm statistics
+ * stay fp32, and every sum accumulates in fp32.  The bf16 TMA boxes need 16-byte row strides, so voxel counts must be
+ * multiples of 8, and the buffers TMA reads (x, W, dy) 16-byte aligned: FZ_ERR_UNSUPPORTED otherwise, before anything
+ * is written. */
+
+/* fz_linear_forward_ex on bf16 activations: r = W x + bias with the same FZ_EPILOGUE_* (aux, y, y2 bf16; bias fp32, may be
+ * NULL), applied to the fp32 sums before the one rounding to bf16.  W is a bf16 (cout, cin) matrix whose rows are ldw
+ * elements apart (ldw >= cin, a multiple of 8), K-major; the input gradient passes the transposed copy written by
+ * fz_bf16_stage_weights.  tcgen05 kind::f16, one MMA per 16 input channels. */
+int fz_linear_forward_bf16_supported(int32_t cout, int32_t cin, int64_t voxels);
+int fz_linear_forward_bf16(const void* x, const void* W, int32_t ldw, const float* bias, void* y, int64_t batch, int32_t cin,
+                           int32_t cout, int64_t voxels, int32_t epilogue, const void* aux, void* y2, void* stream);
+/* fz_linear_wgrad on bf16 dy (batch, cout, voxels) and x (batch, cin, voxels): dW (cout x cin) and db (cout, may be NULL)
+ * fp32, OVERWRITTEN. */
+int fz_linear_wgrad_bf16_supported(int32_t cout, int32_t cin, int64_t voxels);
+int fz_linear_wgrad_bf16(const void* dy, const void* x, float* dW, float* db, int64_t batch, int32_t cout, int32_t cin,
+                         int64_t voxels, void* stream);
+/* One launch converting four fp32 weights W_i (rows_i, cols_i), row-major, to bf16 in `out` (16-byte aligned): for i = 0..3
+ * in turn, W_i as stored with rows ld8(cols_i) elements apart, then W_i^T (cols_i, rows_i) with rows ld8(rows_i) apart,
+ * ld8(n) = n rounded up to a multiple of 8, the padding zero.  fz_bf16_staged_elems(rows, cols) is the number of bf16
+ * elements one matrix takes (both copies). */
+int fz_bf16_stage_weights_supported(int32_t rows, int32_t cols);
+int64_t fz_bf16_staged_elems(int32_t rows, int32_t cols);
+int fz_bf16_stage_weights(const float* w0, int32_t rows0, int32_t cols0, const float* w1, int32_t rows1, int32_t cols1,
+                          const float* w2, int32_t rows2, int32_t cols2, const float* w3, int32_t rows3, int32_t cols3, void* out,
+                          void* stream);
+/* fz_layernorm_cf_forward / fz_layernorm_cf_backward_add on bf16 x, y, dy, add, dx; gamma, beta, d(gamma), d(beta) fp32. */
+int fz_layernorm_cf_bf16_supported(int32_t channels, int64_t voxels);
+int fz_layernorm_cf_forward_bf16(const void* x, const float* gamma, const float* beta, void* y, int64_t batch, int32_t channels,
+                                 int64_t voxels, float eps, void* stream);
+int fz_layernorm_cf_backward_add_bf16(const void* x, const float* gamma, const void* dy, const void* add, void* dx, float* dgamma,
+                                      float* dbeta, int64_t batch, int32_t channels, int64_t voxels, float eps, void* stream);
+/* 1 if fz_swnmf_forward / _backward take bf16 volumes of this geometry and solver (g->dtype is ignored). */
+int fz_swnmf_bf16_supported(const fz_geom* g, const fz_solver* s, int32_t relu_input);
+
 /* (batch, channels, D, H, W) <-> (batch, channels*8, D/2*H/2*W/2) with rows ordered (c, kd, kh, kw): the view on which
  * the reference U-Net's kernel-2 stride-2 down-sampling convolution (factorizer/unet.py:53) and transposed up-sampling
  * convolution (unet.py:97-99) are channel maps.  to_depth != 0: full resolution -> patch rows; 0: the inverse.
