@@ -67,6 +67,13 @@ _SIGNATURES = {
     "fz_conv3d_stem_forward": (c_int, [c_void_p, c_void_p, c_void_p, c_void_p, c_int64, c_int32, c_int32, c_int32, c_int32, c_int32, c_void_p]),
     "fz_space_depth2_supported": (c_int, [c_int32, c_int32, c_int32]),
     "fz_space_depth2": (c_int, [c_void_p, c_void_p, c_int64, c_int32, c_int32, c_int32, c_int32, c_int32, c_void_p]),
+    "fz_space_depth2_bf16_supported": (c_int, [c_int32, c_int32, c_int32]),
+    "fz_space_depth2_bf16": (c_int, [c_void_p, c_void_p, c_int64, c_int32, c_int32, c_int32, c_int32, c_int32, c_void_p]),
+    "fz_conv3d_stem_forward_bf16": (c_int, [c_void_p, c_int32, c_void_p, c_void_p, c_void_p, c_int64, c_int32, c_int32, c_int32, c_int32,
+                                            c_int32, c_void_p]),
+    "fz_conv3d_stem_wgrad_bf16_supported": (c_int, [c_int32, c_int32, c_int32, c_int32, c_int32]),
+    "fz_conv3d_stem_wgrad_bf16": (c_int, [c_void_p, c_void_p, c_int32, c_void_p, c_void_p, c_int64, c_int32, c_int32, c_int32, c_int32,
+                                          c_int32, c_void_p]),
     "fz_layernorm_cf_supported": (c_int, [c_int32, c_int64]),
     "fz_layernorm_cf_forward": (c_int, [c_void_p, c_void_p, c_void_p, c_void_p, c_int64, c_int32, c_int64, c_float, c_void_p]),
     "fz_layernorm_cf_backward": (c_int, [c_void_p, c_void_p, c_void_p, c_void_p, c_void_p, c_void_p, c_int64, c_int32,
@@ -81,6 +88,7 @@ _SIGNATURES = {
     "fz_bf16_stage_weights_supported": (c_int, [c_int32, c_int32]),
     "fz_bf16_staged_elems": (c_int64, [c_int32, c_int32]),
     "fz_bf16_stage_weights": (c_int, [c_void_p, c_int32, c_int32] * 4 + [c_void_p, c_void_p]),
+    "fz_bf16_stage_weight": (c_int, [c_void_p, c_int32, c_int32, c_void_p, c_void_p]),
     "fz_layernorm_cf_bf16_supported": (c_int, [c_int32, c_int64]),
     "fz_layernorm_cf_forward_bf16": (c_int, [c_void_p, c_void_p, c_void_p, c_void_p, c_int64, c_int32, c_int64, c_float, c_void_p]),
     "fz_layernorm_cf_backward_add_bf16": (c_int, [c_void_p, c_void_p, c_void_p, c_void_p, c_void_p, c_void_p, c_void_p, c_int64,

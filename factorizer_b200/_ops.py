@@ -767,19 +767,20 @@ class SpaceDepth2(torch.autograd.Function):
 
     @staticmethod
     def _run(x, B, D, H, W, to_depth):
-        x = L.require_cuda_f32(x, "x")
+        x = L.require_cuda_f32(x, "x", allow_bf16=True)        # bf16: the scaffold's bf16 route (fz_space_depth2_bf16)
         if x.data_ptr() % 16:               # the kernel moves float4 words: the same permutation in torch
             if to_depth:
                 return x.view(B, -1, D // 2, 2, H // 2, 2, W // 2, 2).permute(0, 1, 3, 5, 7, 2, 4, 6).reshape(B, -1, (D // 2) * (H // 2) * (W // 2))
             return x.view(B, -1, 2, 2, 2, D // 2, H // 2, W // 2).permute(0, 1, 5, 2, 6, 3, 7, 4).reshape(B, -1, D, H, W)
         if to_depth:
             C = x.shape[1]
-            out = torch.empty(B, C * 8, (D // 2) * (H // 2) * (W // 2), device=x.device, dtype=torch.float32)
+            out = torch.empty(B, C * 8, (D // 2) * (H // 2) * (W // 2), device=x.device, dtype=x.dtype)
         else:
             C = x.shape[1] // 8
-            out = torch.empty(B, C, D, H, W, device=x.device, dtype=torch.float32)
+            out = torch.empty(B, C, D, H, W, device=x.device, dtype=x.dtype)
+        fn = L.lib().fz_space_depth2_bf16 if x.dtype == torch.bfloat16 else L.lib().fz_space_depth2
         with torch.cuda.device(x.device):
-            _call(L.lib().fz_space_depth2, L.ptr(x), L.ptr(out), B, C, D, H, W, 1 if to_depth else 0, L.stream_ptr(x.device))
+            _call(fn, L.ptr(x), L.ptr(out), B, C, D, H, W, 1 if to_depth else 0, L.stream_ptr(x.device))
         return out
 
     @staticmethod
@@ -787,6 +788,146 @@ class SpaceDepth2(torch.autograd.Function):
     def backward(ctx, g):
         D, H, W = ctx.full_shape
         return SpaceDepth2._run(g, g.shape[0], D, H, W, not ctx.to_depth), None, None
+
+
+# ---- the U-Net scaffold's layers on bf16 activations -----------------------------------------------------------------------------
+def bf16_library_faster(voxels: int, out_channels: int, linear: bool) -> bool:
+    """Shapes on which the library's bf16 kernels beat the bf16 route under autocast (forward + backward measured on a B200 at
+    a 1000 W power limit, bench_probes/bf16_scaffold_time.py): fewer than 16 outputs (the 3-channel head at 128^3: 0.19 ms in
+    cuDNN, 0.39 ms here, where a 64-output tile holds 3 outputs), and a Linear over fewer than 65536 voxels in all (the 16^3
+    and 32^3 decoder adapters: 3 GEMMs against a staging launch, 3 kernels and 2 memsets; 0.79x and 0.94x).  `voxels` counts
+    the whole batch."""
+    return out_channels < 16 or (linear and voxels < 65536)
+
+
+def bf16_layer_supported(x: torch.Tensor, voxels: int, in_channels: int, out_channels: int, linear: bool = False) -> bool:
+    """The bf16 route of Linear, of the kernel-2 stride-2 and kernel-1 patch convolutions, of the transposed kernel-2 stride-2
+    convolution and of the stem: a CUDA input under bf16 autocast, or a bf16 input without autocast (the FactorizerBlock
+    rule); `in_channels` input channels (a mismatch falls through to the stock module, which raises); `voxels`, those of the
+    channel map the layer runs per sample, a multiple of 8; a bf16 input contiguous and 16-byte aligned (an fp32 input under
+    autocast is converted into a fresh buffer).  Under autocast, the shapes bf16_library_faster names keep the library
+    route; a bf16 input without autocast has no other route.  fp16 autocast and fp32 without autocast keep their routes."""
+    if not (isinstance(x, torch.Tensor) and x.is_cuda and x.dtype in (torch.float32, torch.bfloat16) and x.dim() >= 3
+            and x.shape[1] == in_channels):
+        return False
+    autocast = torch.is_autocast_enabled("cuda")
+    if autocast:
+        if torch.get_autocast_dtype("cuda") != torch.bfloat16:
+            return False
+    elif x.dtype != torch.bfloat16:
+        return False
+    if x.dtype == torch.bfloat16 and not (x.is_contiguous() and x.data_ptr() % 16 == 0):
+        return False
+    if not (x.shape[0] > 0 and 0 < int(voxels) < 2 ** 31 and int(voxels) % 8 == 0):
+        return False
+    return not (autocast and bf16_library_faster(x.shape[0] * int(voxels), int(out_channels), linear))
+
+
+def as_bf16(x: torch.Tensor) -> torch.Tensor:
+    """x as a contiguous, 16-byte aligned bf16 tensor (itself when it is one)."""
+    x = x.to(torch.bfloat16, memory_format=torch.contiguous_format)
+    return x if x.data_ptr() % 16 == 0 else x.clone()
+
+
+def _stage_weight_bf16(w: torch.Tensor) -> torch.Tensor:
+    """One launch: the fp32 matrix w (R, C) as bf16, as stored and transposed (see _staged_views)."""
+    lib = L.lib()
+    buf = torch.empty(int(lib.fz_bf16_staged_elems(w.shape[0], w.shape[1])), device=w.device, dtype=torch.bfloat16)
+    _call(lib.fz_bf16_stage_weight, L.ptr(w), w.shape[0], w.shape[1], L.ptr(buf), L.stream_ptr(w.device))
+    return buf
+
+
+class LinearBf16Fn(_GradModeFunction):
+    """y = W x + b on bf16 (B, C_in, voxels) (fz_linear_forward_bf16): W = wmat, or wmat^T with `transposed` (the up-samplers'
+    (C_in, C_out * K) weight read as stored).  Parameters and their gradients stay fp32, the sums are fp32 and rounded to
+    bf16 once, after the bias.  One launch stages wmat in bf16 (as stored and transposed); the backward takes the other copy
+    for dx and fz_linear_wgrad_bf16 for dW and db.  Saves x and the staged weight."""
+
+    @staticmethod
+    def forward(ctx, x, wmat, bias, transposed: bool):
+        wmat = L.require_cuda_f32(wmat, "weight")
+        bias = None if bias is None else L.require_cuda_f32(bias, "bias")
+        R, C = wmat.shape
+        if x.dtype != torch.bfloat16 or x.shape[1] != (R if transposed else C):
+            raise ValueError(f"factorizer_b200: LinearBf16Fn takes bf16 x with {R if transposed else C} channels, got {x.dtype} "
+                             f"{tuple(x.shape)}")
+        with torch.cuda.device(x.device):
+            staged = _stage_weight_bf16(wmat)
+            w, wt = _staged_views(staged, [(R, C)])[0]
+            y = _channel_map_bf16(x, wt if transposed else w, C if transposed else R, bias)
+        if _GradModeFunction.wants_grad(ctx, 3):
+            ctx.save_for_backward(x, staged)
+            ctx.shape, ctx.transposed, ctx.has_bias = (R, C), bool(transposed), bias is not None
+        return y
+
+    @staticmethod
+    @once_differentiable
+    def backward(ctx, gy):
+        x, staged = ctx.saved_tensors
+        gy = as_bf16(gy)
+        w, wt = _staged_views(staged, [ctx.shape])[0]
+        gx = gw = gb = None
+        with torch.cuda.device(x.device):
+            if ctx.needs_input_grad[0]:
+                gx = _channel_map_bf16(gy, w if ctx.transposed else wt, x.shape[1], None)
+            if ctx.needs_input_grad[1] or (ctx.has_bias and ctx.needs_input_grad[2]):
+                gw, gb = _channel_map_wgrad_bf16(gy, x, ctx.has_bias)
+                if ctx.transposed:
+                    gw = gw.t()
+        return gx, gw, gb, None
+
+
+def stem_bf16_supported(x: torch.Tensor, weight: torch.Tensor) -> bool:
+    """StemConvBf16Fn: bf16_layer_supported, and a contiguous, 16-byte aligned x (fp32 or bf16, read as it is) of a 3x3x3
+    1..4 -> 32 channel convolution with W divisible by 8 (the caller checks stride 1, padding 1, dilation, groups)."""
+    if not (isinstance(x, torch.Tensor) and x.dim() == 5 and weight.dim() == 5 and tuple(weight.shape[2:]) == (3, 3, 3)
+            and weight.dtype == torch.float32 and weight.is_contiguous()):
+        return False
+    D, H, W = x.shape[2:]
+    lib = L.lib()
+    return (bf16_layer_supported(x, D * H * W, weight.shape[1], weight.shape[0]) and x.is_contiguous() and x.data_ptr() % 16 == 0
+            and bool(lib.fz_conv3d_stem_supported(x.shape[1], weight.shape[0], D, H, W))
+            and bool(lib.fz_conv3d_stem_wgrad_bf16_supported(x.shape[1], weight.shape[0], D, H, W)))
+
+
+class StemConvBf16Fn(_GradModeFunction):
+    """The 3x3x3 stem with a bf16 output: x is read in the dtype it arrives in (the model's fp32 input is not converted), the
+    sums are fp32 and rounded to bf16 once, after the bias (fz_conv3d_stem_forward_bf16).  The weight gradient is
+    fz_conv3d_stem_wgrad_bf16, without an unfolded copy of x; dx, which the Swin Factorizer never needs, is the library's."""
+
+    @staticmethod
+    def forward(ctx, x, weight, bias):
+        B, cin, D, H, W = x.shape
+        cout = weight.shape[0]
+        b = None if bias is None else L.require_cuda_f32(bias.detach(), "bias")
+        y = torch.empty(B, cout, D, H, W, device=x.device, dtype=torch.bfloat16)
+        dt = L.FZ_DTYPE_BF16 if x.dtype == torch.bfloat16 else L.FZ_DTYPE_F32
+        with torch.cuda.device(x.device):
+            _call(L.lib().fz_conv3d_stem_forward_bf16, L.ptr(x), dt, L.ptr(weight.detach()), L.ptr(b), L.ptr(y), B, cin, cout, D, H, W,
+                  L.stream_ptr(x.device))
+        if _GradModeFunction.wants_grad(ctx):
+            ctx.save_for_backward(x, weight)
+            ctx.has_bias = bias is not None
+        return y
+
+    @staticmethod
+    @once_differentiable
+    def backward(ctx, gy):
+        x, weight = ctx.saved_tensors
+        gy = as_bf16(gy)
+        B, cin, D, H, W = x.shape
+        cout = weight.shape[0]
+        gx = gw = gb = None
+        if ctx.needs_input_grad[0]:
+            gx = torch.nn.grad.conv3d_input(x.shape, weight, gy.float(), padding=1).to(x.dtype)
+        if ctx.needs_input_grad[1] or (ctx.has_bias and ctx.needs_input_grad[2]):
+            gw = torch.empty_like(weight)
+            gb = torch.empty(cout, device=x.device, dtype=torch.float32) if ctx.has_bias else None
+            dt = L.FZ_DTYPE_BF16 if x.dtype == torch.bfloat16 else L.FZ_DTYPE_F32
+            with torch.cuda.device(x.device):
+                _call(L.lib().fz_conv3d_stem_wgrad_bf16, L.ptr(gy), L.ptr(x), dt, L.ptr(gw), L.ptr(gb), B, cin, cout, D, H, W,
+                      L.stream_ptr(x.device))
+        return gx, gw, gb
 
 
 def linear_wgrad_supported(x: torch.Tensor, out_channels: int, min_voxels: int = 4096, rows: Optional[int] = None,
@@ -857,8 +998,8 @@ def stem_conv_supported(x: torch.Tensor, weight: torch.Tensor, padding) -> bool:
     """3x3x3, stride 1, padding 1, 1..4 -> 32 channels on a contiguous CUDA fp32 volume: csrc/fz_linear.cu has a direct
     kernel for the forward (the caller checks stride / dilation / groups)."""
     return (isinstance(x, torch.Tensor) and x.is_cuda and x.dtype == torch.float32 and x.dim() == 5 and x.is_contiguous()
-            and x.data_ptr() % 16 == 0
-            and not torch.is_autocast_enabled() and weight.dim() == 5 and tuple(weight.shape[2:]) == (3, 3, 3) and tuple(padding) == (1, 1, 1)
+            and x.data_ptr() % 16 == 0 and weight.dim() == 5 and x.shape[1] == weight.shape[1]
+            and not torch.is_autocast_enabled() and tuple(weight.shape[2:]) == (3, 3, 3) and tuple(padding) == (1, 1, 1)
             and weight.is_contiguous() and weight.dtype == torch.float32
             and bool(L.lib().fz_conv3d_stem_supported(x.shape[1], weight.shape[0], *x.shape[2:])))
 

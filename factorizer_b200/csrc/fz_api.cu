@@ -32,6 +32,10 @@ int encode_tiled_map(CUtensorMap* m, const char* what, CUtensorMapDataType type,
             enc = reinterpret_cast<EncodeTiledFn>(p);
     }
     if (!enc) return fail(FZ_ERR_CUDA, "cuTensorMapEncodeTiled entry point not available");
+    // the driver call needs the device's context current on the calling thread; a thread that has made no runtime call yet
+    // (autograd's backward thread, when a tensor map is its first CUDA work) has none
+    int dev = 0;
+    if (cudaGetDevice(&dev) != cudaSuccess || cudaSetDevice(dev) != cudaSuccess) return fail(FZ_ERR_CUDA, "no usable CUDA device");
     const cuuint32_t es[5] = {1, 1, 1, 1, 1};
     const CUresult r = enc(m, type, rank, const_cast<void*>(ptr), dims, strides, box, es, CU_TENSOR_MAP_INTERLEAVE_NONE, swizzle,
                            CU_TENSOR_MAP_L2_PROMOTION_L2_128B, CU_TENSOR_MAP_FLOAT_OOB_FILL_NONE);

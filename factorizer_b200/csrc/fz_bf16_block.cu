@@ -1,5 +1,6 @@
 // The bf16 FactorizerBlock's channel maps on the tensor cores (tcgen05 kind::f16: bf16 operands, fp32 accumulator in TMEM),
-// and the launch that stages its weights in bf16.
+// and the launch that stages its weights in bf16.  The U-Net scaffold's bf16 layers use the same channel maps and staging,
+// and the stem's weight gradient below.
 //
 // Channel map  y[b][o][v] = sum_c W[o][c] x[b][c][v] (+ bias[o]), with the five FZ_EPILOGUE_* epilogues of linear_fwd_tc
 // (fz_linear_tc.cu) -- the same persistent walk over (voxel tile, output tile) items, one MMA per 16 channels and no
@@ -364,6 +365,148 @@ linear_wgrad_bf16_tc(const __grid_constant__ CUtensorMap map_dy, const __grid_co
     if (warp == 1) tmem_dealloc<256>(tmem);
 }
 
+// ---- stem weight gradient ---------------------------------------------------------------------------------------------------
+// dW[o][r] = sum over voxels of dy[o][v] col[r][v], with col[r = (c, kd, kh, kw)][v] = x[c][v + (kd-1, kh-1, kw-1)] (zero
+// outside the volume): the 27 cin im2col rows of a 64-voxel tile are built in shared memory, never in global memory, in the
+// K-major SWIZZLE_128B layout TMA writes (row r = 128 bytes, its 16-byte chunk j at (j ^ (r % 8))); row 27 cin is all ones (its
+// sums are db), the rest zero.  D[128 rows x 32 outputs] += col[128 x 64] dy[32 x 64]^T, four MMAs per stage; dy comes by TMA.
+// Warp 0 = TMA, warp 1 = MMA issue, warps 2-9 = im2col builders, then the epilogue (one atomic per element and CTA).  The chain
+// is capped at 32 stages per CTA, as in linear_wgrad_bf16_tc.
+constexpr int kSV = 64;                                 // voxels per stage
+constexpr int kSStages = 3;
+constexpr int kSThreads = 320;
+constexpr int kSBuilders = kSThreads - 64;
+constexpr uint32_t kSA = 128 * 128, kSB = 32 * 128, kSStage = kSA + kSB;     // im2col tile 16 KiB | dy tile 4 KiB
+constexpr uint32_t sBarFull = kSStages * kSStage, sBarEmpty = sBarFull + 8 * kSStages, sBarDone = sBarEmpty + 8 * kSStages,
+                   sTmemSlot = sBarDone + 8, kSSmem = sTmemSlot + 8;
+
+__device__ __forceinline__ float ldx(const float* p) { return __ldg(p); }
+__device__ __forceinline__ float ldx(const bf16* p) { return ldbf(p); }
+__device__ __forceinline__ uint32_t pack_bf16(float a, float b) {
+    const __nv_bfloat162 h = __floats2bfloat162_rn(a, b);
+    return *reinterpret_cast<const uint32_t*>(&h);
+}
+
+template <typename TX>
+__global__ void __launch_bounds__(kSThreads, 1)
+stem_wgrad_bf16_tc(const __grid_constant__ CUtensorMap map_dy, const TX* __restrict__ x, float* __restrict__ dW, float* __restrict__ db,
+                   int cin, int D, int H, int W, int tiles_per_sample, long long total_tiles) {
+    extern __shared__ __align__(1024) unsigned char smem[];
+    const uint32_t sbase = smem_u32(smem);
+    const int tid = threadIdx.x, lane = tid & 31;
+    const int warp = (int)uniform_u32((uint32_t)(tid >> 5));
+    const int R = 27 * cin;
+    const long long vox = (long long)D * H * W;
+    const long long my_tiles = blockIdx.x < total_tiles ? (total_tiles - blockIdx.x + gridDim.x - 1) / gridDim.x : 0;
+
+    if (tid == 0) {
+        for (int s = 0; s < kSStages; ++s) {
+            mbar_init(sbase + sBarFull + 8 * s, 1 + kSBuilders / 32);
+            mbar_init(sbase + sBarEmpty + 8 * s, 1);
+        }
+        mbar_init(sbase + sBarDone, 1);
+        fence_mbarrier_init();
+    }
+    // the constant rows of every stage: R = ones, R+1 .. 127 = zeros (rows of equal values: no swizzle to mind)
+    for (int i = tid; i < kSStages * (128 - R) * 64; i += kSThreads) {
+        const int s = i / ((128 - R) * 64), e = i % ((128 - R) * 64);
+        reinterpret_cast<bf16*>(smem + s * kSStage)[R * 64 + e] = __float2bfloat16_rn(e < 64 ? 1.f : 0.f);
+    }
+    if (warp == 1) {
+        tmem_alloc<32>(sbase + sTmemSlot);
+        tmem_relinquish_alloc_permit();
+    }
+    fence_proxy_async_smem();
+    tc_fence_before();
+    __syncthreads();
+    tc_fence_after();
+    const uint32_t tmem = uniform_u32(*reinterpret_cast<const uint32_t*>(smem + sTmemSlot));
+
+    if (warp == 0) {
+        // ---- TMA producer: the dy tile (32 outputs x 64 voxels) ----
+        if (elect_one()) {
+            for (long long it = 0; it < my_tiles; ++it) {
+                const long long tile = blockIdx.x + it * gridDim.x;
+                const int nb = (int)(tile / tiles_per_sample), nt = (int)(tile - (long long)nb * tiles_per_sample);
+                const int s = (int)(it % kSStages);
+                const uint32_t round = (uint32_t)(it / kSStages);
+                if (round > 0) mbar_wait(sbase + sBarEmpty + 8 * s, (round - 1) & 1);
+                const uint32_t full = sbase + sBarFull + 8 * s;
+                mbar_arrive_expect_tx(full, kSB);
+                tma_load_3d(sbase + s * kSStage + kSA, &map_dy, full, nt * kSV, 0, nb);
+            }
+        }
+        __syncwarp();
+    } else if (warp == 1) {
+        // ---- MMA issue ----
+        const uint32_t idesc = make_idesc_bf16(128, 32, false, false);
+        for (long long it = 0; it < my_tiles; ++it) {
+            const int s = (int)(it % kSStages);
+            const uint32_t round = (uint32_t)(it / kSStages);
+            mbar_wait(sbase + sBarFull + 8 * s, round & 1);
+            tc_fence_after();
+            if (elect_one()) {
+                const uint64_t ad = make_desc(sbase + s * kSStage, 16, 1024, 2);
+                const uint64_t bd = make_desc(sbase + s * kSStage + kSA, 16, 1024, 2);
+#pragma unroll
+                for (int k = 0; k < kSV / 16; ++k) mma_bf16(tmem, desc_at(ad, k * 32), desc_at(bd, k * 32), idesc, it > 0 || k > 0);
+                commit(sbase + sBarEmpty + 8 * s);
+                if (it + 1 == my_tiles) commit(sbase + sBarDone);
+            }
+            __syncwarp();
+        }
+    } else {
+        // ---- im2col builders: a thread fills 16-byte chunks (8 voxels along W, W % 8 == 0) of rows r, r + 32, ... ----
+        const int b = tid - 64, j = b & 7, r0 = b >> 3;
+        for (long long it = 0; it < my_tiles; ++it) {
+            const long long tile = blockIdx.x + it * gridDim.x;
+            const long long nb = tile / tiles_per_sample;
+            const long long v = (tile - nb * tiles_per_sample) * kSV + 8 * j;
+            const int w = (int)(v % W), h = (int)((v / W) % H), d = (int)(v / ((long long)W * H));
+            const bool live = v < vox;
+            const TX* xb = x + nb * cin * vox;
+            const int s = (int)(it % kSStages);
+            const uint32_t round = (uint32_t)(it / kSStages);
+            if (round > 0) mbar_wait(sbase + sBarEmpty + 8 * s, (round - 1) & 1);
+            unsigned char* tileA = smem + s * kSStage;
+            for (int r = r0; r < R; r += kSBuilders / 8) {
+                const int c = r / 27, t = r - 27 * c, kd = t / 9, kh = (t / 3) % 3, kw = t % 3;
+                const int dd = d + kd - 1, hh = h + kh - 1, w0 = w + kw - 1;
+                const bool rowok = live && dd >= 0 && dd < D && hh >= 0 && hh < H;
+                const TX* src = xb + c * vox + ((long long)dd * H + hh) * W + w0;
+                float e[8];
+#pragma unroll
+                for (int i = 0; i < 8; ++i) e[i] = (rowok && w0 + i >= 0 && w0 + i < W) ? ldx(src + i) : 0.f;
+                const uint4 q = make_uint4(pack_bf16(e[0], e[1]), pack_bf16(e[2], e[3]), pack_bf16(e[4], e[5]), pack_bf16(e[6], e[7]));
+                *reinterpret_cast<uint4*>(tileA + r * 128 + ((j ^ (r & 7)) << 4)) = q;
+            }
+            fence_proxy_async_smem();                          // generic-proxy writes -> the tensor core's reads
+            __syncwarp();
+            if (lane == 0) mbar_arrive(sbase + sBarFull + 8 * s);
+        }
+    }
+    // ---- epilogue: TMEM lane r = im2col row r, column o = output channel ----
+    if (warp >= 2 && my_tiles > 0) {
+        mbar_wait(sbase + sBarDone, 0);
+        tc_fence_after();
+        const int q = warp & 3, half = (warp - 2) >> 2;       // TMEM lane quarter; columns [16 half, 16 half + 16)
+        const int r = q * 32 + lane;
+        uint32_t e[16];
+        tmem_ld16_nowait(tmem + ((uint32_t)(q * 32) << 16) + 16 * half, e);
+        tmem_ld_wait();
+        if (r < R) {
+#pragma unroll
+            for (int i = 0; i < 16; ++i) atomicAdd(dW + (16 * half + i) * R + r, __uint_as_float(e[i]));
+        } else if (r == R && db) {
+#pragma unroll
+            for (int i = 0; i < 16; ++i) atomicAdd(db + 16 * half + i, __uint_as_float(e[i]));
+        }
+    }
+    tc_fence_before();
+    __syncthreads();
+    if (warp == 1) tmem_dealloc<32>(tmem);
+}
+
 // ---- weight staging ---------------------------------------------------------------------------------------------------------
 // bf16 rows are padded to whole 16-byte groups: a TMA row stride must be a multiple of 16 bytes
 __host__ __device__ inline long long ld8(long long n) { return (n + 7) & ~7LL; }
@@ -395,6 +538,36 @@ __global__ void __launch_bounds__(256) stage_weights_bf16(StageArgs a, bf16* __r
 }
 
 bool aligned16(const void* p) { return (reinterpret_cast<uintptr_t>(p) & 15) == 0; }
+
+int stage_weights_launch(int n, const float* const* w, const int* r, const int* c, void* out, void* stream) {
+    tls().launches = 0;
+    StageArgs a;
+    long long off = 0;
+    for (int m = 0; m < 4; ++m) {
+        if (m >= n) {                                           // absent weights: empty ranges at the end
+            a.w[m] = nullptr;
+            a.rows[m] = a.cols[m] = 1;
+            a.off[2 * m] = a.off[2 * m + 1] = off;
+            continue;
+        }
+        if (!w[m] || !fz_bf16_stage_weights_supported(r[m], c[m])) return fail(FZ_ERR_INVALID, "weight %d: null or bad shape (%d, %d)", m, r[m], c[m]);
+        a.w[m] = w[m];
+        a.rows[m] = r[m];
+        a.cols[m] = c[m];
+        a.off[2 * m] = off;
+        off += (long long)r[m] * ld8(c[m]);
+        a.off[2 * m + 1] = off;
+        off += (long long)c[m] * ld8(r[m]);
+    }
+    a.off[8] = off;
+    if (!out) return fail(FZ_ERR_INVALID, "null buffer");
+    if (!aligned16(out)) return fail(FZ_ERR_UNSUPPORTED, "staged weights must be 16-byte aligned");
+    long long blocks = (off + 255) / 256;
+    if (blocks > 4LL * num_sms()) blocks = 4LL * num_sms();
+    stage_weights_bf16<<<(unsigned)blocks, 256, 0, (cudaStream_t)stream>>>(a, static_cast<bf16*>(out));
+    FZ_LAUNCH_CHECK();
+    return FZ_OK;
+}
 
 }  // namespace
 }  // namespace fz
@@ -498,27 +671,52 @@ int64_t fz_bf16_staged_elems(int32_t rows, int32_t cols) {
 
 int fz_bf16_stage_weights(const float* w0, int32_t r0, int32_t c0, const float* w1, int32_t r1, int32_t c1, const float* w2, int32_t r2,
                           int32_t c2, const float* w3, int32_t r3, int32_t c3, void* out, void* stream) {
-    tls().launches = 0;
-    StageArgs a;
     const float* w[4] = {w0, w1, w2, w3};
     const int r[4] = {r0, r1, r2, r3}, c[4] = {c0, c1, c2, c3};
-    long long off = 0;
-    for (int m = 0; m < 4; ++m) {
-        if (!w[m] || !fz_bf16_stage_weights_supported(r[m], c[m])) return fail(FZ_ERR_INVALID, "weight %d: null or bad shape (%d, %d)", m, r[m], c[m]);
-        a.w[m] = w[m];
-        a.rows[m] = r[m];
-        a.cols[m] = c[m];
-        a.off[2 * m] = off;
-        off += (long long)r[m] * ld8(c[m]);
-        a.off[2 * m + 1] = off;
-        off += (long long)c[m] * ld8(r[m]);
+    return stage_weights_launch(4, w, r, c, out, stream);
+}
+
+int fz_bf16_stage_weight(const float* w, int32_t rows, int32_t cols, void* out, void* stream) {
+    return stage_weights_launch(1, &w, &rows, &cols, out, stream);
+}
+
+int fz_conv3d_stem_wgrad_bf16_supported(int32_t cin, int32_t cout, int32_t D, int32_t H, int32_t W) {
+    return cin >= 1 && cin <= 4 && cout == 32 && D > 0 && H > 0 && W > 0 && W % 8 == 0 && (long long)D * H * W < (1LL << 31);
+}
+
+int fz_conv3d_stem_wgrad_bf16(const void* dy, const void* x, int32_t x_dtype, float* dW, float* db, int64_t batch, int32_t cin, int32_t cout,
+                              int32_t D, int32_t H, int32_t W, void* stream) {
+    tls().launches = 0;
+    cudaStream_t st = (cudaStream_t)stream;
+    if (!dW) return fail(FZ_ERR_INVALID, "null buffer");
+    if (batch < 0 || batch >= (1LL << 31)) return fail(FZ_ERR_INVALID, "stem weight gradient: bad batch");
+    if (x_dtype != FZ_DTYPE_F32 && x_dtype != FZ_DTYPE_BF16) return fail(FZ_ERR_INVALID, "stem weight gradient: unknown x dtype %d", x_dtype);
+    if (!fz_conv3d_stem_wgrad_bf16_supported(cin, cout, D, H, W))
+        return fail(FZ_ERR_UNSUPPORTED, "stem weight gradient handles 1..4 -> 32 channels, W divisible by 8 (got %d -> %d, W = %d)", cin, cout, W);
+    FZ_CUDA_CHECK(cudaMemsetAsync(dW, 0, sizeof(float) * (size_t)cout * cin * 27, st));
+    if (db) FZ_CUDA_CHECK(cudaMemsetAsync(db, 0, sizeof(float) * (size_t)cout, st));
+    if (batch == 0) return FZ_OK;
+    if (!dy || !x) return fail(FZ_ERR_INVALID, "null buffer");
+    if (!aligned16(dy) || !aligned16(x)) return fail(FZ_ERR_UNSUPPORTED, "stem weight gradient: dy and x must be 16-byte aligned");
+    const long long vox = (long long)D * H * W;
+    CUtensorMap map_dy;
+    if (int e = make_map_rows16(&map_dy, "dy (bf16)", static_cast<const bf16*>(dy), cout, vox, vox, 32, 3, batch)) return e;
+    const int tps = (int)((vox + kSV - 1) / kSV);
+    const long long tiles = batch * tps;
+    long long gx = 2LL * num_sms();
+    constexpr long long kMaxChain = 32;                         // stages per CTA, as fz_linear_wgrad_bf16
+    if (gx * kMaxChain < tiles) gx = (tiles + kMaxChain - 1) / kMaxChain;
+    if (gx > tiles) gx = tiles;
+    if (gx >= (1LL << 31)) return fail(FZ_ERR_UNSUPPORTED, "stem weight gradient: too many voxels");
+    if (x_dtype == FZ_DTYPE_F32) {
+        static SmemConfig cfg;
+        FZ_CUDA_CHECK(cfg.ensure(stem_wgrad_bf16_tc<float>, kSSmem));
+        stem_wgrad_bf16_tc<float><<<(unsigned)gx, kSThreads, kSSmem, st>>>(map_dy, static_cast<const float*>(x), dW, db, cin, D, H, W, tps, tiles);
+    } else {
+        static SmemConfig cfg;
+        FZ_CUDA_CHECK(cfg.ensure(stem_wgrad_bf16_tc<bf16>, kSSmem));
+        stem_wgrad_bf16_tc<bf16><<<(unsigned)gx, kSThreads, kSSmem, st>>>(map_dy, static_cast<const bf16*>(x), dW, db, cin, D, H, W, tps, tiles);
     }
-    a.off[8] = off;
-    if (!out) return fail(FZ_ERR_INVALID, "null buffer");
-    if (!aligned16(out)) return fail(FZ_ERR_UNSUPPORTED, "staged weights must be 16-byte aligned");
-    long long blocks = (off + 255) / 256;
-    if (blocks > 4LL * num_sms()) blocks = 4LL * num_sms();
-    stage_weights_bf16<<<(unsigned)blocks, 256, 0, (cudaStream_t)stream>>>(a, static_cast<bf16*>(out));
     FZ_LAUNCH_CHECK();
     return FZ_OK;
 }

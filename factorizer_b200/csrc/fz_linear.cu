@@ -4,7 +4,8 @@
 //
 //   fz_linear_wgrad          dW[o][i] = sum_{b,v} dy[b][o][v] x[b][i][v],  db[o] = sum_{b,v} dy[b][o][v]
 //   fz_space_depth2          (B,C,D,H,W) <-> (B,8C,DHW/8): the view on which a 2x2x2 stride-2 (transposed) convolution is a channel map
-//   fz_conv3d_stem_forward   3x3x3, padding 1, 1..4 -> 32 channels
+//                            (fz_space_depth2_bf16: the same on bf16)
+//   fz_conv3d_stem_forward   3x3x3, padding 1, 1..4 -> 32 channels (fz_conv3d_stem_forward_bf16: fp32 or bf16 x, bf16 y)
 //
 // Weight gradient: the Swin Factorizer's wider stages give it a 64..1024 x 64..512 result over 512..262144 voxels, a shape
 // library SGEMMs handle badly (sgemm_largek: 340 us for 64 x 64 x 262144, 10 % of the FP32 pipe; cuDNN's fp32 wgrad of the
@@ -12,11 +13,15 @@
 // 256 voxels of its 32 + 32 rows in shared memory, keeps the partial sums in registers (a warp takes every 4th float4 column,
 // a lane an 8 x 4 sub-block read with broadcast LDS.128) and adds them to dW once at the end.  linear_wgrad64 (further down):
 // 64 x 64 or 32 x 128 blocks, cp.async double buffering, 8 x 8 register tiles.  FP32 pipe, exact fp32 products.
+#include <cuda_bf16.h>
+
 #include "fz_device.cuh"
 #include "fz_internal.cuh"
 
 namespace fz {
 namespace {
+
+typedef __nv_bfloat16 bf16;
 
 constexpr int kWT = 128;            // threads
 constexpr int kWV = 256;            // voxels per tile
@@ -229,10 +234,27 @@ __global__ void __launch_bounds__(kW2T, 1) linear_wgrad64(const float* __restric
 // (B, C, D, H, W) <-> (B, C*8, D/2 * H/2 * W/2), rows ordered (c, kd, kh, kw): the view on which a kernel-2 stride-2
 // convolution (or its transpose) is a channel map.  A thread moves one float4 of the full-resolution tensor = two
 // float2 of the patch rows kw = 0 and kw = 1, so both sides are coalesced (torch's strided permute copy gathers 4-byte
-// elements at stride 2).
-template <bool TO_DEPTH>
-__global__ void __launch_bounds__(256) space_depth2(const float* __restrict__ in, float* __restrict__ out, long long total4, int C, int D,
+// elements at stride 2).  On bf16 the same thread moves 8 bytes and two 4-byte pairs.
+template <typename T> struct Quad;          // 4 consecutive elements along W, split into the pairs (0, 2) and (1, 3)
+template <> struct Quad<float> {
+    typedef float4 V4;
+    typedef float2 V2;
+    static __device__ __forceinline__ V2 even(V4 v) { return make_float2(v.x, v.z); }
+    static __device__ __forceinline__ V2 odd(V4 v) { return make_float2(v.y, v.w); }
+    static __device__ __forceinline__ V4 join(V2 a, V2 b) { return make_float4(a.x, b.x, a.y, b.y); }
+};
+template <> struct Quad<bf16> {
+    typedef uint2 V4;                       // (e0 | e1 << 16, e2 | e3 << 16)
+    typedef unsigned int V2;
+    static __device__ __forceinline__ V2 even(V4 v) { return __byte_perm(v.x, v.y, 0x5410); }
+    static __device__ __forceinline__ V2 odd(V4 v) { return __byte_perm(v.x, v.y, 0x7632); }
+    static __device__ __forceinline__ V4 join(V2 a, V2 b) { return make_uint2(__byte_perm(a, b, 0x5410), __byte_perm(a, b, 0x7632)); }
+};
+
+template <typename T, bool TO_DEPTH>
+__global__ void __launch_bounds__(256) space_depth2(const T* __restrict__ in, T* __restrict__ out, long long total4, int C, int D,
                                                     int H, int W4) {
+    typedef Quad<T> Q;
     const int Hh = H >> 1, Wh = 2 * W4;                         // half-resolution height / width
     const long long Vh = (long long)(D >> 1) * Hh * Wh;
     for (long long q = (long long)blockIdx.x * blockDim.x + threadIdx.x; q < total4; q += (long long)gridDim.x * blockDim.x) {
@@ -243,12 +265,13 @@ __global__ void __launch_bounds__(256) space_depth2(const float* __restrict__ in
         const long long row = t * 8 + (d & 1) * 4 + (h & 1) * 2;
         const long long off = row * Vh + ((long long)(d >> 1) * Hh + (h >> 1)) * Wh + 2 * j;
         if (TO_DEPTH) {
-            const float4 v = __ldcs(reinterpret_cast<const float4*>(in) + q);
-            *reinterpret_cast<float2*>(out + off) = make_float2(v.x, v.z);
-            *reinterpret_cast<float2*>(out + off + Vh) = make_float2(v.y, v.w);
+            const typename Q::V4 v = __ldcs(reinterpret_cast<const typename Q::V4*>(in) + q);
+            *reinterpret_cast<typename Q::V2*>(out + off) = Q::even(v);
+            *reinterpret_cast<typename Q::V2*>(out + off + Vh) = Q::odd(v);
         } else {
-            const float2 a = __ldcs(reinterpret_cast<const float2*>(in + off)), b = __ldcs(reinterpret_cast<const float2*>(in + off + Vh));
-            reinterpret_cast<float4*>(out)[q] = make_float4(a.x, b.x, a.y, b.y);
+            const typename Q::V2 a = __ldcs(reinterpret_cast<const typename Q::V2*>(in + off)),
+                                 b = __ldcs(reinterpret_cast<const typename Q::V2*>(in + off + Vh));
+            reinterpret_cast<typename Q::V4*>(out)[q] = Q::join(a, b);
         }
     }
 }
@@ -258,10 +281,25 @@ __global__ void __launch_bounds__(256) space_depth2(const float* __restrict__ in
 // (the Swin Factorizer's stem, reference factorizer/factorizer.py:139-140: 4 -> 32 channels at full resolution; the
 // library's fp32 implicit-GEMM kernel takes 0.98 ms at 128^3 for 7.2 GFMA).  A thread owns 4 consecutive voxels along W
 // and all 32 outputs (64 float2 accumulators); per input row it loads one float4 and its two neighbours, per tap it
-// reads the 32 weights as 8 broadcast LDS.128 and issues 64 FFMA2 (weight broadcast x voxel pair).
-template <int CIN>
-__global__ void __launch_bounds__(128, 2) conv3_stem_fwd(const float* __restrict__ x, const float* __restrict__ wgt, const float* __restrict__ bias,
-                                                         float* __restrict__ y, int D, int H, int W, long long total4) {
+// reads the 32 weights as 8 broadcast LDS.128 and issues 64 FFMA2 (weight broadcast x voxel pair).  x (TI) and y (TO) are
+// fp32 or bf16; weights, bias and sums are fp32, and a bf16 y is the one rounding of the sum.
+__device__ __forceinline__ float4 ld4(const float* p) { return __ldg(reinterpret_cast<const float4*>(p)); }
+__device__ __forceinline__ float4 ld4(const bf16* p) {
+    const uint2 u = __ldg(reinterpret_cast<const uint2*>(p));
+    return make_float4(__uint_as_float(u.x << 16), __uint_as_float(u.x & 0xffff0000u), __uint_as_float(u.y << 16),
+                       __uint_as_float(u.y & 0xffff0000u));
+}
+__device__ __forceinline__ float ld1(const float* p) { return __ldg(p); }
+__device__ __forceinline__ float ld1(const bf16* p) { return __bfloat162float(__ldg(p)); }
+__device__ __forceinline__ void st4(float* p, float4 v) { *reinterpret_cast<float4*>(p) = v; }
+__device__ __forceinline__ void st4(bf16* p, float4 v) {
+    const __nv_bfloat162 a = __floats2bfloat162_rn(v.x, v.y), b = __floats2bfloat162_rn(v.z, v.w);
+    *reinterpret_cast<uint2*>(p) = make_uint2(*reinterpret_cast<const unsigned int*>(&a), *reinterpret_cast<const unsigned int*>(&b));
+}
+
+template <int CIN, typename TI, typename TO>
+__global__ void __launch_bounds__(128, 2) conv3_stem_fwd(const TI* __restrict__ x, const float* __restrict__ wgt, const float* __restrict__ bias,
+                                                         TO* __restrict__ y, int D, int H, int W, long long total4) {
     constexpr int CO = 32;
     __shared__ __align__(16) float ws[CIN * 27 * CO];          // [(ci, kd, kh, kw)][o]
     __shared__ float bs[CO];
@@ -282,7 +320,7 @@ __global__ void __launch_bounds__(128, 2) conv3_stem_fwd(const float* __restrict
         float2 acc[CO][2];
 #pragma unroll
         for (int o = 0; o < CO; ++o) acc[o][0] = acc[o][1] = make_float2(bs[o], bs[o]);
-        const float* xb = x + t * CIN * vox;
+        const TI* xb = x + t * CIN * vox;
         // input row r = (ci, kd, kh): float4 of the thread's 4 voxels and the two neighbours; rows outside the volume are zero.
         // The next row is fetched before the current one is used (the loop is not unrolled: 192 FFMA2 per row).
         auto fetch = [&](int r, float4& c, float& lft, float& rgt) {
@@ -292,10 +330,10 @@ __global__ void __launch_bounds__(128, 2) conv3_stem_fwd(const float* __restrict
                 c = make_float4(0.f, 0.f, 0.f, 0.f); lft = rgt = 0.f;
                 return;
             }
-            const float* row = xb + ci * vox + ((long long)dd * H + hh) * W + w0;
-            c = __ldg(reinterpret_cast<const float4*>(row));
-            lft = w0 > 0 ? __ldg(row - 1) : 0.f;
-            rgt = w0 + 4 < W ? __ldg(row + 4) : 0.f;
+            const TI* row = xb + ci * vox + ((long long)dd * H + hh) * W + w0;
+            c = ld4(row);
+            lft = w0 > 0 ? ld1(row - 1) : 0.f;
+            rgt = w0 + 4 < W ? ld1(row + 4) : 0.f;
         };
         float4 c, cn;
         float lft, rgt, lftn, rgtn;
@@ -321,15 +359,62 @@ __global__ void __launch_bounds__(128, 2) conv3_stem_fwd(const float* __restrict
                 }
             c = cn; lft = lftn; rgt = rgtn;
         }
-        float* yo = y + t * CO * vox + ((long long)d * H + h) * W + w0;
+        TO* yo = y + t * CO * vox + ((long long)d * H + h) * W + w0;
 #pragma unroll
-        for (int o = 0; o < CO; ++o)
-            *reinterpret_cast<float4*>(yo + o * vox) = make_float4(acc[o][0].x, acc[o][0].y, acc[o][1].x, acc[o][1].y);
+        for (int o = 0; o < CO; ++o) st4(yo + o * vox, make_float4(acc[o][0].x, acc[o][0].y, acc[o][1].x, acc[o][1].y));
     }
 }
 
 // the kernels above move float4 (and cp.async 16-byte) words of the caller's buffers
 bool unaligned16(const void* p) { return (reinterpret_cast<uintptr_t>(p) & 15) != 0; }
+
+template <typename T>
+int space_depth2_launch(const void* in, void* out, int64_t batch, int32_t channels, int32_t D, int32_t H, int32_t W, int32_t to_depth,
+                        void* stream) {
+    if (batch < 0 || channels <= 0) return fail(FZ_ERR_INVALID, "space/depth: bad sizes");
+    if (!fz_space_depth2_supported(D, H, W))
+        return fail(FZ_ERR_UNSUPPORTED, "space/depth kernel needs even D, H and W divisible by 4 (got %d x %d x %d)", D, H, W);
+    if (batch == 0) return FZ_OK;
+    if (!in || !out) return fail(FZ_ERR_INVALID, "space/depth: null buffer");
+    if (unaligned16(in) || unaligned16(out)) return fail(FZ_ERR_UNSUPPORTED, "space/depth kernel needs 16-byte aligned buffers");
+    const long long total4 = (long long)batch * channels * D * H * (W / 4);
+    const int sms = num_sms();
+    long long blocks = (total4 + 255) / 256;
+    if (blocks > 16LL * sms) blocks = 16LL * sms;
+    cudaStream_t st = (cudaStream_t)stream;
+    const T* i = static_cast<const T*>(in);
+    T* o = static_cast<T*>(out);
+    if (to_depth) space_depth2<T, true><<<(unsigned)blocks, 256, 0, st>>>(i, o, total4, channels, D, H, W / 4);
+    else space_depth2<T, false><<<(unsigned)blocks, 256, 0, st>>>(i, o, total4, channels, D, H, W / 4);
+    FZ_LAUNCH_CHECK();
+    return FZ_OK;
+}
+
+template <typename TI, typename TO>
+int stem_forward_launch(const void* x, const float* weight, const float* bias, void* y, int64_t batch, int32_t cin, int32_t cout, int32_t D,
+                        int32_t H, int32_t W, void* stream) {
+    if (batch < 0) return fail(FZ_ERR_INVALID, "stem convolution: bad batch");
+    if (!fz_conv3d_stem_supported(cin, cout, D, H, W))
+        return fail(FZ_ERR_UNSUPPORTED, "stem convolution kernel handles 1..4 -> 32 channels, W divisible by 4 (got %d -> %d, W = %d)", cin, cout, W);
+    if (batch == 0) return FZ_OK;
+    if (!x || !weight || !y) return fail(FZ_ERR_INVALID, "stem convolution: null buffer");
+    if (unaligned16(x) || unaligned16(y)) return fail(FZ_ERR_UNSUPPORTED, "stem convolution kernel needs 16-byte aligned x and y");
+    const long long total4 = (long long)batch * D * H * (W / 4);
+    const int sms = num_sms();
+    long long blocks = (total4 + 127) / 128;
+    if (blocks > 16LL * sms) blocks = 16LL * sms;
+    cudaStream_t st = (cudaStream_t)stream;
+    const TI* xi = static_cast<const TI*>(x);
+    TO* yo = static_cast<TO*>(y);
+    switch (cin) {
+        case 1: conv3_stem_fwd<1, TI, TO><<<(unsigned)blocks, 128, 0, st>>>(xi, weight, bias, yo, D, H, W, total4); break;
+        case 2: conv3_stem_fwd<2, TI, TO><<<(unsigned)blocks, 128, 0, st>>>(xi, weight, bias, yo, D, H, W, total4); break;
+        case 3: conv3_stem_fwd<3, TI, TO><<<(unsigned)blocks, 128, 0, st>>>(xi, weight, bias, yo, D, H, W, total4); break;
+        default: conv3_stem_fwd<4, TI, TO><<<(unsigned)blocks, 128, 0, st>>>(xi, weight, bias, yo, D, H, W, total4); break;
+    }
+    FZ_LAUNCH_CHECK();
+    return FZ_OK;
+}
 
 }  // namespace
 }  // namespace fz
@@ -429,21 +514,14 @@ int fz_space_depth2_supported(int32_t D, int32_t H, int32_t W) {
 
 int fz_space_depth2(const float* in, float* out, int64_t batch, int32_t channels, int32_t D, int32_t H, int32_t W, int32_t to_depth,
                     void* stream) {
-    if (batch < 0 || channels <= 0) return fail(FZ_ERR_INVALID, "space/depth: bad sizes");
-    if (!fz_space_depth2_supported(D, H, W))
-        return fail(FZ_ERR_UNSUPPORTED, "space/depth kernel needs even D, H and W divisible by 4 (got %d x %d x %d)", D, H, W);
-    if (batch == 0) return FZ_OK;
-    if (!in || !out) return fail(FZ_ERR_INVALID, "space/depth: null buffer");
-    if (unaligned16(in) || unaligned16(out)) return fail(FZ_ERR_UNSUPPORTED, "space/depth kernel needs 16-byte aligned buffers");
-    const long long total4 = (long long)batch * channels * D * H * (W / 4);
-    const int sms = num_sms();
-    long long blocks = (total4 + 255) / 256;
-    if (blocks > 16LL * sms) blocks = 16LL * sms;
-    cudaStream_t st = (cudaStream_t)stream;
-    if (to_depth) space_depth2<true><<<(unsigned)blocks, 256, 0, st>>>(in, out, total4, channels, D, H, W / 4);
-    else space_depth2<false><<<(unsigned)blocks, 256, 0, st>>>(in, out, total4, channels, D, H, W / 4);
-    FZ_LAUNCH_CHECK();
-    return FZ_OK;
+    return space_depth2_launch<float>(in, out, batch, channels, D, H, W, to_depth, stream);
+}
+
+int fz_space_depth2_bf16_supported(int32_t D, int32_t H, int32_t W) { return fz_space_depth2_supported(D, H, W); }
+
+int fz_space_depth2_bf16(const void* in, void* out, int64_t batch, int32_t channels, int32_t D, int32_t H, int32_t W, int32_t to_depth,
+                         void* stream) {
+    return space_depth2_launch<bf16>(in, out, batch, channels, D, H, W, to_depth, stream);
 }
 
 int fz_conv3d_stem_supported(int32_t cin, int32_t cout, int32_t D, int32_t H, int32_t W) {
@@ -452,25 +530,14 @@ int fz_conv3d_stem_supported(int32_t cin, int32_t cout, int32_t D, int32_t H, in
 
 int fz_conv3d_stem_forward(const float* x, const float* weight, const float* bias, float* y, int64_t batch, int32_t cin, int32_t cout,
                            int32_t D, int32_t H, int32_t W, void* stream) {
-    if (batch < 0) return fail(FZ_ERR_INVALID, "stem convolution: bad batch");
-    if (!fz_conv3d_stem_supported(cin, cout, D, H, W))
-        return fail(FZ_ERR_UNSUPPORTED, "stem convolution kernel handles 1..4 -> 32 channels, W divisible by 4 (got %d -> %d, W = %d)", cin, cout, W);
-    if (batch == 0) return FZ_OK;
-    if (!x || !weight || !y) return fail(FZ_ERR_INVALID, "stem convolution: null buffer");
-    if (unaligned16(x) || unaligned16(y)) return fail(FZ_ERR_UNSUPPORTED, "stem convolution kernel needs 16-byte aligned x and y");
-    const long long total4 = (long long)batch * D * H * (W / 4);
-    const int sms = num_sms();
-    long long blocks = (total4 + 127) / 128;
-    if (blocks > 16LL * sms) blocks = 16LL * sms;
-    cudaStream_t st = (cudaStream_t)stream;
-    switch (cin) {
-        case 1: conv3_stem_fwd<1><<<(unsigned)blocks, 128, 0, st>>>(x, weight, bias, y, D, H, W, total4); break;
-        case 2: conv3_stem_fwd<2><<<(unsigned)blocks, 128, 0, st>>>(x, weight, bias, y, D, H, W, total4); break;
-        case 3: conv3_stem_fwd<3><<<(unsigned)blocks, 128, 0, st>>>(x, weight, bias, y, D, H, W, total4); break;
-        default: conv3_stem_fwd<4><<<(unsigned)blocks, 128, 0, st>>>(x, weight, bias, y, D, H, W, total4); break;
-    }
-    FZ_LAUNCH_CHECK();
-    return FZ_OK;
+    return stem_forward_launch<float, float>(x, weight, bias, y, batch, cin, cout, D, H, W, stream);
+}
+
+int fz_conv3d_stem_forward_bf16(const void* x, int32_t x_dtype, const float* weight, const float* bias, void* y, int64_t batch, int32_t cin,
+                                int32_t cout, int32_t D, int32_t H, int32_t W, void* stream) {
+    if (x_dtype == FZ_DTYPE_F32) return stem_forward_launch<float, bf16>(x, weight, bias, y, batch, cin, cout, D, H, W, stream);
+    if (x_dtype == FZ_DTYPE_BF16) return stem_forward_launch<bf16, bf16>(x, weight, bias, y, batch, cin, cout, D, H, W, stream);
+    return fail(FZ_ERR_INVALID, "stem convolution: unknown x dtype %d", x_dtype);
 }
 
 }  // extern "C"

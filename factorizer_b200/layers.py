@@ -1,7 +1,8 @@
 """Channels-first glue layers around the hot path (SURVEY.md section 8(f) row 1).  LayerNorm runs a
 hand-written channels-first kernel (csrc/fz_layernorm.cu) where it applies; Linear is a cuBLAS GEMM on the
 (C_out, C_in) x (C_in, voxels) view instead of a k=1 cuDNN convolution, with its own weight-gradient kernel
-(csrc/fz_linear.cu) when the contraction over voxels is long; GELU / residual adds are ATen.  Module and parameter names match the reference so its checkpoints load:
+(csrc/fz_linear.cu) when the contraction over voxels is long; GELU / residual adds are ATen.  Under bf16 autocast, or on bf16
+inputs, Linear, the patch convolutions and the stem run this library's bf16 kernels (_ops.bf16_layer_supported).  Module and parameter names match the reference so its checkpoints load:
 ``Linear.linear`` (factorizer/layers/linear.py:43-58), ``LayerNorm.norm`` (layers/norm.py:25-34),
 ``MLP.block.{0,3}`` (layers/mlp.py:40-63), ``PositionalEmbedding.pos`` (layers/pos_embed.py:70-89).
 """
@@ -33,6 +34,9 @@ class Linear(nn.Module):
         w = self.linear.weight.squeeze(-1)
         xf = self.flatten(x)                                  # (B, C_in, voxels): a view, no copy
         from . import _ops
+        if _ops.bf16_layer_supported(x, xf.shape[-1], w.shape[1], w.shape[0], linear=True):
+            # bf16 autocast, or bf16 x: bf16 tensor-core channel map (csrc/fz_bf16_block.cu), fp32 parameters
+            return _ops.LinearBf16Fn.apply(_ops.as_bf16(xf), w, self.linear.bias, False).view(shape[0], -1, *shape[2:])
         if torch.is_grad_enabled() and w.requires_grad and xf.is_contiguous() and _ops.linear_wgrad_supported(xf, w.shape[0]):
             # long contractions over voxels: hand-written weight-gradient kernel (csrc/fz_linear.cu)
             return _ops.LinearCF.apply(xf, w, self.linear.bias).view(shape[0], -1, *shape[2:])
@@ -97,10 +101,40 @@ class _PatchConv:
         return (rows <= 256 and min(out_sp) > 0 and vox % 4 == 0 and x.shape[0] * vox >= 4096
                 and x.shape[0] * rows * vox * 4 <= 2 ** 31)
 
+    def _bf16_forward(self, x: torch.Tensor):
+        """The bf16 route (_ops.bf16_layer_supported): the 3-D kernel-2 stride-2 down-sampler as bf16 space-to-depth + the bf16
+        channel map, a kernel-1 convolution as the bf16 channel map on the flattened view, the 3x3x3 stem as StemConvBf16Fn;
+        None for every other layer or shape."""
+        from . import _ops
+        k, sp = tuple(self.kernel_size), tuple(x.shape[2:])
+        if not (x.dim() == len(k) + 2 and self.groups == 1 and all(d == 1 for d in self.dilation) and not isinstance(self.padding, str)
+                and self.padding_mode == "zeros"):
+            return None
+        B, C, co = x.shape[0], x.shape[1], self.out_channels
+        if tuple(self.stride) == k and all(p == 0 for p in self.padding):
+            out_sp = [n // q for n, q in zip(sp, k)]
+            if all(q == 1 for q in k):
+                if not _ops.bf16_layer_supported(x, math.prod(sp), self.in_channels, co):
+                    return None
+                xf = _ops.as_bf16(x).view(B, C, -1)
+            elif k == (2, 2, 2) and _ops.L.lib().fz_space_depth2_bf16_supported(*sp) and _ops.bf16_layer_supported(x, math.prod(out_sp), self.in_channels, co):
+                xf = _ops.SpaceDepth2.apply(_ops.as_bf16(x), True, sp)                             # bf16 permutation
+            else:
+                return None
+            y = _ops.LinearBf16Fn.apply(xf, self.weight.reshape(co, -1), self.bias, False)
+            return y.view(B, co, *out_sp)
+        if (k == (3, 3, 3) and all(q == 1 for q in self.stride) and tuple(self.padding) == (1, 1, 1)
+                and _ops.stem_bf16_supported(x, self.weight)):
+            return _ops.StemConvBf16Fn.apply(x, self.weight, self.bias)
+        return None
+
     def forward(self, x: torch.Tensor) -> torch.Tensor:
         pv = self._patch_view(x)
         if pv is None:
             from . import _ops
+            y = self._bf16_forward(x)
+            if y is not None:
+                return y
             if self._unfold_ok(x):
                 return _ops.ConvWgradCF.apply(x, self.weight, self.bias, tuple(self.padding))
             if (not (torch.is_grad_enabled() and (x.requires_grad or self.weight.requires_grad)) and self.groups == 1
@@ -141,7 +175,28 @@ class _PatchConvTranspose:
         from . import _ops
         return _ops.linear_wgrad_supported(x.flatten(2), self.out_channels * math.prod(k), min_voxels=64)
 
+    def _bf16_forward(self, x: torch.Tensor):
+        """The bf16 route (_ops.bf16_layer_supported) of the 3-D kernel-2 stride-2 up-sampler: the bf16 channel map with the
+        transposed staged weight (rows (co, k)), then bf16 depth-to-space; None for every other layer or shape."""
+        from . import _ops
+        k = tuple(self.kernel_size)
+        if not (k == (2, 2, 2) and x.dim() == 5 and self.groups == 1 and tuple(self.stride) == k and all(d == 1 for d in self.dilation)
+                and all(p == 0 for p in self.padding) and all(p == 0 for p in self.output_padding)):
+            return None
+        full = tuple(2 * n for n in x.shape[2:])
+        if not (_ops.L.lib().fz_space_depth2_bf16_supported(*full) and _ops.bf16_layer_supported(x, math.prod(x.shape[2:]), self.in_channels, self.out_channels * 8)):
+            return None
+        B, co, K = x.shape[0], self.out_channels, math.prod(k)
+        w = self.weight.reshape(self.in_channels, co * K)                        # (ci, (co, k)) as stored
+        b = None if self.bias is None else self.bias.repeat_interleave(K)
+        y = _ops.LinearBf16Fn.apply(_ops.as_bf16(x).view(B, x.shape[1], -1), w, b, True)
+        return _ops.SpaceDepth2.apply(y, False, full)                           # bf16 permutation
+
     def forward(self, x: torch.Tensor, output_size=None) -> torch.Tensor:
+        if output_size is None:
+            y = self._bf16_forward(x)
+            if y is not None:
+                return y
         if output_size is not None or not self._patch_ok(x):
             return super().forward(x, output_size)
         from . import _ops

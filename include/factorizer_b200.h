@@ -214,6 +214,8 @@ int64_t fz_bf16_staged_elems(int32_t rows, int32_t cols);
 int fz_bf16_stage_weights(const float* w0, int32_t rows0, int32_t cols0, const float* w1, int32_t rows1, int32_t cols1,
                           const float* w2, int32_t rows2, int32_t cols2, const float* w3, int32_t rows3, int32_t cols3, void* out,
                           void* stream);
+/* The same layout for a single weight (the standalone layers): W as stored, then W^T, in one launch. */
+int fz_bf16_stage_weight(const float* w, int32_t rows, int32_t cols, void* out, void* stream);
 /* fz_layernorm_cf_forward / fz_layernorm_cf_backward_add on bf16 x, y, dy, add, dx; gamma, beta, d(gamma), d(beta) fp32. */
 int fz_layernorm_cf_bf16_supported(int32_t channels, int64_t voxels);
 int fz_layernorm_cf_forward_bf16(const void* x, const float* gamma, const float* beta, void* y, int64_t batch, int32_t channels,
@@ -230,6 +232,10 @@ int fz_swnmf_bf16_supported(const fz_geom* g, const fz_solver* s, int32_t relu_i
 int fz_space_depth2_supported(int32_t D, int32_t H, int32_t W);
 int fz_space_depth2(const float* in, float* out, int64_t batch, int32_t channels, int32_t D, int32_t H, int32_t W,
                     int32_t to_depth, void* stream);
+/* The same permutation of bf16 tensors, with the same conditions. */
+int fz_space_depth2_bf16_supported(int32_t D, int32_t H, int32_t W);
+int fz_space_depth2_bf16(const void* in, void* out, int64_t batch, int32_t channels, int32_t D, int32_t H, int32_t W,
+                         int32_t to_depth, void* stream);
 
 /* 3x3x3 convolution, stride 1, zero padding 1, 1..4 input channels -> 32 output channels: the Swin Factorizer's stem
  * (reference factorizer/factorizer.py:139-140).  x (batch, cin, D, H, W), weight (32, cin, 3, 3, 3), bias 32 floats or
@@ -237,6 +243,17 @@ int fz_space_depth2(const float* in, float* out, int64_t batch, int32_t channels
 int fz_conv3d_stem_supported(int32_t cin, int32_t cout, int32_t D, int32_t H, int32_t W);
 int fz_conv3d_stem_forward(const float* x, const float* weight, const float* bias, float* y, int64_t batch, int32_t cin,
                            int32_t cout, int32_t D, int32_t H, int32_t W, void* stream);
+/* The stem with a bf16 y: x is fp32 or bf16 (x_dtype = FZ_DTYPE_F32 / FZ_DTYPE_BF16), weight and bias fp32, the sums fp32
+ * rounded to bf16 once after the bias.  Same conditions as fz_conv3d_stem_forward. */
+int fz_conv3d_stem_forward_bf16(const void* x, int32_t x_dtype, const float* weight, const float* bias, void* y, int64_t batch,
+                                int32_t cin, int32_t cout, int32_t D, int32_t H, int32_t W, void* stream);
+/* The stem's weight gradient on a bf16 dy (batch, 32, D, H, W): dW[o][c][kd][kh][kw] = sum over (batch, voxel v) of
+ * dy[o][v] x[c][v + (kd-1, kh-1, kw-1)] (zero outside the volume) and db[o] = sum of dy[o][v] (db may be NULL), fp32,
+ * OVERWRITTEN.  x is fp32 (read as bf16) or bf16.  tcgen05 kind::f16 on im2col rows built in shared memory, never in
+ * global memory.  1..4 -> 32 channels, W divisible by 8, dy and x 16-byte aligned (FZ_ERR_UNSUPPORTED otherwise). */
+int fz_conv3d_stem_wgrad_bf16_supported(int32_t cin, int32_t cout, int32_t D, int32_t H, int32_t W);
+int fz_conv3d_stem_wgrad_bf16(const void* dy, const void* x, int32_t x_dtype, float* dW, float* db, int64_t batch, int32_t cin,
+                              int32_t cout, int32_t D, int32_t H, int32_t W, void* stream);
 
 /* ---- FactMixer / FactorizerBlock pointwise glue, 32-channel blocks (SURVEY section 8(f) row 1) --------
  * All tensors are (batch, channels, voxels) fp32 = flattened NCDHW; weights are the reference's Conv1d(k=1)
