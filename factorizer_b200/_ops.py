@@ -440,34 +440,41 @@ def _channel_map(x, w, bias, epi=EPI_NONE, aux=None, transposed=False):
 
 
 def _channel_map_wgrad(gy, x, want_bias: bool):
-    """dW = sum over (batch, voxels) of gy x^T, db = sum of gy.  Views the kernels do not take (non-contiguous, or not
-    16-byte aligned) run the same arithmetic in torch."""
+    """dW = sum over (batch, voxels) of gy x^T, db = sum of gy, both fp32.  bf16 gy and x: fz_linear_wgrad_bf16.  fp32 views the
+    kernels do not take (non-contiguous, or not 16-byte aligned) run the same arithmetic in torch."""
     lib = L.lib()
     B, cout, vox = gy.shape
     cin = x.shape[1]
-    if (gy.is_contiguous() and x.is_contiguous() and (gy.data_ptr() | x.data_ptr()) % 16 == 0
-            and lib.fz_linear_wgrad_supported(cout, cin, vox)):
+    bf16 = x.dtype == torch.bfloat16
+    if bf16 or (gy.is_contiguous() and x.is_contiguous() and (gy.data_ptr() | x.data_ptr()) % 16 == 0
+                and lib.fz_linear_wgrad_supported(cout, cin, vox)):
         gw = torch.empty(cout, cin, device=x.device, dtype=torch.float32)
         gb = torch.empty(cout, device=x.device, dtype=torch.float32) if want_bias else None
-        _call(lib.fz_linear_wgrad, L.ptr(gy), L.ptr(x), L.ptr(gw), L.ptr(gb), B, cout, cin, vox, L.stream_ptr(x.device))
+        _call(lib.fz_linear_wgrad_bf16 if bf16 else lib.fz_linear_wgrad, L.ptr(gy), L.ptr(x), L.ptr(gw), L.ptr(gb), B, cout, cin,
+              vox, L.stream_ptr(x.device))
         return gw, gb
     gw = torch.bmm(gy, x.transpose(1, 2)).sum(0)
     return gw, (gy.sum((0, 2)) if want_bias else None)
 
 
 def _ln_forward(x3, gamma, beta, eps):
+    """LayerNorm over the channels of fp32 or bf16 (B, C, voxels); the statistics are fp32."""
+    lib = L.lib()
     B, C, vox = x3.shape
     y = torch.empty_like(x3)
-    _call(L.lib().fz_layernorm_cf_forward, L.ptr(x3), L.ptr(gamma), L.ptr(beta), L.ptr(y), B, C, vox, float(eps), L.stream_ptr(x3.device))
+    fn = lib.fz_layernorm_cf_forward_bf16 if x3.dtype == torch.bfloat16 else lib.fz_layernorm_cf_forward
+    _call(fn, L.ptr(x3), L.ptr(gamma), L.ptr(beta), L.ptr(y), B, C, vox, float(eps), L.stream_ptr(x3.device))
     return y
 
 
 def _ln_backward_add(x3, gamma, gy, add, eps):
-    """dx = add + LN'(gy), d(gamma), d(beta)."""
+    """dx = add + LN'(gy) in the dtype of x3, d(gamma), d(beta) in fp32."""
+    lib = L.lib()
     B, C, vox = x3.shape
     dx, dg, db = torch.empty_like(x3), torch.empty_like(gamma), torch.empty_like(gamma)
-    _call(L.lib().fz_layernorm_cf_backward_add, L.ptr(x3), L.ptr(gamma), L.ptr(gy), L.ptr(add), L.ptr(dx), L.ptr(dg), L.ptr(db),
-          B, C, vox, float(eps), L.stream_ptr(x3.device))
+    fn = lib.fz_layernorm_cf_backward_add_bf16 if x3.dtype == torch.bfloat16 else lib.fz_layernorm_cf_backward_add
+    _call(fn, L.ptr(x3), L.ptr(gamma), L.ptr(gy), L.ptr(add), L.ptr(dx), L.ptr(dg), L.ptr(db), B, C, vox, float(eps),
+          L.stream_ptr(x3.device))
     return dx, dg, db
 
 
@@ -486,16 +493,22 @@ def wide_block_supported(x: torch.Tensor, hidden: int) -> bool:
                 and x.data_ptr() % 16 == 0)
 
 
-class FactorizerBlockWideFn(_GradModeFunction):
+class _WideBlockFn(_GradModeFunction):
     """FactorizerBlock.forward (reference factorizer/factorizer.py:74-77 with FactMixer.forward :34-57, MLP
-    layers/mlp.py:54-60) for norm = LayerNorm, act = ReLU, GELU MLP, no dropout, at any width (the 64..512-channel stages
-    of the Swin Factorizer): every step is a kernel of this library, with the residual sums, the bias + GELU and the GELU
-    derivative folded into the epilogues of the tcgen05 channel map and the residual gradients into the LayerNorm backward
-    -- nine launches forward (norm1 | in_proj | core x3 | out_proj + residual | norm2 | fc1 + GELU | fc2 + residual)."""
+    layers/mlp.py:54-60) for norm = LayerNorm, act = ReLU, GELU MLP, no dropout, at any width: every step is a kernel of this
+    library, with the residual sums, the bias + GELU and the GELU derivative folded into the epilogues of the tensor-core
+    channel map and the residual gradients into the LayerNorm backward -- nine launches forward (norm1 | in_proj | core x3 |
+    out_proj + residual | norm2 | fc1 + GELU | fc2 + residual), the same steps in reverse backward.  Written once for
+    FactorizerBlockWideFn and FactorizerBlockBf16Fn; a subclass names the activations' `dtype` and says how its channel maps
+    read the four weights (w_in, w_out, w1, w2): _stage(ws) returns the tensors the backward keeps for them, _maps(staged,
+    shapes) one channel map per weight, m(x, bias, epi, aux, transposed), transposed = that layer's input gradient."""
+    dtype = None
 
-    @staticmethod
-    def forward(ctx, x, g1, b1n, w_in, w_out, b_out, g2, b2n, w1, bb1, w2, bb2, u0, v0, geom, spec, eps1, eps2):
-        x = _check_vol(x, geom, "x")
+    @classmethod
+    def _forward(cls, ctx, x, g1, b1n, w_in, w_out, b_out, g2, b2n, w1, bb1, w2, bb2, u0, v0, geom, spec, eps1, eps2):
+        if x.dtype != cls.dtype:
+            raise NotImplementedError(f"factorizer_b200: {cls.__name__} takes {cls.dtype} activations, got {x.dtype}")
+        x = _check_vol(x, geom, "x", allow_bf16=True)
         params = [L.require_cuda_f32(t, "parameter") for t in (g1, b1n, w_in, w_out, b_out, g2, b2n, w1, bb1, w2, bb2)]
         g1, b1n, w_in, w_out, b_out, g2, b2n, w1, bb1, w2, bb2 = params
         u0 = L.require_cuda_f32(u0, "u0")
@@ -503,47 +516,72 @@ class FactorizerBlockWideFn(_GradModeFunction):
         B, C = x.shape[0], x.shape[1]
         need_grad = _GradModeFunction.wants_grad(ctx, 12)
         x3 = x.view(B, C, -1)
+        shapes = [tuple(w.shape) for w in (w_in, w_out, w1, w2)]
         with torch.cuda.device(x.device):
+            staged = cls._stage((w_in, w_out, w1, w2))
+            m_in, m_out, m1, m2 = cls._maps(staged, shapes)
             n1 = _ln_forward(x3, g1, b1n, eps1)
-            z = _channel_map(n1, w_in, None)
+            z = m_in(n1, None)
             m, saved = _swnmf_forward(z.view(x.shape), u0, v0, geom, spec, True, need_grad)
             m3 = m.view(B, C, -1)
-            x1 = _channel_map(m3, w_out, b_out, EPI_RESIDUAL, x3)
+            x1 = m_out(m3, b_out, EPI_RESIDUAL, x3)
             n2 = _ln_forward(x1, g2, b2n, eps2)
             if need_grad:
-                h, g = _channel_map(n2, w1, bb1, EPI_GELU)
+                h, g = m1(n2, bb1, EPI_GELU)
             else:                                                       # inference: the pre-activation is not kept
-                h, g = None, _channel_map(n2, w1, bb1, EPI_GELU_ONLY)
-            out = _channel_map(g, w2, bb2, EPI_RESIDUAL, x1)
+                h, g = None, m1(n2, bb1, EPI_GELU_ONLY)
+            out = m2(g, bb2, EPI_RESIDUAL, x1)
         if need_grad:
-            ctx.save_for_backward(x3, n1, z, m3, x1, n2, h, g, saved, g1, w_in, w_out, g2, w1, w2, u0, v0)
+            ctx.save_for_backward(x3, n1, z, m3, x1, n2, h, g, saved, g1, g2, u0, v0, *staged)
+            ctx.block, ctx.shapes = cls, shapes
             ctx.geom, ctx.spec, ctx.eps = geom, spec, (float(eps1), float(eps2))
         return out.view(x.shape)
 
     @staticmethod
     @once_differentiable
     def backward(ctx, gout):
-        x3, n1, z, m3, x1, n2, h, g, saved, g1, w_in, w_out, g2, w1, w2, u0, v0 = ctx.saved_tensors
+        x3, n1, z, m3, x1, n2, h, g, saved, g1, g2, u0, v0, *staged = ctx.saved_tensors
         geom = ctx.geom
-        gout = _check_vol(gout, geom, "grad")
+        gout = _check_vol(gout.to(x3.dtype), geom, "grad", allow_bf16=True)
         B, C = x3.shape[0], x3.shape[1]
         eps1, eps2 = ctx.eps
+        m_in, m_out, m1, m2 = ctx.block._maps(staged, ctx.shapes)
         go3 = gout.view(B, C, -1)
         with torch.cuda.device(x3.device):
-            dh = _channel_map(go3, w2, None, EPI_GELU_GRAD, h, True)        # (W2^T dOut) * gelu'(h)
+            dh = m2(go3, None, EPI_GELU_GRAD, h, True)                      # (W2^T dOut) * gelu'(h)
             dw2, dbb2 = _channel_map_wgrad(go3, g, True)
             dw1, dbb1 = _channel_map_wgrad(dh, n2, True)
-            dn2 = _channel_map(dh, w1, None, transposed=True)
+            dn2 = m1(dh, None, transposed=True)
             dx1, dg2, db2n = _ln_backward_add(x1, g2, dn2, go3, eps2)       # dOut + norm2'(..)
-            dm = _channel_map(dx1, w_out, None, transposed=True)
+            dm = m_out(dx1, None, transposed=True)
             dw_out, db_out = _channel_map_wgrad(dx1, m3, True)
             vol = (B, C, *geom.size)
             dz = _swnmf_backward(z.view(vol), dm.view(vol), u0, v0, saved, geom, ctx.spec, True).view(B, C, -1)
             dw_in, _ = _channel_map_wgrad(dz, n1, False)
-            dn1 = _channel_map(dz, w_in, None, transposed=True)
+            dn1 = m_in(dz, None, transposed=True)
             dx, dg1, db1n = _ln_backward_add(x3, g1, dn1, dx1, eps1)        # dx1 + norm1'(..)
         return (dx.view(vol), dg1, db1n, dw_in, dw_out, db_out, dg2, db2n, dw1, dbb1, dw2, dbb2,
                 None, None, None, None, None, None)
+
+
+class FactorizerBlockWideFn(_WideBlockFn):
+    """_WideBlockFn on fp32 activations (the 64..512-channel stages of the Swin Factorizer): the tcgen05 channel map
+    (fz_linear_forward_ex, 3xTF32) reads the four weights as stored, and transposed in place for the input gradients."""
+    dtype = torch.float32
+
+    @staticmethod
+    def forward(ctx, *args):
+        return FactorizerBlockWideFn._forward(ctx, *args)
+
+    @staticmethod
+    def _stage(ws):
+        return ws
+
+    @staticmethod
+    def _maps(ws, shapes):
+        def bind(w):
+            return lambda x, bias, epi=EPI_NONE, aux=None, transposed=False: _channel_map(x, w, bias, epi, aux, transposed)
+        return [bind(w) for w in ws]
 
 
 # ---- FactorizerBlock on bf16 activations: bf16 tensor-core channel maps around the bf16 fused core ------------------
@@ -585,15 +623,16 @@ def _staged_views(buf, shapes):
     return views
 
 
-def _stage_weights_bf16(ws):
-    """One launch: the four fp32 weights as bf16, each as stored and transposed; returns the buffer."""
+def _stage_weights_bf16(*ws):
+    """One launch: the fp32 matrices (one, or a block's four: the C entries take exactly those counts) as bf16, each as
+    stored and transposed; returns the buffer (see _staged_views)."""
+    if len(ws) not in (1, 4):
+        raise ValueError(f"factorizer_b200: bf16 weight staging takes one or four weights, got {len(ws)}")
     lib = L.lib()
     n = sum(int(lib.fz_bf16_staged_elems(w.shape[0], w.shape[1])) for w in ws)
     buf = torch.empty(n, device=ws[0].device, dtype=torch.bfloat16)
-    args = []
-    for w in ws:
-        args += [L.ptr(w), w.shape[0], w.shape[1]]
-    _call(lib.fz_bf16_stage_weights, *args, L.ptr(buf), L.stream_ptr(buf.device))
+    args = [a for w in ws for a in (L.ptr(w), w.shape[0], w.shape[1])]
+    _call(lib.fz_bf16_stage_weight if len(ws) == 1 else lib.fz_bf16_stage_weights, *args, L.ptr(buf), L.stream_ptr(buf.device))
     return buf
 
 
@@ -609,97 +648,28 @@ def _channel_map_bf16(x, w, cout, bias, epi=EPI_NONE, aux=None):
     return (y, y2) if epi == EPI_GELU else y
 
 
-def _channel_map_wgrad_bf16(gy, x, want_bias: bool):
-    B, cout, vox = gy.shape
-    cin = x.shape[1]
-    gw = torch.empty(cout, cin, device=x.device, dtype=torch.float32)
-    gb = torch.empty(cout, device=x.device, dtype=torch.float32) if want_bias else None
-    _call(L.lib().fz_linear_wgrad_bf16, L.ptr(gy), L.ptr(x), L.ptr(gw), L.ptr(gb), B, cout, cin, vox, L.stream_ptr(x.device))
-    return gw, gb
-
-
-def _ln_forward_bf16(x3, gamma, beta, eps):
-    B, C, vox = x3.shape
-    y = torch.empty_like(x3)
-    _call(L.lib().fz_layernorm_cf_forward_bf16, L.ptr(x3), L.ptr(gamma), L.ptr(beta), L.ptr(y), B, C, vox, float(eps),
-          L.stream_ptr(x3.device))
-    return y
-
-
-def _ln_backward_add_bf16(x3, gamma, gy, add, eps):
-    """dx = add + LN'(gy) in bf16, d(gamma), d(beta) in fp32."""
-    B, C, vox = x3.shape
-    dx, dg, db = torch.empty_like(x3), torch.empty_like(gamma), torch.empty_like(gamma)
-    _call(L.lib().fz_layernorm_cf_backward_add_bf16, L.ptr(x3), L.ptr(gamma), L.ptr(gy), L.ptr(add), L.ptr(dx), L.ptr(dg),
-          L.ptr(db), B, C, vox, float(eps), L.stream_ptr(x3.device))
-    return dx, dg, db
-
-
-class FactorizerBlockBf16Fn(_GradModeFunction):
-    """FactorizerBlockWideFn's steps on bf16 activations: every activation (n1, z, m, x1, n2, h, g, the output, dx) is bf16 in
-    memory and in the saved tensors; the parameters and their gradients stay fp32 (master weights), every sum accumulates
-    in fp32, the LayerNorm statistics are fp32, and bias, residual, GELU and GELU' are applied before the one rounding to
-    bf16.  One launch stages the four weights in bf16 (as stored and transposed), then norm1 | in_proj | core x3 |
-    out_proj + residual | norm2 | fc1 + GELU | fc2 + residual; the backward runs the same steps in reverse with the
-    weight gradients from fz_linear_wgrad_bf16."""
+class FactorizerBlockBf16Fn(_WideBlockFn):
+    """_WideBlockFn on bf16 activations: every activation (n1, z, m, x1, n2, h, g, the output, dx) is bf16 in memory and in the
+    saved tensors; the parameters and their gradients stay fp32 (master weights), every sum accumulates in fp32, the
+    LayerNorm statistics are fp32, and bias, residual, GELU and GELU' are applied before the one rounding to bf16.  One launch
+    stages the four weights in bf16, as stored and transposed (fz_bf16_stage_weights), before the nine steps; the backward
+    keeps the staged buffer and reads the transposed copies, and its weight gradients are fz_linear_wgrad_bf16."""
+    dtype = torch.bfloat16
 
     @staticmethod
-    def forward(ctx, x, g1, b1n, w_in, w_out, b_out, g2, b2n, w1, bb1, w2, bb2, u0, v0, geom, spec, eps1, eps2):
-        if x.dtype != torch.bfloat16:
-            raise NotImplementedError(f"factorizer_b200: FactorizerBlockBf16Fn takes bf16 activations, got {x.dtype}")
-        x = _check_vol(x, geom, "x", allow_bf16=True)
-        params = [L.require_cuda_f32(t, "parameter") for t in (g1, b1n, w_in, w_out, b_out, g2, b2n, w1, bb1, w2, bb2)]
-        g1, b1n, w_in, w_out, b_out, g2, b2n, w1, bb1, w2, bb2 = params
-        u0 = L.require_cuda_f32(u0, "u0")
-        v0 = L.require_cuda_f32(v0, "v0")
-        B, C = x.shape[0], x.shape[1]
-        H = w1.shape[0]
-        need_grad = _GradModeFunction.wants_grad(ctx, 12)
-        x3 = x.view(B, C, -1)
-        with torch.cuda.device(x.device):
-            staged = _stage_weights_bf16((w_in, w_out, w1, w2))
-            (wi, _), (wo, _), (f1, _), (f2, _) = _staged_views(staged, [tuple(w.shape) for w in (w_in, w_out, w1, w2)])
-            n1 = _ln_forward_bf16(x3, g1, b1n, eps1)
-            z = _channel_map_bf16(n1, wi, C, None)
-            m, saved = _swnmf_forward(z.view(x.shape), u0, v0, geom, spec, True, need_grad)
-            m3 = m.view(B, C, -1)
-            x1 = _channel_map_bf16(m3, wo, C, b_out, EPI_RESIDUAL, x3)
-            n2 = _ln_forward_bf16(x1, g2, b2n, eps2)
-            if need_grad:
-                h, g = _channel_map_bf16(n2, f1, H, bb1, EPI_GELU)
-            else:                                                       # inference: the pre-activation is not kept
-                h, g = None, _channel_map_bf16(n2, f1, H, bb1, EPI_GELU_ONLY)
-            out = _channel_map_bf16(g, f2, C, bb2, EPI_RESIDUAL, x1)
-        if need_grad:
-            ctx.save_for_backward(x3, n1, z, m3, x1, n2, h, g, saved, g1, g2, u0, v0, staged)
-            ctx.geom, ctx.spec, ctx.eps, ctx.C, ctx.H = geom, spec, (float(eps1), float(eps2)), C, H
-        return out.view(x.shape)
+    def forward(ctx, *args):
+        return FactorizerBlockBf16Fn._forward(ctx, *args)
 
     @staticmethod
-    @once_differentiable
-    def backward(ctx, gout):
-        x3, n1, z, m3, x1, n2, h, g, saved, g1, g2, u0, v0, staged = ctx.saved_tensors
-        geom, H = ctx.geom, ctx.H
-        gout = _check_vol(gout.to(torch.bfloat16), geom, "grad", allow_bf16=True)
-        B, C = x3.shape[0], x3.shape[1]
-        eps1, eps2 = ctx.eps
-        (_, wit), (_, wot), (_, f1t), (_, f2t) = _staged_views(staged, [(C, C), (C, C), (H, C), (C, H)])
-        go3 = gout.view(B, C, -1)
-        with torch.cuda.device(x3.device):
-            dh = _channel_map_bf16(go3, f2t, H, None, EPI_GELU_GRAD, h)     # (W2^T dOut) * gelu'(h)
-            dw2, dbb2 = _channel_map_wgrad_bf16(go3, g, True)
-            dw1, dbb1 = _channel_map_wgrad_bf16(dh, n2, True)
-            dn2 = _channel_map_bf16(dh, f1t, C, None)
-            dx1, dg2, db2n = _ln_backward_add_bf16(x1, g2, dn2, go3, eps2)   # dOut + norm2'(..)
-            dm = _channel_map_bf16(dx1, wot, C, None)
-            dw_out, db_out = _channel_map_wgrad_bf16(dx1, m3, True)
-            vol = (B, C, *geom.size)
-            dz = _swnmf_backward(z.view(vol), dm.view(vol), u0, v0, saved, geom, ctx.spec, True).view(B, C, -1)
-            dw_in, _ = _channel_map_wgrad_bf16(dz, n1, False)
-            dn1 = _channel_map_bf16(dz, wit, C, None)
-            dx, dg1, db1n = _ln_backward_add_bf16(x3, g1, dn1, dx1, eps1)   # dx1 + norm1'(..)
-        return (dx.view(vol), dg1, db1n, dw_in, dw_out, db_out, dg2, db2n, dw1, dbb1, dw2, dbb2,
-                None, None, None, None, None, None)
+    def _stage(ws):
+        return (_stage_weights_bf16(*ws),)
+
+    @staticmethod
+    def _maps(staged, shapes):
+        def bind(views, shape):
+            return lambda x, bias, epi=EPI_NONE, aux=None, transposed=False: _channel_map_bf16(
+                x, views[transposed], shape[transposed], bias, epi, aux)
+        return [bind(v, shape) for v, shape in zip(_staged_views(staged[0], shapes), shapes)]
 
 
 # ---- channels-first LayerNorm (glue around the mixer) --------------------------------------------
@@ -829,14 +799,6 @@ def as_bf16(x: torch.Tensor) -> torch.Tensor:
     return x if x.data_ptr() % 16 == 0 else x.clone()
 
 
-def _stage_weight_bf16(w: torch.Tensor) -> torch.Tensor:
-    """One launch: the fp32 matrix w (R, C) as bf16, as stored and transposed (see _staged_views)."""
-    lib = L.lib()
-    buf = torch.empty(int(lib.fz_bf16_staged_elems(w.shape[0], w.shape[1])), device=w.device, dtype=torch.bfloat16)
-    _call(lib.fz_bf16_stage_weight, L.ptr(w), w.shape[0], w.shape[1], L.ptr(buf), L.stream_ptr(w.device))
-    return buf
-
-
 class LinearBf16Fn(_GradModeFunction):
     """y = W x + b on bf16 (B, C_in, voxels) (fz_linear_forward_bf16): W = wmat, or wmat^T with `transposed` (the up-samplers'
     (C_in, C_out * K) weight read as stored).  Parameters and their gradients stay fp32, the sums are fp32 and rounded to
@@ -852,7 +814,7 @@ class LinearBf16Fn(_GradModeFunction):
             raise ValueError(f"factorizer_b200: LinearBf16Fn takes bf16 x with {R if transposed else C} channels, got {x.dtype} "
                              f"{tuple(x.shape)}")
         with torch.cuda.device(x.device):
-            staged = _stage_weight_bf16(wmat)
+            staged = _stage_weights_bf16(wmat)
             w, wt = _staged_views(staged, [(R, C)])[0]
             y = _channel_map_bf16(x, wt if transposed else w, C if transposed else R, bias)
         if _GradModeFunction.wants_grad(ctx, 3):
@@ -871,7 +833,7 @@ class LinearBf16Fn(_GradModeFunction):
             if ctx.needs_input_grad[0]:
                 gx = _channel_map_bf16(gy, w if ctx.transposed else wt, x.shape[1], None)
             if ctx.needs_input_grad[1] or (ctx.has_bias and ctx.needs_input_grad[2]):
-                gw, gb = _channel_map_wgrad_bf16(gy, x, ctx.has_bias)
+                gw, gb = _channel_map_wgrad(gy, x, ctx.has_bias)
                 if ctx.transposed:
                     gw = gw.t()
         return gx, gw, gb, None

@@ -2,9 +2,8 @@
 // and the launch that stages its weights in bf16.  The U-Net scaffold's bf16 layers use the same channel maps and staging,
 // and the stem's weight gradient below.
 //
-// Channel map  y[b][o][v] = sum_c W[o][c] x[b][c][v] (+ bias[o]), with the five FZ_EPILOGUE_* epilogues of linear_fwd_tc
-// (fz_linear_tc.cu) -- the same persistent walk over (voxel tile, output tile) items, one MMA per 16 channels and no
-// remainder tiles:
+// Channel map  y[b][o][v] = sum_c W[o][c] x[b][c][v] (+ bias[o]), with the item walk, the 2/4-stage launch policy and the five
+// FZ_EPILOGUE_* epilogues it shares with linear_fwd_tc (fz_channel_map.cuh) -- one MMA per 16 channels and no remainder tiles:
 //   D[128 voxels x 64 outputs] += A[128 x 64 channels] B[64 x 64]^T per K chunk (four MMAs),
 // A = x, voxel-contiguous = MN-major: two TMA boxes of (64 channels x 64 voxels), each channel one 128-byte row in the
 // 128-byte swizzle; B = W, K-major, one box of (64 outputs x 64 channels).  The weight is always K-major: the input
@@ -17,9 +16,10 @@
 // Weight gradient  dW[o][c] = sum over (batch, voxel) of dy[o][v] x[c][v], db[o] = sum of dy[o][v]: as linear_wgrad_tc,
 // with bf16 K-major boxes of (128 channels x 64 voxels) and no remainder tiles: A = dy (M = 128 outputs), B = [x ; ones]
 // (N = 128 inputs + the bias column), four MMAs per stage; dW, db fp32 with one atomic per element and CTA; the chain is
-// capped at 32 stages per CTA as there.
+// capped at 32 stages per CTA as there (cmap::wgrad_ctas).
 #include <cuda_bf16.h>
 
+#include "fz_channel_map.cuh"
 #include "fz_internal.cuh"
 #include "fz_tc.cuh"
 
@@ -29,11 +29,8 @@ namespace {
 using namespace tc;
 typedef __nv_bfloat16 bf16;
 
-__device__ __forceinline__ float ldbf(const bf16* p) { return __bfloat162float(__ldg(p)); }
-
 // ---- channel map ------------------------------------------------------------------------------------------------------------
-constexpr int kHM = 128, kHN = 64, kHK = 64;          // voxels x outputs per item, channels per K chunk (one 128-byte row)
-constexpr int kHThreads = 320;
+constexpr int kHM = cmap::kM, kHN = cmap::kN, kHK = 64;   // voxels x outputs per item, channels per K chunk (one 128-byte row)
 constexpr uint32_t kHA = kHK * kHM * 2;               // x chunk: two boxes of (64 channels x 64 voxels) = 16 KiB
 constexpr uint32_t kHB = kHN * kHK * 2;               // W chunk: 64 rows x 128 bytes = 8 KiB
 constexpr uint32_t hA = 0, hB = kHA, kHStage = kHA + kHB;
@@ -59,7 +56,7 @@ int make_map_rows16(CUtensorMap* m, const char* what, const bf16* ptr, long long
 }
 
 template <int STAGES>
-__global__ void __launch_bounds__(kHThreads, STAGES <= 2 ? 2 : 1)
+__global__ void __launch_bounds__(cmap::kThreads, STAGES <= 2 ? 2 : 1)
 linear_fwd_bf16_tc(const __grid_constant__ CUtensorMap map_x, const __grid_constant__ CUtensorMap map_w, const float* __restrict__ bias,
                    bf16* __restrict__ y, const bf16* __restrict__ aux, bf16* __restrict__ y2, int epi, int cout, int cin, long long vox,
                    int vtiles_per_sample, int otiles, long long total_items) {
@@ -144,31 +141,13 @@ linear_fwd_bf16_tc(const __grid_constant__ CUtensorMap map_x, const __grid_const
     } else {
         // ---- workers: drain an item's accumulator, apply the epilogue in fp32, store bf16 ----
         const int wq = warp & 3, wh = (warp - 2) >> 2;                     // TMEM lane quarter this warp may read; half of the columns
+        const cmap::Epilogue<bf16> ep{bias, y, aux, y2, epi, cout, otiles, vtiles_per_sample, vox, wq, wh, lane};
         for (long long it = 0; it < my_items; ++it) {
-            // (32-bit index arithmetic: the launcher keeps the item count below 2^31)
-            const unsigned item = blockIdx.x + (unsigned)it * gridDim.x;
-            const unsigned vt_all = item / (unsigned)otiles, ot = item - vt_all * (unsigned)otiles;
-            const unsigned b = vt_all / (unsigned)vtiles_per_sample;
-            const long long v = (long long)(vt_all - b * (unsigned)vtiles_per_sample) * kHM + wq * 32 + lane;
-            const int o0 = (int)ot * kHN + wh * 32;
-            const long long off = ((long long)b * cout + o0) * vox + v;
-            const bool live = v < vox, full = o0 + 32 <= cout;
             // the running sums start from the residual or the bias; their loads are in flight while the MMAs finish
             float sum[32];
 #pragma unroll
             for (int o = 0; o < 32; ++o) sum[o] = 0.f;
-            if (live && epi == FZ_EPILOGUE_RESIDUAL) {
-                const bf16* pa = aux + off;
-#pragma unroll
-                for (int o = 0; o < 32; ++o) {
-                    if (full || o0 + o < cout) sum[o] = ldbf(pa);
-                    pa += vox;
-                }
-            } else if (bias) {
-#pragma unroll
-                for (int o = 0; o < 32; ++o)
-                    if (full || o0 + o < cout) sum[o] = __ldg(bias + o0 + o);
-            }
+            ep.start(sum, it, false);
             const uint32_t acc = (uint32_t)(it & 1), use = (uint32_t)(it >> 1);
             mbar_wait(sbase + hBarAccFull + 8 * acc, use & 1);
             tc_fence_after();
@@ -185,58 +164,7 @@ linear_fwd_bf16_tc(const __grid_constant__ CUtensorMap map_x, const __grid_const
                 sum[i] += __uint_as_float(d0[i]);
                 sum[16 + i] += __uint_as_float(d1[i]);
             }
-            if (!live) continue;
-            if (epi == FZ_EPILOGUE_RESIDUAL && bias) {
-#pragma unroll
-                for (int o = 0; o < 32; ++o)
-                    if (full || o0 + o < cout) sum[o] += __ldg(bias + o0 + o);
-            }
-            bf16* py = y + off;
-            if (epi == FZ_EPILOGUE_GELU) {
-                bf16* pg = y2 + off;
-#pragma unroll
-                for (int o = 0; o < 32; o += 2) {
-                    float2 e;
-                    const float2 r = make_float2(sum[o], sum[o + 1]);
-                    const float2 gl = __fmul2_rn(r, gauss_cdf2(r, e));
-                    if (full || o0 + o < cout) { *py = __float2bfloat16_rn(r.x); *pg = __float2bfloat16_rn(gl.x); }
-                    py += vox; pg += vox;
-                    if (full || o0 + o + 1 < cout) { *py = __float2bfloat16_rn(r.y); *pg = __float2bfloat16_rn(gl.y); }
-                    py += vox; pg += vox;
-                }
-                continue;
-            }
-            if (epi == FZ_EPILOGUE_GELU_ONLY) {
-#pragma unroll
-                for (int o = 0; o < 32; o += 2) {
-                    float2 e;
-                    const float2 r = make_float2(sum[o], sum[o + 1]);
-                    const float2 gl = __fmul2_rn(r, gauss_cdf2(r, e));
-                    sum[o] = gl.x;
-                    sum[o + 1] = gl.y;
-                }
-            }
-            if (epi == FZ_EPILOGUE_GELU_GRAD) {
-                float h[32];
-                const bf16* pa = aux + off;
-#pragma unroll
-                for (int o = 0; o < 32; ++o) {
-                    h[o] = (full || o0 + o < cout) ? ldbf(pa) : 0.f;
-                    pa += vox;
-                }
-#pragma unroll
-                for (int o = 0; o < 32; o += 2) {
-                    float2 gl, gp;
-                    gelu_grad2(make_float2(h[o], h[o + 1]), gl, gp);
-                    sum[o] *= gp.x;
-                    sum[o + 1] *= gp.y;
-                }
-            }
-#pragma unroll
-            for (int o = 0; o < 32; ++o) {
-                if (full || o0 + o < cout) *py = __float2bfloat16_rn(sum[o]);
-                py += vox;
-            }
+            ep.finish(sum, it);
         }
     }
     tc_fence_before();
@@ -380,8 +308,6 @@ constexpr uint32_t kSA = 128 * 128, kSB = 32 * 128, kSStage = kSA + kSB;     // 
 constexpr uint32_t sBarFull = kSStages * kSStage, sBarEmpty = sBarFull + 8 * kSStages, sBarDone = sBarEmpty + 8 * kSStages,
                    sTmemSlot = sBarDone + 8, kSSmem = sTmemSlot + 8;
 
-__device__ __forceinline__ float ldx(const float* p) { return __ldg(p); }
-__device__ __forceinline__ float ldx(const bf16* p) { return ldbf(p); }
 __device__ __forceinline__ uint32_t pack_bf16(float a, float b) {
     const __nv_bfloat162 h = __floats2bfloat162_rn(a, b);
     return *reinterpret_cast<const uint32_t*>(&h);
@@ -476,7 +402,7 @@ stem_wgrad_bf16_tc(const __grid_constant__ CUtensorMap map_dy, const TX* __restr
                 const TX* src = xb + c * vox + ((long long)dd * H + hh) * W + w0;
                 float e[8];
 #pragma unroll
-                for (int i = 0; i < 8; ++i) e[i] = (rowok && w0 + i >= 0 && w0 + i < W) ? ldx(src + i) : 0.f;
+                for (int i = 0; i < 8; ++i) e[i] = (rowok && w0 + i >= 0 && w0 + i < W) ? cmap::ldg_f(src + i) : 0.f;
                 const uint4 q = make_uint4(pack_bf16(e[0], e[1]), pack_bf16(e[2], e[3]), pack_bf16(e[4], e[5]), pack_bf16(e[6], e[7]));
                 *reinterpret_cast<uint4*>(tileA + r * 128 + ((j ^ (r & 7)) << 4)) = q;
             }
@@ -586,9 +512,7 @@ int fz_linear_forward_bf16(const void* x, const void* W, int32_t ldw, const floa
     if (batch == 0) return FZ_OK;
     if (!x || !W || !y) return fail(FZ_ERR_INVALID, "null buffer");
     if (batch < 0 || batch >= (1LL << 31)) return fail(FZ_ERR_INVALID, "batch=%lld", (long long)batch);
-    if (epilogue < FZ_EPILOGUE_NONE || epilogue > FZ_EPILOGUE_GELU_ONLY) return fail(FZ_ERR_INVALID, "unknown epilogue %d", epilogue);
-    if ((epilogue == FZ_EPILOGUE_RESIDUAL || epilogue == FZ_EPILOGUE_GELU_GRAD) && !aux) return fail(FZ_ERR_INVALID, "epilogue %d needs aux", epilogue);
-    if (epilogue == FZ_EPILOGUE_GELU && !y2) return fail(FZ_ERR_INVALID, "FZ_EPILOGUE_GELU needs y2");
+    if (int e = cmap::check_epilogue("bf16 channel map", epilogue, aux, y2)) return e;
     if (!fz_linear_forward_bf16_supported(cout, cin, voxels))
         return fail(FZ_ERR_UNSUPPORTED, "bf16 channel map: voxels must be a positive multiple of 8 below 2^31 (got %lld)", (long long)voxels);
     if (ldw < cin || ldw % 8) return fail(FZ_ERR_UNSUPPORTED, "bf16 channel map: ldw=%d must be >= cin=%d and a multiple of 8", ldw, cin);
@@ -608,18 +532,17 @@ int fz_linear_forward_bf16(const void* x, const void* W, int32_t ldw, const floa
     bf16* y2b = static_cast<bf16*>(y2);
     const bf16* ab = static_cast<const bf16*>(aux);
     cudaStream_t st = (cudaStream_t)stream;
-    if (items <= num_sms() && cin > 2 * kHK) {            // fewer items than SMs and more than two K chunks: deeper pipeline, one CTA per SM
+    const cmap::Launch ls = cmap::launch_shape(items, (cin + kHK - 1) / kHK);
+    if (ls.stages == 4) {
         static SmemConfig cfg4;
         FZ_CUDA_CHECK(cfg4.ensure(linear_fwd_bf16_tc<4>, h_smem_bytes(4)));
-        linear_fwd_bf16_tc<4><<<(unsigned)items, kHThreads, h_smem_bytes(4), st>>>(map_x, map_w, bias, yb, ab, y2b, epilogue, cout, cin, voxels,
-                                                                                  vtps, otiles, items);
+        linear_fwd_bf16_tc<4><<<ls.blocks, cmap::kThreads, h_smem_bytes(4), st>>>(map_x, map_w, bias, yb, ab, y2b, epilogue, cout, cin, voxels,
+                                                                                 vtps, otiles, items);
     } else {
         static SmemConfig cfg2;
         FZ_CUDA_CHECK(cfg2.ensure(linear_fwd_bf16_tc<2>, h_smem_bytes(2)));
-        const long long cap = 2LL * num_sms();
-        const unsigned blocks = (unsigned)(items < cap ? items : cap);
-        linear_fwd_bf16_tc<2><<<blocks, kHThreads, h_smem_bytes(2), st>>>(map_x, map_w, bias, yb, ab, y2b, epilogue, cout, cin, voxels, vtps,
-                                                                         otiles, items);
+        linear_fwd_bf16_tc<2><<<ls.blocks, cmap::kThreads, h_smem_bytes(2), st>>>(map_x, map_w, bias, yb, ab, y2b, epilogue, cout, cin, voxels,
+                                                                                 vtps, otiles, items);
     }
     FZ_LAUNCH_CHECK();
     return FZ_OK;
@@ -650,12 +573,7 @@ int fz_linear_wgrad_bf16(const void* dy, const void* x, float* dW, float* db, in
     const int tps = (int)((voxels + kWVT - 1) / kWVT);
     const long long tiles = batch * tps;
     const int bo = (cout + kWBlk - 1) / kWBlk, bi = (cin + kWBlk - 1) / kWBlk;
-    long long gx = (2LL * num_sms() + bo * bi - 1) / (bo * bi);
-    // the tensor core truncates as it accumulates: at most kMaxChain stages (4 MMAs each) per CTA, as linear_wgrad_tc
-    constexpr long long kMaxChain = 32;
-    if (gx * kMaxChain < tiles) gx = (tiles + kMaxChain - 1) / kMaxChain;
-    if (gx > tiles) gx = tiles;
-    if (gx < 1) gx = 1;
+    const long long gx = cmap::wgrad_ctas((2LL * num_sms() + bo * bi - 1) / (bo * bi), tiles);
     linear_wgrad_bf16_tc<<<dim3((unsigned)gx, bo, bi), kWThreads, kWSmem, st>>>(map_dy, map_x, dW, db, cout, cin, tps, tiles);
     FZ_LAUNCH_CHECK();
     return FZ_OK;
@@ -703,10 +621,7 @@ int fz_conv3d_stem_wgrad_bf16(const void* dy, const void* x, int32_t x_dtype, fl
     if (int e = make_map_rows16(&map_dy, "dy (bf16)", static_cast<const bf16*>(dy), cout, vox, vox, 32, 3, batch)) return e;
     const int tps = (int)((vox + kSV - 1) / kSV);
     const long long tiles = batch * tps;
-    long long gx = 2LL * num_sms();
-    constexpr long long kMaxChain = 32;                         // stages per CTA, as fz_linear_wgrad_bf16
-    if (gx * kMaxChain < tiles) gx = (tiles + kMaxChain - 1) / kMaxChain;
-    if (gx > tiles) gx = tiles;
+    const long long gx = cmap::wgrad_ctas(2LL * num_sms(), tiles);
     if (gx >= (1LL << 31)) return fail(FZ_ERR_UNSUPPORTED, "stem weight gradient: too many voxels");
     if (x_dtype == FZ_DTYPE_F32) {
         static SmemConfig cfg;

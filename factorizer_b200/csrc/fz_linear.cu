@@ -15,6 +15,7 @@
 // 64 x 64 or 32 x 128 blocks, cp.async double buffering, 8 x 8 register tiles.  FP32 pipe, exact fp32 products.
 #include <cuda_bf16.h>
 
+#include "fz_channel_map.cuh"
 #include "fz_device.cuh"
 #include "fz_internal.cuh"
 
@@ -497,9 +498,7 @@ int fz_linear_forward_ex(const float* x, const float* W, const float* bias, floa
     if (epilogue < FZ_EPILOGUE_NONE || epilogue > FZ_EPILOGUE_GELU_ONLY) return fail(FZ_ERR_INVALID, "linear forward: unknown epilogue %d", epilogue);
     if (batch == 0) return FZ_OK;
     if (!x || !W || !y) return fail(FZ_ERR_INVALID, "linear forward: null buffer");
-    if ((epilogue == FZ_EPILOGUE_RESIDUAL || epilogue == FZ_EPILOGUE_GELU_GRAD) && !aux)
-        return fail(FZ_ERR_INVALID, "linear forward: this epilogue reads `aux`");
-    if (epilogue == FZ_EPILOGUE_GELU && !y2) return fail(FZ_ERR_INVALID, "linear forward: the GELU epilogue writes `y2`");
+    if (int e = cmap::check_epilogue("linear forward", epilogue, aux, y2)) return e;
     if (!fz_linear_forward_supported(cout, cin, voxels) || !linear_fwd_tc_supported(x, W, batch, cout, cin, voxels) ||
         (w_transposed && cout % 4))
         return fail(FZ_ERR_UNSUPPORTED, "linear forward kernel needs voxels and input channels (with a transposed weight: output "

@@ -9,9 +9,11 @@
 // Four warps compute the remainder tiles lo = v - hi(v) element by element (same shared-memory offsets, so the swizzle is
 // never decoded), and ONE MMA per 8 voxels with A = [dy ; dy_lo] (M = 128) and B = [x ; x_lo ; ones] (N = 144) produces all
 // four hi / lo blocks of a 64 x 64 block of dW plus the bias column; they accumulate in TMEM over the CTA's share of the
-// voxels and are added up, then added to the global gradient with one atomic per element and CTA.
+// voxels and are added up, then added to the global gradient with one atomic per element and CTA (the chain is capped at
+// cmap::wgrad_ctas's 32 stages per CTA).
 // Warp roles: warp 0 = TMA producer, warp 1 = MMA issue (warp-uniform code under elect.sync), warps 2-5 = remainder tiles and
 // epilogue.  Three stages of 32 KB, two CTAs per SM.
+#include "fz_channel_map.cuh"
 #include "fz_tc.cuh"
 
 namespace fz {
@@ -179,18 +181,18 @@ linear_wgrad_tc(const __grid_constant__ CUtensorMap map_dy, const __grid_constan
 //   D[128 voxels x 64 outputs] += A[128 x 32 channels] B[64 x 32]^T per K chunk,
 // A = x, voxel-contiguous = MN-major: TMA boxes of (32 channels x 32 voxels) with SWIZZLE_128B_ATOM_32B are exactly the atoms
 // of the one swizzle 32-bit MN-major operands accept; B = W, K-major, SWIZZLE_128B boxes as in the weight-gradient kernel.
-// The fp32 tiles are the hi operands; eight warps write the remainder tiles and later run the epilogue (thread = voxel = TMEM
-// lane; bias / residual loaded into the running sums an item ahead; FZ_EPILOGUE_*: + residual, GELU, GELU derivative;
-// coalesced stores along the voxel axis).  Persistent CTAs walk (voxel tile, output tile) items; K chunks flow
-// through a two-stage (four-stage for launches with fewer items than SMs) TMA -> remainder -> MMA pipeline that runs across items.  The tensor core adds into its accumulator with
+// The fp32 tiles are the hi operands; eight warps write the remainder tiles and later run the epilogue (cmap::Epilogue in
+// fz_channel_map.cuh, shared with the bf16 channel map: thread = voxel = TMEM lane; bias / residual loaded into the running
+// sums an item ahead; FZ_EPILOGUE_*: + residual, GELU, GELU derivative; coalesced stores along the voxel axis).  Persistent
+// CTAs walk (voxel tile, output tile) items; K chunks flow through a two-stage (four-stage for launches with fewer items than
+// SMs: cmap::launch_shape) TMA -> remainder -> MMA pipeline that runs across items.  The tensor core adds into its accumulator with
 // truncation, so a long accumulation chain loses accuracy (1.4e-5 after the 192 MMAs of 512 input channels): an item is cut
 // into SEGMENTS of 4 K chunks, the a_hi b_hi products (16 MMAs per segment) and the two cross terms go to separate accumulators,
 // and the workers add the segments up in registers (round to nearest).  The accumulator pair is double-buffered in TMEM, so
 // draining a segment overlaps the MMAs of the next one.  Warp 0 = TMA producer, warp 1 = MMA issue, warps 2-9 workers.
 // =====================================================================================================================
-constexpr int kGM = 128, kGN = 64, kGK = 32;         // voxels x outputs per item, channels per K chunk
+constexpr int kGM = cmap::kM, kGN = cmap::kN, kGK = 32;   // voxels x outputs per item, channels per K chunk
 constexpr int kGSeg = 4;                              // K chunks per accumulation segment
-constexpr int kGThreads = 320;
 constexpr uint32_t kGA = kGK * kGM * 4;              // x chunk: 4 atoms of (32 channels x 32 voxels) = 16 KiB
 constexpr uint32_t kGB = kGN * kGK * 4;              // W chunk: 64 rows x 128 bytes = 8 KiB
 constexpr uint32_t gA = 0, gAlo = kGA, gB = 2 * kGA, gBlo = 2 * kGA + kGB, kGStage = 2 * kGA + 2 * kGB;   // 48 KiB
@@ -224,10 +226,9 @@ int make_map_wt(CUtensorMap* m, const float* ptr, int cout, int cin) {
                             CU_TENSOR_MAP_SWIZZLE_128B_ATOM_32B);
 }
 
-// STAGES = 2: two CTAs per SM (the streaming shapes); STAGES = 4: one CTA per SM with four K chunks in flight, for launches with
-// fewer items than SMs (the 8^3 / 16^3 stages: few voxel tiles, long K), which are bound by the chunk hand-over latency
+// STAGES = 2: two CTAs per SM; STAGES = 4: one CTA per SM with four K chunks in flight (cmap::launch_shape)
 template <int STAGES>
-__global__ void __launch_bounds__(kGThreads, STAGES <= 2 ? 2 : 1)
+__global__ void __launch_bounds__(cmap::kThreads, STAGES <= 2 ? 2 : 1)
 linear_fwd_tc(const __grid_constant__ CUtensorMap map_x, const __grid_constant__ CUtensorMap map_w, const float* __restrict__ bias,
               float* __restrict__ y, const float* __restrict__ aux, float* __restrict__ y2, int epi, int wt, int cout, int cin, long long vox,
               int vtiles_per_sample, int otiles, long long total_items) {
@@ -333,49 +334,12 @@ linear_fwd_tc(const __grid_constant__ CUtensorMap map_x, const __grid_constant__
         const int wq = warp & 3, wh = (warp - 2) >> 2;                     // TMEM lane quarter this warp may read; half of the columns
         const int spi = (kchunks + kGSeg - 1) / kGSeg;                     // segments per item
         float sum[32];
-        // where this thread's 32 outputs of item `it` live: y[off + o * vox], o0 + o < cout, voxel inside the sample
-        // (32-bit index arithmetic: the launcher keeps the item count below 2^31)
-        auto item_pos = [&](long long it, long long& off, int& o0) -> bool {
-            const unsigned item = blockIdx.x + (unsigned)it * gridDim.x;
-            const unsigned vt_all = item / (unsigned)otiles, ot = item - vt_all * (unsigned)otiles;
-            const unsigned b = vt_all / (unsigned)vtiles_per_sample;
-            const long long v = (long long)(vt_all - b * (unsigned)vtiles_per_sample) * kGM + wq * 32 + lane;
-            o0 = (int)ot * kGN + wh * 32;
-            off = ((long long)b * cout + o0) * vox + v;
-            return v < vox;
-        };
-        // an item's running sums start from the bias -- or from the residual (FZ_EPILOGUE_RESIDUAL; the bias is added at the
-        // end then): the loads are issued an item ahead of their first use and cost no registers; FZ_EPILOGUE_GELU_GRAD pulls
-        // its aux values into L2 meanwhile
+        const cmap::Epilogue<float> ep{bias, y, aux, y2, epi, cout, otiles, vtiles_per_sample, vox, wq, wh, lane};
+        // an item's running sums are loaded an item ahead of their first use and cost no registers
         auto start_item = [&](long long it) {
 #pragma unroll
             for (int i = 0; i < 32; ++i) sum[i] = 0.f;
-            if (it >= my_items) return;
-            long long off;
-            int o0;
-            const bool live = item_pos(it, off, o0);
-            if (epi != FZ_EPILOGUE_RESIDUAL) {
-                if (bias) {
-#pragma unroll
-                    for (int o = 0; o < 32; ++o)
-                        if (o0 + o < cout) sum[o] = __ldg(bias + o0 + o);
-                }
-                if (epi == FZ_EPILOGUE_GELU_GRAD && live) {
-                    const float* pa = aux + off;
-#pragma unroll
-                    for (int o = 0; o < 32; ++o) {
-                        if (o0 + o < cout) asm volatile("prefetch.global.L2 [%0];" :: "l"(pa));
-                        pa += vox;
-                    }
-                }
-            } else if (live) {
-                const float* pa = aux + off;
-#pragma unroll
-                for (int o = 0; o < 32; ++o) {
-                    if (o0 + o < cout) sum[o] = __ldg(pa);
-                    pa += vox;
-                }
-            }
+            if (it < my_items) ep.start(sum, it, true);
         };
         start_item(0);
         auto drain = [&](long long seg) {
@@ -397,68 +361,7 @@ linear_fwd_tc(const __grid_constant__ CUtensorMap map_x, const __grid_constant__
             if (lane == 0) mbar_arrive(sbase + gBarAccFree + 8 * acc);
             if (seg % spi == spi - 1) {                                    // the item's last segment: epilogue, store, start over
                 const long long it = seg / spi;
-                long long off;
-                int o0;
-                if (item_pos(it, off, o0)) {
-                    // FZ_EPILOGUE_*: (bias / residual already in the sums) | y = r, y2 = gelu(r) | y = r * gelu'(aux)
-                    const bool full = o0 + 32 <= cout;                     // no channel predicates on whole groups of 32
-                    if (epi == FZ_EPILOGUE_RESIDUAL && bias) {
-#pragma unroll
-                        for (int o = 0; o < 32; ++o)
-                            if (full || o0 + o < cout) sum[o] += __ldg(bias + o0 + o);
-                    }
-                    float* py = y + off;
-                    if (epi == FZ_EPILOGUE_GELU) {
-                        float* pg = y2 + off;
-#pragma unroll
-                        for (int o = 0; o < 32; o += 2) {
-                            float2 e;
-                            const float2 r = make_float2(sum[o], sum[o + 1]);
-                            const float2 gl = __fmul2_rn(r, gauss_cdf2(r, e));
-                            if (full || o0 + o < cout) { *py = r.x; *pg = gl.x; }
-                            py += vox; pg += vox;
-                            if (full || o0 + o + 1 < cout) { *py = r.y; *pg = gl.y; }
-                            py += vox; pg += vox;
-                        }
-                    } else {
-                        if (epi == FZ_EPILOGUE_GELU_ONLY) {
-#pragma unroll
-                            for (int o = 0; o < 32; o += 2) {
-                                float2 e;
-                                const float2 r = make_float2(sum[o], sum[o + 1]);
-                                const float2 gl = __fmul2_rn(r, gauss_cdf2(r, e));
-                                sum[o] = gl.x;
-                                sum[o + 1] = gl.y;
-                            }
-                        }
-                        if (epi == FZ_EPILOGUE_GELU_GRAD) {
-                            float h[32];
-                            const float* pa = aux + off;
-#pragma unroll
-                            for (int o = 0; o < 32; ++o) {
-                                h[o] = (full || o0 + o < cout) ? __ldg(pa) : 0.f;
-                                pa += vox;
-                            }
-#pragma unroll
-                            for (int o = 0; o < 32; o += 2) {
-                                float2 gl, gp;
-                                gelu_grad2(make_float2(h[o], h[o + 1]), gl, gp);
-                                sum[o] *= gp.x;
-                                sum[o + 1] *= gp.y;
-                            }
-                        }
-                        if (full) {
-#pragma unroll
-                            for (int o = 0; o < 32; ++o) { *py = sum[o]; py += vox; }
-                        } else {
-#pragma unroll
-                            for (int o = 0; o < 32; ++o) {
-                                if (o0 + o < cout) *py = sum[o];
-                                py += vox;
-                            }
-                        }
-                    }
-                }
+                ep.finish(sum, it);
                 start_item(it + 1);
             }
         };
@@ -519,16 +422,7 @@ int linear_wgrad_tc_launch(const float* dy, const float* x, float* dW, float* db
     const int tps = (int)((voxels + kVT - 1) / kVT);
     const long long tiles = batch * tps;
     const int bo = (cout + kBlk - 1) / kBlk, bi = (cin + kBlk - 1) / kBlk;
-    long long gx = (2LL * num_sms() + bo * bi - 1) / (bo * bi);
-    // The tensor core adds into its fp32 accumulator with truncation, so the error of a TMEM accumulation chain grows linearly
-    // with its length: on same-sign operands about 2^-24 S per MMA of the chain, S = sum |dy| |x| (B200: 1.7e-5 S after 64
-    // stages, 9.8e-5 S after 443; the FP32-pipe kernels stay below 1.1e-6 S).  At most kMaxChain stages (4 MMAs each) per
-    // CTA, more CTAs along the voxel axis instead: 32 stages keep the error at 0.8-1.04e-5 S
-    // (tests/test_gpu_channel_map_scale.py holds it to 2e-5 S).
-    constexpr long long kMaxChain = 32;
-    if (gx * kMaxChain < tiles) gx = (tiles + kMaxChain - 1) / kMaxChain;
-    if (gx > tiles) gx = tiles;
-    if (gx < 1) gx = 1;
+    const long long gx = cmap::wgrad_ctas((2LL * num_sms() + bo * bi - 1) / (bo * bi), tiles);
     linear_wgrad_tc<<<dim3((unsigned)gx, bo, bi), kThreads, kSmemW, st>>>(map_dy, map_x, dW, db, cout, cin, tps, tiles);
     FZ_LAUNCH_CHECK();
     return FZ_OK;
@@ -551,18 +445,17 @@ int linear_fwd_tc_launch(const float* x, const float* W, const float* bias, floa
     const int otiles = (cout + kGN - 1) / kGN;
     const long long items = batch * vtps * otiles;
     if (items >= (1LL << 31)) return fail(FZ_ERR_UNSUPPORTED, "linear forward: more than 2^31 (voxel tile, output tile) items");
-    if (items <= num_sms() && cin > 2 * kGK) {            // fewer items than SMs and more than two K chunks: deeper pipeline, one CTA per SM
+    const cmap::Launch ls = cmap::launch_shape(items, (cin + kGK - 1) / kGK);
+    if (ls.stages == 4) {
         static SmemConfig cfg4;
         FZ_CUDA_CHECK(cfg4.ensure(linear_fwd_tc<4>, g_smem_bytes(4)));
-        linear_fwd_tc<4><<<(unsigned)items, kGThreads, g_smem_bytes(4), st>>>(map_x, map_w, bias, y, aux, y2, epi, wt, cout, cin, voxels, vtps,
-                                                                             otiles, items);
+        linear_fwd_tc<4><<<ls.blocks, cmap::kThreads, g_smem_bytes(4), st>>>(map_x, map_w, bias, y, aux, y2, epi, wt, cout, cin, voxels, vtps,
+                                                                            otiles, items);
     } else {
         static SmemConfig cfg2;
         FZ_CUDA_CHECK(cfg2.ensure(linear_fwd_tc<2>, g_smem_bytes(2)));
-        const long long cap = 2LL * num_sms();
-        const unsigned blocks = (unsigned)(items < cap ? items : cap);
-        linear_fwd_tc<2><<<blocks, kGThreads, g_smem_bytes(2), st>>>(map_x, map_w, bias, y, aux, y2, epi, wt, cout, cin, voxels, vtps, otiles,
-                                                                    items);
+        linear_fwd_tc<2><<<ls.blocks, cmap::kThreads, g_smem_bytes(2), st>>>(map_x, map_w, bias, y, aux, y2, epi, wt, cout, cin, voxels, vtps,
+                                                                            otiles, items);
     }
     FZ_LAUNCH_CHECK();
     return FZ_OK;

@@ -56,6 +56,28 @@ def test_geometry_validation_through_abi(ft):
     assert code == _lib.FZ_ERR_UNSUPPORTED
 
 
+def test_channel_map_epilogue_arguments_through_abi(ft):
+    """Return codes of the two channel-map entries on bad epilogue arguments (refused before any device work).  The fp32
+    entry rejects an unknown epilogue even for a zero batch; the bf16 entry returns early on a zero batch."""
+    from factorizer_b200 import _lib
+    lib = _lib.lib()
+    p = 256                                       # a non-null address the refused calls never dereference
+    fwd = lambda batch, epi, aux, y2: lib.fz_linear_forward_ex(p, p, None, p, batch, 8, 8, 64, epi, 0, aux, y2, None)
+    bf16 = lambda batch, epi, aux, y2: lib.fz_linear_forward_bf16(p, p, 8, None, p, batch, 8, 8, 64, epi, aux, y2, None)
+    assert fwd(0, 7, p, p) == _lib.FZ_ERR_INVALID
+    assert fwd(0, -1, p, p) == _lib.FZ_ERR_INVALID
+    assert fwd(0, 1, None, None) == _lib.FZ_OK
+    assert fwd(1, 7, p, p) == _lib.FZ_ERR_INVALID
+    assert fwd(1, 1, None, p) == _lib.FZ_ERR_INVALID
+    assert fwd(1, 3, None, p) == _lib.FZ_ERR_INVALID
+    assert fwd(1, 2, p, None) == _lib.FZ_ERR_INVALID
+    assert bf16(0, 7, None, None) == _lib.FZ_OK
+    assert bf16(1, 7, p, p) == _lib.FZ_ERR_INVALID
+    assert bf16(1, 1, None, p) == _lib.FZ_ERR_INVALID
+    assert bf16(1, 3, None, p) == _lib.FZ_ERR_INVALID
+    assert bf16(1, 2, p, None) == _lib.FZ_ERR_INVALID
+
+
 def test_readme_shapes_and_state_dict_keys(ft, golden):
     sw = ft.SWMatricize((None, 32, 128, 128, 128), head_dim=8, patch_size=8)
     assert sw.output_size == (None, 4096, 8, 512)          # reference README.md:43-47
