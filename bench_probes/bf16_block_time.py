@@ -10,7 +10,13 @@ eagerly for fp32, bf16-old and bf16-new.  Achieved bandwidth is against the bloc
 each step reads or writes once, 32 C + 8 H elements per voxel for forward + backward (C channels, H hidden), 4 bytes each
 in fp32, 2 in bf16.  Writes JSON (the card's name and power limit included) to --out.
 
+--shifts bundle, --mlp-ratio 4 --batch 2 configure blocks and model like the BraTS23 bundle (shifts [None, 2, 4, 6]).  At
+those shifts the fused core took bf16 volumes only after the paired path learnt bf16, so bf16-old also switches the bf16
+core off there (FactMixer casts the core's input to fp32, as it did before).  --core adds the core alone at
+(--batch, 32, 128^3), fp32 against bf16 on the same path, forward and backward, each as one CUDA graph.
+
     python bench_probes/bf16_block_time.py --out /tmp/bf16_block_time.json
+    python bench_probes/bf16_block_time.py --shifts bundle --mlp-ratio 4 --batch 2 --core --out /tmp/bundle.json
 """
 import argparse
 import json
@@ -25,7 +31,8 @@ sys.path.insert(0, os.path.dirname(os.path.dirname(os.path.abspath(__file__))))
 import factorizer_b200 as ft  # noqa: E402
 from factorizer_b200 import _ops  # noqa: E402
 
-SHAPES = [(1, 32, 128), (1, 64, 64), (1, 128, 32), (1, 256, 16)]
+SHAPES = [(32, 128), (64, 64), (128, 32), (256, 16)]
+SHIFTS = {"default": None, "bundle": [None, 2, 4, 6]}
 
 
 def card():
@@ -37,26 +44,35 @@ def card():
 
 
 class _Route:
-    def __init__(self, name):
-        self.name = name
-        self.saved = _ops.bf16_block_supported
+    def __init__(self, name, shifts=None):
+        self.name, self.core_off = name, name == "bf16-old" and shifts is not None
+        self.saved = _ops.bf16_block_supported, _ops.bf16_core_supported
 
     def __enter__(self):
         if self.name == "bf16-old":
             _ops.bf16_block_supported = lambda x, hidden: False
+        if self.core_off:
+            _ops.bf16_core_supported = lambda *a, **k: False
         self.ac = torch.autocast("cuda", dtype=torch.bfloat16, enabled=self.name == "bf16-old")
         self.ac.__enter__()
 
     def __exit__(self, *exc):
         self.ac.__exit__(*exc)
-        _ops.bf16_block_supported = self.saved
+        _ops.bf16_block_supported, _ops.bf16_core_supported = self.saved
 
 
-def block(C, n, ratio=2):
+def reshape(shifts):
+    kw = {"head_dim": 8, "patch_size": 8}
+    if shifts is not None:
+        kw["shifts"] = shifts
+    return (ft.SWMatricize, kw)
+
+
+def block(C, n, ratio=2, shifts=None):
     torch.manual_seed(0)
-    return ft.FactorizerBlock(channels=C, spatial_size=(n, n, n), norm=ft.LayerNorm,
-                              reshape=(ft.SWMatricize, {"head_dim": 8, "patch_size": 8}), act=nn.ReLU, factorize=ft.NMF, rank=1,
-                              num_iters=5, init="uniform", solver="hals", mlp_ratio=ratio, dropout=0.0).cuda()
+    return ft.FactorizerBlock(channels=C, spatial_size=(n, n, n), norm=ft.LayerNorm, reshape=reshape(shifts), act=nn.ReLU,
+                              factorize=ft.NMF, rank=1, num_iters=5, init="uniform", solver="hals", mlp_ratio=ratio,
+                              dropout=0.0).cuda()
 
 
 def time_graph(fn, warmup, reps):
@@ -80,8 +96,8 @@ def time_graph(fn, warmup, reps):
     return a.elapsed_time(b) / reps
 
 
-def block_leg(B, C, n, route, warmup, reps):
-    blk = block(C, n)
+def block_leg(B, C, n, route, warmup, reps, ratio=2, shifts=None):
+    blk = block(C, n, ratio, shifts)
     H = blk.mlp.block[0].linear.out_channels
     dtype = torch.float32 if route == "fp32" else torch.bfloat16
     x = torch.randn(B, C, n, n, n, device="cuda").to(dtype).requires_grad_(True)
@@ -92,12 +108,12 @@ def block_leg(B, C, n, route, warmup, reps):
         for p in params:
             p.grad = None
         x.grad = None
-        with _Route(route):
+        with _Route(route, shifts):
             out = blk(x)
         out.backward(gout.to(out.dtype))
         return out
 
-    with _Route(route):
+    with _Route(route, shifts):
         node = type(blk(x).grad_fn).__name__
     ms = time_graph(step, warmup, reps)
     nbytes = (32 * C + 8 * H) * B * n ** 3 * (4 if route == "fp32" else 2)
@@ -106,19 +122,19 @@ def block_leg(B, C, n, route, warmup, reps):
             "achieved_GBps": nbytes / ms / 1e6}
 
 
-def model_leg(route, warmup, reps, n=128):
+def model_leg(route, warmup, reps, n=128, B=1, ratio=2, shifts=None):
     torch.manual_seed(1234)
     net = ft.Factorizer(in_channels=4, out_channels=3, spatial_size=(n, n, n), encoder_depth=(1, 1, 1, 1, 1),
                         encoder_width=(32, 64, 128, 256, 512), strides=(1, 2, 2, 2, 2), decoder_depth=(1, 1, 1, 1),
-                        norm=ft.LayerNorm, reshape=(ft.SWMatricize, {"head_dim": 8, "patch_size": 8}), act=nn.ReLU,
-                        factorize=ft.NMF, rank=1, num_iters=5, init="uniform", solver="hals", mlp_ratio=2, dropout=0.1).cuda()
+                        norm=ft.LayerNorm, reshape=reshape(shifts), act=nn.ReLU, factorize=ft.NMF, rank=1, num_iters=5,
+                        init="uniform", solver="hals", mlp_ratio=ratio, dropout=0.1).cuda()
     net.train()
-    x = torch.rand(1, 4, n, n, n, device="cuda")
-    target = torch.randint(0, 2, (1, 3, n, n, n), device="cuda").float()
+    x = torch.rand(B, 4, n, n, n, device="cuda")
+    target = torch.randint(0, 2, (B, 3, n, n, n), device="cuda").float()
 
     def step():
         net.zero_grad(set_to_none=True)
-        with _Route(route), torch.autocast("cuda", dtype=torch.bfloat16, enabled=route != "fp32"):
+        with _Route(route, shifts), torch.autocast("cuda", dtype=torch.bfloat16, enabled=route != "fp32"):
             logits = net(x).float()
         p = torch.sigmoid(logits)
         dice = 1 - (2 * (p * target).sum((2, 3, 4)) + 1e-5) / (p.sum((2, 3, 4)) + target.sum((2, 3, 4)) + 1e-5)
@@ -137,25 +153,49 @@ def model_leg(route, warmup, reps, n=128):
     return {"route": route, "train_step_ms_eager": a.elapsed_time(b) / reps}
 
 
+def core_leg(B, shifts, dtype, warmup, reps, C=32, n=128):
+    """the fused core alone (SWMatricize -> ReLU -> HALS -> inverse), forward and backward as separate graphs"""
+    from factorizer_b200 import _lib
+    geom = reshape(shifts)[0]((None, C, n, n, n), **reshape(shifts)[1])._geom
+    nmf = ft.NMF((8, 512), rank=1, num_iters=5, init="uniform", solver="hals").cuda()
+    spec, u0, v0 = nmf.solver_spec(), nmf.init.u0, nmf.init.v0
+    x = torch.randn(B, C, n, n, n, device="cuda").to(dtype)
+    gy = torch.randn(B, C, n, n, n, device="cuda").to(dtype)
+    _, saved = _ops._swnmf_forward(x, u0, v0, geom, spec, True, True)
+    path = _lib.lib().fz_last_path()
+    fwd = time_graph(lambda: _ops._swnmf_forward(x, u0, v0, geom, spec, True, True), warmup, reps)
+    bwd = time_graph(lambda: _ops._swnmf_backward(x, gy, u0, v0, saved, geom, spec, True), warmup, reps)
+    return {"shape": [B, C, n, n, n], "dtype": str(dtype), "path": path, "fwd_ms": fwd, "bwd_ms": bwd}
+
+
 def main():
     ap = argparse.ArgumentParser()
     ap.add_argument("--out", required=True, help="JSON file to write")
     ap.add_argument("--warmup", type=int, default=5)
     ap.add_argument("--reps", type=int, default=30)
     ap.add_argument("--no-model", action="store_true")
+    ap.add_argument("--shifts", choices=sorted(SHIFTS), default="default")
+    ap.add_argument("--mlp-ratio", type=int, default=2)
+    ap.add_argument("--batch", type=int, default=1)
+    ap.add_argument("--core", action="store_true", help="also time the core alone, fp32 against bf16")
     args = ap.parse_args()
     torch.backends.cuda.matmul.allow_tf32 = False
     torch.backends.cudnn.allow_tf32 = False
-    res = {"card": card(), "blocks": [], "model": []}
-    for B, C, n in SHAPES:
-        row = {r: block_leg(B, C, n, r, args.warmup, args.reps) for r in ("fp32", "bf16-old", "bf16-new")}
+    shifts, B = SHIFTS[args.shifts], args.batch
+    res = {"card": card(), "shifts": args.shifts, "mlp_ratio": args.mlp_ratio, "batch": B, "core": [], "blocks": [], "model": []}
+    if args.core:
+        for dtype in (torch.float32, torch.bfloat16):
+            res["core"].append(core_leg(B, shifts, dtype, args.warmup, args.reps))
+            print(json.dumps(res["core"][-1]), flush=True)
+    for C, n in SHAPES:
+        row = {r: block_leg(B, C, n, r, args.warmup, args.reps, args.mlp_ratio, shifts) for r in ("fp32", "bf16-old", "bf16-new")}
         row["new_vs_old"] = row["bf16-old"]["ms"] / row["bf16-new"]["ms"]
         row["new_vs_fp32"] = row["fp32"]["ms"] / row["bf16-new"]["ms"]
         res["blocks"].append(row)
         print(json.dumps(row), flush=True)
     if not args.no_model:
         for r in ("fp32", "bf16-old", "bf16-new"):
-            res["model"].append(model_leg(r, 3, 5))
+            res["model"].append(model_leg(r, 3, 5, B=B, ratio=args.mlp_ratio, shifts=shifts))
             print(json.dumps(res["model"][-1]), flush=True)
     os.makedirs(os.path.dirname(os.path.abspath(args.out)), exist_ok=True)
     with open(args.out, "w") as f:

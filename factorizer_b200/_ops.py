@@ -590,8 +590,9 @@ def _ld8(n: int) -> int:
 
 
 def bf16_core_supported(geom: Geometry, spec: SolverSpec, relu: bool = True) -> bool:
-    """The fused core takes bf16 volumes of this geometry (the octant kernels: head_dim 8, patch 8^3, shifts [0, 4], rank-1
-    HALS, an even number of patches along W)."""
+    """The fused core takes bf16 volumes of this geometry: the octant kernels (head_dim 8, patch 8^3, rank-1 HALS, an even
+    number of patches along W) at shifts [0, 4], or at window sets that pair up as (a, a + 4) with even base shifts along W,
+    such as the BraTS23 bundle's [0, 2, 4, 6]."""
     g, s = geom.c_geom(1, torch.bfloat16), spec.c_solver()
     return bool(L.lib().fz_swnmf_bf16_supported(ctypes.byref(g), ctypes.byref(s), int(relu)))
 

@@ -184,6 +184,11 @@ size_t fz_swnmf_workspace_bytes(const fz_geom* g, const fz_solver* s) {
     return a;
 }
 
+static const char* const kBf16Coverage =
+    "bf16 volumes are served by the octant kernels only (head_dim 8, patch 8x8x8, ReLU, rank-1 HALS, an even number of "
+    "patches along W, and window sets that pair up as (a, a + 4) with every base shift a even along W, e.g. shifts "
+    "[0, 4] or [0, 2, 4, 6])";
+
 int fz_swnmf_bf16_supported(const fz_geom* g, const fz_solver* s, int32_t relu_input) {
     if (!g || !s) return 0;
     fz_geom gb = *g;
@@ -191,7 +196,7 @@ int fz_swnmf_bf16_supported(const fz_geom* g, const fz_solver* s, int32_t relu_i
     DevGeom G;
     int K;
     if (make_dev_geom(&gb, &G) || check_solver(s, G.d, G.P, &K)) return 0;
-    return phase_supported(G, *s, relu_input) ? 1 : 0;
+    return phase_supported(G, *s, relu_input) || pairs_supported(G, *s, relu_input) ? 1 : 0;
 }
 
 int fz_swnmf_forward(const float* x, const float* u0, const float* v0, float* y, void* saved,
@@ -214,15 +219,13 @@ int fz_swnmf_forward(const float* x, const float* u0, const float* v0, float* y,
         tls().path = 2;
         return phase_forward(x, v0, y, saved, workspace, G, *s, (cudaStream_t)stream);
     }
-    if (G.dtype != FZ_DTYPE_F32)
-        return fail(FZ_ERR_UNSUPPORTED, "bf16 volumes are served by the octant kernels only (head_dim 8, patch 8x8x8, shifts "
-                    "[0, 4], ReLU, rank-1 HALS, an even number of patches along W)");
     if (octant_ok && pairs_supported(G, *s, relu_input)) {
         tls().path = 4;
         const int e = pairs_forward(x, v0, y, saved, workspace, G, *s, (cudaStream_t)stream);
         tls().path = 4;
         return e;
     }
+    if (G.dtype != FZ_DTYPE_F32) return fail(FZ_ERR_UNSUPPORTED, "%s", kBf16Coverage);
     if (fast_ok && fast_supported(G, *s)) {
         tls().path = 1;
         return fast_forward(x, u0, v0, y, saved, workspace, G, *s, relu_input, (cudaStream_t)stream);
@@ -264,13 +267,11 @@ int fz_swnmf_backward(const float* x, const float* gy, const float* u0, const fl
         tls().path = 2;
         return phase_backward(x, gy, v0, saved, gx, workspace, G, *s, K, (cudaStream_t)stream);
     }
-    if (G.dtype != FZ_DTYPE_F32)
-        return fail(FZ_ERR_UNSUPPORTED, "bf16 volumes are served by the octant kernels only (head_dim 8, patch 8x8x8, shifts "
-                    "[0, 4], ReLU, rank-1 HALS, an even number of patches along W)");
     if (octant_ok && pairs_supported(G, *s, relu_input)) {
         tls().path = 4;
         return pairs_backward(x, gy, v0, saved, gx, workspace, G, *s, K, (cudaStream_t)stream);
     }
+    if (G.dtype != FZ_DTYPE_F32) return fail(FZ_ERR_UNSUPPORTED, "%s", kBf16Coverage);
     if (fast_ok && fast_supported(G, *s)) {
         tls().path = 1;
         return fast_backward(x, gy, u0, v0, saved, gx, workspace, G, *s, K, relu_input,

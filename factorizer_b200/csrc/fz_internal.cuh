@@ -52,13 +52,14 @@ int small_direct(const float* x, const float* u0, const float* v0, const float* 
 int small_window(const float* x, const float* u0, const float* v0, const float* gy, float* out, const DevGeom& G,
                  const fz_solver& s, int K, int relu, bool bwd, cudaStream_t st);
 
-// fz_swnmf_phase.cu: three-pass "octant" formulation for [unshifted, shifted by patch/2], act = ReLU
+// fz_swnmf_phase.cu: three-pass "octant" formulation for [unshifted, shifted by patch/2], act = ReLU.  y / gx have the
+// volume's element type, or fp32 with f32_out (the partial sums of the paired variant below)
 bool phase_supported(const DevGeom& G, const fz_solver& s, int relu);
 size_t phase_workspace_bytes(const DevGeom& G, const fz_solver& s);
 int phase_forward(const float* x, const float* v0, float* y, void* saved, void* workspace,
-                  const DevGeom& G, const fz_solver& s, cudaStream_t st);
+                  const DevGeom& G, const fz_solver& s, cudaStream_t st, bool f32_out = false);
 int phase_backward(const float* x, const float* gy, const float* v0, const void* saved, float* gx,
-                   void* workspace, const DevGeom& G, const fz_solver& s, int K, cudaStream_t st);
+                   void* workspace, const DevGeom& G, const fz_solver& s, int K, cudaStream_t st, bool f32_out = false);
 
 // fz_swnmf_pipe.cu: the same formulation as ONE persistent, software-pipelined launch per direction (large volumes)
 bool pipe_supported(const DevGeom& G, const fz_solver& s, int relu, int force);

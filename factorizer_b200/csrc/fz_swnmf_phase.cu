@@ -3,6 +3,8 @@
 // whole volume.  Used for volumes that fit the L2 anyway (nothing to gain from pipelining the passes), as the inner
 // step of the paired-window-set variant at the end of this file, and as the reference the pipelined scheme
 // (fz_swnmf_pipe.cu, the production path for large volumes) is tested against.
+#include <initializer_list>
+
 #include "fz_swnmf_octant.cuh"
 
 namespace fz {
@@ -116,8 +118,9 @@ __global__ void __launch_bounds__(128) phase_fwd_solve(const __grid_constant__ P
 
 // =====================================================================================================
 // forward pass 3: y = 1/2 (u_0 v_0^T + u_1 v_1^T) voxel by voxel, v_s = relu(rd_s (X^T u_s + eps))
+// OutT: the volume's own type, or fp32 for a bf16 volume whose y is a partial sum (the paired window sets below)
 // =====================================================================================================
-template <bool BF16>
+template <bool BF16, typename OutT = typename TileOf<BF16>::out_t>
 __global__ void __launch_bounds__(kW3 * 32, 1) phase_fwd_apply(const __grid_constant__ PhaseParams P) {
     extern __shared__ __align__(1024) unsigned char smem_raw[];
     __shared__ uint64_t bars[kW3][2];
@@ -172,7 +175,7 @@ __global__ void __launch_bounds__(kW3 * 32, 1) phase_fwd_apply(const __grid_cons
                 mbar_wait(&bars[warp][st], parity[st]);
                 parity[st] ^= 1;
             }
-            fwd_tile_apply_t<!BF16, false, typename TileOf<BF16>::type, typename TileOf<BF16>::out_t>(P, tile_at<BF16>(buf + st * 4096, half), f0, f1, c, lane);
+            fwd_tile_apply_t<!BF16, false, typename TileOf<BF16>::type, OutT>(P, tile_at<BF16>(buf + st * 4096, half), f0, f1, c, lane);
         }
     }
 }
@@ -256,8 +259,9 @@ __global__ void __launch_bounds__(kSolveThreads) phase_bwd_solve(const __grid_co
 
 // =====================================================================================================
 // backward pass 3: dx = [x > 0] sum_s ( rd_s u_s (u_s . g)/2 + M_s x + m_s + abar1_s v0[col_s] ) voxel by voxel
+// OutT as in forward pass 3
 // =====================================================================================================
-template <bool BF16>
+template <bool BF16, typename OutT = typename TileOf<BF16>::out_t>
 __global__ void __launch_bounds__(kWB * 32, 1) phase_bwd_apply(const __grid_constant__ PhaseParams P) {
     constexpr int kPer = BF16 ? 2 : 1;
     extern __shared__ __align__(1024) unsigned char smem_raw[];
@@ -316,7 +320,7 @@ __global__ void __launch_bounds__(kWB * 32, 1) phase_bwd_apply(const __grid_cons
                 parity[st] ^= 1;
             }
             const TileCoord c = tile_coord(P, tile_of(q));
-            bwd_tile_apply_t<false, typename TileOf<BF16>::type, typename TileOf<BF16>::out_t>(
+            bwd_tile_apply_t<false, typename TileOf<BF16>::type, OutT>(
                 P, tile_at<BF16>(buf + st * 8192, half), tile_at<BF16>(buf + st * 8192 + 4096, half), mbs_all[warp][q & 1], v0s, c, lane);
             __syncwarp();                                             // records of tile q are free for tile q + 2
         }
@@ -375,7 +379,7 @@ size_t phase_workspace_bytes(const DevGeom& G, const fz_solver& s) {
 }
 
 int phase_forward(const float* x, const float* v0, float* y, void* saved, void* workspace,
-                  const DevGeom& G, const fz_solver& s, cudaStream_t st) {
+                  const DevGeom& G, const fz_solver& s, cudaStream_t st, bool f32_out) {
     if (!workspace) return fail(FZ_ERR_INVALID, "fz_swnmf_forward: workspace of %zu bytes required", phase_workspace_bytes(G, s));
     if (reinterpret_cast<uintptr_t>(y) & 15) return fail(FZ_ERR_INVALID, "output pointer %p is not 16-byte aligned", (void*)y);
     static thread_local PhaseParams P;
@@ -383,10 +387,11 @@ int phase_forward(const float* x, const float* v0, float* y, void* saved, void* 
     if (int e = make_tile_map(&P.tm_x, x, G)) return e;
     P.x = x; P.out = y; P.v0 = v0; P.saved = static_cast<float*>(saved);
     const bool bf16 = G.dtype == FZ_DTYPE_BF16;
-    static SmemConfig cfg_gram, cfg_apply, cfg_gram_h, cfg_apply_h;
+    static SmemConfig cfg_gram, cfg_apply, cfg_gram_h, cfg_apply_h, cfg_apply_hf;
     if (bf16) {
         FZ_CUDA_CHECK(cfg_gram_h.ensure(phase_fwd_gram<true>, kW1 * 2 * kTileBytes));
-        FZ_CUDA_CHECK(cfg_apply_h.ensure(phase_fwd_apply<true>, kW3 * 2 * kTileBytes));
+        if (f32_out) FZ_CUDA_CHECK(cfg_apply_hf.ensure(phase_fwd_apply<true, float>, kW3 * 2 * kTileBytes));
+        else FZ_CUDA_CHECK(cfg_apply_h.ensure(phase_fwd_apply<true>, kW3 * 2 * kTileBytes));
     } else {
         FZ_CUDA_CHECK(cfg_gram.ensure(phase_fwd_gram<false>, kW1 * 2 * kTileBytes));
         FZ_CUDA_CHECK(cfg_apply.ensure(phase_fwd_apply<false>, kW3 * 2 * kTileBytes));
@@ -401,14 +406,15 @@ int phase_forward(const float* x, const float* v0, float* y, void* saved, void* 
     const long long groups = 2LL * P.t_count;
     phase_fwd_solve<<<(unsigned)((groups * 8 + 127) / 128), 128, 0, st>>>(P);
     FZ_LAUNCH_CHECK();
-    if (bf16) phase_fwd_apply<true><<<grid_for(units, kW3), kW3 * 32, kW3 * 2 * kTileBytes, st>>>(P);
+    if (bf16 && f32_out) phase_fwd_apply<true, float><<<grid_for(units, kW3), kW3 * 32, kW3 * 2 * kTileBytes, st>>>(P);
+    else if (bf16) phase_fwd_apply<true><<<grid_for(units, kW3), kW3 * 32, kW3 * 2 * kTileBytes, st>>>(P);
     else phase_fwd_apply<false><<<grid_for(units, kW3), kW3 * 32, kW3 * 2 * kTileBytes, st>>>(P);
     FZ_LAUNCH_CHECK();
     return FZ_OK;
 }
 
 int phase_backward(const float* x, const float* gy, const float* v0, const void* saved, float* gx,
-                   void* workspace, const DevGeom& G, const fz_solver& s, int K, cudaStream_t st) {
+                   void* workspace, const DevGeom& G, const fz_solver& s, int K, cudaStream_t st, bool f32_out) {
     if (!workspace) return fail(FZ_ERR_INVALID, "fz_swnmf_backward: workspace of %zu bytes required", phase_workspace_bytes(G, s));
     if (!saved) return fail(FZ_ERR_INVALID, "fz_swnmf_backward: the `saved` buffer written by fz_swnmf_forward is required");
     if (reinterpret_cast<uintptr_t>(gx) & 15) return fail(FZ_ERR_INVALID, "output pointer %p is not 16-byte aligned", (void*)gx);
@@ -419,10 +425,11 @@ int phase_backward(const float* x, const float* gy, const float* v0, const void*
     P.x = x; P.gy = gy; P.out = gx; P.v0 = v0;
     P.saved = const_cast<float*>(static_cast<const float*>(saved));
     const bool bf16 = G.dtype == FZ_DTYPE_BF16;
-    static SmemConfig cfg_reduce, cfg_apply, cfg_reduce_h, cfg_apply_h;
+    static SmemConfig cfg_reduce, cfg_apply, cfg_reduce_h, cfg_apply_h, cfg_apply_hf;
     if (bf16) {
         FZ_CUDA_CHECK(cfg_reduce_h.ensure(phase_bwd_reduce<true>, kWB * 4 * kTileBytes));
-        FZ_CUDA_CHECK(cfg_apply_h.ensure(phase_bwd_apply<true>, kWB * 4 * kTileBytes));
+        if (f32_out) FZ_CUDA_CHECK(cfg_apply_hf.ensure(phase_bwd_apply<true, float>, kWB * 4 * kTileBytes));
+        else FZ_CUDA_CHECK(cfg_apply_h.ensure(phase_bwd_apply<true>, kWB * 4 * kTileBytes));
     } else {
         FZ_CUDA_CHECK(cfg_reduce.ensure(phase_bwd_reduce<false>, kWB * 4 * kTileBytes));
         FZ_CUDA_CHECK(cfg_apply.ensure(phase_bwd_apply<false>, kWB * 4 * kTileBytes));
@@ -437,7 +444,8 @@ int phase_backward(const float* x, const float* gy, const float* v0, const void*
     const long long groups = 2LL * P.t_count;
     phase_bwd_solve<<<(unsigned)((groups + kSolveThreads - 1) / kSolveThreads), kSolveThreads, 0, st>>>(P);
     FZ_LAUNCH_CHECK();
-    if (bf16) phase_bwd_apply<true><<<grid_for(units, kWB), kWB * 32, kWB * 4 * kTileBytes, st>>>(P);
+    if (bf16 && f32_out) phase_bwd_apply<true, float><<<grid_for(units, kWB), kWB * 32, kWB * 4 * kTileBytes, st>>>(P);
+    else if (bf16) phase_bwd_apply<true><<<grid_for(units, kWB), kWB * 32, kWB * 4 * kTileBytes, st>>>(P);
     else phase_bwd_apply<false><<<grid_for(units, kWB), kWB * 32, kWB * 4 * kTileBytes, st>>>(P);
     FZ_LAUNCH_CHECK();
     return FZ_OK;
@@ -449,25 +457,33 @@ int phase_backward(const float* x, const float* gy, const float* v0, const void*
 //   sum_{s in {a, a+4}} inv_s(NMF(win(roll(x, s)))) = roll( octant(roll(x, a)), -a )
 // (torch.roll composes: roll(x, a + 4) = roll(roll(x, a), 4); operations.py:266-280), so e.g. the brats23
 // bundle's shifts [0, 2, 4, 6] (model_zoo/factorizer_brats23/configs/train.yaml:50-54) run as two octant
-// problems plus one roll and one roll-and-combine pass per pair instead of four window-at-a-time sweeps.
+// problems plus one roll and one roll-and-combine pass per pair instead of four window-at-a-time sweeps.  A bf16 volume
+// is rolled as bf16 (an exact copy) and the pairs' partial sums stay fp32 until the last combine writes the bf16 result.
 // =====================================================================================================
 namespace {
 
 struct RollParams { int n0, n1, n2, s0, s1, s2; long long rows, vox; };
 
-// out[r][i] = in[r][(i - s) mod n]   (torch.roll).  One CTA per (row, i0) plane; V = 2 or 4 neighbouring voxels per
-// thread (n2 and s2 multiples of V), 32-bit index math.
-template <int V>
-__global__ void __launch_bounds__(256) roll_volume(const float* __restrict__ in, float* __restrict__ out, const RollParams R) {
-    typedef typename std::conditional<V == 4, float4, float2>::type vec;
+// V neighbouring elements as one access: fp32 8 or 16 bytes, bf16 4 or 8 bytes
+template <typename T, int V> struct VecOf;
+template <> struct VecOf<float, 2> { typedef float2 type; };
+template <> struct VecOf<float, 4> { typedef float4 type; };
+template <> struct VecOf<__nv_bfloat16, 2> { typedef unsigned int type; };
+template <> struct VecOf<__nv_bfloat16, 4> { typedef uint2 type; };
+
+// out[r][i] = in[r][(i - s) mod n]   (torch.roll), an exact copy for either element type.  One CTA per (row, i0) plane;
+// V = 2 or 4 neighbouring voxels per thread (n2 and s2 multiples of V), 32-bit index math.
+template <typename T, int V>
+__global__ void __launch_bounds__(256) roll_volume(const T* __restrict__ in, T* __restrict__ out, const RollParams R) {
+    typedef typename VecOf<T, V>::type vec;
     const int hv = R.n2 / V, per_plane = R.n1 * hv;
     for (long long pl = blockIdx.x; pl < R.rows * R.n0; pl += gridDim.x) {
         const long long r = pl / R.n0;
         const int i0 = (int)(pl - r * R.n0);
         int j0 = i0 - R.s0;
         if (j0 < 0) j0 += R.n0;
-        const float* src = in + r * R.vox + (long long)j0 * R.n1 * R.n2;
-        float* dst = out + r * R.vox + (long long)i0 * R.n1 * R.n2;
+        const T* src = in + r * R.vox + (long long)j0 * R.n1 * R.n2;
+        T* dst = out + r * R.vox + (long long)i0 * R.n1 * R.n2;
         for (int t = threadIdx.x; t < per_plane; t += blockDim.x) {
             const int i1 = t / hv, i2 = (t - i1 * hv) * V;
             int j1 = i1 - R.s1, j2 = i2 - R.s2;
@@ -478,10 +494,12 @@ __global__ void __launch_bounds__(256) roll_volume(const float* __restrict__ in,
     }
 }
 
-// acc[r][i] = ((first ? 0 : acc[r][i]) + part[r][(i + s) mod n]) * scale   (the inverse roll, summed over the pairs)
-template <int V>
+// acc[r][i] = ((first ? 0 : acc[r][i]) + part[r][(i + s) mod n]) * scale   (the inverse roll, summed over the pairs).
+// T = bf16: the last call for a bf16 volume, which writes that sum to y[r][i] instead of acc, rounded to bf16 once
+// (T = float leaves y unused).
+template <int V, typename T>
 __global__ void __launch_bounds__(256) unroll_combine(float* __restrict__ acc, const float* __restrict__ part, const RollParams R,
-                                                      int first, float scale) {
+                                                      int first, float scale, T* __restrict__ y) {
     typedef typename std::conditional<V == 4, float4, float2>::type vec;
     const int hv = R.n2 / V, per_plane = R.n1 * hv;
     for (long long pl = blockIdx.x; pl < R.rows * R.n0; pl += gridDim.x) {
@@ -507,7 +525,15 @@ __global__ void __launch_bounds__(256) unroll_combine(float* __restrict__ acc, c
             }
 #pragma unroll
             for (int q = 0; q < V; ++q) vf[q] *= scale;
-            *d = v;
+            if constexpr (std::is_same<T, float>::value) {
+                *d = v;
+            } else {
+                typename VecOf<T, V>::type h;
+                __nv_bfloat162* hp = reinterpret_cast<__nv_bfloat162*>(&h);
+#pragma unroll
+                for (int q = 0; q < V / 2; ++q) hp[q] = __floats2bfloat162_rn(vf[2 * q], vf[2 * q + 1]);
+                *reinterpret_cast<typename VecOf<T, V>::type*>(y + r * R.vox + (long long)i0 * R.n1 * R.n2 + i1 * R.n2 + i2) = h;
+            }
         }
     }
 }
@@ -545,31 +571,69 @@ DevGeom pair_geom(const DevGeom& G) {
     return P;
 }
 
-size_t vol_bytes(const DevGeom& G) { return align_up((size_t)G.B * G.C * G.vox * sizeof(float), 256); }
+size_t vol_bytes(const DevGeom& G, size_t elem) { return align_up((size_t)G.B * G.C * G.vox * elem, 256); }
+size_t elem_bytes(const DevGeom& G) { return G.dtype == FZ_DTYPE_BF16 ? sizeof(__nv_bfloat16) : sizeof(float); }
+
+// The workspace of the paired scheme: the octant kernels' own, then the rolled x and the rolled dY (the volume's element
+// type), the partial sum of one pair (fp32) and, for bf16 volumes, the fp32 sum over the pairs (fp32 volumes sum in y / dX).
+struct PairBufs { float *xr, *gr, *part, *acc; };
+PairBufs pair_bufs(void* workspace, const DevGeom& G, const fz_solver& s, float* out) {
+    char* p = static_cast<char*>(workspace) + align_up(phase_workspace_bytes(pair_geom(G), s), 256);
+    PairBufs b;
+    b.xr = reinterpret_cast<float*>(p);
+    p += vol_bytes(G, elem_bytes(G));
+    b.gr = reinterpret_cast<float*>(p);
+    p += vol_bytes(G, elem_bytes(G));
+    b.part = reinterpret_cast<float*>(p);
+    p += vol_bytes(G, sizeof(float));
+    b.acc = G.dtype == FZ_DTYPE_BF16 ? reinterpret_cast<float*>(p) : out;
+    return b;
+}
 
 int launch_roll(const float* in, float* out, const DevGeom& G, const int* a, cudaStream_t st) {
     RollParams R = {G.n[0], G.n[1], G.n[2], a[0], a[1], a[2], (long long)G.B * G.C, G.vox};
     const long long planes = R.rows * R.n0;
     const unsigned grid = (unsigned)(planes < 65535LL * 16 ? planes : 65535LL * 16);
-    if (R.n2 % 4 == 0 && R.s2 % 4 == 0) roll_volume<4><<<grid, 256, 0, st>>>(in, out, R);
-    else roll_volume<2><<<grid, 256, 0, st>>>(in, out, R);
+    const bool v4 = R.n2 % 4 == 0 && R.s2 % 4 == 0;
+    if (G.dtype == FZ_DTYPE_BF16) {
+        const __nv_bfloat16* i = reinterpret_cast<const __nv_bfloat16*>(in);
+        __nv_bfloat16* o = reinterpret_cast<__nv_bfloat16*>(out);
+        if (v4) roll_volume<__nv_bfloat16, 4><<<grid, 256, 0, st>>>(i, o, R);
+        else roll_volume<__nv_bfloat16, 2><<<grid, 256, 0, st>>>(i, o, R);
+    } else {
+        if (v4) roll_volume<float, 4><<<grid, 256, 0, st>>>(in, out, R);
+        else roll_volume<float, 2><<<grid, 256, 0, st>>>(in, out, R);
+    }
     FZ_LAUNCH_CHECK();
     return FZ_OK;
 }
-int launch_combine(float* acc, const float* part, const DevGeom& G, const int* a, int first, float scale, cudaStream_t st) {
+// adds pair partial `part` into acc; y: the last call for a bf16 volume, which writes the finished bf16 sum there
+int launch_combine(float* acc, const float* part, const DevGeom& G, const int* a, int first, float scale, float* y, cudaStream_t st) {
     RollParams R = {G.n[0], G.n[1], G.n[2], a[0], a[1], a[2], (long long)G.B * G.C, G.vox};
     const long long planes = R.rows * R.n0;
     const unsigned grid = (unsigned)(planes < 65535LL * 16 ? planes : 65535LL * 16);
-    if (R.n2 % 4 == 0 && R.s2 % 4 == 0) unroll_combine<4><<<grid, 256, 0, st>>>(acc, part, R, first, scale);
-    else unroll_combine<2><<<grid, 256, 0, st>>>(acc, part, R, first, scale);
+    const bool v4 = R.n2 % 4 == 0 && R.s2 % 4 == 0;
+    if (y) {
+        __nv_bfloat16* h = reinterpret_cast<__nv_bfloat16*>(y);
+        if (v4) unroll_combine<4, __nv_bfloat16><<<grid, 256, 0, st>>>(acc, part, R, first, scale, h);
+        else unroll_combine<2, __nv_bfloat16><<<grid, 256, 0, st>>>(acc, part, R, first, scale, h);
+    } else {
+        if (v4) unroll_combine<4, float><<<grid, 256, 0, st>>>(acc, part, R, first, scale, nullptr);
+        else unroll_combine<2, float><<<grid, 256, 0, st>>>(acc, part, R, first, scale, nullptr);
+    }
     FZ_LAUNCH_CHECK();
+    return FZ_OK;
+}
+
+int check_bf16_pointers(std::initializer_list<const void*> ptrs) {
+    for (const void* p : ptrs)
+        if (reinterpret_cast<uintptr_t>(p) & 15) return fail(FZ_ERR_INVALID, "bf16 volume pointer %p is not 16-byte aligned", p);
     return FZ_OK;
 }
 
 }  // namespace
 
 bool pairs_supported(const DevGeom& G, const fz_solver& s, int relu) {
-    if (G.dtype != FZ_DTYPE_F32) return false;        // the roll / combine passes are fp32
     if (G.S < 2 || G.S % 2 || G.n[2] % 2) return false;
     int base[FZ_MAX_SHIFTS][3];
     if (!find_pairs(G, base)) return false;
@@ -583,36 +647,38 @@ size_t pairs_saved_bytes(const DevGeom& G, const fz_solver& s) {
 }
 
 size_t pairs_workspace_bytes(const DevGeom& G, const fz_solver& s) {
-    return align_up(phase_workspace_bytes(pair_geom(G), s), 256) + 3 * vol_bytes(G);
+    const size_t f32_vols = G.dtype == FZ_DTYPE_BF16 ? 2 : 1;
+    return align_up(phase_workspace_bytes(pair_geom(G), s), 256) + 2 * vol_bytes(G, elem_bytes(G)) + f32_vols * vol_bytes(G, sizeof(float));
 }
 
+// Every pair's octant kernels write an fp32 partial sum (the unshifted pair's straight into the sum); a bf16 volume's y is
+// written once, by the last combine, so the partial sums are never rounded to bf16.
 int pairs_forward(const float* x, const float* v0, float* y, void* saved, void* workspace, const DevGeom& G,
                   const fz_solver& s, cudaStream_t st) {
     if (!workspace) return fail(FZ_ERR_INVALID, "fz_swnmf_forward: workspace of %zu bytes required", pairs_workspace_bytes(G, s));
+    const bool bf16 = G.dtype == FZ_DTYPE_BF16;
+    if (bf16) if (int e = check_bf16_pointers({x, y})) return e;
     const DevGeom Gp = pair_geom(G);
     int base[FZ_MAX_SHIFTS][3];
     find_pairs(G, base);
     const int np = G.S / 2;
-    char* ws = static_cast<char*>(workspace);
-    float* bufA = reinterpret_cast<float*>(ws + align_up(phase_workspace_bytes(Gp, s), 256));
-    float* bufB = reinterpret_cast<float*>(reinterpret_cast<char*>(bufA) + vol_bytes(G));
+    const PairBufs b = pair_bufs(workspace, G, s, y);
     const size_t saved_stride = (size_t)2 * Gp.mats_per_shift * (rec_head_for(s.num_iters) + 72) * sizeof(float);
     for (int k = 0; k < np; ++k) {
         const bool rolled = base[k][0] || base[k][1] || base[k][2];
         const float* xin = x;
         if (rolled) {
-            if (int e = launch_roll(x, bufA, G, base[k], st)) return e;
-            xin = bufA;
+            if (int e = launch_roll(x, b.xr, G, base[k], st)) return e;
+            xin = b.xr;
         }
-        const bool direct = !rolled && k == 0;       // the unshifted pair writes (the start of) the sum in place
         void* sv = saved ? static_cast<char*>(saved) + k * saved_stride : nullptr;
-        if (int e = phase_forward(xin, v0, direct ? y : bufB, sv, workspace, Gp, s, st)) return e;
-        const float scale = k == np - 1 ? 1.f / (float)np : 1.f;
-        if (!direct) {
-            if (int e = launch_combine(y, bufB, G, base[k], k == 0, scale, st)) return e;
-        } else if (np == 1) {
-            return FZ_OK;
-        }
+        if (!rolled && np == 1) return phase_forward(xin, v0, y, sv, workspace, Gp, s, st);
+        const bool direct = !rolled && k == 0;       // the unshifted pair writes (the start of) the sum in place
+        if (int e = phase_forward(xin, v0, direct ? b.acc : b.part, sv, workspace, Gp, s, st, true)) return e;
+        const bool last = k == np - 1;
+        if (!direct)
+            if (int e = launch_combine(b.acc, b.part, G, base[k], k == 0, last ? 1.f / (float)np : 1.f, bf16 && last ? y : nullptr, st))
+                return e;
     }
     return FZ_OK;
 }
@@ -621,31 +687,30 @@ int pairs_backward(const float* x, const float* gy, const float* v0, const void*
                    const DevGeom& G, const fz_solver& s, int K, cudaStream_t st) {
     if (!workspace) return fail(FZ_ERR_INVALID, "fz_swnmf_backward: workspace of %zu bytes required", pairs_workspace_bytes(G, s));
     if (!saved) return fail(FZ_ERR_INVALID, "fz_swnmf_backward: the `saved` buffer written by fz_swnmf_forward is required");
+    const bool bf16 = G.dtype == FZ_DTYPE_BF16;
+    if (bf16) if (int e = check_bf16_pointers({x, gy, gx})) return e;
     const DevGeom Gp = pair_geom(G);
     int base[FZ_MAX_SHIFTS][3];
     find_pairs(G, base);
     const int np = G.S / 2;
-    char* ws = static_cast<char*>(workspace);
-    float* bufA = reinterpret_cast<float*>(ws + align_up(phase_workspace_bytes(Gp, s), 256));
-    float* bufB = reinterpret_cast<float*>(reinterpret_cast<char*>(bufA) + vol_bytes(G));
-    float* bufC = reinterpret_cast<float*>(reinterpret_cast<char*>(bufB) + vol_bytes(G));
+    const PairBufs b = pair_bufs(workspace, G, s, gx);
     const size_t saved_stride = (size_t)2 * Gp.mats_per_shift * (rec_head_for(s.num_iters) + 72) * sizeof(float);
-    const float inv_np = 1.f / (float)np;
     for (int k = 0; k < np; ++k) {
         const bool rolled = base[k][0] || base[k][1] || base[k][2];
         const float *xin = x, *gin = gy;
         if (rolled) {
-            if (int e = launch_roll(x, bufA, G, base[k], st)) return e;
-            if (int e = launch_roll(gy, bufB, G, base[k], st)) return e;
-            xin = bufA; gin = bufB;
+            if (int e = launch_roll(x, b.xr, G, base[k], st)) return e;
+            if (int e = launch_roll(gy, b.gr, G, base[k], st)) return e;
+            xin = b.xr; gin = b.gr;
         }
-        const bool direct = !rolled && k == 0;
         const void* sv = static_cast<const char*>(saved) + k * saved_stride;
-        if (int e = phase_backward(xin, gin, v0, sv, direct ? gx : bufC, workspace, Gp, s, K, st)) return e;
-        const float scale = k == np - 1 ? inv_np : 1.f;
-        if (!direct) {
-            if (int e = launch_combine(gx, bufC, G, base[k], k == 0, scale, st)) return e;
-        }
+        if (!rolled && np == 1) return phase_backward(xin, gin, v0, sv, gx, workspace, Gp, s, K, st);
+        const bool direct = !rolled && k == 0;
+        if (int e = phase_backward(xin, gin, v0, sv, direct ? b.acc : b.part, workspace, Gp, s, K, st, true)) return e;
+        const bool last = k == np - 1;
+        if (!direct)
+            if (int e = launch_combine(b.acc, b.part, G, base[k], k == 0, last ? 1.f / (float)np : 1.f, bf16 && last ? gx : nullptr, st))
+                return e;
     }
     return FZ_OK;
 }

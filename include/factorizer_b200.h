@@ -55,8 +55,10 @@ typedef struct fz_geom {
     int32_t dtype;                      /* FZ_DTYPE_F32 (0) or FZ_DTYPE_BF16: element type of the VOLUMES handed to
                                            fz_swnmf_forward / _backward (x, y, dy, dx); u0, v0, the saved records and
                                            all arithmetic stay fp32.  bf16 is served by the octant kernels only
-                                           (head_dim 8, patch 8^3, shifts [0, 4], ReLU, rank-1 HALS, an even number of
-                                           patches along W); anything else returns FZ_ERR_UNSUPPORTED              */
+                                           (head_dim 8, patch 8^3, ReLU, rank-1 HALS, an even number of patches along
+                                           W) at shifts [0, 4] or at window sets that pair up as (a, a + 4) with even
+                                           base shifts along W, e.g. [0, 2, 4, 6]; anything else returns
+                                           FZ_ERR_UNSUPPORTED                                                      */
     int32_t path;                       /* FZ_PATH_AUTO (0), or one of FZ_PATH_* to restrict the
                                            kernel family fz_swnmf_* may pick for this call (tests
                                            and measurements; a per-call argument, no global state) */
