@@ -15,8 +15,13 @@ those shifts the fused core took bf16 volumes only after the paired path learnt 
 core off there (FactMixer casts the core's input to fp32, as it did before).  --core adds the core alone at
 (--batch, 32, 128^3), fp32 against bf16 on the same path, forward and backward, each as one CUDA graph.
 
+--shifts isles22 configures the ISLES22 bundle's geometry instead: patch 4 (8 x 64 windows on the sub-warp kernels) at shifts
+[None, 1, 2, 3], blocks at the stages of a 64^3 ROI, the model at 64^3, the core at (--batch, 32, 64^3); use it with --batch 8.
+The fused core took bf16 volumes at patch 4 only after the sub-warp kernels learnt bf16, so bf16-old switches it off there too.
+
     python bench_probes/bf16_block_time.py --out /tmp/bf16_block_time.json
     python bench_probes/bf16_block_time.py --shifts bundle --mlp-ratio 4 --batch 2 --core --out /tmp/bundle.json
+    python bench_probes/bf16_block_time.py --shifts isles22 --batch 8 --core --out /tmp/isles22.json
 """
 import argparse
 import json
@@ -32,7 +37,12 @@ import factorizer_b200 as ft  # noqa: E402
 from factorizer_b200 import _ops  # noqa: E402
 
 SHAPES = [(32, 128), (64, 64), (128, 32), (256, 16)]
-SHIFTS = {"default": None, "bundle": [None, 2, 4, 6]}
+SHIFTS = {"default": None, "bundle": [None, 2, 4, 6], "isles22": [None, 1, 2, 3]}
+ISLES22_SHAPES = [(32, 64), (64, 32), (128, 16), (256, 8), (512, 4)]      # (channels, n) of the stages of a 64^3 ROI
+
+
+def patch_of(shifts):
+    return 4 if shifts == SHIFTS["isles22"] else 8
 
 
 def card():
@@ -62,7 +72,7 @@ class _Route:
 
 
 def reshape(shifts):
-    kw = {"head_dim": 8, "patch_size": 8}
+    kw = {"head_dim": 8, "patch_size": patch_of(shifts)}
     if shifts is not None:
         kw["shifts"] = shifts
     return (ft.SWMatricize, kw)
@@ -157,7 +167,7 @@ def core_leg(B, shifts, dtype, warmup, reps, C=32, n=128):
     """the fused core alone (SWMatricize -> ReLU -> HALS -> inverse), forward and backward as separate graphs"""
     from factorizer_b200 import _lib
     geom = reshape(shifts)[0]((None, C, n, n, n), **reshape(shifts)[1])._geom
-    nmf = ft.NMF((8, 512), rank=1, num_iters=5, init="uniform", solver="hals").cuda()
+    nmf = ft.NMF((8, patch_of(shifts) ** 3), rank=1, num_iters=5, init="uniform", solver="hals").cuda()
     spec, u0, v0 = nmf.solver_spec(), nmf.init.u0, nmf.init.v0
     x = torch.randn(B, C, n, n, n, device="cuda").to(dtype)
     gy = torch.randn(B, C, n, n, n, device="cuda").to(dtype)
@@ -182,12 +192,14 @@ def main():
     torch.backends.cuda.matmul.allow_tf32 = False
     torch.backends.cudnn.allow_tf32 = False
     shifts, B = SHIFTS[args.shifts], args.batch
+    isles = args.shifts == "isles22"
+    n_model = 64 if isles else 128
     res = {"card": card(), "shifts": args.shifts, "mlp_ratio": args.mlp_ratio, "batch": B, "core": [], "blocks": [], "model": []}
     if args.core:
         for dtype in (torch.float32, torch.bfloat16):
-            res["core"].append(core_leg(B, shifts, dtype, args.warmup, args.reps))
+            res["core"].append(core_leg(B, shifts, dtype, args.warmup, args.reps, n=n_model))
             print(json.dumps(res["core"][-1]), flush=True)
-    for C, n in SHAPES:
+    for C, n in ISLES22_SHAPES if isles else SHAPES:
         row = {r: block_leg(B, C, n, r, args.warmup, args.reps, args.mlp_ratio, shifts) for r in ("fp32", "bf16-old", "bf16-new")}
         row["new_vs_old"] = row["bf16-old"]["ms"] / row["bf16-new"]["ms"]
         row["new_vs_fp32"] = row["fp32"]["ms"] / row["bf16-new"]["ms"]
@@ -195,7 +207,7 @@ def main():
         print(json.dumps(row), flush=True)
     if not args.no_model:
         for r in ("fp32", "bf16-old", "bf16-new"):
-            res["model"].append(model_leg(r, 3, 5, B=B, ratio=args.mlp_ratio, shifts=shifts))
+            res["model"].append(model_leg(r, 3, 5, n=n_model, B=B, ratio=args.mlp_ratio, shifts=shifts))
             print(json.dumps(res["model"][-1]), flush=True)
     os.makedirs(os.path.dirname(os.path.abspath(args.out)), exist_ok=True)
     with open(args.out, "w") as f:

@@ -316,8 +316,8 @@ class SWNMF(_GradModeFunction):
 
     @staticmethod
     def forward(ctx, x, u0, v0, geom: Geometry, spec: SolverSpec, relu: bool):
-        # bf16 volumes (an extension: the reference runs fp32) are read and written as bf16 by the octant kernels; u0, v0,
-        # the saved records and all arithmetic stay fp32
+        # bf16 volumes (an extension: the reference runs fp32) are read and written as bf16 by the octant and sub-warp
+        # kernels; u0, v0, the saved records and all arithmetic stay fp32
         x = _check_vol(x, geom, "x", allow_bf16=True)
         u0 = L.require_cuda_f32(u0.float(), "u0")
         v0 = L.require_cuda_f32(v0.float(), "v0")
@@ -592,7 +592,8 @@ def _ld8(n: int) -> int:
 def bf16_core_supported(geom: Geometry, spec: SolverSpec, relu: bool = True) -> bool:
     """The fused core takes bf16 volumes of this geometry: the octant kernels (head_dim 8, patch 8^3, rank-1 HALS, an even
     number of patches along W) at shifts [0, 4], or at window sets that pair up as (a, a + 4) with even base shifts along W,
-    such as the BraTS23 bundle's [0, 2, 4, 6]."""
+    such as the BraTS23 bundle's [0, 2, 4, 6]; or the sub-warp kernels (64-column windows with head_dim 4..32, such as the
+    ISLES22 bundle's patch 4 at shifts [None, 1, 2, 3], and 8 x 16 / 128 / 256 windows) at any shifts, rank-1 HALS or MU."""
     g, s = geom.c_geom(1, torch.bfloat16), spec.c_solver()
     return bool(L.lib().fz_swnmf_bf16_supported(ctypes.byref(g), ctypes.byref(s), int(relu)))
 

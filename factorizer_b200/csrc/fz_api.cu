@@ -177,6 +177,10 @@ size_t fz_swnmf_workspace_bytes(const fz_geom* g, const fz_solver* s) {
         const size_t b = pairs_workspace_bytes(G, *s);
         if (b > a) a = b;
     }
+    if (small_window_supported(G, *s)) {
+        const size_t b = small_workspace_bytes(G);
+        if (b > a) a = b;
+    }
     if (big_window(G, *s)) {
         const size_t b = big_workspace_bytes(G.mats_per_shift, G.d, G.P, *s);
         if (b > a) a = b;
@@ -185,9 +189,15 @@ size_t fz_swnmf_workspace_bytes(const fz_geom* g, const fz_solver* s) {
 }
 
 static const char* const kBf16Coverage =
-    "bf16 volumes are served by the octant kernels only (head_dim 8, patch 8x8x8, ReLU, rank-1 HALS, an even number of "
+    "bf16 volumes are served by the octant kernels (head_dim 8, patch 8x8x8, ReLU, rank-1 HALS, an even number of "
     "patches along W, and window sets that pair up as (a, a + 4) with every base shift a even along W, e.g. shifts "
-    "[0, 4] or [0, 2, 4, 6])";
+    "[0, 4] or [0, 2, 4, 6]) and by the sub-warp kernels (64-column windows with head_dim 4, 8, 16 or 32, or 8 x 16, "
+    "8 x 128 or 8 x 256 windows, at any shifts, rank-1 HALS or MU with up to 5 iterations, ReLU or not)";
+
+// The window-at-a-time 8x512 kernels (path 1), the grid-wide (5) and the generic (0) kernels take fp32 volumes only.
+static bool bf16_small_ok(const DevGeom& G, const fz_solver& s) {
+    return G.path != FZ_PATH_GENERIC && small_window_supported(G, s);
+}
 
 int fz_swnmf_bf16_supported(const fz_geom* g, const fz_solver* s, int32_t relu_input) {
     if (!g || !s) return 0;
@@ -196,7 +206,7 @@ int fz_swnmf_bf16_supported(const fz_geom* g, const fz_solver* s, int32_t relu_i
     DevGeom G;
     int K;
     if (make_dev_geom(&gb, &G) || check_solver(s, G.d, G.P, &K)) return 0;
-    return phase_supported(G, *s, relu_input) || pairs_supported(G, *s, relu_input) ? 1 : 0;
+    return phase_supported(G, *s, relu_input) || pairs_supported(G, *s, relu_input) || bf16_small_ok(G, *s) ? 1 : 0;
 }
 
 int fz_swnmf_forward(const float* x, const float* u0, const float* v0, float* y, void* saved,
@@ -225,14 +235,18 @@ int fz_swnmf_forward(const float* x, const float* u0, const float* v0, float* y,
         tls().path = 4;
         return e;
     }
-    if (G.dtype != FZ_DTYPE_F32) return fail(FZ_ERR_UNSUPPORTED, "%s", kBf16Coverage);
+    if (G.dtype != FZ_DTYPE_F32) {
+        if (!bf16_small_ok(G, *s)) return fail(FZ_ERR_UNSUPPORTED, "%s", kBf16Coverage);
+        tls().path = 3;
+        return small_window(x, u0, v0, nullptr, y, workspace, G, *s, K, relu_input, false, (cudaStream_t)stream);
+    }
     if (fast_ok && fast_supported(G, *s)) {
         tls().path = 1;
         return fast_forward(x, u0, v0, y, saved, workspace, G, *s, relu_input, (cudaStream_t)stream);
     }
     if (fast_ok && small_window_supported(G, *s)) {
         tls().path = 3;
-        return small_window(x, u0, v0, nullptr, y, G, *s, K, relu_input, false, (cudaStream_t)stream);
+        return small_window(x, u0, v0, nullptr, y, workspace, G, *s, K, relu_input, false, (cudaStream_t)stream);
     }
     if (big_window(G, *s)) {
         tls().path = 5;
@@ -271,7 +285,11 @@ int fz_swnmf_backward(const float* x, const float* gy, const float* u0, const fl
         tls().path = 4;
         return pairs_backward(x, gy, v0, saved, gx, workspace, G, *s, K, (cudaStream_t)stream);
     }
-    if (G.dtype != FZ_DTYPE_F32) return fail(FZ_ERR_UNSUPPORTED, "%s", kBf16Coverage);
+    if (G.dtype != FZ_DTYPE_F32) {
+        if (!bf16_small_ok(G, *s)) return fail(FZ_ERR_UNSUPPORTED, "%s", kBf16Coverage);
+        tls().path = 3;
+        return small_window(x, u0, v0, gy, gx, workspace, G, *s, K, relu_input, true, (cudaStream_t)stream);
+    }
     if (fast_ok && fast_supported(G, *s)) {
         tls().path = 1;
         return fast_backward(x, gy, u0, v0, saved, gx, workspace, G, *s, K, relu_input,
@@ -279,7 +297,7 @@ int fz_swnmf_backward(const float* x, const float* gy, const float* u0, const fl
     }
     if (fast_ok && small_window_supported(G, *s)) {
         tls().path = 3;
-        return small_window(x, u0, v0, gy, gx, G, *s, K, relu_input, true, (cudaStream_t)stream);
+        return small_window(x, u0, v0, gy, gx, workspace, G, *s, K, relu_input, true, (cudaStream_t)stream);
     }
     if (big_window(G, *s)) {
         tls().path = 5;

@@ -44,13 +44,15 @@ int fast_backward(const float* x, const float* gy, const float* u0, const float*
                   const void* saved, float* gx, void* workspace, const DevGeom& G,
                   const fz_solver& s, int K, int relu, cudaStream_t st);
 
-// fz_swnmf_small.cu: rank-1 HALS / MU on small matrices (N = 64 with M = 4, 8, 16, 32; 8x16, 8x128, 8x256), a sub-warp each
+// fz_swnmf_small.cu: rank-1 HALS / MU on small matrices (N = 64 with M = 4, 8, 16, 32; 8x16, 8x128, 8x256), a sub-warp each.
+// Window mode takes fp32 or bf16 volumes; a bf16 volume at S >= 2 sums the window sets in an fp32 volume in the workspace
 bool small_supported(int M, int N, const fz_solver& s);
 bool small_window_supported(const DevGeom& G, const fz_solver& s);
+size_t small_workspace_bytes(const DevGeom& G);
 int small_direct(const float* x, const float* u0, const float* v0, const float* gy, float* out, long long n, int M, int N,
                  const fz_solver& s, int K, bool bwd, cudaStream_t st);
-int small_window(const float* x, const float* u0, const float* v0, const float* gy, float* out, const DevGeom& G,
-                 const fz_solver& s, int K, int relu, bool bwd, cudaStream_t st);
+int small_window(const float* x, const float* u0, const float* v0, const float* gy, float* out, void* workspace,
+                 const DevGeom& G, const fz_solver& s, int K, int relu, bool bwd, cudaStream_t st);
 
 // fz_swnmf_phase.cu: three-pass "octant" formulation for [unshifted, shifted by patch/2], act = ReLU.  y / gx have the
 // volume's element type, or fp32 with f32_out (the partial sums of the paired variant below)

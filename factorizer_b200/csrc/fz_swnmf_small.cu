@@ -17,6 +17,13 @@
 // (operations.py:426-433); consecutive sub-warps take windows that are neighbours along W, so a warp-wide
 // load still covers whole 32-byte sectors.  Division is reciprocal (MUFU + one Newton step) times numerator,
 // <= 1 ulp from the reference's true division (same deviation as the 8x512 kernels, DESIGN.md section 2).
+// Window mode also takes bf16 volumes (x, dL/dy in, y, dL/dx out; u, v, the iterates, the history and every sum stay fp32).
+// Their elements are read and written 2 bytes at a time: shifts 1 and 3 put window origins at odd W indices, where a column
+// pair is not 4-byte aligned.  The window sets then sum in an fp32 accumulator volume in the caller's workspace: set 0 writes
+// it, later sets read-add-store it, and the last set writes the finished sum to the bf16 output, rounded once.  So y / dL/dx
+// are the fp32 kernels' results on the same (bf16-representable) inputs, rounded to bf16.
+#include <cuda_bf16.h>
+
 #include "fz_device.cuh"
 #include "fz_internal.cuh"
 
@@ -26,17 +33,48 @@ namespace {
 constexpr int kTMax = 5;          // iterates kept (in shared memory) by the backward
 constexpr int kSmallThreads = 128;
 
+template <typename E>     // element type of the volumes: float, or __nv_bfloat16 in window mode
 struct SmallParams {
-    const float* x;       // window mode: volume; direct mode: (n, M, N)
-    const float* gy;      // backward: dL/dy, same layout as x
-    float* out;           // forward: y; backward: dL/dx
+    const E* x;           // window mode: volume; direct mode: (n, M, N)
+    const E* gy;          // backward: dL/dy, same layout as x
+    E* out;               // forward: y; backward: dL/dx
     const float* u0;      // (M)
     const float* v0;      // (N)
     long long n;          // matrices in this launch (windows of ONE set in window mode)
     int T, K, kind, relu, set, S, window;
     float eps;
     DevGeom G;
+    float* acc;           // bf16 volume, S >= 2: the fp32 sum over the window sets, laid out as the volume
 };
+
+// Where a window set's sums go.  `acc` is where a set > 0 reads the sums so far.  An fp32 volume read-add-stores in `out`.  A
+// bf16 volume at S >= 2 sums in the fp32 accumulator, and its last set writes `out`, rounded once; at S == 1, set 0 writes
+// `out` directly.
+template <typename E>
+struct SetSums;
+template <>
+struct SetSums<float> {
+    float* acc;
+    __device__ __forceinline__ SetSums(const SmallParams<float>& P, long long base) : acc(P.out + base) {}
+    // v before i: the evaluation order of `acc[i] = v`, which keeps the fp32 kernels' code as it was
+    __device__ __forceinline__ void store(float v, int i) const { acc[i] = v; }
+};
+template <>
+struct SetSums<__nv_bfloat16> {
+    const SmallParams<__nv_bfloat16>& P;      // `out` is addressed from P at each store: two more live pointers spill
+    long long base;
+    float* acc;
+    __device__ __forceinline__ SetSums(const SmallParams<__nv_bfloat16>& P_, long long base_) : P(P_), base(base_), acc(P_.acc + base_) {}
+    __device__ __forceinline__ void store(float v, int i) const {
+        if (P.set < P.S - 1) acc[i] = v;
+        else P.out[base + i] = __float2bfloat16_rn(v);
+    }
+};
+
+// element i of a volume, as float; the unsigned bf16 index gives one IMAD.WIDE.U32 per address (a signed one takes three
+// instructions and a register more)
+__device__ __forceinline__ float ld_at(const float* p, int i) { return __ldg(p + i); }
+__device__ __forceinline__ float ld_at(const __nv_bfloat16* p, int i) { return __bfloat162float(__ldg(p + (unsigned)i)); }
 
 template <int L>
 __device__ __forceinline__ float group_sum(float v) {
@@ -46,11 +84,11 @@ __device__ __forceinline__ float group_sum(float v) {
 }
 
 // element offsets (relative to the (batch, head) base) of this lane's CPL columns of matrix `mid`
-template <int M, int CPL, int L>
+template <typename E, int M, int CPL, int L>
 struct Locator {
     int rel[CPL];     // offset of column 2 ((k >> 1) L + lane) + (k & 1) relative to the window origin (no wrap)
     int lane_;
-    __device__ __forceinline__ void init(const SmallParams& P, int lane) {
+    __device__ __forceinline__ void init(const SmallParams<E>& P, int lane) {
         lane_ = lane;
 #pragma unroll
         for (int k = 0; k < CPL; ++k) {
@@ -66,7 +104,7 @@ struct Locator {
         }
     }
     // returns the base offset (channel row 0) and fills off[]
-    __device__ __forceinline__ long long locate(const SmallParams& P, long long mid, int (&off)[CPL]) const {
+    __device__ __forceinline__ long long locate(const SmallParams<E>& P, long long mid, int (&off)[CPL]) const {
         if (!P.window) {
 #pragma unroll
             for (int k = 0; k < CPL; ++k) off[k] = rel[k];
@@ -161,13 +199,13 @@ __device__ __forceinline__ void step_v(const f2 (&x)[M][H], const float (&u)[M],
     }
 }
 
-template <int M, int CPL, int L>
-__global__ void __launch_bounds__(kSmallThreads, 3) small_fwd(const SmallParams P) {
+template <typename E, int M, int CPL, int L>
+__global__ void __launch_bounds__(kSmallThreads, 3) small_fwd(const SmallParams<E> P) {
     constexpr int H = CPL / 2;
     const int lane = threadIdx.x & (L - 1);
     const long long groups = (long long)gridDim.x * (kSmallThreads / L);
     const long long g0 = ((long long)blockIdx.x * kSmallThreads + threadIdx.x) / L;
-    Locator<M, CPL, L> loc;
+    Locator<E, M, CPL, L> loc;
     loc.init(P, lane);
     const int istride = P.window ? (int)P.G.vox : CPL * L;
     const float invS = 1.f / (float)P.S;
@@ -179,7 +217,7 @@ __global__ void __launch_bounds__(kSmallThreads, 3) small_fwd(const SmallParams 
         const long long base = loc.locate(P, valid ? mid : 0, off);
         // every load is issued unconditionally (an idle sub-warp re-reads matrix 0) and back to back: the kernel lives
         // on memory-level parallelism; 32-bit element offsets, one IMAD.WIDE per address
-        const float* src = P.x + base;
+        const E* src = P.x + base;
         f2 x[M][H];
         constexpr int RB = 16 / CPL > 0 ? 16 / CPL : 1;      // rows per batch of 16 loads
 #pragma unroll
@@ -188,7 +226,7 @@ __global__ void __launch_bounds__(kSmallThreads, 3) small_fwd(const SmallParams 
             for (int i = ib; i < ib + RB; ++i)
 #pragma unroll
                 for (int k = 0; k < H; ++k)
-                    x[i][k] = make_float2(__ldg(src + (i * istride + off[2 * k])), __ldg(src + (i * istride + off[2 * k + 1])));
+                    x[i][k] = make_float2(ld_at(src, i * istride + off[2 * k]), ld_at(src, i * istride + off[2 * k + 1]));
             asm volatile("" ::: "memory");              // keep the batches (and their 64-bit addresses) apart
         }
 #pragma unroll
@@ -207,7 +245,7 @@ __global__ void __launch_bounds__(kSmallThreads, 3) small_fwd(const SmallParams 
         }
         if (valid) {
             const bool add = P.window && P.set > 0, last = P.window && P.set == P.S - 1 && P.S > 1;
-            float* dstb = P.out + base;
+            const SetSums<E> dst(P, base);
             const float fin = last ? ((P.S & (P.S - 1)) ? 0.f : invS) : 1.f;    // 0: true division below
             int is2 = istride;
             asm volatile("" : "+r"(is2));                 // recompute the 64 offsets here instead of carrying them in registers
@@ -218,15 +256,15 @@ __global__ void __launch_bounds__(kSmallThreads, 3) small_fwd(const SmallParams 
                 for (int k = 0; k < H; ++k) y[k] = make_float2(0.f, 0.f);
                 if (add) {
 #pragma unroll
-                    for (int k = 0; k < H; ++k) y[k] = make_float2(dstb[i * is2 + off[2 * k]], dstb[i * is2 + off[2 * k + 1]]);
+                    for (int k = 0; k < H; ++k) y[k] = make_float2(dst.acc[i * is2 + off[2 * k]], dst.acc[i * is2 + off[2 * k + 1]]);
                 }
 #pragma unroll
                 for (int k = 0; k < H; ++k) {
                     float y0 = __fadd_rn(y[k].x, u[i] * v[k].x), y1 = __fadd_rn(y[k].y, u[i] * v[k].y);
                     if (fin == 0.f) { y0 = __fdiv_rn(y0, (float)P.S); y1 = __fdiv_rn(y1, (float)P.S); }
                     else { y0 *= fin; y1 *= fin; }
-                    dstb[i * is2 + off[2 * k]] = y0;
-                    dstb[i * is2 + off[2 * k + 1]] = y1;
+                    dst.store(y0, i * is2 + off[2 * k]);
+                    dst.store(y1, i * is2 + off[2 * k + 1]);
                 }
             }
         }
@@ -240,8 +278,8 @@ struct Hist {
     static constexpr int floats = L < 32 ? raw + ((L - raw % 32) + 32) % 32 : raw;
 };
 
-template <int M, int CPL, int L>
-__global__ void __launch_bounds__(kSmallThreads) small_bwd(const SmallParams P) {
+template <typename E, int M, int CPL, int L>
+__global__ void __launch_bounds__(kSmallThreads) small_bwd(const SmallParams<E> P) {
     extern __shared__ __align__(8) float hist_all[];
     constexpr int H = CPL / 2;
     constexpr int kHS = M + CPL * L;
@@ -249,7 +287,7 @@ __global__ void __launch_bounds__(kSmallThreads) small_bwd(const SmallParams P) 
     const int lane = threadIdx.x & (L - 1);
     const long long groups = (long long)gridDim.x * (kSmallThreads / L);
     const long long g0 = ((long long)blockIdx.x * kSmallThreads + threadIdx.x) / L;
-    Locator<M, CPL, L> loc;
+    Locator<E, M, CPL, L> loc;
     loc.init(P, lane);
     float u0r[M];
     f2 v0r[H];
@@ -269,7 +307,7 @@ __global__ void __launch_bounds__(kSmallThreads) small_bwd(const SmallParams P) 
         const bool valid = mid < P.n;
         int off[CPL];
         const long long base = loc.locate(P, valid ? mid : 0, off);
-        const float* src = P.x + base;
+        const E* src = P.x + base;
         f2 x[M][H];
         constexpr int RB = 16 / CPL > 0 ? 16 / CPL : 1;      // rows per batch of 16 loads
 #pragma unroll
@@ -278,7 +316,7 @@ __global__ void __launch_bounds__(kSmallThreads) small_bwd(const SmallParams P) 
             for (int i = ib; i < ib + RB; ++i)
 #pragma unroll
                 for (int k = 0; k < H; ++k)
-                    x[i][k] = make_float2(__ldg(src + (i * istride + off[2 * k])), __ldg(src + (i * istride + off[2 * k + 1])));
+                    x[i][k] = make_float2(ld_at(src, i * istride + off[2 * k]), ld_at(src, i * istride + off[2 * k + 1]));
             asm volatile("" ::: "memory");              // keep the batches (and their 64-bit addresses) apart
         }
         unsigned long long mask = 0;       // x > 0 before the ReLU (M*CPL = 64 bits)
@@ -318,7 +356,7 @@ __global__ void __launch_bounds__(kSmallThreads) small_bwd(const SmallParams P) 
         // ---- seed: y = u_T v_T^T ----
         f2 xb[M][H];                       // dL/dx accumulator; first holds dL/dy
         {
-            const float* gsrc = P.gy + base;
+            const E* gsrc = P.gy + base;
             int is3 = istride;
             asm volatile("" : "+r"(is3));
 #pragma unroll
@@ -327,7 +365,7 @@ __global__ void __launch_bounds__(kSmallThreads) small_bwd(const SmallParams P) 
                 for (int i = ib; i < ib + RB; ++i)
 #pragma unroll
                     for (int k = 0; k < H; ++k)
-                        xb[i][k] = make_float2(__ldg(gsrc + (i * is3 + off[2 * k])), __ldg(gsrc + (i * is3 + off[2 * k + 1])));
+                        xb[i][k] = make_float2(ld_at(gsrc, i * is3 + off[2 * k]), ld_at(gsrc, i * is3 + off[2 * k + 1]));
                 asm volatile("" ::: "memory");
             }
             if (P.window) {
@@ -480,7 +518,7 @@ __global__ void __launch_bounds__(kSmallThreads) small_bwd(const SmallParams P) 
         }
         if (valid) {
             const bool add = P.window && P.set > 0;
-            float* dstb = P.out + base;
+            const SetSums<E> dst(P, base);
             int is2 = istride;
             asm volatile("" : "+r"(is2));
 #pragma unroll
@@ -490,22 +528,22 @@ __global__ void __launch_bounds__(kSmallThreads) small_bwd(const SmallParams P) 
                 for (int k = 0; k < H; ++k) o[k] = make_float2(0.f, 0.f);
                 if (add) {
 #pragma unroll
-                    for (int k = 0; k < H; ++k) o[k] = make_float2(dstb[i * is2 + off[2 * k]], dstb[i * is2 + off[2 * k + 1]]);
+                    for (int k = 0; k < H; ++k) o[k] = make_float2(dst.acc[i * is2 + off[2 * k]], dst.acc[i * is2 + off[2 * k + 1]]);
                 }
 #pragma unroll
                 for (int k = 0; k < H; ++k) {
                     const float g0v = ((mask >> (i * CPL + 2 * k)) & 1ULL) ? xb[i][k].x : 0.f;
                     const float g1v = ((mask >> (i * CPL + 2 * k + 1)) & 1ULL) ? xb[i][k].y : 0.f;
-                    dstb[i * is2 + off[2 * k]] = __fadd_rn(o[k].x, g0v);
-                    dstb[i * is2 + off[2 * k + 1]] = __fadd_rn(o[k].y, g1v);
+                    dst.store(__fadd_rn(o[k].x, g0v), i * is2 + off[2 * k]);
+                    dst.store(__fadd_rn(o[k].y, g1v), i * is2 + off[2 * k + 1]);
                 }
             }
         }
     }
 }
 
-template <int M, int CPL, int L>
-int launch_small(const SmallParams& P, bool bwd, cudaStream_t st) {
+template <typename E, int M, int CPL, int L>
+int launch_small(const SmallParams<E>& P, bool bwd, cudaStream_t st) {
     const long long per_cta = kSmallThreads / L;
     long long ctas = (P.n + per_cta - 1) / per_cta;
     const long long cap = 8LL * num_sms();
@@ -513,27 +551,28 @@ int launch_small(const SmallParams& P, bool bwd, cudaStream_t st) {
     if (bwd) {
         const size_t smem = sizeof(float) * Hist<M, CPL, L>::floats * (kSmallThreads / L);
         static SmemConfig cfg;
-        FZ_CUDA_CHECK(cfg.ensure(small_bwd<M, CPL, L>, smem));
-        small_bwd<M, CPL, L><<<(unsigned)ctas, kSmallThreads, smem, st>>>(P);
+        FZ_CUDA_CHECK(cfg.ensure(small_bwd<E, M, CPL, L>, smem));
+        small_bwd<E, M, CPL, L><<<(unsigned)ctas, kSmallThreads, smem, st>>>(P);
     } else {
-        small_fwd<M, CPL, L><<<(unsigned)ctas, kSmallThreads, 0, st>>>(P);
+        small_fwd<E, M, CPL, L><<<(unsigned)ctas, kSmallThreads, 0, st>>>(P);
     }
     FZ_LAUNCH_CHECK();
     return FZ_OK;
 }
 
-int dispatch_small(const SmallParams& P, int M, int N, bool bwd, cudaStream_t st) {
+template <typename E>
+int dispatch_small(const SmallParams<E>& P, int M, int N, bool bwd, cudaStream_t st) {
     if (N == 64) {
         switch (M) {
-            case 4: return launch_small<4, 16, 4>(P, bwd, st);
-            case 8: return launch_small<8, 8, 8>(P, bwd, st);
-            case 16: return launch_small<16, 4, 16>(P, bwd, st);
-            case 32: return launch_small<32, 2, 32>(P, bwd, st);
+            case 4: return launch_small<E, 4, 16, 4>(P, bwd, st);
+            case 8: return launch_small<E, 8, 8, 8>(P, bwd, st);
+            case 16: return launch_small<E, 16, 4, 16>(P, bwd, st);
+            case 32: return launch_small<E, 32, 2, 32>(P, bwd, st);
         }
     }
-    if (N == 128 && M == 8) return launch_small<8, 8, 16>(P, bwd, st);
-    if (N == 256 && M == 8) return launch_small<8, 8, 32>(P, bwd, st);
-    if (N == 16 && M == 8) return launch_small<8, 4, 4>(P, bwd, st);
+    if (N == 128 && M == 8) return launch_small<E, 8, 8, 16>(P, bwd, st);
+    if (N == 256 && M == 8) return launch_small<E, 8, 8, 32>(P, bwd, st);
+    if (N == 16 && M == 8) return launch_small<E, 8, 4, 4>(P, bwd, st);
     return fail(FZ_ERR_UNSUPPORTED, "no small-matrix kernel for %dx%d", M, N);
 }
 
@@ -554,9 +593,14 @@ bool small_window_supported(const DevGeom& G, const fz_solver& s) {
     return G.mats_per_shift > 0;
 }
 
+size_t small_workspace_bytes(const DevGeom& G) {
+    if (G.dtype != FZ_DTYPE_BF16 || G.S < 2) return 0;
+    return ((size_t)G.B * G.C * G.vox * sizeof(float) + 255) / 256 * 256;
+}
+
 int small_direct(const float* x, const float* u0, const float* v0, const float* gy, float* out, long long n, int M, int N,
                  const fz_solver& s, int K, bool bwd, cudaStream_t st) {
-    SmallParams P;
+    SmallParams<float> P;
     memset(&P, 0, sizeof(P));
     P.x = x; P.gy = gy; P.out = out; P.u0 = u0; P.v0 = v0; P.n = n;
     P.T = s.num_iters; P.K = K; P.kind = s.kind; P.eps = s.eps; P.S = 1;
@@ -564,11 +608,13 @@ int small_direct(const float* x, const float* u0, const float* v0, const float* 
     return dispatch_small(P, M, N, bwd, st);
 }
 
-int small_window(const float* x, const float* u0, const float* v0, const float* gy, float* out, const DevGeom& G,
-                 const fz_solver& s, int K, int relu, bool bwd, cudaStream_t st) {
-    SmallParams P;
+namespace {
+template <typename E>
+int small_window_sets(const E* x, const float* u0, const float* v0, const E* gy, E* out, float* acc, const DevGeom& G,
+                      const fz_solver& s, int K, int relu, bool bwd, cudaStream_t st) {
+    SmallParams<E> P;
     memset(&P, 0, sizeof(P));
-    P.x = x; P.gy = gy; P.out = out; P.u0 = u0; P.v0 = v0; P.n = G.mats_per_shift;
+    P.x = x; P.gy = gy; P.out = out; P.u0 = u0; P.v0 = v0; P.n = G.mats_per_shift; P.acc = acc;
     P.T = s.num_iters; P.K = K; P.kind = s.kind; P.eps = s.eps; P.S = G.S; P.window = 1; P.relu = relu;
     P.G = G;
     for (int q = 0; q < G.S; ++q)       // torch.roll semantics: any integer shift, reduced to [0, n)
@@ -583,6 +629,18 @@ int small_window(const float* x, const float* u0, const float* v0, const float* 
         if (int e = dispatch_small(P, G.d, G.P, bwd, st)) return e;
     }
     return FZ_OK;
+}
+}  // namespace
+
+int small_window(const float* x, const float* u0, const float* v0, const float* gy, float* out, void* workspace,
+                 const DevGeom& G, const fz_solver& s, int K, int relu, bool bwd, cudaStream_t st) {
+    if (G.dtype != FZ_DTYPE_BF16) return small_window_sets(x, u0, v0, gy, out, nullptr, G, s, K, relu, bwd, st);
+    if (small_workspace_bytes(G) && !workspace)
+        return fail(FZ_ERR_INVALID, "%s: workspace of %zu bytes required", bwd ? "fz_swnmf_backward" : "fz_swnmf_forward",
+                    small_workspace_bytes(G));
+    typedef __nv_bfloat16 bf;
+    return small_window_sets(reinterpret_cast<const bf*>(x), u0, v0, reinterpret_cast<const bf*>(gy), reinterpret_cast<bf*>(out),
+                             static_cast<float*>(workspace), G, s, K, relu, bwd, st);
 }
 
 }  // namespace fz

@@ -8,7 +8,8 @@ any other combination runs the same steps through the standalone kernels.  A Fac
 and no active dropout runs entirely in hand-written kernels: 32 channels in the fused glue kernels (csrc/fz_block_glue*.cu)
 around the fused core, any other width in the tcgen05 channel-map kernel with fused epilogues (csrc/fz_linear_tc.cu) and the
 channels-first LayerNorm kernels, bf16 inputs (bf16 autocast) in the bf16 channel maps (csrc/fz_bf16_block.cu) around the
-bf16 core (shifts [0, 4] or paired window sets such as [0, 2, 4, 6]); other blocks run the glue layer by layer.
+bf16 core (patch 8^3 at shifts [0, 4] or paired window sets such as [0, 2, 4, 6]; 64-column windows such as patch 4^3 at any
+shifts); other blocks run the glue layer by layer.
 """
 from __future__ import annotations
 
@@ -52,7 +53,7 @@ class FactMixer(nn.Module):
             f = self.factorize
             relu = isinstance(self.act, nn.ReLU)
             if out.dtype == torch.bfloat16 and not _ops.bf16_core_supported(self.reshape._geom, f.solver_spec(), relu):
-                out = out.float()           # the bf16 core covers the octant geometries only (not the 8^3 bottleneck)
+                out = out.float()           # geometries the bf16 core does not cover, such as the 8^3 bottleneck at patch 8
             out = _ops.SWNMF.apply(out, f.init.u0, f.init.v0, self.reshape._geom, f.solver_spec(), relu)
         else:
             out = self.reshape(out)

@@ -54,11 +54,13 @@ typedef struct fz_geom {
     int32_t shifts[FZ_MAX_SHIFTS][3];   /* torch.roll shifts per window set; 0 = unshifted     */
     int32_t dtype;                      /* FZ_DTYPE_F32 (0) or FZ_DTYPE_BF16: element type of the VOLUMES handed to
                                            fz_swnmf_forward / _backward (x, y, dy, dx); u0, v0, the saved records and
-                                           all arithmetic stay fp32.  bf16 is served by the octant kernels only
+                                           all arithmetic stay fp32.  bf16 is served by the octant kernels
                                            (head_dim 8, patch 8^3, ReLU, rank-1 HALS, an even number of patches along
                                            W) at shifts [0, 4] or at window sets that pair up as (a, a + 4) with even
-                                           base shifts along W, e.g. [0, 2, 4, 6]; anything else returns
-                                           FZ_ERR_UNSUPPORTED                                                      */
+                                           base shifts along W, e.g. [0, 2, 4, 6]; and by the sub-warp kernels at
+                                           64-column windows with head_dim 4..32 (e.g. patch 4^3) and 8 x 16 / 128 /
+                                           256 windows, at any shifts, rank-1 HALS or MU, up to 5 iterations, ReLU
+                                           or not.  Anything else returns FZ_ERR_UNSUPPORTED                        */
     int32_t path;                       /* FZ_PATH_AUTO (0), or one of FZ_PATH_* to restrict the
                                            kernel family fz_swnmf_* may pick for this call (tests
                                            and measurements; a per-call argument, no global state) */
@@ -122,7 +124,8 @@ int fz_nmf_backward(const float* x, const float* u0, const float* v0, const floa
 /* ---- fused FactMixer core: reshape -> act -> factorize -> inverse (factorizer.py:41-50) ----- */
 
 /* Bytes of the `saved` buffer fz_swnmf_forward fills for fz_swnmf_backward (per-window iterate
- * summaries), and of the scratch `workspace` both directions need (tile-order counters). */
+ * summaries), and of the scratch `workspace` both directions need (tile-order counters; for bf16
+ * volumes on the sub-warp kernels with two or more window sets, an fp32 sum over the sets). */
 size_t fz_swnmf_saved_bytes(const fz_geom* g, const fz_solver* s);
 size_t fz_swnmf_workspace_bytes(const fz_geom* g, const fz_solver* s);
 
