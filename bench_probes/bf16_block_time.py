@@ -22,6 +22,13 @@ The fused core took bf16 volumes at patch 4 only after the sub-warp kernels lear
     python bench_probes/bf16_block_time.py --out /tmp/bf16_block_time.json
     python bench_probes/bf16_block_time.py --shifts bundle --mlp-ratio 4 --batch 2 --core --out /tmp/bundle.json
     python bench_probes/bf16_block_time.py --shifts isles22 --batch 8 --core --out /tmp/isles22.json
+
+--dtype f16 times fp16 activations instead (FactorizerBlockF16Fn, fp16 autocast: torch.autocast("cuda")'s default).  Its
+routes are fp32, f16-old (fp16 autocast layer by layer with the core cast to fp32, the only fp16 route before the fp16
+kernels) and f16-new; the model is timed for fp32, bf16-new (bf16 autocast) and f16-new (fp16 autocast), and --core
+compares fp32 with fp16.
+
+    python bench_probes/bf16_block_time.py --dtype f16 --core --out /tmp/f16_block_time.json
 """
 import argparse
 import json
@@ -38,6 +45,7 @@ from factorizer_b200 import _ops  # noqa: E402
 
 SHAPES = [(32, 128), (64, 64), (128, 32), (256, 16)]
 SHIFTS = {"default": None, "bundle": [None, 2, 4, 6], "isles22": [None, 1, 2, 3]}
+DTYPES = {"bf16": torch.bfloat16, "f16": torch.float16}
 ISLES22_SHAPES = [(32, 64), (64, 32), (128, 16), (256, 8), (512, 4)]      # (channels, n) of the stages of a 64^3 ROI
 
 
@@ -53,22 +61,30 @@ def card():
         return f"{torch.cuda.get_device_name()} (power limit not read: {e})"
 
 
+def route_dtype(route):
+    return torch.float32 if route == "fp32" else DTYPES[route.split("-")[0]]
+
+
 class _Route:
+    """`route` = fp32, or <bf16|f16>-<old|new>; -old runs under that dtype's autocast with its block path switched off (and its
+    core: at the bundle / isles22 shifts for bf16, always for fp16), -new feeds the block that dtype"""
     def __init__(self, name, shifts=None):
-        self.name, self.core_off = name, name == "bf16-old" and shifts is not None
-        self.saved = _ops.bf16_block_supported, _ops.bf16_core_supported
+        self.name, self.tag = name, name.split("-")[0]
+        self.old = name.endswith("-old")
+        self.core_off = self.old and (shifts is not None or self.tag == "f16")
+        self.saved = (_ops.bf16_block_supported, _ops.bf16_core_supported, _ops.f16_block_supported, _ops.f16_core_supported)
 
     def __enter__(self):
-        if self.name == "bf16-old":
-            _ops.bf16_block_supported = lambda x, hidden: False
+        if self.old:
+            setattr(_ops, f"{self.tag}_block_supported", lambda x, hidden: False)
         if self.core_off:
-            _ops.bf16_core_supported = lambda *a, **k: False
-        self.ac = torch.autocast("cuda", dtype=torch.bfloat16, enabled=self.name == "bf16-old")
+            setattr(_ops, f"{self.tag}_core_supported", lambda *a, **k: False)
+        self.ac = torch.autocast("cuda", dtype=route_dtype(self.name), enabled=self.old)
         self.ac.__enter__()
 
     def __exit__(self, *exc):
         self.ac.__exit__(*exc)
-        _ops.bf16_block_supported, _ops.bf16_core_supported = self.saved
+        _ops.bf16_block_supported, _ops.bf16_core_supported, _ops.f16_block_supported, _ops.f16_core_supported = self.saved
 
 
 def reshape(shifts):
@@ -109,7 +125,7 @@ def time_graph(fn, warmup, reps):
 def block_leg(B, C, n, route, warmup, reps, ratio=2, shifts=None):
     blk = block(C, n, ratio, shifts)
     H = blk.mlp.block[0].linear.out_channels
-    dtype = torch.float32 if route == "fp32" else torch.bfloat16
+    dtype = route_dtype(route)
     x = torch.randn(B, C, n, n, n, device="cuda").to(dtype).requires_grad_(True)
     gout = torch.randn(B, C, n, n, n, device="cuda").to(dtype)
     params = list(blk.parameters())
@@ -144,7 +160,7 @@ def model_leg(route, warmup, reps, n=128, B=1, ratio=2, shifts=None):
 
     def step():
         net.zero_grad(set_to_none=True)
-        with _Route(route, shifts), torch.autocast("cuda", dtype=torch.bfloat16, enabled=route != "fp32"):
+        with _Route(route, shifts), torch.autocast("cuda", dtype=route_dtype(route), enabled=route != "fp32"):
             logits = net(x).float()
         p = torch.sigmoid(logits)
         dice = 1 - (2 * (p * target).sum((2, 3, 4)) + 1e-5) / (p.sum((2, 3, 4)) + target.sum((2, 3, 4)) + 1e-5)
@@ -187,26 +203,28 @@ def main():
     ap.add_argument("--shifts", choices=sorted(SHIFTS), default="default")
     ap.add_argument("--mlp-ratio", type=int, default=2)
     ap.add_argument("--batch", type=int, default=1)
-    ap.add_argument("--core", action="store_true", help="also time the core alone, fp32 against bf16")
+    ap.add_argument("--core", action="store_true", help="also time the core alone, fp32 against --dtype")
+    ap.add_argument("--dtype", choices=sorted(DTYPES), default="bf16", help="the 16-bit activation type of the -old / -new routes")
     args = ap.parse_args()
+    old, new = f"{args.dtype}-old", f"{args.dtype}-new"
     torch.backends.cuda.matmul.allow_tf32 = False
     torch.backends.cudnn.allow_tf32 = False
     shifts, B = SHIFTS[args.shifts], args.batch
     isles = args.shifts == "isles22"
     n_model = 64 if isles else 128
-    res = {"card": card(), "shifts": args.shifts, "mlp_ratio": args.mlp_ratio, "batch": B, "core": [], "blocks": [], "model": []}
+    res = {"card": card(), "dtype": args.dtype, "shifts": args.shifts, "mlp_ratio": args.mlp_ratio, "batch": B, "core": [], "blocks": [], "model": []}
     if args.core:
-        for dtype in (torch.float32, torch.bfloat16):
+        for dtype in (torch.float32, DTYPES[args.dtype]):
             res["core"].append(core_leg(B, shifts, dtype, args.warmup, args.reps, n=n_model))
             print(json.dumps(res["core"][-1]), flush=True)
     for C, n in ISLES22_SHAPES if isles else SHAPES:
-        row = {r: block_leg(B, C, n, r, args.warmup, args.reps, args.mlp_ratio, shifts) for r in ("fp32", "bf16-old", "bf16-new")}
-        row["new_vs_old"] = row["bf16-old"]["ms"] / row["bf16-new"]["ms"]
-        row["new_vs_fp32"] = row["fp32"]["ms"] / row["bf16-new"]["ms"]
+        row = {r: block_leg(B, C, n, r, args.warmup, args.reps, args.mlp_ratio, shifts) for r in ("fp32", old, new)}
+        row["new_vs_old"] = row[old]["ms"] / row[new]["ms"]
+        row["new_vs_fp32"] = row["fp32"]["ms"] / row[new]["ms"]
         res["blocks"].append(row)
         print(json.dumps(row), flush=True)
     if not args.no_model:
-        for r in ("fp32", "bf16-old", "bf16-new"):
+        for r in ("fp32", "bf16-old", "bf16-new") if args.dtype == "bf16" else ("fp32", "bf16-new", "f16-new"):
             res["model"].append(model_leg(r, 3, 5, n=n_model, B=B, ratio=args.mlp_ratio, shifts=shifts))
             print(json.dumps(res["model"][-1]), flush=True)
     os.makedirs(os.path.dirname(os.path.abspath(args.out)), exist_ok=True)

@@ -1,13 +1,15 @@
-// Pins the shared-memory layouts of the bf16 tensor-core kernels (csrc/fz_bf16_block.cu) before they are built on:
-// tcgen05.mma kind::f16 with BF16 A and B, an F32 accumulator, the 128-byte swizzle (descriptor layout type 2) that TMA
+// Pins the shared-memory layouts of the bf16 and fp16 tensor-core kernels (csrc/fz_bf16_block.cu) before they are built on:
+// tcgen05.mma kind::f16 with BF16 or FP16 A and B (instruction-descriptor A / B format 1 or 0), an F32 accumulator, the 128-byte swizzle (descriptor layout type 2) that TMA
 // writes for 16-bit boxes whose rows are 128 bytes, and the K steps of 16 values.  Two configurations, each four MMAs
 // (K = 64) into one accumulator:
 //   fwd:   A MN-major (128 voxels x 64 channels, two 64-voxel atoms LBO = 8192 apart, SBO = 1024, K step +2048 bytes),
 //          B K-major (64 outputs x 64 channels, SBO = 1024, K step +32 bytes), N = 64   -- the channel map
 //   wgrad: A K-major (128 rows), B K-major (144 rows), N = 144                              -- the weight gradient
 // The operands are small integers (every product and sum exact in fp32); the result is compared with the host product
-// element by element.  Not part of the product.
+// element by element.  The fp16 operands go up to +-511, which bf16 cannot hold, so a wrong format field shows.  Each
+// configuration runs for both types.  Not part of the product.
 #include <cuda_bf16.h>
+#include <cuda_fp16.h>
 #include <cuda_runtime.h>
 #include <cstdint>
 #include <cstdio>
@@ -26,8 +28,10 @@ __host__ __device__ inline uint32_t sw128(int r, int c) { return r * 128 + (((c 
 constexpr int M = 128, K = 64, NMAX = 144;
 constexpr uint32_t kA = 16384, kB = NMAX * 128;
 
-// mode 0: A MN-major (fwd), N = 64; mode 1: A K-major (wgrad), N = 144.  a: [M][K], b: [N][K] as bf16 bit patterns
-__global__ void __launch_bounds__(128) probe(int mode, const uint16_t* __restrict__ a, const uint16_t* __restrict__ b, float* __restrict__ D) {
+// mode 0: A MN-major (fwd), N = 64; mode 1: A K-major (wgrad), N = 144.  a: [M][K], b: [N][K] as 16-bit patterns of the
+// format `fmt` (1 = bf16, 0 = fp16)
+__global__ void __launch_bounds__(128) probe(int mode, uint32_t fmt, const uint16_t* __restrict__ a, const uint16_t* __restrict__ b,
+                                             float* __restrict__ D) {
     extern __shared__ __align__(1024) unsigned char smem[];
     unsigned char* sa = smem;
     unsigned char* sb = smem + kA;
@@ -51,7 +55,7 @@ __global__ void __launch_bounds__(128) probe(int mode, const uint16_t* __restric
     __syncthreads();
     asm volatile("tcgen05.fence::after_thread_sync;" ::: "memory");
     const uint32_t tmem = tmem_base;
-    const uint32_t idesc = (1u << 4) | (1u << 7) | (1u << 10) | ((uint32_t)(mode ? 0 : 1) << 15) | ((uint32_t)(N >> 3) << 17) | ((uint32_t)(M >> 4) << 24);
+    const uint32_t idesc = (1u << 4) | (fmt << 7) | (fmt << 10) | ((uint32_t)(mode ? 0 : 1) << 15) | ((uint32_t)(N >> 3) << 17) | ((uint32_t)(M >> 4) << 24);
     if (tid == 0) {
         const uint64_t ad = mode ? make_desc(smem_u32(sa), 16, 1024, 2) : make_desc(smem_u32(sa), 8192, 1024, 2);
         const uint64_t bd = make_desc(smem_u32(sb), 16, 1024, 2);
@@ -81,43 +85,47 @@ __global__ void __launch_bounds__(128) probe(int mode, const uint16_t* __restric
 }
 
 static uint16_t bf16_bits(float v) { __nv_bfloat16 h = __float2bfloat16(v); uint16_t u; memcpy(&u, &h, 2); return u; }
+static uint16_t f16_bits(float v) { __half h = __float2half(v); uint16_t u; memcpy(&u, &h, 2); return u; }
 
 int main() {
-    std::vector<float> A(M * K), B(NMAX * K);
-    std::vector<uint16_t> Ab(M * K), Bb(NMAX * K);
-    srand(12345);
-    for (int i = 0; i < M * K; ++i) { A[i] = (float)(rand() % 7 - 3); Ab[i] = bf16_bits(A[i]); }
-    for (int i = 0; i < NMAX * K; ++i) { B[i] = (float)(rand() % 7 - 3); Bb[i] = bf16_bits(B[i]); }
     uint16_t *dA, *dB;
     float* dD;
-    CK(cudaMalloc(&dA, Ab.size() * 2));
-    CK(cudaMalloc(&dB, Bb.size() * 2));
+    CK(cudaMalloc(&dA, M * K * 2));
+    CK(cudaMalloc(&dB, NMAX * K * 2));
     CK(cudaMalloc(&dD, M * NMAX * 4));
-    CK(cudaMemcpy(dA, Ab.data(), Ab.size() * 2, cudaMemcpyHostToDevice));
-    CK(cudaMemcpy(dB, Bb.data(), Bb.size() * 2, cudaMemcpyHostToDevice));
     const int smem = kA + kB + 1024;
     CK(cudaFuncSetAttribute(probe, cudaFuncAttributeMaxDynamicSharedMemorySize, smem));
     int bad_total = 0;
-    for (int mode = 0; mode < 2; ++mode) {
-        const int N = mode ? 144 : 64;
-        CK(cudaMemset(dD, 0, M * NMAX * 4));
-        probe<<<1, 128, smem>>>(mode, dA, dB, dD);
-        CK(cudaDeviceSynchronize());
-        std::vector<float> D(M * NMAX);
-        CK(cudaMemcpy(D.data(), dD, D.size() * 4, cudaMemcpyDeviceToHost));
-        int bad = 0;
-        for (int m = 0; m < M; ++m)
-            for (int n = 0; n < N; ++n) {
-                float ref = 0.f;
-                for (int k = 0; k < K; ++k) ref += A[m * K + k] * B[n * K + k];
-                if (D[m * NMAX + n] != ref) {
-                    if (bad < 8) printf("  mode %d: D[%d][%d] = %g, expected %g\n", mode, m, n, D[m * NMAX + n], ref);
-                    ++bad;
+    for (uint32_t fmt = 1; fmt != ~0u; --fmt) {                      // bf16, then fp16
+        const int range = fmt ? 3 : 511;                             // |operand| <= range: 64 products sum exactly in fp32
+        std::vector<float> A(M * K), B(NMAX * K);
+        std::vector<uint16_t> Ab(M * K), Bb(NMAX * K);
+        srand(12345);
+        for (int i = 0; i < M * K; ++i) { A[i] = (float)(rand() % (2 * range + 1) - range); Ab[i] = fmt ? bf16_bits(A[i]) : f16_bits(A[i]); }
+        for (int i = 0; i < NMAX * K; ++i) { B[i] = (float)(rand() % (2 * range + 1) - range); Bb[i] = fmt ? bf16_bits(B[i]) : f16_bits(B[i]); }
+        CK(cudaMemcpy(dA, Ab.data(), Ab.size() * 2, cudaMemcpyHostToDevice));
+        CK(cudaMemcpy(dB, Bb.data(), Bb.size() * 2, cudaMemcpyHostToDevice));
+        for (int mode = 0; mode < 2; ++mode) {
+            const int N = mode ? 144 : 64;
+            CK(cudaMemset(dD, 0, M * NMAX * 4));
+            probe<<<1, 128, smem>>>(mode, fmt, dA, dB, dD);
+            CK(cudaDeviceSynchronize());
+            std::vector<float> D(M * NMAX);
+            CK(cudaMemcpy(D.data(), dD, D.size() * 4, cudaMemcpyDeviceToHost));
+            int bad = 0;
+            for (int m = 0; m < M; ++m)
+                for (int n = 0; n < N; ++n) {
+                    float ref = 0.f;
+                    for (int k = 0; k < K; ++k) ref += A[m * K + k] * B[n * K + k];
+                    if (D[m * NMAX + n] != ref) {
+                        if (bad < 8) printf("  %s mode %d: D[%d][%d] = %g, expected %g\n", fmt ? "bf16" : "fp16", mode, m, n, D[m * NMAX + n], ref);
+                        ++bad;
+                    }
                 }
-            }
-        printf("%s (A %s, N = %d): %d of %d entries differ -> %s\n", mode ? "wgrad" : "fwd", mode ? "K-major" : "MN-major", N, bad,
-               M * N, bad ? "FAIL" : "PASS");
-        bad_total += bad;
+            printf("%s %s (A %s, N = %d): %d of %d entries differ -> %s\n", fmt ? "bf16" : "fp16", mode ? "wgrad" : "fwd",
+                   mode ? "K-major" : "MN-major", N, bad, M * N, bad ? "FAIL" : "PASS");
+            bad_total += bad;
+        }
     }
     return bad_total ? 1 : 0;
 }

@@ -15,7 +15,7 @@ FZ_MAX_SHIFTS = 8
 FZ_MAX_RANK = 8
 FZ_SOLVER_MU, FZ_SOLVER_HALS = 0, 1
 FZ_OK, FZ_ERR_INVALID, FZ_ERR_UNSUPPORTED, FZ_ERR_CUDA = 0, 1, 2, 3
-FZ_DTYPE_F32, FZ_DTYPE_BF16 = 0, 1
+FZ_DTYPE_F32, FZ_DTYPE_BF16, FZ_DTYPE_F16 = 0, 1, 2
 FZ_PATH_AUTO, FZ_PATH_GENERIC, FZ_PATH_NO_OCTANT, FZ_PATH_OCTANT_3LAUNCH, FZ_PATH_OCTANT_PIPELINE = 0, 1, 2, 3, 4
 
 
@@ -94,6 +94,20 @@ _SIGNATURES = {
     "fz_layernorm_cf_backward_add_bf16": (c_int, [c_void_p, c_void_p, c_void_p, c_void_p, c_void_p, c_void_p, c_void_p, c_int64,
                                                   c_int32, c_int64, c_float, c_void_p]),
     "fz_swnmf_bf16_supported": (c_int, [POINTER(FzGeom), POINTER(FzSolver), c_int32]),
+    "fz_linear_forward_f16_supported": (c_int, [c_int32, c_int32, c_int64]),
+    "fz_linear_forward_f16": (c_int, [c_void_p, c_void_p, c_int32, c_void_p, c_void_p, c_int64, c_int32, c_int32, c_int64, c_int32,
+                                      c_void_p, c_void_p, c_void_p]),
+    "fz_linear_wgrad_f16_supported": (c_int, [c_int32, c_int32, c_int64]),
+    "fz_linear_wgrad_f16": (c_int, [c_void_p, c_void_p, c_void_p, c_void_p, c_int64, c_int32, c_int32, c_int64, c_void_p]),
+    "fz_f16_stage_weights_supported": (c_int, [c_int32, c_int32]),
+    "fz_f16_staged_elems": (c_int64, [c_int32, c_int32]),
+    "fz_f16_stage_weights": (c_int, [c_void_p, c_int32, c_int32] * 4 + [c_void_p, c_void_p]),
+    "fz_f16_stage_weight": (c_int, [c_void_p, c_int32, c_int32, c_void_p, c_void_p]),
+    "fz_layernorm_cf_f16_supported": (c_int, [c_int32, c_int64]),
+    "fz_layernorm_cf_forward_f16": (c_int, [c_void_p, c_void_p, c_void_p, c_void_p, c_int64, c_int32, c_int64, c_float, c_void_p]),
+    "fz_layernorm_cf_backward_add_f16": (c_int, [c_void_p, c_void_p, c_void_p, c_void_p, c_void_p, c_void_p, c_void_p, c_int64,
+                                                 c_int32, c_int64, c_float, c_void_p]),
+    "fz_swnmf_f16_supported": (c_int, [POINTER(FzGeom), POINTER(FzSolver), c_int32]),
     "fz_set_glue_mode": (None, [c_int32]),
     "fz_get_glue_mode": (c_int, []),
     "fz_glue_supported": (c_int, [c_int32, c_int32, c_int64]),
@@ -145,14 +159,14 @@ def check(code: int) -> None:
     raise RuntimeError(f"factorizer_b200: {msg}")
 
 
-def require_cuda_f32(t: torch.Tensor, name: str, allow_bf16: bool = False) -> torch.Tensor:
+def require_cuda_f32(t: torch.Tensor, name: str, allow_bf16: bool = False, allow_f16: bool = False) -> torch.Tensor:
     if not isinstance(t, torch.Tensor):
         raise TypeError(f"{name} must be a torch.Tensor")
     if not t.is_cuda:
         raise RuntimeError(
             f"factorizer_b200: `{name}` is on {t.device}; this package has CUDA kernels only "
             "(no CPU fallback) - move the module and its inputs to a CUDA device")
-    if t.dtype != torch.float32 and not (allow_bf16 and t.dtype == torch.bfloat16):
+    if t.dtype != torch.float32 and not (allow_bf16 and t.dtype == torch.bfloat16) and not (allow_f16 and t.dtype == torch.float16):
         raise NotImplementedError(
             f"factorizer_b200: `{name}` has dtype {t.dtype}; only float32 is implemented "
             "(the reference runs this path in fp32, amp: false)")

@@ -33,7 +33,7 @@ class Geometry:
 
     def c_geom(self, batch: int, dtype: torch.dtype = torch.float32) -> L.FzGeom:
         return L.make_geom(batch, self.channels, self.size, self.patch, self.head_dim, self.shifts, self.path,
-                           L.FZ_DTYPE_BF16 if dtype == torch.bfloat16 else L.FZ_DTYPE_F32)
+                           {torch.bfloat16: L.FZ_DTYPE_BF16, torch.float16: L.FZ_DTYPE_F16}.get(dtype, L.FZ_DTYPE_F32))
 
     def mat_shape(self, batch: int) -> Tuple[int, int, int, int]:
         return (len(self.shifts) * batch * self.heads, self.num_windows, self.head_dim, self.num_cols)
@@ -68,8 +68,8 @@ class _GradModeFunction(torch.autograd.Function):
         return bool(getattr(_GradModeFunction._caller, "grad", True)) and any(flags)
 
 
-def _check_vol(x: torch.Tensor, geom: Geometry, name: str, allow_bf16: bool = False) -> torch.Tensor:
-    x = L.require_cuda_f32(x, name, allow_bf16)
+def _check_vol(x: torch.Tensor, geom: Geometry, name: str, allow_16bit: bool = False) -> torch.Tensor:
+    x = L.require_cuda_f32(x, name, allow_bf16=allow_16bit, allow_f16=allow_16bit)
     if tuple(x.shape[1:]) != (geom.channels, *geom.size):
         raise ValueError(f"{name}: expected (B, {geom.channels}, {', '.join(map(str, geom.size))}), "
                          f"got {tuple(x.shape)}")
@@ -316,9 +316,9 @@ class SWNMF(_GradModeFunction):
 
     @staticmethod
     def forward(ctx, x, u0, v0, geom: Geometry, spec: SolverSpec, relu: bool):
-        # bf16 volumes (an extension: the reference runs fp32) are read and written as bf16 by the octant and sub-warp
-        # kernels; u0, v0, the saved records and all arithmetic stay fp32
-        x = _check_vol(x, geom, "x", allow_bf16=True)
+        # bf16 and fp16 volumes (an extension: the reference runs fp32) are read and written in their type by the octant and
+        # sub-warp kernels; u0, v0, the saved records and all arithmetic stay fp32
+        x = _check_vol(x, geom, "x", allow_16bit=True)
         u0 = L.require_cuda_f32(u0.float(), "u0")
         v0 = L.require_cuda_f32(v0.float(), "v0")
         y, saved = _swnmf_forward(x, u0, v0, geom, spec, relu, _GradModeFunction.wants_grad(ctx, 1))
@@ -330,7 +330,7 @@ class SWNMF(_GradModeFunction):
     @once_differentiable
     def backward(ctx, gy):
         x, u0, v0, saved = ctx.saved_tensors
-        gy = _check_vol(gy.to(x.dtype), ctx.geom, "grad", allow_bf16=True)
+        gy = _check_vol(gy.to(x.dtype), ctx.geom, "grad", allow_16bit=True)
         gx = _swnmf_backward(x, gy, u0, v0, saved, ctx.geom, ctx.spec, ctx.relu)
         return gx, None, None, None, None, None
 
@@ -439,30 +439,36 @@ def _channel_map(x, w, bias, epi=EPI_NONE, aux=None, transposed=False):
     return r
 
 
+# the suffix of the C entry points of each 16-bit activation type (fz_linear_forward_bf16 / _f16, fz_bf16_stage_weights /
+# fz_f16_stage_weights, ...)
+_HALF = {torch.bfloat16: "bf16", torch.float16: "f16"}
+
+
 def _channel_map_wgrad(gy, x, want_bias: bool):
-    """dW = sum over (batch, voxels) of gy x^T, db = sum of gy, both fp32.  bf16 gy and x: fz_linear_wgrad_bf16.  fp32 views the
-    kernels do not take (non-contiguous, or not 16-byte aligned) run the same arithmetic in torch."""
+    """dW = sum over (batch, voxels) of gy x^T, db = sum of gy, both fp32.  bf16 / fp16 gy and x: fz_linear_wgrad_bf16 / _f16.
+    fp32 views the kernels do not take (non-contiguous, or not 16-byte aligned) run the same arithmetic in torch."""
     lib = L.lib()
     B, cout, vox = gy.shape
     cin = x.shape[1]
-    bf16 = x.dtype == torch.bfloat16
-    if bf16 or (gy.is_contiguous() and x.is_contiguous() and (gy.data_ptr() | x.data_ptr()) % 16 == 0
+    half = _HALF.get(x.dtype)
+    if half or (gy.is_contiguous() and x.is_contiguous() and (gy.data_ptr() | x.data_ptr()) % 16 == 0
                 and lib.fz_linear_wgrad_supported(cout, cin, vox)):
         gw = torch.empty(cout, cin, device=x.device, dtype=torch.float32)
         gb = torch.empty(cout, device=x.device, dtype=torch.float32) if want_bias else None
-        _call(lib.fz_linear_wgrad_bf16 if bf16 else lib.fz_linear_wgrad, L.ptr(gy), L.ptr(x), L.ptr(gw), L.ptr(gb), B, cout, cin,
-              vox, L.stream_ptr(x.device))
+        fn = getattr(lib, f"fz_linear_wgrad_{half}") if half else lib.fz_linear_wgrad
+        _call(fn, L.ptr(gy), L.ptr(x), L.ptr(gw), L.ptr(gb), B, cout, cin, vox, L.stream_ptr(x.device))
         return gw, gb
     gw = torch.bmm(gy, x.transpose(1, 2)).sum(0)
     return gw, (gy.sum((0, 2)) if want_bias else None)
 
 
 def _ln_forward(x3, gamma, beta, eps):
-    """LayerNorm over the channels of fp32 or bf16 (B, C, voxels); the statistics are fp32."""
+    """LayerNorm over the channels of fp32, bf16 or fp16 (B, C, voxels); the statistics are fp32."""
     lib = L.lib()
     B, C, vox = x3.shape
     y = torch.empty_like(x3)
-    fn = lib.fz_layernorm_cf_forward_bf16 if x3.dtype == torch.bfloat16 else lib.fz_layernorm_cf_forward
+    half = _HALF.get(x3.dtype)
+    fn = getattr(lib, f"fz_layernorm_cf_forward_{half}") if half else lib.fz_layernorm_cf_forward
     _call(fn, L.ptr(x3), L.ptr(gamma), L.ptr(beta), L.ptr(y), B, C, vox, float(eps), L.stream_ptr(x3.device))
     return y
 
@@ -472,7 +478,8 @@ def _ln_backward_add(x3, gamma, gy, add, eps):
     lib = L.lib()
     B, C, vox = x3.shape
     dx, dg, db = torch.empty_like(x3), torch.empty_like(gamma), torch.empty_like(gamma)
-    fn = lib.fz_layernorm_cf_backward_add_bf16 if x3.dtype == torch.bfloat16 else lib.fz_layernorm_cf_backward_add
+    half = _HALF.get(x3.dtype)
+    fn = getattr(lib, f"fz_layernorm_cf_backward_add_{half}") if half else lib.fz_layernorm_cf_backward_add
     _call(fn, L.ptr(x3), L.ptr(gamma), L.ptr(gy), L.ptr(add), L.ptr(dx), L.ptr(dg), L.ptr(db), B, C, vox, float(eps),
           L.stream_ptr(x3.device))
     return dx, dg, db
@@ -499,7 +506,7 @@ class _WideBlockFn(_GradModeFunction):
     library, with the residual sums, the bias + GELU and the GELU derivative folded into the epilogues of the tensor-core
     channel map and the residual gradients into the LayerNorm backward -- nine launches forward (norm1 | in_proj | core x3 |
     out_proj + residual | norm2 | fc1 + GELU | fc2 + residual), the same steps in reverse backward.  Written once for
-    FactorizerBlockWideFn and FactorizerBlockBf16Fn; a subclass names the activations' `dtype` and says how its channel maps
+    FactorizerBlockWideFn, FactorizerBlockBf16Fn and FactorizerBlockF16Fn; a subclass names the activations' `dtype` and says how its channel maps
     read the four weights (w_in, w_out, w1, w2): _stage(ws) returns the tensors the backward keeps for them, _maps(staged,
     shapes) one channel map per weight, m(x, bias, epi, aux, transposed), transposed = that layer's input gradient."""
     dtype = None
@@ -508,7 +515,7 @@ class _WideBlockFn(_GradModeFunction):
     def _forward(cls, ctx, x, g1, b1n, w_in, w_out, b_out, g2, b2n, w1, bb1, w2, bb2, u0, v0, geom, spec, eps1, eps2):
         if x.dtype != cls.dtype:
             raise NotImplementedError(f"factorizer_b200: {cls.__name__} takes {cls.dtype} activations, got {x.dtype}")
-        x = _check_vol(x, geom, "x", allow_bf16=True)
+        x = _check_vol(x, geom, "x", allow_16bit=True)
         params = [L.require_cuda_f32(t, "parameter") for t in (g1, b1n, w_in, w_out, b_out, g2, b2n, w1, bb1, w2, bb2)]
         g1, b1n, w_in, w_out, b_out, g2, b2n, w1, bb1, w2, bb2 = params
         u0 = L.require_cuda_f32(u0, "u0")
@@ -542,7 +549,7 @@ class _WideBlockFn(_GradModeFunction):
     def backward(ctx, gout):
         x3, n1, z, m3, x1, n2, h, g, saved, g1, g2, u0, v0, *staged = ctx.saved_tensors
         geom = ctx.geom
-        gout = _check_vol(gout.to(x3.dtype), geom, "grad", allow_bf16=True)
+        gout = _check_vol(gout.to(x3.dtype), geom, "grad", allow_16bit=True)
         B, C = x3.shape[0], x3.shape[1]
         eps1, eps2 = ctx.eps
         m_in, m_out, m1, m2 = ctx.block._maps(staged, ctx.shapes)
@@ -594,29 +601,47 @@ def bf16_core_supported(geom: Geometry, spec: SolverSpec, relu: bool = True) -> 
     number of patches along W) at shifts [0, 4], or at window sets that pair up as (a, a + 4) with even base shifts along W,
     such as the BraTS23 bundle's [0, 2, 4, 6]; or the sub-warp kernels (64-column windows with head_dim 4..32, such as the
     ISLES22 bundle's patch 4 at shifts [None, 1, 2, 3], and 8 x 16 / 128 / 256 windows) at any shifts, rank-1 HALS or MU."""
-    g, s = geom.c_geom(1, torch.bfloat16), spec.c_solver()
-    return bool(L.lib().fz_swnmf_bf16_supported(ctypes.byref(g), ctypes.byref(s), int(relu)))
+    return _core16_supported(geom, spec, relu, torch.bfloat16)
+
+
+def f16_core_supported(geom: Geometry, spec: SolverSpec, relu: bool = True) -> bool:
+    """The fused core takes fp16 volumes of this geometry: the same geometries as bf16_core_supported."""
+    return _core16_supported(geom, spec, relu, torch.float16)
+
+
+def _core16_supported(geom: Geometry, spec: SolverSpec, relu: bool, dtype: torch.dtype) -> bool:
+    g, s = geom.c_geom(1, dtype), spec.c_solver()
+    return bool(getattr(L.lib(), f"fz_swnmf_{_HALF[dtype]}_supported")(ctypes.byref(g), ctypes.byref(s), int(relu)))
 
 
 def bf16_block_supported(x: torch.Tensor, hidden: int) -> bool:
     """FactorizerBlockBf16Fn: a contiguous, 16-byte aligned bf16 CUDA volume whose voxel count is a multiple of 8 (the bf16
     TMA boxes need 16-byte row strides), channel counts the LayerNorm kernels take (up to 512); with or without autocast.
     The caller checks the core's geometry (bf16_core_supported)."""
-    if not (isinstance(x, torch.Tensor) and x.is_cuda and x.dtype == torch.bfloat16 and x.dim() >= 3 and x.is_contiguous()
+    return _block16_supported(x, hidden, torch.bfloat16)
+
+
+def f16_block_supported(x: torch.Tensor, hidden: int) -> bool:
+    """FactorizerBlockF16Fn: bf16_block_supported's conditions on an fp16 volume (fp16 autocast, or fp16 inputs).  The caller
+    checks the core's geometry (f16_core_supported)."""
+    return _block16_supported(x, hidden, torch.float16)
+
+
+def _block16_supported(x: torch.Tensor, hidden: int, dtype: torch.dtype) -> bool:
+    if not (isinstance(x, torch.Tensor) and x.is_cuda and x.dtype == dtype and x.dim() >= 3 and x.is_contiguous()
             and x.data_ptr() % 16 == 0):
         return False
     B, C = x.shape[0], x.shape[1]
     vox = x.numel() // max(B * C, 1)
-    lib, H = L.lib(), int(hidden)
-    return bool(B > 0 and vox > 0 and lib.fz_layernorm_cf_bf16_supported(C, vox)
-                and lib.fz_linear_forward_bf16_supported(C, C, vox) and lib.fz_linear_forward_bf16_supported(H, C, vox)
-                and lib.fz_linear_forward_bf16_supported(C, H, vox) and lib.fz_linear_wgrad_bf16_supported(H, C, vox)
-                and lib.fz_linear_wgrad_bf16_supported(C, H, vox))
+    lib, H, t = L.lib(), int(hidden), _HALF[dtype]
+    fwd, wgrad = getattr(lib, f"fz_linear_forward_{t}_supported"), getattr(lib, f"fz_linear_wgrad_{t}_supported")
+    return bool(B > 0 and vox > 0 and getattr(lib, f"fz_layernorm_cf_{t}_supported")(C, vox)
+                and fwd(C, C, vox) and fwd(H, C, vox) and fwd(C, H, vox) and wgrad(H, C, vox) and wgrad(C, H, vox))
 
 
 def _staged_views(buf, shapes):
-    """Per weight of shape (R, C) in `buf`, the (W, W^T) bf16 copies fz_bf16_stage_weights wrote there, each as (view, row
-    stride)."""
+    """Per weight of shape (R, C) in `buf`, the (W, W^T) 16-bit copies fz_bf16_stage_weights / fz_f16_stage_weights wrote
+    there, each as (view, row stride)."""
     views, off = [], 0
     for R, C in shapes:
         n = R * _ld8(C) + C * _ld8(R)
@@ -625,32 +650,50 @@ def _staged_views(buf, shapes):
     return views
 
 
-def _stage_weights_bf16(*ws):
-    """One launch: the fp32 matrices (one, or a block's four: the C entries take exactly those counts) as bf16, each as
-    stored and transposed; returns the buffer (see _staged_views)."""
+def _stage_weights_bf16(*ws, dtype=torch.bfloat16):
+    """One launch: the fp32 matrices (one, or a block's four: the C entries take exactly those counts) as bf16 (or fp16 with
+    `dtype`), each as stored and transposed; returns the buffer (see _staged_views)."""
     if len(ws) not in (1, 4):
-        raise ValueError(f"factorizer_b200: bf16 weight staging takes one or four weights, got {len(ws)}")
-    lib = L.lib()
-    n = sum(int(lib.fz_bf16_staged_elems(w.shape[0], w.shape[1])) for w in ws)
-    buf = torch.empty(n, device=ws[0].device, dtype=torch.bfloat16)
+        raise ValueError(f"factorizer_b200: 16-bit weight staging takes one or four weights, got {len(ws)}")
+    lib, t = L.lib(), _HALF[dtype]
+    n = sum(int(getattr(lib, f"fz_{t}_staged_elems")(w.shape[0], w.shape[1])) for w in ws)
+    buf = torch.empty(n, device=ws[0].device, dtype=dtype)
     args = [a for w in ws for a in (L.ptr(w), w.shape[0], w.shape[1])]
-    _call(lib.fz_bf16_stage_weight if len(ws) == 1 else lib.fz_bf16_stage_weights, *args, L.ptr(buf), L.stream_ptr(buf.device))
+    fn = getattr(lib, f"fz_{t}_stage_weight" if len(ws) == 1 else f"fz_{t}_stage_weights")
+    _call(fn, *args, L.ptr(buf), L.stream_ptr(buf.device))
     return buf
 
 
 def _channel_map_bf16(x, w, cout, bias, epi=EPI_NONE, aux=None):
-    """r = W x + bias on bf16 (B, C_in, voxels), w = (staged bf16 weight, row stride); returns y, or (y, gelu(y)) for
-    EPI_GELU (fz_linear_forward_bf16)."""
+    """r = W x + bias on bf16 or fp16 (B, C_in, voxels), w = (staged weight of x's dtype, row stride); returns y, or
+    (y, gelu(y)) for EPI_GELU (fz_linear_forward_bf16 / _f16)."""
     B, cin, vox = x.shape
-    y = torch.empty(B, cout, vox, device=x.device, dtype=torch.bfloat16)
+    y = torch.empty(B, cout, vox, device=x.device, dtype=x.dtype)
     y2 = torch.empty_like(y) if epi == EPI_GELU else None
     wb, ldw = w
-    _call(L.lib().fz_linear_forward_bf16, L.ptr(x), L.ptr(wb), ldw, L.ptr(bias), L.ptr(y), B, cin, cout, vox, epi, L.ptr(aux),
-          L.ptr(y2), L.stream_ptr(x.device))
+    _call(getattr(L.lib(), f"fz_linear_forward_{_HALF[x.dtype]}"), L.ptr(x), L.ptr(wb), ldw, L.ptr(bias), L.ptr(y), B, cin, cout,
+          vox, epi, L.ptr(aux), L.ptr(y2), L.stream_ptr(x.device))
     return (y, y2) if epi == EPI_GELU else y
 
 
-class FactorizerBlockBf16Fn(_WideBlockFn):
+class _Block16Fn(_WideBlockFn):
+    """_WideBlockFn on 16-bit activations (`dtype` = bf16 or fp16): one launch stages the four weights in that type, as stored
+    and transposed (fz_bf16_stage_weights / fz_f16_stage_weights), before the nine steps; the backward keeps the staged buffer
+    and reads the transposed copies."""
+
+    @classmethod
+    def _stage(cls, ws):
+        return (_stage_weights_bf16(*ws, dtype=cls.dtype),)
+
+    @staticmethod
+    def _maps(staged, shapes):
+        def bind(views, shape):
+            return lambda x, bias, epi=EPI_NONE, aux=None, transposed=False: _channel_map_bf16(
+                x, views[transposed], shape[transposed], bias, epi, aux)
+        return [bind(v, shape) for v, shape in zip(_staged_views(staged[0], shapes), shapes)]
+
+
+class FactorizerBlockBf16Fn(_Block16Fn):
     """_WideBlockFn on bf16 activations: every activation (n1, z, m, x1, n2, h, g, the output, dx) is bf16 in memory and in the
     saved tensors; the parameters and their gradients stay fp32 (master weights), every sum accumulates in fp32, the
     LayerNorm statistics are fp32, and bias, residual, GELU and GELU' are applied before the one rounding to bf16.  One launch
@@ -662,16 +705,18 @@ class FactorizerBlockBf16Fn(_WideBlockFn):
     def forward(ctx, *args):
         return FactorizerBlockBf16Fn._forward(ctx, *args)
 
-    @staticmethod
-    def _stage(ws):
-        return (_stage_weights_bf16(*ws),)
+
+# ---- FactorizerBlock on fp16 activations (fp16 autocast: torch.autocast("cuda")'s default, MONAI's amp) --------------
+class FactorizerBlockF16Fn(_Block16Fn):
+    """FactorizerBlockBf16Fn with fp16 activations: the same nine steps on the same kernels (tcgen05 kind::f16 with fp16
+    operands, fz_linear_forward_f16 / fz_linear_wgrad_f16, the fp16 LayerNorm, the fp16 fused core), fp32 parameters,
+    gradients and sums, one rounding to fp16 after bias, residual and GELU.  fp16 has 3 more mantissa bits than bf16 and
+    a range up to 65504: a sum beyond it is stored as +-inf, which torch.amp.GradScaler detects and skips the step."""
+    dtype = torch.float16
 
     @staticmethod
-    def _maps(staged, shapes):
-        def bind(views, shape):
-            return lambda x, bias, epi=EPI_NONE, aux=None, transposed=False: _channel_map_bf16(
-                x, views[transposed], shape[transposed], bias, epi, aux)
-        return [bind(v, shape) for v, shape in zip(_staged_views(staged[0], shapes), shapes)]
+    def forward(ctx, *args):
+        return FactorizerBlockF16Fn._forward(ctx, *args)
 
 
 # ---- channels-first LayerNorm (glue around the mixer) --------------------------------------------

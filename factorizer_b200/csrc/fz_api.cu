@@ -88,7 +88,7 @@ int make_dev_geom(const fz_geom* g, DevGeom* o) {
     if (g->path < FZ_PATH_AUTO || g->path > FZ_PATH_OCTANT_PIPELINE)
         return fail(FZ_ERR_INVALID, "fz_geom.path=%d is not one of FZ_PATH_*", g->path);
     o->path = g->path;
-    if (g->dtype != FZ_DTYPE_F32 && g->dtype != FZ_DTYPE_BF16)
+    if (g->dtype != FZ_DTYPE_F32 && g->dtype != FZ_DTYPE_BF16 && g->dtype != FZ_DTYPE_F16)
         return fail(FZ_ERR_INVALID, "fz_geom.dtype=%d is not one of FZ_DTYPE_*", g->dtype);
     o->dtype = g->dtype;
     return FZ_OK;
@@ -188,25 +188,34 @@ size_t fz_swnmf_workspace_bytes(const fz_geom* g, const fz_solver* s) {
     return a;
 }
 
-static const char* const kBf16Coverage =
-    "bf16 volumes are served by the octant kernels (head_dim 8, patch 8x8x8, ReLU, rank-1 HALS, an even number of "
+static const char* const k16BitCoverage =
+    "bf16 and fp16 volumes are served by the octant kernels (head_dim 8, patch 8x8x8, ReLU, rank-1 HALS, an even number of "
     "patches along W, and window sets that pair up as (a, a + 4) with every base shift a even along W, e.g. shifts "
     "[0, 4] or [0, 2, 4, 6]) and by the sub-warp kernels (64-column windows with head_dim 4, 8, 16 or 32, or 8 x 16, "
     "8 x 128 or 8 x 256 windows, at any shifts, rank-1 HALS or MU with up to 5 iterations, ReLU or not)";
 
 // The window-at-a-time 8x512 kernels (path 1), the grid-wide (5) and the generic (0) kernels take fp32 volumes only.
-static bool bf16_small_ok(const DevGeom& G, const fz_solver& s) {
+static bool half_small_ok(const DevGeom& G, const fz_solver& s) {
     return G.path != FZ_PATH_GENERIC && small_window_supported(G, s);
 }
 
-int fz_swnmf_bf16_supported(const fz_geom* g, const fz_solver* s, int32_t relu_input) {
+// bf16 and fp16 volumes take the same kernels at the same geometries
+static int half_supported(const fz_geom* g, const fz_solver* s, int32_t relu_input, int dtype) {
     if (!g || !s) return 0;
     fz_geom gb = *g;
-    gb.dtype = FZ_DTYPE_BF16;
+    gb.dtype = dtype;
     DevGeom G;
     int K;
     if (make_dev_geom(&gb, &G) || check_solver(s, G.d, G.P, &K)) return 0;
-    return phase_supported(G, *s, relu_input) || pairs_supported(G, *s, relu_input) || bf16_small_ok(G, *s) ? 1 : 0;
+    return phase_supported(G, *s, relu_input) || pairs_supported(G, *s, relu_input) || half_small_ok(G, *s) ? 1 : 0;
+}
+
+int fz_swnmf_bf16_supported(const fz_geom* g, const fz_solver* s, int32_t relu_input) {
+    return half_supported(g, s, relu_input, FZ_DTYPE_BF16);
+}
+
+int fz_swnmf_f16_supported(const fz_geom* g, const fz_solver* s, int32_t relu_input) {
+    return half_supported(g, s, relu_input, FZ_DTYPE_F16);
 }
 
 int fz_swnmf_forward(const float* x, const float* u0, const float* v0, float* y, void* saved,
@@ -236,7 +245,7 @@ int fz_swnmf_forward(const float* x, const float* u0, const float* v0, float* y,
         return e;
     }
     if (G.dtype != FZ_DTYPE_F32) {
-        if (!bf16_small_ok(G, *s)) return fail(FZ_ERR_UNSUPPORTED, "%s", kBf16Coverage);
+        if (!half_small_ok(G, *s)) return fail(FZ_ERR_UNSUPPORTED, "%s", k16BitCoverage);
         tls().path = 3;
         return small_window(x, u0, v0, nullptr, y, workspace, G, *s, K, relu_input, false, (cudaStream_t)stream);
     }
@@ -286,7 +295,7 @@ int fz_swnmf_backward(const float* x, const float* gy, const float* u0, const fl
         return pairs_backward(x, gy, v0, saved, gx, workspace, G, *s, K, (cudaStream_t)stream);
     }
     if (G.dtype != FZ_DTYPE_F32) {
-        if (!bf16_small_ok(G, *s)) return fail(FZ_ERR_UNSUPPORTED, "%s", kBf16Coverage);
+        if (!half_small_ok(G, *s)) return fail(FZ_ERR_UNSUPPORTED, "%s", k16BitCoverage);
         tls().path = 3;
         return small_window(x, u0, v0, gy, gx, workspace, G, *s, K, relu_input, true, (cudaStream_t)stream);
     }

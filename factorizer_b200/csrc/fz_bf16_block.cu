@@ -1,6 +1,7 @@
-// The bf16 FactorizerBlock's channel maps on the tensor cores (tcgen05 kind::f16: bf16 operands, fp32 accumulator in TMEM),
-// and the launch that stages its weights in bf16.  The U-Net scaffold's bf16 layers use the same channel maps and staging,
-// and the stem's weight gradient below.
+// The bf16 and fp16 FactorizerBlocks' channel maps on the tensor cores (tcgen05 kind::f16: bf16 or fp16 operands, fp32
+// accumulator in TMEM), and the launch that stages their weights in 16 bits.  The U-Net scaffold's bf16 layers use the same
+// channel maps and staging, and the stem's weight gradient below.  The kernels are templated on the 16-bit element type E,
+// which sets the TMA data type, the MMA's operand format and the conversions (Elem16 below); nothing else differs.
 //
 // Channel map  y[b][o][v] = sum_c W[o][c] x[b][c][v] (+ bias[o]), with the item walk, the 2/4-stage launch policy and the five
 // FZ_EPILOGUE_* epilogues it shares with linear_fwd_tc (fz_channel_map.cuh) -- one MMA per 16 channels and no remainder tiles:
@@ -18,6 +19,7 @@
 // (N = 128 inputs + the bias column), four MMAs per stage; dW, db fp32 with one atomic per element and CTA; the chain is
 // capped at 32 stages per CTA as there (cmap::wgrad_ctas).
 #include <cuda_bf16.h>
+#include <cuda_fp16.h>
 
 #include "fz_channel_map.cuh"
 #include "fz_internal.cuh"
@@ -29,6 +31,20 @@ namespace {
 using namespace tc;
 typedef __nv_bfloat16 bf16;
 
+template <typename E> struct Elem16;
+template <> struct Elem16<bf16> {
+    static constexpr CUtensorMapDataType kTma = CU_TENSOR_MAP_DATA_TYPE_BFLOAT16;
+    static constexpr uint32_t kFormat = 1;             // instruction descriptor, A / B format
+    static constexpr const char* kName = "bf16";
+    static __device__ __forceinline__ bf16 from(float v) { return __float2bfloat16_rn(v); }
+};
+template <> struct Elem16<__half> {
+    static constexpr CUtensorMapDataType kTma = CU_TENSOR_MAP_DATA_TYPE_FLOAT16;
+    static constexpr uint32_t kFormat = 0;
+    static constexpr const char* kName = "fp16";
+    static __device__ __forceinline__ __half from(float v) { return __float2half_rn(v); }
+};
+
 // ---- channel map ------------------------------------------------------------------------------------------------------------
 constexpr int kHM = cmap::kM, kHN = cmap::kN, kHK = 64;   // voxels x outputs per item, channels per K chunk (one 128-byte row)
 constexpr uint32_t kHA = kHK * kHM * 2;               // x chunk: two boxes of (64 channels x 64 voxels) = 16 KiB
@@ -37,28 +53,30 @@ constexpr uint32_t hA = 0, hB = kHA, kHStage = kHA + kHB;
 // barriers behind the stages: full / empty per stage, accumulator full / free per accumulator, the TMEM slot
 __host__ __device__ constexpr uint32_t h_smem_bytes(int stages) { return stages * kHStage + 2 * 8 * stages + 16 + 16 + 8; }
 
-// x as (batch, channels, voxels) bf16: box (1, 64, 64)
-int make_map_x16(CUtensorMap* m, const bf16* ptr, long long batch, int channels, long long voxels) {
+// x as (batch, channels, voxels) of E: box (1, 64, 64)
+template <typename E>
+int make_map_x16(CUtensorMap* m, const E* ptr, long long batch, int channels, long long voxels) {
     cuuint64_t dims[3] = {(cuuint64_t)voxels, (cuuint64_t)channels, (cuuint64_t)batch};
     cuuint64_t strides[2] = {(cuuint64_t)voxels * 2, (cuuint64_t)voxels * channels * 2};
     cuuint32_t box[3] = {64, kHK, 1};
-    return encode_tiled_map(m, "x (bf16)", CU_TENSOR_MAP_DATA_TYPE_BFLOAT16, 3, ptr, dims, strides, box, CU_TENSOR_MAP_SWIZZLE_128B);
+    return encode_tiled_map(m, "x (16-bit)", Elem16<E>::kTma, 3, ptr, dims, strides, box, CU_TENSOR_MAP_SWIZZLE_128B);
 }
-// a K-major bf16 matrix (rows, cols) with rows `ld` elements apart: box (box_rows, 64 columns)
+// a K-major matrix of E (rows, cols) with rows `ld` elements apart: box (box_rows, 64 columns)
 // (rank 2, or rank 3 with `batch` such matrices rows * ld elements apart)
-int make_map_rows16(CUtensorMap* m, const char* what, const bf16* ptr, long long rows, long long cols, long long ld, int box_rows,
+template <typename E>
+int make_map_rows16(CUtensorMap* m, const char* what, const E* ptr, long long rows, long long cols, long long ld, int box_rows,
                     int rank, long long batch = 1) {
     cuuint64_t dims[3] = {(cuuint64_t)cols, (cuuint64_t)rows, (cuuint64_t)batch};
     cuuint64_t strides[2] = {(cuuint64_t)ld * 2, (cuuint64_t)ld * rows * 2};
     cuuint32_t box[3] = {64, (cuuint32_t)box_rows, 1};
-    return encode_tiled_map(m, what, CU_TENSOR_MAP_DATA_TYPE_BFLOAT16, rank, ptr, dims, strides, box,
+    return encode_tiled_map(m, what, Elem16<E>::kTma, rank, ptr, dims, strides, box,
                             CU_TENSOR_MAP_SWIZZLE_128B);
 }
 
-template <int STAGES>
+template <typename E, int STAGES>
 __global__ void __launch_bounds__(cmap::kThreads, STAGES <= 2 ? 2 : 1)
 linear_fwd_bf16_tc(const __grid_constant__ CUtensorMap map_x, const __grid_constant__ CUtensorMap map_w, const float* __restrict__ bias,
-                   bf16* __restrict__ y, const bf16* __restrict__ aux, bf16* __restrict__ y2, int epi, int cout, int cin, long long vox,
+                   E* __restrict__ y, const E* __restrict__ aux, E* __restrict__ y2, int epi, int cout, int cin, long long vox,
                    int vtiles_per_sample, int otiles, long long total_items) {
     constexpr uint32_t hBarFull = STAGES * kHStage, hBarEmpty = hBarFull + 8 * STAGES, hBarAccFull = hBarEmpty + 8 * STAGES,
                        hBarAccFree = hBarAccFull + 16, hTmemSlot = hBarAccFree + 16;
@@ -115,7 +133,7 @@ linear_fwd_bf16_tc(const __grid_constant__ CUtensorMap map_x, const __grid_const
         __syncwarp();
     } else if (warp == 1) {
         // ---- MMA issue: one accumulator per item, two in TMEM ----
-        const uint32_t idesc = make_idesc_bf16(kHM, kHN, true, false);         // A MN-major, B K-major
+        const uint32_t idesc = make_idesc_16bit(kHM, kHN, true, false, Elem16<E>::kFormat);   // A MN-major, B K-major
         long long g = 0;
         for (long long it = 0; it < my_items; ++it) {
             const uint32_t acc = (uint32_t)(it & 1), use = (uint32_t)(it >> 1);
@@ -139,9 +157,9 @@ linear_fwd_bf16_tc(const __grid_constant__ CUtensorMap map_x, const __grid_const
             }
         }
     } else {
-        // ---- workers: drain an item's accumulator, apply the epilogue in fp32, store bf16 ----
+        // ---- workers: drain an item's accumulator, apply the epilogue in fp32, store E ----
         const int wq = warp & 3, wh = (warp - 2) >> 2;                     // TMEM lane quarter this warp may read; half of the columns
-        const cmap::Epilogue<bf16> ep{bias, y, aux, y2, epi, cout, otiles, vtiles_per_sample, vox, wq, wh, lane};
+        const cmap::Epilogue<E> ep{bias, y, aux, y2, epi, cout, otiles, vtiles_per_sample, vox, wq, wh, lane};
         for (long long it = 0; it < my_items; ++it) {
             // the running sums start from the residual or the bias; their loads are in flight while the MMAs finish
             float sum[32];
@@ -177,7 +195,7 @@ constexpr int kWBlk = 128;                              // channels per block of
 constexpr int kWVT = 64;                                // voxels per stage = one 128-byte swizzle row
 constexpr int kWStages = 3;
 constexpr int kWThreads = 192;
-constexpr uint32_t kWTile = kWBlk * 128;                // one (128 x 64) bf16 tile: 16 KiB
+constexpr uint32_t kWTile = kWBlk * 128;                // one (128 x 64) 16-bit tile: 16 KiB
 // stage: dy | x | ones block (16 rows: the first all ones)
 constexpr uint32_t wA = 0, wB = kWTile, wOnes = 2 * kWTile, kWStage = 2 * kWTile + 16 * 128;
 constexpr uint32_t wBarFull = kWStages * kWStage, wBarEmpty = wBarFull + 8 * kWStages, wBarDone = wBarEmpty + 8 * kWStages,
@@ -185,6 +203,7 @@ constexpr uint32_t wBarFull = kWStages * kWStage, wBarEmpty = wBarFull + 8 * kWS
 constexpr int kWN = kWBlk + 16;                         // 144 accumulator columns
 static_assert(kWBlk * (kWBlk + 17) * 4 <= kWStages * kWStage, "the epilogue's scratch copy fits in the stages");
 
+template <typename E>
 __global__ void __launch_bounds__(kWThreads, 2)
 linear_wgrad_bf16_tc(const __grid_constant__ CUtensorMap map_dy, const __grid_constant__ CUtensorMap map_x, float* __restrict__ dW,
                      float* __restrict__ db, int cout, int cin, int tiles_per_sample, long long total_tiles) {
@@ -206,7 +225,7 @@ linear_wgrad_bf16_tc(const __grid_constant__ CUtensorMap map_dy, const __grid_co
     // the ones block of every stage (constant): row 0 = ones, rows 1 .. 15 = zeros (a 128-byte row of equal values: no swizzle to mind)
     for (int i = tid; i < kWStages * 16 * 64; i += kWThreads) {
         const int s = i / (16 * 64), r = (i / 64) % 16;
-        reinterpret_cast<bf16*>(smem + s * kWStage + wOnes)[i % (16 * 64)] = __float2bfloat16_rn(r == 0 ? 1.f : 0.f);
+        reinterpret_cast<E*>(smem + s * kWStage + wOnes)[i % (16 * 64)] = Elem16<E>::from(r == 0 ? 1.f : 0.f);
     }
     if (warp == 1) {
         tmem_alloc<256>(sbase + wTmemSlot);
@@ -238,7 +257,7 @@ linear_wgrad_bf16_tc(const __grid_constant__ CUtensorMap map_dy, const __grid_co
         __syncwarp();
     } else if (warp == 1) {
         // ---- MMA issue: D[128 x 144] += dy (rows) x [x ; ones] (columns) over the stage's 4 groups of 16 voxels ----
-        const uint32_t idesc = make_idesc_bf16(kWBlk, kWN, false, false);
+        const uint32_t idesc = make_idesc_16bit(kWBlk, kWN, false, false, Elem16<E>::kFormat);
         for (long long it = 0; it < my_tiles; ++it) {
             const int s = (int)(it % kWStages);
             const uint32_t round = (uint32_t)(it / kWStages);
@@ -434,7 +453,7 @@ stem_wgrad_bf16_tc(const __grid_constant__ CUtensorMap map_dy, const TX* __restr
 }
 
 // ---- weight staging ---------------------------------------------------------------------------------------------------------
-// bf16 rows are padded to whole 16-byte groups: a TMA row stride must be a multiple of 16 bytes
+// 16-bit rows are padded to whole 16-byte groups: a TMA row stride must be a multiple of 16 bytes
 __host__ __device__ inline long long ld8(long long n) { return (n + 7) & ~7LL; }
 
 struct StageArgs {
@@ -443,7 +462,8 @@ struct StageArgs {
     long long off[9];                                           // start of each of the 8 outputs (W_i, W_i^T), and the total
 };
 
-__global__ void __launch_bounds__(256) stage_weights_bf16(StageArgs a, bf16* __restrict__ out) {
+template <typename E>
+__global__ void __launch_bounds__(256) stage_weights_bf16(StageArgs a, E* __restrict__ out) {
     for (long long i = (long long)blockIdx.x * blockDim.x + threadIdx.x; i < a.off[8]; i += (long long)gridDim.x * blockDim.x) {
         int j = 0;
 #pragma unroll
@@ -459,12 +479,13 @@ __global__ void __launch_bounds__(256) stage_weights_bf16(StageArgs a, bf16* __r
             const long long ld = ld8(R), c = local / ld, r = local - c * ld;
             if (r < R) v = __ldg(a.w[m] + r * C + c);
         }
-        out[i] = __float2bfloat16_rn(v);
+        out[i] = Elem16<E>::from(v);
     }
 }
 
 bool aligned16(const void* p) { return (reinterpret_cast<uintptr_t>(p) & 15) == 0; }
 
+template <typename E>
 int stage_weights_launch(int n, const float* const* w, const int* r, const int* c, void* out, void* stream) {
     tls().launches = 0;
     StageArgs a;
@@ -490,7 +511,85 @@ int stage_weights_launch(int n, const float* const* w, const int* r, const int* 
     if (!aligned16(out)) return fail(FZ_ERR_UNSUPPORTED, "staged weights must be 16-byte aligned");
     long long blocks = (off + 255) / 256;
     if (blocks > 4LL * num_sms()) blocks = 4LL * num_sms();
-    stage_weights_bf16<<<(unsigned)blocks, 256, 0, (cudaStream_t)stream>>>(a, static_cast<bf16*>(out));
+    stage_weights_bf16<<<(unsigned)blocks, 256, 0, (cudaStream_t)stream>>>(a, static_cast<E*>(out));
+    FZ_LAUNCH_CHECK();
+    return FZ_OK;
+}
+
+bool channel_map16_supported(int32_t cout, int32_t cin, int64_t voxels) {
+    return cout > 0 && cin > 0 && voxels > 0 && voxels % 8 == 0 && voxels < (1LL << 31);
+}
+
+template <typename E>
+int linear_forward16(const void* x, const void* W, int32_t ldw, const float* bias, void* y, int64_t batch, int32_t cin, int32_t cout,
+                     int64_t voxels, int32_t epilogue, const void* aux, void* y2, void* stream) {
+    const char* nm = Elem16<E>::kName;
+    tls().launches = 0;
+    if (batch == 0) return FZ_OK;
+    if (!x || !W || !y) return fail(FZ_ERR_INVALID, "null buffer");
+    if (batch < 0 || batch >= (1LL << 31)) return fail(FZ_ERR_INVALID, "batch=%lld", (long long)batch);
+    char what[32];
+    snprintf(what, sizeof(what), "%s channel map", nm);
+    if (int e = cmap::check_epilogue(what, epilogue, aux, y2)) return e;
+    if (!channel_map16_supported(cout, cin, voxels))
+        return fail(FZ_ERR_UNSUPPORTED, "%s channel map: voxels must be a positive multiple of 8 below 2^31 (got %lld)", nm, (long long)voxels);
+    if (ldw < cin || ldw % 8) return fail(FZ_ERR_UNSUPPORTED, "%s channel map: ldw=%d must be >= cin=%d and a multiple of 8", nm, ldw, cin);
+    if (!aligned16(x) || !aligned16(W))
+        return fail(FZ_ERR_UNSUPPORTED, "%s channel map: x and W must be 16-byte aligned", nm);
+    if (((reinterpret_cast<uintptr_t>(y) | reinterpret_cast<uintptr_t>(aux) | reinterpret_cast<uintptr_t>(y2)) & 1))
+        return fail(FZ_ERR_UNSUPPORTED, "%s channel map: y, aux and y2 must be 2-byte aligned", nm);
+    CUtensorMap map_x, map_w;
+    if (int e = make_map_x16(&map_x, static_cast<const E*>(x), batch, cin, voxels)) return e;
+    if (int e = make_map_rows16(&map_w, "W (16-bit)", static_cast<const E*>(W), cout, cin, ldw, kHN, 2)) return e;
+    const int vtps = (int)((voxels + kHM - 1) / kHM);
+    const int otiles = (cout + kHN - 1) / kHN;
+    const long long items = batch * vtps * otiles;
+    if (items >= (1LL << 31)) return fail(FZ_ERR_UNSUPPORTED, "%s channel map: more than 2^31 (voxel tile, output tile) items", nm);
+    E* ye = static_cast<E*>(y);
+    E* y2e = static_cast<E*>(y2);
+    const E* ae = static_cast<const E*>(aux);
+    cudaStream_t st = (cudaStream_t)stream;
+    const cmap::Launch ls = cmap::launch_shape(items, (cin + kHK - 1) / kHK);
+    if (ls.stages == 4) {
+        static SmemConfig cfg4;
+        FZ_CUDA_CHECK(cfg4.ensure(linear_fwd_bf16_tc<E, 4>, h_smem_bytes(4)));
+        linear_fwd_bf16_tc<E, 4><<<ls.blocks, cmap::kThreads, h_smem_bytes(4), st>>>(map_x, map_w, bias, ye, ae, y2e, epilogue, cout, cin,
+                                                                                    voxels, vtps, otiles, items);
+    } else {
+        static SmemConfig cfg2;
+        FZ_CUDA_CHECK(cfg2.ensure(linear_fwd_bf16_tc<E, 2>, h_smem_bytes(2)));
+        linear_fwd_bf16_tc<E, 2><<<ls.blocks, cmap::kThreads, h_smem_bytes(2), st>>>(map_x, map_w, bias, ye, ae, y2e, epilogue, cout, cin,
+                                                                                    voxels, vtps, otiles, items);
+    }
+    FZ_LAUNCH_CHECK();
+    return FZ_OK;
+}
+
+template <typename E>
+int linear_wgrad16(const void* dy, const void* x, float* dW, float* db, int64_t batch, int32_t cout, int32_t cin, int64_t voxels,
+                   void* stream) {
+    const char* nm = Elem16<E>::kName;
+    tls().launches = 0;
+    cudaStream_t st = (cudaStream_t)stream;
+    if (!dW) return fail(FZ_ERR_INVALID, "null buffer");
+    if (cout < 1 || cin < 1 || batch < 0 || batch >= (1LL << 31)) return fail(FZ_ERR_INVALID, "bad sizes");
+    FZ_CUDA_CHECK(cudaMemsetAsync(dW, 0, sizeof(float) * (size_t)cout * cin, st));
+    if (db) FZ_CUDA_CHECK(cudaMemsetAsync(db, 0, sizeof(float) * (size_t)cout, st));
+    if (batch == 0 || voxels == 0) return FZ_OK;
+    if (!dy || !x) return fail(FZ_ERR_INVALID, "null buffer");
+    if (!channel_map16_supported(cout, cin, voxels))
+        return fail(FZ_ERR_UNSUPPORTED, "%s weight gradient: voxels must be a positive multiple of 8 below 2^31 (got %lld)", nm, (long long)voxels);
+    if (!aligned16(dy) || !aligned16(x)) return fail(FZ_ERR_UNSUPPORTED, "%s weight gradient: dy and x must be 16-byte aligned", nm);
+    CUtensorMap map_dy, map_x;
+    if (int e = make_map_rows16(&map_dy, "dy (16-bit)", static_cast<const E*>(dy), cout, voxels, voxels, kWBlk, 3, batch)) return e;
+    if (int e = make_map_rows16(&map_x, "x (16-bit)", static_cast<const E*>(x), cin, voxels, voxels, kWBlk, 3, batch)) return e;
+    static SmemConfig cfg;
+    FZ_CUDA_CHECK(cfg.ensure(linear_wgrad_bf16_tc<E>, kWSmem));
+    const int tps = (int)((voxels + kWVT - 1) / kWVT);
+    const long long tiles = batch * tps;
+    const int bo = (cout + kWBlk - 1) / kWBlk, bi = (cin + kWBlk - 1) / kWBlk;
+    const long long gx = cmap::wgrad_ctas((2LL * num_sms() + bo * bi - 1) / (bo * bi), tiles);
+    linear_wgrad_bf16_tc<E><<<dim3((unsigned)gx, bo, bi), kWThreads, kWSmem, st>>>(map_dy, map_x, dW, db, cout, cin, tps, tiles);
     FZ_LAUNCH_CHECK();
     return FZ_OK;
 }
@@ -502,81 +601,18 @@ using namespace fz;
 
 extern "C" {
 
-int fz_linear_forward_bf16_supported(int32_t cout, int32_t cin, int64_t voxels) {
-    return cout > 0 && cin > 0 && voxels > 0 && voxels % 8 == 0 && voxels < (1LL << 31);
-}
+int fz_linear_forward_bf16_supported(int32_t cout, int32_t cin, int64_t voxels) { return channel_map16_supported(cout, cin, voxels); }
 
 int fz_linear_forward_bf16(const void* x, const void* W, int32_t ldw, const float* bias, void* y, int64_t batch, int32_t cin, int32_t cout,
                            int64_t voxels, int32_t epilogue, const void* aux, void* y2, void* stream) {
-    tls().launches = 0;
-    if (batch == 0) return FZ_OK;
-    if (!x || !W || !y) return fail(FZ_ERR_INVALID, "null buffer");
-    if (batch < 0 || batch >= (1LL << 31)) return fail(FZ_ERR_INVALID, "batch=%lld", (long long)batch);
-    if (int e = cmap::check_epilogue("bf16 channel map", epilogue, aux, y2)) return e;
-    if (!fz_linear_forward_bf16_supported(cout, cin, voxels))
-        return fail(FZ_ERR_UNSUPPORTED, "bf16 channel map: voxels must be a positive multiple of 8 below 2^31 (got %lld)", (long long)voxels);
-    if (ldw < cin || ldw % 8) return fail(FZ_ERR_UNSUPPORTED, "bf16 channel map: ldw=%d must be >= cin=%d and a multiple of 8", ldw, cin);
-    if (!aligned16(x) || !aligned16(W))
-        return fail(FZ_ERR_UNSUPPORTED, "bf16 channel map: x and W must be 16-byte aligned");
-    if (((reinterpret_cast<uintptr_t>(y) | reinterpret_cast<uintptr_t>(aux) | reinterpret_cast<uintptr_t>(y2)) & 1))
-        return fail(FZ_ERR_UNSUPPORTED, "bf16 channel map: y, aux and y2 must be 2-byte aligned");
-    CUtensorMap map_x, map_w;
-    const bf16* xb = static_cast<const bf16*>(x);
-    if (int e = make_map_x16(&map_x, xb, batch, cin, voxels)) return e;
-    if (int e = make_map_rows16(&map_w, "W (bf16)", static_cast<const bf16*>(W), cout, cin, ldw, kHN, 2)) return e;
-    const int vtps = (int)((voxels + kHM - 1) / kHM);
-    const int otiles = (cout + kHN - 1) / kHN;
-    const long long items = batch * vtps * otiles;
-    if (items >= (1LL << 31)) return fail(FZ_ERR_UNSUPPORTED, "bf16 channel map: more than 2^31 (voxel tile, output tile) items");
-    bf16* yb = static_cast<bf16*>(y);
-    bf16* y2b = static_cast<bf16*>(y2);
-    const bf16* ab = static_cast<const bf16*>(aux);
-    cudaStream_t st = (cudaStream_t)stream;
-    const cmap::Launch ls = cmap::launch_shape(items, (cin + kHK - 1) / kHK);
-    if (ls.stages == 4) {
-        static SmemConfig cfg4;
-        FZ_CUDA_CHECK(cfg4.ensure(linear_fwd_bf16_tc<4>, h_smem_bytes(4)));
-        linear_fwd_bf16_tc<4><<<ls.blocks, cmap::kThreads, h_smem_bytes(4), st>>>(map_x, map_w, bias, yb, ab, y2b, epilogue, cout, cin, voxels,
-                                                                                 vtps, otiles, items);
-    } else {
-        static SmemConfig cfg2;
-        FZ_CUDA_CHECK(cfg2.ensure(linear_fwd_bf16_tc<2>, h_smem_bytes(2)));
-        linear_fwd_bf16_tc<2><<<ls.blocks, cmap::kThreads, h_smem_bytes(2), st>>>(map_x, map_w, bias, yb, ab, y2b, epilogue, cout, cin, voxels,
-                                                                                 vtps, otiles, items);
-    }
-    FZ_LAUNCH_CHECK();
-    return FZ_OK;
+    return linear_forward16<bf16>(x, W, ldw, bias, y, batch, cin, cout, voxels, epilogue, aux, y2, stream);
 }
 
-int fz_linear_wgrad_bf16_supported(int32_t cout, int32_t cin, int64_t voxels) {
-    return cout > 0 && cin > 0 && voxels > 0 && voxels % 8 == 0 && voxels < (1LL << 31);
-}
+int fz_linear_wgrad_bf16_supported(int32_t cout, int32_t cin, int64_t voxels) { return channel_map16_supported(cout, cin, voxels); }
 
 int fz_linear_wgrad_bf16(const void* dy, const void* x, float* dW, float* db, int64_t batch, int32_t cout, int32_t cin, int64_t voxels,
                          void* stream) {
-    tls().launches = 0;
-    cudaStream_t st = (cudaStream_t)stream;
-    if (!dW) return fail(FZ_ERR_INVALID, "null buffer");
-    if (cout < 1 || cin < 1 || batch < 0 || batch >= (1LL << 31)) return fail(FZ_ERR_INVALID, "bad sizes");
-    FZ_CUDA_CHECK(cudaMemsetAsync(dW, 0, sizeof(float) * (size_t)cout * cin, st));
-    if (db) FZ_CUDA_CHECK(cudaMemsetAsync(db, 0, sizeof(float) * (size_t)cout, st));
-    if (batch == 0 || voxels == 0) return FZ_OK;
-    if (!dy || !x) return fail(FZ_ERR_INVALID, "null buffer");
-    if (!fz_linear_wgrad_bf16_supported(cout, cin, voxels))
-        return fail(FZ_ERR_UNSUPPORTED, "bf16 weight gradient: voxels must be a positive multiple of 8 below 2^31 (got %lld)", (long long)voxels);
-    if (!aligned16(dy) || !aligned16(x)) return fail(FZ_ERR_UNSUPPORTED, "bf16 weight gradient: dy and x must be 16-byte aligned");
-    CUtensorMap map_dy, map_x;
-    if (int e = make_map_rows16(&map_dy, "dy (bf16)", static_cast<const bf16*>(dy), cout, voxels, voxels, kWBlk, 3, batch)) return e;
-    if (int e = make_map_rows16(&map_x, "x (bf16)", static_cast<const bf16*>(x), cin, voxels, voxels, kWBlk, 3, batch)) return e;
-    static SmemConfig cfg;
-    FZ_CUDA_CHECK(cfg.ensure(linear_wgrad_bf16_tc, kWSmem));
-    const int tps = (int)((voxels + kWVT - 1) / kWVT);
-    const long long tiles = batch * tps;
-    const int bo = (cout + kWBlk - 1) / kWBlk, bi = (cin + kWBlk - 1) / kWBlk;
-    const long long gx = cmap::wgrad_ctas((2LL * num_sms() + bo * bi - 1) / (bo * bi), tiles);
-    linear_wgrad_bf16_tc<<<dim3((unsigned)gx, bo, bi), kWThreads, kWSmem, st>>>(map_dy, map_x, dW, db, cout, cin, tps, tiles);
-    FZ_LAUNCH_CHECK();
-    return FZ_OK;
+    return linear_wgrad16<bf16>(dy, x, dW, db, batch, cout, cin, voxels, stream);
 }
 
 int fz_bf16_stage_weights_supported(int32_t rows, int32_t cols) {
@@ -591,11 +627,40 @@ int fz_bf16_stage_weights(const float* w0, int32_t r0, int32_t c0, const float* 
                           int32_t c2, const float* w3, int32_t r3, int32_t c3, void* out, void* stream) {
     const float* w[4] = {w0, w1, w2, w3};
     const int r[4] = {r0, r1, r2, r3}, c[4] = {c0, c1, c2, c3};
-    return stage_weights_launch(4, w, r, c, out, stream);
+    return stage_weights_launch<bf16>(4, w, r, c, out, stream);
 }
 
 int fz_bf16_stage_weight(const float* w, int32_t rows, int32_t cols, void* out, void* stream) {
-    return stage_weights_launch(1, &w, &rows, &cols, out, stream);
+    return stage_weights_launch<bf16>(1, &w, &rows, &cols, out, stream);
+}
+
+int fz_linear_forward_f16_supported(int32_t cout, int32_t cin, int64_t voxels) { return channel_map16_supported(cout, cin, voxels); }
+
+int fz_linear_forward_f16(const void* x, const void* W, int32_t ldw, const float* bias, void* y, int64_t batch, int32_t cin, int32_t cout,
+                          int64_t voxels, int32_t epilogue, const void* aux, void* y2, void* stream) {
+    return linear_forward16<__half>(x, W, ldw, bias, y, batch, cin, cout, voxels, epilogue, aux, y2, stream);
+}
+
+int fz_linear_wgrad_f16_supported(int32_t cout, int32_t cin, int64_t voxels) { return channel_map16_supported(cout, cin, voxels); }
+
+int fz_linear_wgrad_f16(const void* dy, const void* x, float* dW, float* db, int64_t batch, int32_t cout, int32_t cin, int64_t voxels,
+                        void* stream) {
+    return linear_wgrad16<__half>(dy, x, dW, db, batch, cout, cin, voxels, stream);
+}
+
+int fz_f16_stage_weights_supported(int32_t rows, int32_t cols) { return fz_bf16_stage_weights_supported(rows, cols); }
+
+int64_t fz_f16_staged_elems(int32_t rows, int32_t cols) { return fz_bf16_staged_elems(rows, cols); }
+
+int fz_f16_stage_weights(const float* w0, int32_t r0, int32_t c0, const float* w1, int32_t r1, int32_t c1, const float* w2, int32_t r2,
+                         int32_t c2, const float* w3, int32_t r3, int32_t c3, void* out, void* stream) {
+    const float* w[4] = {w0, w1, w2, w3};
+    const int r[4] = {r0, r1, r2, r3}, c[4] = {c0, c1, c2, c3};
+    return stage_weights_launch<__half>(4, w, r, c, out, stream);
+}
+
+int fz_f16_stage_weight(const float* w, int32_t rows, int32_t cols, void* out, void* stream) {
+    return stage_weights_launch<__half>(1, &w, &rows, &cols, out, stream);
 }
 
 int fz_conv3d_stem_wgrad_bf16_supported(int32_t cin, int32_t cout, int32_t D, int32_t H, int32_t W) {

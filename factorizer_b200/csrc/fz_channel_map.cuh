@@ -4,6 +4,7 @@
 // and Epilogue is what it does with their running sums.  And the host side of both launchers and of the weight gradients.
 #pragma once
 #include <cuda_bf16.h>
+#include <cuda_fp16.h>
 
 #include "fz_device.cuh"
 
@@ -13,11 +14,13 @@ namespace cmap {
 constexpr int kM = 128, kN = 64;                      // voxels x outputs per item
 constexpr int kThreads = 320;
 
-// load as float, store from float (bf16: rounded to nearest once)
+// load as float, store from float (bf16, fp16: rounded to nearest once; an fp16 value beyond 65504 becomes +-inf)
 __device__ __forceinline__ float ldg_f(const float* p) { return __ldg(p); }
 __device__ __forceinline__ float ldg_f(const __nv_bfloat16* p) { return __bfloat162float(__ldg(p)); }
+__device__ __forceinline__ float ldg_f(const __half* p) { return __half2float(__ldg(p)); }
 __device__ __forceinline__ void st_f(float* p, float v) { *p = v; }
 __device__ __forceinline__ void st_f(__nv_bfloat16* p, float v) { *p = __float2bfloat16_rn(v); }
+__device__ __forceinline__ void st_f(__half* p, float v) { *p = __float2half_rn(v); }
 
 // A worker's epilogue: y, aux and y2 hold T (bias is fp32); FZ_EPILOGUE_*: + residual | y = r, y2 = gelu(r) |
 // y = r * gelu'(aux) | y = gelu(r)

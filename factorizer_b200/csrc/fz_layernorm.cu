@@ -9,9 +9,10 @@
 // issues one atomicAdd per channel and CTA.  HBM-bound: forward reads x and writes y once, backward reads
 // x and dy once and writes dx once.
 //
-// The kernels are templated on the element type T of x, y, dy, add and dx: float, or bf16 (the bf16 FactorizerBlock), which is
-// read and written as bf16 pairs and computed in fp32; gamma, beta, their gradients and the statistics stay fp32.
+// The kernels are templated on the element type T of x, y, dy, add and dx: float, or bf16 / fp16 (the 16-bit FactorizerBlocks),
+// which is read and written as pairs and computed in fp32; gamma, beta, their gradients and the statistics stay fp32.
 #include <cuda_bf16.h>
+#include <cuda_fp16.h>
 
 #include "fz_common.cuh"
 
@@ -21,14 +22,23 @@ namespace {
 template <typename T> struct Pair2;
 template <> struct Pair2<float> { typedef float2 type; };
 template <> struct Pair2<__nv_bfloat16> { typedef __nv_bfloat162 type; };
+template <> struct Pair2<__half> { typedef __half2 type; };
 template <typename T> using pair_t = typename Pair2<T>::type;   // two neighbouring voxels of one channel
 
 __device__ __forceinline__ float2 ld2(const float2* p) { return __ldg(p); }
 __device__ __forceinline__ float2 ld2(const __nv_bfloat162* p) { return __bfloat1622float2(__ldg(p)); }
+__device__ __forceinline__ float2 ld2(const __half2* p) { return __half22float2(__ldg(p)); }
 __device__ __forceinline__ float2 ld2cs(const float2* p) { return __ldcs(p); }
 __device__ __forceinline__ float2 ld2cs(const __nv_bfloat162* p) { return __bfloat1622float2(__ldcs(p)); }
+// fp16 streaming loads as one 32-bit word and two scalar conversions: in the 32-channel backward this keeps 256 bytes fewer
+// of spills than __half22float2 (sm_100a, -Xptxas -v)
+__device__ __forceinline__ float2 ld2cs(const __half2* p) {
+    const unsigned u = __ldcs(reinterpret_cast<const unsigned*>(p));
+    return make_float2(__half2float(__ushort_as_half((unsigned short)(u & 0xffffu))), __half2float(__ushort_as_half((unsigned short)(u >> 16))));
+}
 __device__ __forceinline__ void st2(float2* p, float2 v) { *p = v; }
 __device__ __forceinline__ void st2(__nv_bfloat162* p, float2 v) { *p = __float22bfloat162_rn(v); }
+__device__ __forceinline__ void st2(__half2* p, float2 v) { *p = __float22half2_rn(v); }
 
 constexpr int kLnThreads = 256;
 
@@ -593,6 +603,19 @@ int fz_layernorm_cf_backward_add_bf16(const void* x, const float* gamma, const v
     typedef __nv_bfloat16 bf16;
     return ln_backward_add(static_cast<const bf16*>(x), gamma, static_cast<const bf16*>(dy), static_cast<const bf16*>(add),
                            static_cast<bf16*>(dx), dgamma, dbeta, batch, channels, voxels, eps, stream);
+}
+
+int fz_layernorm_cf_f16_supported(int32_t channels, int64_t voxels) { return fz_layernorm_cf_supported(channels, voxels); }
+
+int fz_layernorm_cf_forward_f16(const void* x, const float* gamma, const float* beta, void* y, int64_t batch, int32_t channels,
+                                int64_t voxels, float eps, void* stream) {
+    return ln_forward(static_cast<const __half*>(x), gamma, beta, static_cast<__half*>(y), batch, channels, voxels, eps, stream);
+}
+
+int fz_layernorm_cf_backward_add_f16(const void* x, const float* gamma, const void* dy, const void* add, void* dx, float* dgamma,
+                                     float* dbeta, int64_t batch, int32_t channels, int64_t voxels, float eps, void* stream) {
+    return ln_backward_add(static_cast<const __half*>(x), gamma, static_cast<const __half*>(dy), static_cast<const __half*>(add),
+                           static_cast<__half*>(dx), dgamma, dbeta, batch, channels, voxels, eps, stream);
 }
 
 }  // extern "C"

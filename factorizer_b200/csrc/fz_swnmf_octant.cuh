@@ -21,6 +21,7 @@
 // There are no wrapped or misaligned boxes and no partial-sum round trip through the volume.
 #pragma once
 #include <cuda_bf16.h>
+#include <cuda_fp16.h>
 #include <type_traits>
 #include <stdlib.h>
 #include <string.h>
@@ -144,8 +145,8 @@ __device__ __forceinline__ int chunk_f4_shifted(int lane, int j) {
     return 16 * (4 * (1 - o0) + j) + 2 * (4 * (1 - o1) + t) + (1 - o2);
 }
 
-// How a streaming warp sees one tile in shared memory.  fp32: an (8,8,8,8) box, rows of 32 bytes.  bf16 activations: two
-// tiles side by side along W travel as one (16,8,8,8) box -- again rows of 32 bytes, the row granularity TMA and the L2
+// How a streaming warp sees one tile in shared memory.  fp32: an (8,8,8,8) box, rows of 32 bytes.  bf16 / fp16 activations:
+// two tiles side by side along W travel as one (16,8,8,8) box -- again rows of 32 bytes, the row granularity TMA and the L2
 // sectors like -- and a tile is one 16-byte column of that box.  ld(i, lane, j): the lane's chunk j of channel i as floats.
 struct TileF32 {
     const float* p;
@@ -153,13 +154,22 @@ struct TileF32 {
         return reinterpret_cast<const float4*>(p)[i * 128 + chunk_f4(lane, j)];
     }
 };
-struct TileBf16 {
+// four 16-bit values (two 32-bit words, the lower half first) as floats
+__device__ __forceinline__ float4 widen4(uint2 r, const __nv_bfloat16*) {
+    return make_float4(__uint_as_float(r.x << 16), __uint_as_float(r.x & 0xffff0000u),
+                       __uint_as_float(r.y << 16), __uint_as_float(r.y & 0xffff0000u));
+}
+__device__ __forceinline__ float4 widen4(uint2 r, const __half*) {
+    const float2 a = __half22float2(*reinterpret_cast<const __half2*>(&r.x)), b = __half22float2(*reinterpret_cast<const __half2*>(&r.y));
+    return make_float4(a.x, a.y, b.x, b.y);
+}
+template <typename E>             // E = __nv_bfloat16 or __half
+struct Tile16 {
     const unsigned char* p;       // pair buffer + 16 * (which tile of the pair)
     __device__ __forceinline__ float4 ld(int i, int lane, int j) const {
         const int o0 = lane >> 4, o1 = (lane >> 3) & 1, o2 = (lane >> 2) & 1, t = lane & 3;
         const uint2 r = *reinterpret_cast<const uint2*>(p + (i * 64 + (4 * o0 + j) * 8 + 4 * o1 + t) * 32 + o2 * 8);
-        return make_float4(__uint_as_float(r.x << 16), __uint_as_float(r.x & 0xffff0000u),
-                           __uint_as_float(r.y << 16), __uint_as_float(r.y & 0xffff0000u));
+        return widen4(r, static_cast<const E*>(nullptr));
     }
 };
 // four neighbouring voxels of the output
@@ -169,6 +179,14 @@ __device__ __forceinline__ void store_out(float* p, float4 v, bool streaming) {
 }
 __device__ __forceinline__ void store_out(__nv_bfloat16* p, float4 v, bool streaming) {
     const __nv_bfloat162 a = __floats2bfloat162_rn(v.x, v.y), b = __floats2bfloat162_rn(v.z, v.w);
+    uint2 r;
+    r.x = *reinterpret_cast<const uint32_t*>(&a);
+    r.y = *reinterpret_cast<const uint32_t*>(&b);
+    if (streaming) __stcs(reinterpret_cast<uint2*>(p), r);
+    else *reinterpret_cast<uint2*>(p) = r;
+}
+__device__ __forceinline__ void store_out(__half* p, float4 v, bool streaming) {
+    const __half2 a = __floats2half2_rn(v.x, v.y), b = __floats2half2_rn(v.z, v.w);
     uint2 r;
     r.x = *reinterpret_cast<const uint32_t*>(&a);
     r.y = *reinterpret_cast<const uint32_t*>(&b);
@@ -865,16 +883,18 @@ __device__ __forceinline__ void bwd_tile_apply(const PhaseParams& P, const float
 }
 
 // ---- host helpers shared by both launch schemes ---------------------------------------------------------
-// box (8,8,8,8,1) of fp32, or -- bf16 activations -- (16,8,8,8,1) of bf16: two tiles side by side along W
+// box (8,8,8,8,1) of fp32, or -- bf16 / fp16 activations -- (16,8,8,8,1) of 16-bit values: two tiles side by side along W
 inline int make_tile_map(CUtensorMap* m, const void* ptr, const DevGeom& G) {
     if (reinterpret_cast<uintptr_t>(ptr) & 15) return fail(FZ_ERR_INVALID, "volume pointer %p is not 16-byte aligned", ptr);
     cuuint64_t dims[5] = {(cuuint64_t)G.n[2], (cuuint64_t)G.n[1], (cuuint64_t)G.n[0], (cuuint64_t)G.C, (cuuint64_t)G.B};
-    const cuuint64_t e = G.dtype == FZ_DTYPE_BF16 ? 2 : 4;
+    const bool h16 = G.dtype != FZ_DTYPE_F32;
+    const cuuint64_t e = h16 ? 2 : 4;
     cuuint64_t strides[4] = {(cuuint64_t)G.n[2] * e, (cuuint64_t)G.n[2] * G.n[1] * e, (cuuint64_t)G.vox * e,
                              (cuuint64_t)G.vox * G.C * e};
-    cuuint32_t box[5] = {G.dtype == FZ_DTYPE_BF16 ? 16u : 8u, 8, 8, 8, 1};
-    return encode_tiled_map(m, "volume tile", G.dtype == FZ_DTYPE_BF16 ? CU_TENSOR_MAP_DATA_TYPE_BFLOAT16 : CU_TENSOR_MAP_DATA_TYPE_FLOAT32,
-                            5, ptr, dims, strides, box, CU_TENSOR_MAP_SWIZZLE_NONE);
+    cuuint32_t box[5] = {h16 ? 16u : 8u, 8, 8, 8, 1};
+    const CUtensorMapDataType type = G.dtype == FZ_DTYPE_BF16 ? CU_TENSOR_MAP_DATA_TYPE_BFLOAT16
+                                     : G.dtype == FZ_DTYPE_F16 ? CU_TENSOR_MAP_DATA_TYPE_FLOAT16 : CU_TENSOR_MAP_DATA_TYPE_FLOAT32;
+    return encode_tiled_map(m, "volume tile", type, 5, ptr, dims, strides, box, CU_TENSOR_MAP_SWIZZLE_NONE);
 }
 inline size_t align_up(size_t v, size_t a) { return (v + a - 1) / a * a; }
 inline int rec_head_for(int T) { return ((9 * T + 3) / 4) * 4; }

@@ -4,6 +4,7 @@
 // step of the paired-window-set variant at the end of this file, and as the reference the pipelined scheme
 // (fz_swnmf_pipe.cu, the production path for large volumes) is tested against.
 #include <initializer_list>
+#include <type_traits>
 
 #include "fz_swnmf_octant.cuh"
 
@@ -27,22 +28,24 @@ struct Stream {
     }
 };
 
-// With bf16 activations (BF16 = true) a streaming warp's unit of work is a PAIR of tiles side by side along W, fetched as
-// one (16,8,8,8) box of bf16 = the same 16 KiB and the same 32-byte rows as one fp32 tile; the pair is then worked on
-// as two tiles, and whatever is prefetched for "the next tile" (window factors) is prefetched per tile of the pair.
-// Stream::tile(k) counts units: tiles (fp32) or pairs (bf16); a pair is tiles 2u and 2u + 1 (t2 is the fastest index).
-template <bool BF16> struct TileOf { typedef TileF32 type; typedef float out_t; };
-template <> struct TileOf<true> { typedef TileBf16 type; typedef __nv_bfloat16 out_t; };
-template <bool BF16>
-__device__ __forceinline__ typename TileOf<BF16>::type tile_at(const float* buf, int half) {
-    if constexpr (BF16) return TileBf16{reinterpret_cast<const unsigned char*>(buf) + 16 * half};
+// The kernels are templated on the volume's element type E: float, or 16-bit activations (__nv_bfloat16, __half).  With 16-bit
+// activations a streaming warp's unit of work is a PAIR of tiles side by side along W, fetched as one (16,8,8,8) box of 16-bit
+// values = the same 16 KiB and the same 32-byte rows as one fp32 tile; the pair is then worked on as two tiles, and whatever
+// is prefetched for "the next tile" (window factors) is prefetched per tile of the pair.
+// Stream::tile(k) counts units: tiles (fp32) or pairs (16-bit); a pair is tiles 2u and 2u + 1 (t2 is the fastest index).
+template <typename E> constexpr int kPerUnit = std::is_same<E, float>::value ? 1 : 2;    // tiles per unit
+template <typename E> struct TileOf { typedef Tile16<E> type; };
+template <> struct TileOf<float> { typedef TileF32 type; };
+template <typename E>
+__device__ __forceinline__ typename TileOf<E>::type tile_at(const float* buf, int half) {
+    if constexpr (kPerUnit<E> == 2) return Tile16<E>{reinterpret_cast<const unsigned char*>(buf) + 16 * half};
     else return TileF32{buf};
 }
 
 // =====================================================================================================
 // forward pass 1: per-octant Gram partials of every unshifted tile
 // =====================================================================================================
-template <bool BF16>
+template <typename E>
 __global__ void __launch_bounds__(kW1 * 32, 1) phase_fwd_gram(const __grid_constant__ PhaseParams P) {
     extern __shared__ __align__(1024) unsigned char smem_raw[];
     __shared__ __align__(16) float v0s[512];
@@ -64,7 +67,7 @@ __global__ void __launch_bounds__(kW1 * 32, 1) phase_fwd_gram(const __grid_const
         sq = warp_sum_f(sq);
         if (lane == 0) *P.b1 = sq;
     }
-    constexpr int kPer = BF16 ? 2 : 1;
+    constexpr int kPer = kPerUnit<E>;
     const int units = P.t_count / kPer;
     Stream S; S.gw = blockIdx.x * kW1 + warp; S.nw = gridDim.x * kW1; S.lane = lane; S.begin = P.t_begin / kPer; S.count = units; S.reverse = 0;
     int dst[15];
@@ -85,12 +88,12 @@ __global__ void __launch_bounds__(kW1 * 32, 1) phase_fwd_gram(const __grid_const
         const int u = S.tile(k), st = k & 1;
         mbar_wait(&bars[warp][st], parity[st]);
         parity[st] ^= 1;
-        if constexpr (BF16) {
+        if constexpr (kPer == 2) {
 #pragma unroll 1
             for (int half = 0; half < 2; ++half) {
                 // the record is assembled in the pair buffer's first 16-byte column: tile 0 of the pair is in registers
                 // by then (half 0) or long consumed (half 1)
-                fwd_tile_gram<TileBf16, 2>(tile_at<true>(buf + st * 4096, half), buf + st * 4096, v0s, dst, lane,
+                fwd_tile_gram<Tile16<E>, 2>(tile_at<E>(buf + st * 4096, half), buf + st * 4096, v0s, dst, lane,
                                            P.oct + (size_t)(2 * u + half) * kTileRec);
                 __syncwarp();
             }
@@ -118,9 +121,9 @@ __global__ void __launch_bounds__(128) phase_fwd_solve(const __grid_constant__ P
 
 // =====================================================================================================
 // forward pass 3: y = 1/2 (u_0 v_0^T + u_1 v_1^T) voxel by voxel, v_s = relu(rd_s (X^T u_s + eps))
-// OutT: the volume's own type, or fp32 for a bf16 volume whose y is a partial sum (the paired window sets below)
+// OutT: the volume's own type, or fp32 for a 16-bit volume whose y is a partial sum (the paired window sets below)
 // =====================================================================================================
-template <bool BF16, typename OutT = typename TileOf<BF16>::out_t>
+template <typename E, typename OutT = E>
 __global__ void __launch_bounds__(kW3 * 32, 1) phase_fwd_apply(const __grid_constant__ PhaseParams P) {
     extern __shared__ __align__(1024) unsigned char smem_raw[];
     __shared__ uint64_t bars[kW3][2];
@@ -132,7 +135,7 @@ __global__ void __launch_bounds__(kW3 * 32, 1) phase_fwd_apply(const __grid_cons
         fence_mbarrier_init();
     }
     __syncthreads();
-    constexpr int kPer = BF16 ? 2 : 1;
+    constexpr int kPer = kPerUnit<E>;
     Stream S; S.gw = blockIdx.x * kW3 + warp; S.nw = gridDim.x * kW3; S.lane = lane; S.begin = P.t_begin / kPer; S.count = P.t_count / kPer; S.reverse = P.reverse;
     const int oct = lane >> 2;
 
@@ -144,7 +147,7 @@ __global__ void __launch_bounds__(kW3 * 32, 1) phase_fwd_apply(const __grid_cons
             tma_load_tile(buf + (k & 1) * 4096, &P.tm_x, &bars[warp][k & 1], c.t2 * 8, c.t1 * 8, c.t0 * 8, c.h * 8, c.b);
         }
     };
-    // tile number q of this warp's sequence of TILES (fp32: unit q; bf16: tile q % 2 of unit q / 2)
+    // tile number q of this warp's sequence of TILES (fp32: unit q; 16-bit: tile q % 2 of unit q / 2)
     auto tile_of = [&](int q) -> int {
         const int u = S.tile(q / kPer);
         return u < P.tiles ? u * kPer + (q % kPer) : 0x7fffffff;
@@ -175,7 +178,7 @@ __global__ void __launch_bounds__(kW3 * 32, 1) phase_fwd_apply(const __grid_cons
                 mbar_wait(&bars[warp][st], parity[st]);
                 parity[st] ^= 1;
             }
-            fwd_tile_apply_t<!BF16, false, typename TileOf<BF16>::type, OutT>(P, tile_at<BF16>(buf + st * 4096, half), f0, f1, c, lane);
+            fwd_tile_apply_t<kPer == 1, false, typename TileOf<E>::type, OutT>(P, tile_at<E>(buf + st * 4096, half), f0, f1, c, lane);
         }
     }
 }
@@ -183,7 +186,7 @@ __global__ void __launch_bounds__(kW3 * 32, 1) phase_fwd_apply(const __grid_cons
 // =====================================================================================================
 // backward pass 1: per octant and window set, lane-partials of  w = G v_T / 2 + X cbar_T  and  e = qbar_T . v_T
 // =====================================================================================================
-template <bool BF16>
+template <typename E>
 __global__ void __launch_bounds__(kWB * 32, 1) phase_bwd_reduce(const __grid_constant__ PhaseParams P) {
     extern __shared__ __align__(1024) unsigned char smem_raw[];
     __shared__ uint64_t bars[kWB][2];
@@ -195,7 +198,7 @@ __global__ void __launch_bounds__(kWB * 32, 1) phase_bwd_reduce(const __grid_con
         fence_mbarrier_init();
     }
     __syncthreads();
-    constexpr int kPer = BF16 ? 2 : 1;
+    constexpr int kPer = kPerUnit<E>;
     Stream S; S.gw = blockIdx.x * kWB + warp; S.nw = gridDim.x * kWB; S.lane = lane; S.begin = P.t_begin / kPer; S.count = P.t_count / kPer; S.reverse = 0;
     const int oct = lane >> 2;
 
@@ -239,7 +242,7 @@ __global__ void __launch_bounds__(kWB * 32, 1) phase_bwd_reduce(const __grid_con
                 mbar_wait(&bars[warp][st], parity[st]);
                 parity[st] ^= 1;
             }
-            bwd_tile_reduce_t(P, tile_at<BF16>(buf + st * 8192, half), tile_at<BF16>(buf + st * 8192 + 4096, half), f0, f1, lane,
+            bwd_tile_reduce_t(P, tile_at<E>(buf + st * 8192, half), tile_at<E>(buf + st * 8192 + 4096, half), f0, f1, lane,
                               P.oct + (size_t)tid * kBwdTileRec);
         }
     }
@@ -261,9 +264,9 @@ __global__ void __launch_bounds__(kSolveThreads) phase_bwd_solve(const __grid_co
 // backward pass 3: dx = [x > 0] sum_s ( rd_s u_s (u_s . g)/2 + M_s x + m_s + abar1_s v0[col_s] ) voxel by voxel
 // OutT as in forward pass 3
 // =====================================================================================================
-template <bool BF16, typename OutT = typename TileOf<BF16>::out_t>
+template <typename E, typename OutT = E>
 __global__ void __launch_bounds__(kWB * 32, 1) phase_bwd_apply(const __grid_constant__ PhaseParams P) {
-    constexpr int kPer = BF16 ? 2 : 1;
+    constexpr int kPer = kPerUnit<E>;
     extern __shared__ __align__(1024) unsigned char smem_raw[];
     __shared__ __align__(16) float v0s[512];
     __shared__ __align__(16) float mbs_all[kWB][2][9 * kMbF];     // [tile parity][window record: 0 = unshifted, 1 + o = shifted window of octant o]
@@ -279,7 +282,7 @@ __global__ void __launch_bounds__(kWB * 32, 1) phase_bwd_apply(const __grid_cons
     __syncthreads();
     Stream S; S.gw = blockIdx.x * kWB + warp; S.nw = gridDim.x * kWB; S.lane = lane; S.begin = P.t_begin / kPer; S.count = P.t_count / kPer; S.reverse = P.reverse;
 
-    // the tile data of unit k (a tile, or a pair of bf16 tiles): one TMA box each for X and dY
+    // the tile data of unit k (a tile, or a pair of 16-bit tiles): one TMA box each for X and dY
     auto issue = [&](int k) {
         const int u = S.tile(k);
         if (u < P.tiles && lane == 0) {
@@ -291,7 +294,7 @@ __global__ void __launch_bounds__(kWB * 32, 1) phase_bwd_apply(const __grid_cons
             tma_load_tile(b + 4096, &P.tm_g, bar, c.t2 * 8, c.t1 * 8, c.t0 * 8, c.h * 8, c.b);
         }
     };
-    // tile number q of this warp's sequence of TILES (fp32: unit q; bf16: tile q % 2 of unit q / 2)
+    // tile number q of this warp's sequence of TILES (fp32: unit q; 16-bit: tile q % 2 of unit q / 2)
     auto tile_of = [&](int q) -> int {
         const int u = S.tile(q / kPer);
         return u < P.tiles ? u * kPer + (q % kPer) : 0x7fffffff;
@@ -320,8 +323,8 @@ __global__ void __launch_bounds__(kWB * 32, 1) phase_bwd_apply(const __grid_cons
                 parity[st] ^= 1;
             }
             const TileCoord c = tile_coord(P, tile_of(q));
-            bwd_tile_apply_t<false, typename TileOf<BF16>::type, OutT>(
-                P, tile_at<BF16>(buf + st * 8192, half), tile_at<BF16>(buf + st * 8192 + 4096, half), mbs_all[warp][q & 1], v0s, c, lane);
+            bwd_tile_apply_t<false, typename TileOf<E>::type, OutT>(
+                P, tile_at<E>(buf + st * 8192, half), tile_at<E>(buf + st * 8192 + 4096, half), mbs_all[warp][q & 1], v0s, c, lane);
             __syncwarp();                                             // records of tile q are free for tile q + 2
         }
     }
@@ -356,6 +359,43 @@ int grid_for(int tiles, int warps) {
     return ctas < num_sms() ? ctas : num_sms();
 }
 
+// the three forward / backward passes over P's tiles for volumes of E; f32_out: y / dX are fp32 partial sums
+template <typename E>
+int forward_passes(const PhaseParams& P, bool f32_out, cudaStream_t st) {
+    static SmemConfig cfg_gram, cfg_apply, cfg_apply_f;
+    FZ_CUDA_CHECK(cfg_gram.ensure(phase_fwd_gram<E>, kW1 * 2 * kTileBytes));
+    if (f32_out) FZ_CUDA_CHECK(cfg_apply_f.ensure(phase_fwd_apply<E, float>, kW3 * 2 * kTileBytes));
+    else FZ_CUDA_CHECK(cfg_apply.ensure(phase_fwd_apply<E>, kW3 * 2 * kTileBytes));
+    const int units = P.t_count / kPerUnit<E>;           // streaming warps work on tiles (fp32) or pairs of tiles (16-bit)
+    phase_fwd_gram<E><<<grid_for(units, kW1), kW1 * 32, kW1 * 2 * kTileBytes, st>>>(P);
+    FZ_LAUNCH_CHECK();
+    const long long groups = 2LL * P.t_count;
+    phase_fwd_solve<<<(unsigned)((groups * 8 + 127) / 128), 128, 0, st>>>(P);
+    FZ_LAUNCH_CHECK();
+    if (f32_out) phase_fwd_apply<E, float><<<grid_for(units, kW3), kW3 * 32, kW3 * 2 * kTileBytes, st>>>(P);
+    else phase_fwd_apply<E><<<grid_for(units, kW3), kW3 * 32, kW3 * 2 * kTileBytes, st>>>(P);
+    FZ_LAUNCH_CHECK();
+    return FZ_OK;
+}
+
+template <typename E>
+int backward_passes(const PhaseParams& P, bool f32_out, cudaStream_t st) {
+    static SmemConfig cfg_reduce, cfg_apply, cfg_apply_f;
+    FZ_CUDA_CHECK(cfg_reduce.ensure(phase_bwd_reduce<E>, kWB * 4 * kTileBytes));
+    if (f32_out) FZ_CUDA_CHECK(cfg_apply_f.ensure(phase_bwd_apply<E, float>, kWB * 4 * kTileBytes));
+    else FZ_CUDA_CHECK(cfg_apply.ensure(phase_bwd_apply<E>, kWB * 4 * kTileBytes));
+    const int units = P.t_count / kPerUnit<E>;
+    phase_bwd_reduce<E><<<grid_for(units, kWB), kWB * 32, kWB * 4 * kTileBytes, st>>>(P);
+    FZ_LAUNCH_CHECK();
+    const long long groups = 2LL * P.t_count;
+    phase_bwd_solve<<<(unsigned)((groups + kSolveThreads - 1) / kSolveThreads), kSolveThreads, 0, st>>>(P);
+    FZ_LAUNCH_CHECK();
+    if (f32_out) phase_bwd_apply<E, float><<<grid_for(units, kWB), kWB * 32, kWB * 4 * kTileBytes, st>>>(P);
+    else phase_bwd_apply<E><<<grid_for(units, kWB), kWB * 32, kWB * 4 * kTileBytes, st>>>(P);
+    FZ_LAUNCH_CHECK();
+    return FZ_OK;
+}
+
 }  // namespace
 
 bool phase_supported(const DevGeom& G, const fz_solver& s, int relu) {
@@ -363,7 +403,7 @@ bool phase_supported(const DevGeom& G, const fz_solver& s, int relu) {
     if (s.num_iters < 1 || s.num_iters > 8) return false;
     if (G.d != 8 || G.p[0] != 8 || G.p[1] != 8 || G.p[2] != 8 || G.S != 2) return false;
     if (G.mats_per_shift == 0 || G.mats_per_shift >= (1LL << 28)) return false;
-    if (G.dtype == FZ_DTYPE_BF16 && (G.g[2] % 2)) return false;       // bf16 tiles travel in pairs along W
+    if (G.dtype != FZ_DTYPE_F32 && (G.g[2] % 2)) return false;       // 16-bit tiles travel in pairs along W
     for (int k = 0; k < 3; ++k) {
         int a = G.sh[0][k] % G.n[k], b = G.sh[1][k] % G.n[k];
         if (a < 0) a += G.n[k];
@@ -386,31 +426,12 @@ int phase_forward(const float* x, const float* v0, float* y, void* saved, void* 
     fill(P, G, s, 0, workspace);
     if (int e = make_tile_map(&P.tm_x, x, G)) return e;
     P.x = x; P.out = y; P.v0 = v0; P.saved = static_cast<float*>(saved);
-    const bool bf16 = G.dtype == FZ_DTYPE_BF16;
-    static SmemConfig cfg_gram, cfg_apply, cfg_gram_h, cfg_apply_h, cfg_apply_hf;
-    if (bf16) {
-        FZ_CUDA_CHECK(cfg_gram_h.ensure(phase_fwd_gram<true>, kW1 * 2 * kTileBytes));
-        if (f32_out) FZ_CUDA_CHECK(cfg_apply_hf.ensure(phase_fwd_apply<true, float>, kW3 * 2 * kTileBytes));
-        else FZ_CUDA_CHECK(cfg_apply_h.ensure(phase_fwd_apply<true>, kW3 * 2 * kTileBytes));
-    } else {
-        FZ_CUDA_CHECK(cfg_gram.ensure(phase_fwd_gram<false>, kW1 * 2 * kTileBytes));
-        FZ_CUDA_CHECK(cfg_apply.ensure(phase_fwd_apply<false>, kW3 * 2 * kTileBytes));
-    }
     P.t_begin = 0;
     P.t_count = P.tiles;
     P.reverse = 1;          // pass 3 walks the tiles backwards: the tail of pass 1 is what L2 still holds
-    const int units = bf16 ? P.t_count / 2 : P.t_count;        // streaming warps work on tiles (fp32) or pairs of tiles (bf16)
-    if (bf16) phase_fwd_gram<true><<<grid_for(units, kW1), kW1 * 32, kW1 * 2 * kTileBytes, st>>>(P);
-    else phase_fwd_gram<false><<<grid_for(units, kW1), kW1 * 32, kW1 * 2 * kTileBytes, st>>>(P);
-    FZ_LAUNCH_CHECK();
-    const long long groups = 2LL * P.t_count;
-    phase_fwd_solve<<<(unsigned)((groups * 8 + 127) / 128), 128, 0, st>>>(P);
-    FZ_LAUNCH_CHECK();
-    if (bf16 && f32_out) phase_fwd_apply<true, float><<<grid_for(units, kW3), kW3 * 32, kW3 * 2 * kTileBytes, st>>>(P);
-    else if (bf16) phase_fwd_apply<true><<<grid_for(units, kW3), kW3 * 32, kW3 * 2 * kTileBytes, st>>>(P);
-    else phase_fwd_apply<false><<<grid_for(units, kW3), kW3 * 32, kW3 * 2 * kTileBytes, st>>>(P);
-    FZ_LAUNCH_CHECK();
-    return FZ_OK;
+    if (G.dtype == FZ_DTYPE_BF16) return forward_passes<__nv_bfloat16>(P, f32_out, st);
+    if (G.dtype == FZ_DTYPE_F16) return forward_passes<__half>(P, f32_out, st);
+    return forward_passes<float>(P, false, st);
 }
 
 int phase_backward(const float* x, const float* gy, const float* v0, const void* saved, float* gx,
@@ -424,31 +445,12 @@ int phase_backward(const float* x, const float* gy, const float* v0, const void*
     if (int e = make_tile_map(&P.tm_g, gy, G)) return e;
     P.x = x; P.gy = gy; P.out = gx; P.v0 = v0;
     P.saved = const_cast<float*>(static_cast<const float*>(saved));
-    const bool bf16 = G.dtype == FZ_DTYPE_BF16;
-    static SmemConfig cfg_reduce, cfg_apply, cfg_reduce_h, cfg_apply_h, cfg_apply_hf;
-    if (bf16) {
-        FZ_CUDA_CHECK(cfg_reduce_h.ensure(phase_bwd_reduce<true>, kWB * 4 * kTileBytes));
-        if (f32_out) FZ_CUDA_CHECK(cfg_apply_hf.ensure(phase_bwd_apply<true, float>, kWB * 4 * kTileBytes));
-        else FZ_CUDA_CHECK(cfg_apply_h.ensure(phase_bwd_apply<true>, kWB * 4 * kTileBytes));
-    } else {
-        FZ_CUDA_CHECK(cfg_reduce.ensure(phase_bwd_reduce<false>, kWB * 4 * kTileBytes));
-        FZ_CUDA_CHECK(cfg_apply.ensure(phase_bwd_apply<false>, kWB * 4 * kTileBytes));
-    }
     P.t_begin = 0;
     P.t_count = P.tiles;
     P.reverse = 1;
-    const int units = bf16 ? P.t_count / 2 : P.t_count;
-    if (bf16) phase_bwd_reduce<true><<<grid_for(units, kWB), kWB * 32, kWB * 4 * kTileBytes, st>>>(P);
-    else phase_bwd_reduce<false><<<grid_for(units, kWB), kWB * 32, kWB * 4 * kTileBytes, st>>>(P);
-    FZ_LAUNCH_CHECK();
-    const long long groups = 2LL * P.t_count;
-    phase_bwd_solve<<<(unsigned)((groups + kSolveThreads - 1) / kSolveThreads), kSolveThreads, 0, st>>>(P);
-    FZ_LAUNCH_CHECK();
-    if (bf16 && f32_out) phase_bwd_apply<true, float><<<grid_for(units, kWB), kWB * 32, kWB * 4 * kTileBytes, st>>>(P);
-    else if (bf16) phase_bwd_apply<true><<<grid_for(units, kWB), kWB * 32, kWB * 4 * kTileBytes, st>>>(P);
-    else phase_bwd_apply<false><<<grid_for(units, kWB), kWB * 32, kWB * 4 * kTileBytes, st>>>(P);
-    FZ_LAUNCH_CHECK();
-    return FZ_OK;
+    if (G.dtype == FZ_DTYPE_BF16) return backward_passes<__nv_bfloat16>(P, f32_out, st);
+    if (G.dtype == FZ_DTYPE_F16) return backward_passes<__half>(P, f32_out, st);
+    return backward_passes<float>(P, false, st);
 }
 
 
@@ -457,19 +459,22 @@ int phase_backward(const float* x, const float* gy, const float* v0, const void*
 //   sum_{s in {a, a+4}} inv_s(NMF(win(roll(x, s)))) = roll( octant(roll(x, a)), -a )
 // (torch.roll composes: roll(x, a + 4) = roll(roll(x, a), 4); operations.py:266-280), so e.g. the brats23
 // bundle's shifts [0, 2, 4, 6] (model_zoo/factorizer_brats23/configs/train.yaml:50-54) run as two octant
-// problems plus one roll and one roll-and-combine pass per pair instead of four window-at-a-time sweeps.  A bf16 volume
-// is rolled as bf16 (an exact copy) and the pairs' partial sums stay fp32 until the last combine writes the bf16 result.
+// problems plus one roll and one roll-and-combine pass per pair instead of four window-at-a-time sweeps.  A bf16 or fp16
+// volume is rolled in its own type (an exact 2-byte copy) and the pairs' partial sums stay fp32 until the last combine writes
+// the 16-bit result.
 // =====================================================================================================
 namespace {
 
 struct RollParams { int n0, n1, n2, s0, s1, s2; long long rows, vox; };
 
-// V neighbouring elements as one access: fp32 8 or 16 bytes, bf16 4 or 8 bytes
-template <typename T, int V> struct VecOf;
+// V neighbouring elements as one access: fp32 8 or 16 bytes, bf16 / fp16 4 or 8 bytes
+template <typename T, int V> struct VecOf { typedef typename std::conditional<V == 4, uint2, unsigned int>::type type; };
 template <> struct VecOf<float, 2> { typedef float2 type; };
 template <> struct VecOf<float, 4> { typedef float4 type; };
-template <> struct VecOf<__nv_bfloat16, 2> { typedef unsigned int type; };
-template <> struct VecOf<__nv_bfloat16, 4> { typedef uint2 type; };
+
+// two fp32 sums rounded once to a 16-bit pair
+__device__ __forceinline__ void round_pair(__nv_bfloat162* p, float a, float b) { *p = __floats2bfloat162_rn(a, b); }
+__device__ __forceinline__ void round_pair(__half2* p, float a, float b) { *p = __floats2half2_rn(a, b); }
 
 // out[r][i] = in[r][(i - s) mod n]   (torch.roll), an exact copy for either element type.  One CTA per (row, i0) plane;
 // V = 2 or 4 neighbouring voxels per thread (n2 and s2 multiples of V), 32-bit index math.
@@ -495,7 +500,7 @@ __global__ void __launch_bounds__(256) roll_volume(const T* __restrict__ in, T* 
 }
 
 // acc[r][i] = ((first ? 0 : acc[r][i]) + part[r][(i + s) mod n]) * scale   (the inverse roll, summed over the pairs).
-// T = bf16: the last call for a bf16 volume, which writes that sum to y[r][i] instead of acc, rounded to bf16 once
+// T = bf16 / fp16: the last call for a 16-bit volume, which writes that sum to y[r][i] instead of acc, rounded to T once
 // (T = float leaves y unused).
 template <int V, typename T>
 __global__ void __launch_bounds__(256) unroll_combine(float* __restrict__ acc, const float* __restrict__ part, const RollParams R,
@@ -528,10 +533,11 @@ __global__ void __launch_bounds__(256) unroll_combine(float* __restrict__ acc, c
             if constexpr (std::is_same<T, float>::value) {
                 *d = v;
             } else {
+                typedef typename std::conditional<std::is_same<T, __half>::value, __half2, __nv_bfloat162>::type T2;
                 typename VecOf<T, V>::type h;
-                __nv_bfloat162* hp = reinterpret_cast<__nv_bfloat162*>(&h);
+                T2* hp = reinterpret_cast<T2*>(&h);
 #pragma unroll
-                for (int q = 0; q < V / 2; ++q) hp[q] = __floats2bfloat162_rn(vf[2 * q], vf[2 * q + 1]);
+                for (int q = 0; q < V / 2; ++q) round_pair(hp + q, vf[2 * q], vf[2 * q + 1]);
                 *reinterpret_cast<typename VecOf<T, V>::type*>(y + r * R.vox + (long long)i0 * R.n1 * R.n2 + i1 * R.n2 + i2) = h;
             }
         }
@@ -572,10 +578,10 @@ DevGeom pair_geom(const DevGeom& G) {
 }
 
 size_t vol_bytes(const DevGeom& G, size_t elem) { return align_up((size_t)G.B * G.C * G.vox * elem, 256); }
-size_t elem_bytes(const DevGeom& G) { return G.dtype == FZ_DTYPE_BF16 ? sizeof(__nv_bfloat16) : sizeof(float); }
+size_t elem_bytes(const DevGeom& G) { return G.dtype != FZ_DTYPE_F32 ? 2 : sizeof(float); }
 
 // The workspace of the paired scheme: the octant kernels' own, then the rolled x and the rolled dY (the volume's element
-// type), the partial sum of one pair (fp32) and, for bf16 volumes, the fp32 sum over the pairs (fp32 volumes sum in y / dX).
+// type), the partial sum of one pair (fp32) and, for 16-bit volumes, the fp32 sum over the pairs (fp32 volumes sum in y / dX).
 struct PairBufs { float *xr, *gr, *part, *acc; };
 PairBufs pair_bufs(void* workspace, const DevGeom& G, const fz_solver& s, float* out) {
     char* p = static_cast<char*>(workspace) + align_up(phase_workspace_bytes(pair_geom(G), s), 256);
@@ -586,37 +592,45 @@ PairBufs pair_bufs(void* workspace, const DevGeom& G, const fz_solver& s, float*
     p += vol_bytes(G, elem_bytes(G));
     b.part = reinterpret_cast<float*>(p);
     p += vol_bytes(G, sizeof(float));
-    b.acc = G.dtype == FZ_DTYPE_BF16 ? reinterpret_cast<float*>(p) : out;
+    b.acc = G.dtype != FZ_DTYPE_F32 ? reinterpret_cast<float*>(p) : out;
     return b;
 }
 
+template <typename T>
+void roll_as(const float* in, float* out, const RollParams& R, bool v4, unsigned grid, cudaStream_t st) {
+    const T* i = reinterpret_cast<const T*>(in);
+    T* o = reinterpret_cast<T*>(out);
+    if (v4) roll_volume<T, 4><<<grid, 256, 0, st>>>(i, o, R);
+    else roll_volume<T, 2><<<grid, 256, 0, st>>>(i, o, R);
+}
 int launch_roll(const float* in, float* out, const DevGeom& G, const int* a, cudaStream_t st) {
     RollParams R = {G.n[0], G.n[1], G.n[2], a[0], a[1], a[2], (long long)G.B * G.C, G.vox};
     const long long planes = R.rows * R.n0;
     const unsigned grid = (unsigned)(planes < 65535LL * 16 ? planes : 65535LL * 16);
     const bool v4 = R.n2 % 4 == 0 && R.s2 % 4 == 0;
-    if (G.dtype == FZ_DTYPE_BF16) {
-        const __nv_bfloat16* i = reinterpret_cast<const __nv_bfloat16*>(in);
-        __nv_bfloat16* o = reinterpret_cast<__nv_bfloat16*>(out);
-        if (v4) roll_volume<__nv_bfloat16, 4><<<grid, 256, 0, st>>>(i, o, R);
-        else roll_volume<__nv_bfloat16, 2><<<grid, 256, 0, st>>>(i, o, R);
-    } else {
-        if (v4) roll_volume<float, 4><<<grid, 256, 0, st>>>(in, out, R);
-        else roll_volume<float, 2><<<grid, 256, 0, st>>>(in, out, R);
-    }
+    if (G.dtype == FZ_DTYPE_BF16) roll_as<__nv_bfloat16>(in, out, R, v4, grid, st);
+    else if (G.dtype == FZ_DTYPE_F16) roll_as<__half>(in, out, R, v4, grid, st);
+    else roll_as<float>(in, out, R, v4, grid, st);
     FZ_LAUNCH_CHECK();
     return FZ_OK;
 }
-// adds pair partial `part` into acc; y: the last call for a bf16 volume, which writes the finished bf16 sum there
+template <typename T>
+void combine_into(float* acc, const float* part, const RollParams& R, int first, float scale, float* y, bool v4, unsigned grid,
+                  cudaStream_t st) {
+    T* h = reinterpret_cast<T*>(y);
+    if (v4) unroll_combine<4, T><<<grid, 256, 0, st>>>(acc, part, R, first, scale, h);
+    else unroll_combine<2, T><<<grid, 256, 0, st>>>(acc, part, R, first, scale, h);
+}
+// adds pair partial `part` into acc; y: the last call for a 16-bit volume, which writes the finished sum there in its type
 int launch_combine(float* acc, const float* part, const DevGeom& G, const int* a, int first, float scale, float* y, cudaStream_t st) {
     RollParams R = {G.n[0], G.n[1], G.n[2], a[0], a[1], a[2], (long long)G.B * G.C, G.vox};
     const long long planes = R.rows * R.n0;
     const unsigned grid = (unsigned)(planes < 65535LL * 16 ? planes : 65535LL * 16);
     const bool v4 = R.n2 % 4 == 0 && R.s2 % 4 == 0;
-    if (y) {
-        __nv_bfloat16* h = reinterpret_cast<__nv_bfloat16*>(y);
-        if (v4) unroll_combine<4, __nv_bfloat16><<<grid, 256, 0, st>>>(acc, part, R, first, scale, h);
-        else unroll_combine<2, __nv_bfloat16><<<grid, 256, 0, st>>>(acc, part, R, first, scale, h);
+    if (y && G.dtype == FZ_DTYPE_F16) {
+        combine_into<__half>(acc, part, R, first, scale, y, v4, grid, st);
+    } else if (y) {
+        combine_into<__nv_bfloat16>(acc, part, R, first, scale, y, v4, grid, st);
     } else {
         if (v4) unroll_combine<4, float><<<grid, 256, 0, st>>>(acc, part, R, first, scale, nullptr);
         else unroll_combine<2, float><<<grid, 256, 0, st>>>(acc, part, R, first, scale, nullptr);
@@ -625,9 +639,9 @@ int launch_combine(float* acc, const float* part, const DevGeom& G, const int* a
     return FZ_OK;
 }
 
-int check_bf16_pointers(std::initializer_list<const void*> ptrs) {
+int check_16bit_pointers(std::initializer_list<const void*> ptrs) {
     for (const void* p : ptrs)
-        if (reinterpret_cast<uintptr_t>(p) & 15) return fail(FZ_ERR_INVALID, "bf16 volume pointer %p is not 16-byte aligned", p);
+        if (reinterpret_cast<uintptr_t>(p) & 15) return fail(FZ_ERR_INVALID, "16-bit volume pointer %p is not 16-byte aligned", p);
     return FZ_OK;
 }
 
@@ -647,17 +661,17 @@ size_t pairs_saved_bytes(const DevGeom& G, const fz_solver& s) {
 }
 
 size_t pairs_workspace_bytes(const DevGeom& G, const fz_solver& s) {
-    const size_t f32_vols = G.dtype == FZ_DTYPE_BF16 ? 2 : 1;
+    const size_t f32_vols = G.dtype != FZ_DTYPE_F32 ? 2 : 1;
     return align_up(phase_workspace_bytes(pair_geom(G), s), 256) + 2 * vol_bytes(G, elem_bytes(G)) + f32_vols * vol_bytes(G, sizeof(float));
 }
 
-// Every pair's octant kernels write an fp32 partial sum (the unshifted pair's straight into the sum); a bf16 volume's y is
-// written once, by the last combine, so the partial sums are never rounded to bf16.
+// Every pair's octant kernels write an fp32 partial sum (the unshifted pair's straight into the sum); a 16-bit volume's y is
+// written once, by the last combine, so the partial sums are never rounded to 16 bits.
 int pairs_forward(const float* x, const float* v0, float* y, void* saved, void* workspace, const DevGeom& G,
                   const fz_solver& s, cudaStream_t st) {
     if (!workspace) return fail(FZ_ERR_INVALID, "fz_swnmf_forward: workspace of %zu bytes required", pairs_workspace_bytes(G, s));
-    const bool bf16 = G.dtype == FZ_DTYPE_BF16;
-    if (bf16) if (int e = check_bf16_pointers({x, y})) return e;
+    const bool h16 = G.dtype != FZ_DTYPE_F32;
+    if (h16) if (int e = check_16bit_pointers({x, y})) return e;
     const DevGeom Gp = pair_geom(G);
     int base[FZ_MAX_SHIFTS][3];
     find_pairs(G, base);
@@ -677,7 +691,7 @@ int pairs_forward(const float* x, const float* v0, float* y, void* saved, void* 
         if (int e = phase_forward(xin, v0, direct ? b.acc : b.part, sv, workspace, Gp, s, st, true)) return e;
         const bool last = k == np - 1;
         if (!direct)
-            if (int e = launch_combine(b.acc, b.part, G, base[k], k == 0, last ? 1.f / (float)np : 1.f, bf16 && last ? y : nullptr, st))
+            if (int e = launch_combine(b.acc, b.part, G, base[k], k == 0, last ? 1.f / (float)np : 1.f, h16 && last ? y : nullptr, st))
                 return e;
     }
     return FZ_OK;
@@ -687,8 +701,8 @@ int pairs_backward(const float* x, const float* gy, const float* v0, const void*
                    const DevGeom& G, const fz_solver& s, int K, cudaStream_t st) {
     if (!workspace) return fail(FZ_ERR_INVALID, "fz_swnmf_backward: workspace of %zu bytes required", pairs_workspace_bytes(G, s));
     if (!saved) return fail(FZ_ERR_INVALID, "fz_swnmf_backward: the `saved` buffer written by fz_swnmf_forward is required");
-    const bool bf16 = G.dtype == FZ_DTYPE_BF16;
-    if (bf16) if (int e = check_bf16_pointers({x, gy, gx})) return e;
+    const bool h16 = G.dtype != FZ_DTYPE_F32;
+    if (h16) if (int e = check_16bit_pointers({x, gy, gx})) return e;
     const DevGeom Gp = pair_geom(G);
     int base[FZ_MAX_SHIFTS][3];
     find_pairs(G, base);
@@ -709,7 +723,7 @@ int pairs_backward(const float* x, const float* gy, const float* v0, const void*
         if (int e = phase_backward(xin, gin, v0, sv, direct ? b.acc : b.part, workspace, Gp, s, K, st, true)) return e;
         const bool last = k == np - 1;
         if (!direct)
-            if (int e = launch_combine(b.acc, b.part, G, base[k], k == 0, last ? 1.f / (float)np : 1.f, bf16 && last ? gx : nullptr, st))
+            if (int e = launch_combine(b.acc, b.part, G, base[k], k == 0, last ? 1.f / (float)np : 1.f, h16 && last ? gx : nullptr, st))
                 return e;
     }
     return FZ_OK;

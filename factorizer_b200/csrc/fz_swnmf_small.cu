@@ -17,12 +17,13 @@
 // (operations.py:426-433); consecutive sub-warps take windows that are neighbours along W, so a warp-wide
 // load still covers whole 32-byte sectors.  Division is reciprocal (MUFU + one Newton step) times numerator,
 // <= 1 ulp from the reference's true division (same deviation as the 8x512 kernels, DESIGN.md section 2).
-// Window mode also takes bf16 volumes (x, dL/dy in, y, dL/dx out; u, v, the iterates, the history and every sum stay fp32).
-// Their elements are read and written 2 bytes at a time: shifts 1 and 3 put window origins at odd W indices, where a column
-// pair is not 4-byte aligned.  The window sets then sum in an fp32 accumulator volume in the caller's workspace: set 0 writes
-// it, later sets read-add-store it, and the last set writes the finished sum to the bf16 output, rounded once.  So y / dL/dx
-// are the fp32 kernels' results on the same (bf16-representable) inputs, rounded to bf16.
+// Window mode also takes bf16 and fp16 volumes (x, dL/dy in, y, dL/dx out; u, v, the iterates, the history and every sum stay
+// fp32).  Their elements are read and written 2 bytes at a time: shifts 1 and 3 put window origins at odd W indices, where a
+// column pair is not 4-byte aligned.  The window sets then sum in an fp32 accumulator volume in the caller's workspace: set 0
+// writes it, later sets read-add-store it, and the last set writes the finished sum to the 16-bit output, rounded once.  So
+// y / dL/dx are the fp32 kernels' results on the same (16-bit-representable) inputs, rounded to the volume's type.
 #include <cuda_bf16.h>
+#include <cuda_fp16.h>
 
 #include "fz_device.cuh"
 #include "fz_internal.cuh"
@@ -33,7 +34,7 @@ namespace {
 constexpr int kTMax = 5;          // iterates kept (in shared memory) by the backward
 constexpr int kSmallThreads = 128;
 
-template <typename E>     // element type of the volumes: float, or __nv_bfloat16 in window mode
+template <typename E>     // element type of the volumes: float, or __nv_bfloat16 / __half in window mode
 struct SmallParams {
     const E* x;           // window mode: volume; direct mode: (n, M, N)
     const E* gy;          // backward: dL/dy, same layout as x
@@ -44,11 +45,15 @@ struct SmallParams {
     int T, K, kind, relu, set, S, window;
     float eps;
     DevGeom G;
-    float* acc;           // bf16 volume, S >= 2: the fp32 sum over the window sets, laid out as the volume
+    float* acc;           // 16-bit volume, S >= 2: the fp32 sum over the window sets, laid out as the volume
 };
 
+// one rounding of an fp32 sum to the volume's 16-bit type
+__device__ __forceinline__ __nv_bfloat16 round_to(float v, const __nv_bfloat16*) { return __float2bfloat16_rn(v); }
+__device__ __forceinline__ __half round_to(float v, const __half*) { return __float2half_rn(v); }
+
 // Where a window set's sums go.  `acc` is where a set > 0 reads the sums so far.  An fp32 volume read-add-stores in `out`.  A
-// bf16 volume at S >= 2 sums in the fp32 accumulator, and its last set writes `out`, rounded once; at S == 1, set 0 writes
+// 16-bit volume at S >= 2 sums in the fp32 accumulator, and its last set writes `out`, rounded once; at S == 1, set 0 writes
 // `out` directly.
 template <typename E>
 struct SetSums;
@@ -59,22 +64,23 @@ struct SetSums<float> {
     // v before i: the evaluation order of `acc[i] = v`, which keeps the fp32 kernels' code as it was
     __device__ __forceinline__ void store(float v, int i) const { acc[i] = v; }
 };
-template <>
-struct SetSums<__nv_bfloat16> {
-    const SmallParams<__nv_bfloat16>& P;      // `out` is addressed from P at each store: two more live pointers spill
+template <typename E>                         // E = __nv_bfloat16 or __half
+struct SetSums {
+    const SmallParams<E>& P;                  // `out` is addressed from P at each store: two more live pointers spill
     long long base;
     float* acc;
-    __device__ __forceinline__ SetSums(const SmallParams<__nv_bfloat16>& P_, long long base_) : P(P_), base(base_), acc(P_.acc + base_) {}
+    __device__ __forceinline__ SetSums(const SmallParams<E>& P_, long long base_) : P(P_), base(base_), acc(P_.acc + base_) {}
     __device__ __forceinline__ void store(float v, int i) const {
         if (P.set < P.S - 1) acc[i] = v;
-        else P.out[base + i] = __float2bfloat16_rn(v);
+        else P.out[base + i] = round_to(v, P.out);
     }
 };
 
-// element i of a volume, as float; the unsigned bf16 index gives one IMAD.WIDE.U32 per address (a signed one takes three
+// element i of a volume, as float; the unsigned 16-bit index gives one IMAD.WIDE.U32 per address (a signed one takes three
 // instructions and a register more)
 __device__ __forceinline__ float ld_at(const float* p, int i) { return __ldg(p + i); }
 __device__ __forceinline__ float ld_at(const __nv_bfloat16* p, int i) { return __bfloat162float(__ldg(p + (unsigned)i)); }
+__device__ __forceinline__ float ld_at(const __half* p, int i) { return __half2float(__ldg(p + (unsigned)i)); }
 
 template <int L>
 __device__ __forceinline__ float group_sum(float v) {
@@ -594,7 +600,7 @@ bool small_window_supported(const DevGeom& G, const fz_solver& s) {
 }
 
 size_t small_workspace_bytes(const DevGeom& G) {
-    if (G.dtype != FZ_DTYPE_BF16 || G.S < 2) return 0;
+    if (G.dtype == FZ_DTYPE_F32 || G.S < 2) return 0;
     return ((size_t)G.B * G.C * G.vox * sizeof(float) + 255) / 256 * 256;
 }
 
@@ -634,10 +640,13 @@ int small_window_sets(const E* x, const float* u0, const float* v0, const E* gy,
 
 int small_window(const float* x, const float* u0, const float* v0, const float* gy, float* out, void* workspace,
                  const DevGeom& G, const fz_solver& s, int K, int relu, bool bwd, cudaStream_t st) {
-    if (G.dtype != FZ_DTYPE_BF16) return small_window_sets(x, u0, v0, gy, out, nullptr, G, s, K, relu, bwd, st);
+    if (G.dtype == FZ_DTYPE_F32) return small_window_sets(x, u0, v0, gy, out, nullptr, G, s, K, relu, bwd, st);
     if (small_workspace_bytes(G) && !workspace)
         return fail(FZ_ERR_INVALID, "%s: workspace of %zu bytes required", bwd ? "fz_swnmf_backward" : "fz_swnmf_forward",
                     small_workspace_bytes(G));
+    if (G.dtype == FZ_DTYPE_F16)
+        return small_window_sets(reinterpret_cast<const __half*>(x), u0, v0, reinterpret_cast<const __half*>(gy),
+                                 reinterpret_cast<__half*>(out), static_cast<float*>(workspace), G, s, K, relu, bwd, st);
     typedef __nv_bfloat16 bf;
     return small_window_sets(reinterpret_cast<const bf*>(x), u0, v0, reinterpret_cast<const bf*>(gy), reinterpret_cast<bf*>(out),
                              static_cast<float*>(workspace), G, s, K, relu, bwd, st);

@@ -43,10 +43,14 @@ __device__ __forceinline__ void mma_tf32(uint32_t tmem_d, uint64_t adesc, uint64
 // kind::f16 with A = B = BF16 and D = F32 (bench_probes/tcgen05_bf16_layout_probe.cu): one MMA per 16 values of K.  16-bit
 // operands use the plain SWIZZLE_128B layout (type 2) in both majors -- K-major: 128-byte rows of 64 K values, SBO = 1024
 // between groups of 8 rows, a K step of 16 is +32 bytes; MN-major: 128-byte rows of 64 MN values, one row per K, SBO = 1024
-// between groups of 8 K, LBO between groups of 64 MN, a K step of 16 is +2048 bytes
-__device__ __forceinline__ uint32_t make_idesc_bf16(int m, int n, bool a_mn_major, bool b_mn_major) {
-    return (1u << 4) | (1u << 7) | (1u << 10) | ((a_mn_major ? 1u : 0u) << 15) | ((b_mn_major ? 1u : 0u) << 16) |
+// between groups of 8 K, LBO between groups of 64 MN, a K step of 16 is +2048 bytes.  fp16 operands are the same MMA with
+// A / B format 0 in bits 7-12 (bf16: 1), pinned by the same probe; the layouts are those of any 2-byte type.
+__device__ __forceinline__ uint32_t make_idesc_16bit(int m, int n, bool a_mn_major, bool b_mn_major, uint32_t ab_format) {
+    return (1u << 4) | (ab_format << 7) | (ab_format << 10) | ((a_mn_major ? 1u : 0u) << 15) | ((b_mn_major ? 1u : 0u) << 16) |
            ((uint32_t)(n >> 3) << 17) | ((uint32_t)(m >> 4) << 24);
+}
+__device__ __forceinline__ uint32_t make_idesc_bf16(int m, int n, bool a_mn_major, bool b_mn_major) {
+    return make_idesc_16bit(m, n, a_mn_major, b_mn_major, 1u);
 }
 __device__ __forceinline__ void mma_bf16(uint32_t tmem_d, uint64_t adesc, uint64_t bdesc, uint32_t idesc, uint32_t accumulate) {
     asm volatile(

@@ -7,9 +7,9 @@ reference's constructor signatures and parameter names (factorizer/factorizer.py
 any other combination runs the same steps through the standalone kernels.  A FactorizerBlock with LayerNorm / ReLU / GELU
 and no active dropout runs entirely in hand-written kernels: 32 channels in the fused glue kernels (csrc/fz_block_glue*.cu)
 around the fused core, any other width in the tcgen05 channel-map kernel with fused epilogues (csrc/fz_linear_tc.cu) and the
-channels-first LayerNorm kernels, bf16 inputs (bf16 autocast) in the bf16 channel maps (csrc/fz_bf16_block.cu) around the
-bf16 core (patch 8^3 at shifts [0, 4] or paired window sets such as [0, 2, 4, 6]; 64-column windows such as patch 4^3 at any
-shifts); other blocks run the glue layer by layer.
+channels-first LayerNorm kernels, bf16 or fp16 inputs (bf16 or fp16 autocast) in the 16-bit channel maps
+(csrc/fz_bf16_block.cu) around the 16-bit core (patch 8^3 at shifts [0, 4] or paired window sets such as [0, 2, 4, 6];
+64-column windows such as patch 4^3 at any shifts); other blocks run the glue layer by layer.
 """
 from __future__ import annotations
 
@@ -54,6 +54,8 @@ class FactMixer(nn.Module):
             relu = isinstance(self.act, nn.ReLU)
             if out.dtype == torch.bfloat16 and not _ops.bf16_core_supported(self.reshape._geom, f.solver_spec(), relu):
                 out = out.float()           # geometries the bf16 core does not cover, such as the 8^3 bottleneck at patch 8
+            elif out.dtype == torch.float16 and not _ops.f16_core_supported(self.reshape._geom, f.solver_spec(), relu):
+                out = out.float()           # the same for fp16
             out = _ops.SWNMF.apply(out, f.init.u0, f.init.v0, self.reshape._geom, f.solver_spec(), relu)
         else:
             out = self.reshape(out)
@@ -100,6 +102,12 @@ class FactorizerBlock(nn.Module):
                     and _ops.bf16_core_supported(f.reshape._geom, f.factorize.solver_spec())):
                 return None
             fn = _ops.FactorizerBlockBf16Fn
+        elif isinstance(x, torch.Tensor) and x.dtype == torch.float16:
+            # fp16 activations (fp16 autocast, or fp16 inputs): the same kernels on fp16, under the same rule
+            if not (_ops.f16_block_supported(x, fc1.linear.out_channels)
+                    and _ops.f16_core_supported(f.reshape._geom, f.factorize.solver_spec())):
+                return None
+            fn = _ops.FactorizerBlockF16Fn
         elif _ops.block_glue_supported(x, fc1.linear.out_channels):
             fn = _ops.FactorizerBlockFn            # 32 channels: fused glue kernels (csrc/fz_block_glue*.cu)
         elif _ops.wide_block_supported(x, fc1.linear.out_channels):

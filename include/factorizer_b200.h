@@ -40,7 +40,7 @@ enum {
 };
 
 enum { FZ_SOLVER_MU = 0, FZ_SOLVER_HALS = 1 };
-enum { FZ_DTYPE_F32 = 0, FZ_DTYPE_BF16 = 1 };
+enum { FZ_DTYPE_F32 = 0, FZ_DTYPE_BF16 = 1, FZ_DTYPE_F16 = 2 };
 
 /* Window geometry of Matricize / SWMatricize
  * (factorizer/factorization/operations.py:299-355 and :381-415). */
@@ -52,9 +52,10 @@ typedef struct fz_geom {
     int32_t head_dim;                   /* d = rows M of every matrix                          */
     int32_t num_shifts;                 /* S (1 for a plain Matricize)                         */
     int32_t shifts[FZ_MAX_SHIFTS][3];   /* torch.roll shifts per window set; 0 = unshifted     */
-    int32_t dtype;                      /* FZ_DTYPE_F32 (0) or FZ_DTYPE_BF16: element type of the VOLUMES handed to
-                                           fz_swnmf_forward / _backward (x, y, dy, dx); u0, v0, the saved records and
-                                           all arithmetic stay fp32.  bf16 is served by the octant kernels
+    int32_t dtype;                      /* FZ_DTYPE_F32 (0), FZ_DTYPE_BF16 or FZ_DTYPE_F16: element type of the VOLUMES
+                                           handed to fz_swnmf_forward / _backward (x, y, dy, dx); u0, v0, the saved
+                                           records and all arithmetic stay fp32, and a 16-bit y / dx is the fp32 result
+                                           rounded once.  bf16 and fp16 are served by the octant kernels
                                            (head_dim 8, patch 8^3, ReLU, rank-1 HALS, an even number of patches along
                                            W) at shifts [0, 4] or at window sets that pair up as (a, a + 4) with even
                                            base shifts along W, e.g. [0, 2, 4, 6]; and by the sub-warp kernels at
@@ -125,7 +126,7 @@ int fz_nmf_backward(const float* x, const float* u0, const float* v0, const floa
 
 /* Bytes of the `saved` buffer fz_swnmf_forward fills for fz_swnmf_backward (per-window iterate
  * summaries), and of the scratch `workspace` both directions need (tile-order counters; for bf16
- * volumes on the sub-warp kernels with two or more window sets, an fp32 sum over the sets). */
+ * and fp16 volumes on the sub-warp kernels with two or more window sets, an fp32 sum over the sets). */
 size_t fz_swnmf_saved_bytes(const fz_geom* g, const fz_solver* s);
 size_t fz_swnmf_workspace_bytes(const fz_geom* g, const fz_solver* s);
 
@@ -229,6 +230,31 @@ int fz_layernorm_cf_backward_add_bf16(const void* x, const float* gamma, const v
                                       float* dbeta, int64_t batch, int32_t channels, int64_t voxels, float eps, void* stream);
 /* 1 if fz_swnmf_forward / _backward take bf16 volumes of this geometry and solver (g->dtype is ignored). */
 int fz_swnmf_bf16_supported(const fz_geom* g, const fz_solver* s, int32_t relu_input);
+
+/* ---- fp16 activations (the FactorizerBlock under fp16 autocast, torch.autocast("cuda")'s default, or fed fp16 tensors) ----
+ * The bf16 entry points above with fp16 (torch.float16) in every `void*` buffer: the same kernels, shapes, conditions and
+ * FZ_ERR_UNSUPPORTED refusals.  Sums stay fp32 and are rounded to fp16 once (round to nearest even): a result beyond
+ * +-65504 becomes +-inf, not a saturated value, so a loss scaler sees the overflow. */
+int fz_linear_forward_f16_supported(int32_t cout, int32_t cin, int64_t voxels);
+int fz_linear_forward_f16(const void* x, const void* W, int32_t ldw, const float* bias, void* y, int64_t batch, int32_t cin,
+                          int32_t cout, int64_t voxels, int32_t epilogue, const void* aux, void* y2, void* stream);
+int fz_linear_wgrad_f16_supported(int32_t cout, int32_t cin, int64_t voxels);
+int fz_linear_wgrad_f16(const void* dy, const void* x, float* dW, float* db, int64_t batch, int32_t cout, int32_t cin,
+                        int64_t voxels, void* stream);
+/* fz_bf16_stage_weights' layout (and element counts) with fp16 values. */
+int fz_f16_stage_weights_supported(int32_t rows, int32_t cols);
+int64_t fz_f16_staged_elems(int32_t rows, int32_t cols);
+int fz_f16_stage_weights(const float* w0, int32_t rows0, int32_t cols0, const float* w1, int32_t rows1, int32_t cols1,
+                         const float* w2, int32_t rows2, int32_t cols2, const float* w3, int32_t rows3, int32_t cols3, void* out,
+                         void* stream);
+int fz_f16_stage_weight(const float* w, int32_t rows, int32_t cols, void* out, void* stream);
+int fz_layernorm_cf_f16_supported(int32_t channels, int64_t voxels);
+int fz_layernorm_cf_forward_f16(const void* x, const float* gamma, const float* beta, void* y, int64_t batch, int32_t channels,
+                                int64_t voxels, float eps, void* stream);
+int fz_layernorm_cf_backward_add_f16(const void* x, const float* gamma, const void* dy, const void* add, void* dx, float* dgamma,
+                                     float* dbeta, int64_t batch, int32_t channels, int64_t voxels, float eps, void* stream);
+/* 1 if fz_swnmf_forward / _backward take fp16 volumes of this geometry and solver: the same geometries as bf16. */
+int fz_swnmf_f16_supported(const fz_geom* g, const fz_solver* s, int32_t relu_input);
 
 /* (batch, channels, D, H, W) <-> (batch, channels*8, D/2*H/2*W/2) with rows ordered (c, kd, kh, kw): the view on which
  * the reference U-Net's kernel-2 stride-2 down-sampling convolution (factorizer/unet.py:53) and transposed up-sampling
